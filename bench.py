@@ -3,7 +3,7 @@
 images/s masked-ViT encode+rate.
 
     python bench.py --gpus N --steps K --warmup W [--impl reference] [--workload NAME] [--precise all|rate]
-                    [--scaling weak|strong]
+                    [--scaling weak|strong] [--dump-outputs DIR]
 
 One "step" = one pass of the path (mask-select -> gather -> ViT encoder -> g_a/h_a/h_s/slice nets -> quantise ->
 likelihoods -> bpp) over one batch of images.  Default workload = BASELINE.json configs[1]: synthetic 224x224, batch 64
@@ -18,10 +18,13 @@ SURVEY 0.2 #4), bf16 tensor-core operands, fp32 accumulate.  The other BASELINE 
 Images are sharded across ranks, weights replicated; the only collective is the 16-byte rate all-reduce per step.
 `--scaling weak` (default): every rank runs the workload's batch; `--scaling strong`: the workload's batch is the
 GLOBAL batch, sharded with distributed.shard_range.
+`--dump-outputs DIR`: after the timed steps, rank 0 writes what the last timed step returned to its caller as DIR/<name>.npy
+(see dump_outputs); inputs and weights are seeded, so two builds run with the same arguments can be compared array by array.
+With --impl reference it writes the fp32 oracle's outputs, under the same names, for the inputs of the B200 path's last
+timed step with the same arguments (the reference arm times a sample of other images), minus rate_sums and ids_shuffle.
 
 --impl reference: the reference's CPU implementation of the same path (the in-repo fp32 oracle, bit-identical to the
-reference's MCM.forward executed from /root/reference - tests/test_reference_exec.py; the reference tree itself does not
-exist on the GPU box) on all host cores, same images per step.
+reference's MCM.forward - tests/test_reference_exec.py) on all host cores, same images per step.
 """
 from __future__ import annotations
 
@@ -155,6 +158,41 @@ def make_inputs(kwargs, batch, seed, n_rot, kind="uniform"):
     return imgs, scores
 
 
+DUMP_BUDGET_BYTES = 64 * 10**6
+
+
+def dump_outputs(out, dirname):
+    """Writes every tensor of a forward's result dict as <dirname>/<name>.npy, nested keys joined by "_"
+    (likelihoods_y, latents_y_sym, bpp, ids_restore, ...): float32 outputs as float32, the rest (fp64 rate sums, integer
+    symbols and indices) as float64, which holds them exactly.  When the files would exceed DUMP_BUDGET_BYTES in all,
+    each array above 1 MiB is replaced by the same fraction of its elements, flattened, at indices drawn from a fixed
+    seed: the same arguments give the same sample."""
+    import numpy as np
+    arrays = {}
+
+    def collect(prefix, v):
+        if isinstance(v, dict):
+            for k, x in v.items():
+                collect(f"{prefix}{k}_", x)
+        elif torch.is_tensor(v):
+            dt = torch.float32 if v.dtype == torch.float32 else torch.float64
+            arrays[prefix[:-1]] = np.ascontiguousarray(v.detach().to("cpu", dt).numpy())
+
+    collect("", out)
+    room = DUMP_BUDGET_BYTES - 1024 * len(arrays)               # .npy headers
+    if sum(a.nbytes for a in arrays.values()) > room:
+        big = [n for n, a in arrays.items() if a.nbytes > 2**20]
+        frac = (room - sum(a.nbytes for n, a in arrays.items() if n not in big)) / sum(arrays[n].nbytes for n in big)
+        for name in big:
+            a = arrays[name]
+            idx = np.random.default_rng(0).choice(a.size, int(a.size * frac), replace=False)
+            arrays[name] = a.reshape(-1)[np.sort(idx)]
+    d = Path(dirname)
+    d.mkdir(parents=True, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(d / f"{name}.npy", a)
+
+
 def algo_gflop_per_image(cfg, wl):
     """Reference-algorithmic GFLOP per image (2 x MAC; SURVEY 6.2 closed forms)."""
     if wl in ALGO_GFLOP_PER_IMG:
@@ -178,6 +216,12 @@ def algo_gflop_per_image(cfg, wl):
 
 
 # ----------------------------------------------------------------------------------------------------------
+def rotation_count(kwargs, batch):
+    """Input batches the timed B200 loop rotates over: together > 126 MB L2 (with the weights)."""
+    img_bytes = batch * 3 * kwargs["img_size"] ** 2 * 4
+    return max(2, min(8, int(320e6 // max(img_bytes, 1)) + 1))
+
+
 def run_reference(args, kwargs, batch, desc, kind):
     """The reference's CPU path (fp32 oracle == reference MCM.forward bit for bit) on the host cores; rank 0 only."""
     rank = int(os.environ.get("RANK", "0"))
@@ -230,6 +274,12 @@ def run_reference(args, kwargs, batch, desc, kind):
         "gpu_launches": 0,
     }
     print(json.dumps(line), flush=True)
+    if args.dump_outputs:
+        n_rot = rotation_count(kwargs, batch)
+        imgs_b, scores_b = make_inputs(kwargs, batch, 1000, n_rot, kind)
+        r = ref_model.forward_rate(sd, cfg, imgs_b[(args.steps - 1) % n_rot], scores_b[(args.steps - 1) % n_rot])
+        dump_outputs({"likelihoods": r["likelihoods"], "bpp": r["bpp"], "ids_restore": r["ids_restore"], "ids_keep": r["ids_keep"],
+                      "latents": {k: r[k] for k in ("y_sym", "z_sym", "y_hat", "z_hat")}}, args.dump_outputs)
 
 
 # ----------------------------------------------------------------------------------------------------------
@@ -308,8 +358,7 @@ def run_b200(args, kwargs, batch_named, desc, wl, kind):
     S = max(1, args.streams)
     R = Runner(kwargs, max(batch, 1), S, args.precise, dev, world)
     cfg, models, model = R.cfg, R.models, R.models[0]
-    img_bytes = batch * 3 * kwargs["img_size"] ** 2 * 4
-    n_rot = max(2, min(8, int(320e6 // max(img_bytes, 1)) + 1))   # rotating input batches: together > 126 MB L2 (with the weights)
+    n_rot = rotation_count(kwargs, batch)
     imgs_h, scores_h = make_inputs(kwargs, batch, 1000 + rank, n_rot, kind)
     imgs_d = [t.cuda() for t in imgs_h]
     scores_d = [t.cuda() for t in scores_h]
@@ -351,6 +400,8 @@ def run_b200(args, kwargs, batch_named, desc, wl, kind):
     warm_eff += extra
     ms_max, out = R.timed(step_dev, args.steps)
     value = global_batch * args.steps / (ms_max / 1e3)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(out, args.dump_outputs)
 
     # ---- end to end through the host-buffer entry -------------------------------------------------------------------
     # pinned host images + scores -> H2D -> forward -> D2H of what the reference's forward returns to its caller
@@ -568,6 +619,7 @@ def run_b200(args, kwargs, batch_named, desc, wl, kind):
 
 
 def main():
+    sys.dont_write_bytecode = True          # the benchmark writes nothing into the tree, which may be read-only
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
     ap.add_argument("--steps", type=int, default=100)
@@ -582,7 +634,11 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--streams", type=int, default=4, help="batches in flight per GPU (independent handles/streams)")
     ap.add_argument("--batch", type=int, default=0, help="experiment only: images per step instead of the workload's batch")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the arrays the last timed step returned as DIR/<name>.npy (rank 0)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     kwargs, batch, desc, kind = WORKLOADS[args.workload]
     if args.batch > 0:
         desc = desc.replace(f"batch {batch}", f"batch {args.batch} (EXPERIMENT, not the named workload)")

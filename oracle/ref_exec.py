@@ -2,26 +2,24 @@
 
 Executes the REFERENCE's own `models/Compression/MCM.py` (class MCM: `__init__` topology, `forward_encoder`,
 `random_masking`, `get_ids_shuffle`, `forward` incl. the slice loop, `forward_decoder`, `unpatchify`,
-`forward_loss`) verbatim from /root/reference, with only the absent third-party leaf classes supplied by
-oracle/ref_stubs.py (timm / compressai / pytorch_msssim restated from their published definitions) and
-the pretrained-VGG feature loss replaced by zero (it needs a download).  This is the strongest pin of the
-in-repo oracle (oracle/ref_model.py) available in this container: every line of MCM.py on the path runs
-as written.  Used by `-m "not gpu"` tests and by tests/golden/make_golden.py (the reference tree does not
-exist on the GPU box; its outputs travel as fixtures tests/golden/refexec_*.pt).
+`forward_loss`) verbatim from the reference checkout (oracle.REFERENCE_ROOT), with only the absent
+third-party leaf classes supplied by oracle/ref_stubs.py (timm / compressai / pytorch_msssim restated from
+their published definitions) and the pretrained-VGG feature loss replaced by zero (it needs a download).
+This is the strongest pin of the in-repo oracle (oracle/ref_model.py): every line of MCM.py on the path runs as written.  Used by the
+`-m "not gpu"` tests that skip without the checkout and by tests/golden/make_refexec_golden.py, whose
+outputs (tests/golden/refexec_*) let every other machine compare against the reference.
 """
 from __future__ import annotations
 
 import contextlib
 import sys
 import types
-from pathlib import Path
 
 import numpy as np
 import torch
 
-from . import ref_stubs
+from . import REFERENCE_ROOT, SKIP_REASON, ref_stubs, reference_has
 
-REFERENCE_ROOT = Path("/root/reference")
 _STUBBED = ("compressai", "compressai.ans", "compressai.entropy_models", "compressai.layers", "compressai.models",
             "compressai.ops", "pytorch_msssim", "timm", "timm.models", "timm.models.vision_transformer",
             "models.Compression.loss.vgg")
@@ -29,7 +27,7 @@ _cached_cls = None
 
 
 def reference_available() -> bool:
-    return (REFERENCE_ROOT / "models/Compression/MCM.py").exists()
+    return reference_has("models/Compression/MCM.py")
 
 
 def _mod(name, **attrs):
@@ -39,12 +37,12 @@ def _mod(name, **attrs):
 
 
 def load_reference_mcm_class():
-    """Import /root/reference/models/Compression/MCM.py as written and return its `MCM` class."""
+    """Import the reference's models/Compression/MCM.py as written and return its `MCM` class."""
     global _cached_cls
     if _cached_cls is not None:
         return _cached_cls
     if not reference_available():
-        raise RuntimeError("/root/reference is not mounted")
+        raise RuntimeError(SKIP_REASON)
     S = ref_stubs
     stubs = {
         "compressai": _mod("compressai"),

@@ -1,8 +1,8 @@
 """TEST INFRASTRUCTURE - the reference's HuffmanCoding (utils/huffman.py) for checking the host-side coder (SURVEY 8 f-4).
 
 Only tests/ may import this.  `load_reference_class()` executes the reference file where it lies (it needs only torch and the
-standard library); `HuffmanOracle` is a restatement for boxes without /root/reference: the same algorithm on Python's own
-`heapq` (the library the reference calls, so the tie-breaking is the reference's by construction), nodes ordered by
+standard library); `HuffmanOracle` is a restatement for machines without the reference checkout: the same algorithm on
+Python's own `heapq` (the library the reference calls, so the tie-breaking is the reference's by construction), nodes ordered by
 frequency only (utils/huffman.py:28-38), values in first-appearance order (:55-62), pre-order walk left "0" / right "1"
 (:76-93), decode by growing the current code (:120-139).  Pinned by tests/test_huffman.py against the executed reference
 class and the committed goldens (tests/golden/huffman_refexec.pt).
@@ -11,9 +11,14 @@ from __future__ import annotations
 
 import heapq
 import importlib.util
-from pathlib import Path
 
-REF_FILE = Path("/root/reference/utils/huffman.py")
+from . import REFERENCE_ROOT, reference_has
+
+REF_FILE = REFERENCE_ROOT / "utils/huffman.py"
+
+
+def reference_available() -> bool:
+    return reference_has("utils/huffman.py")
 
 
 def load_reference_class():

@@ -1,15 +1,15 @@
 """ORACLE (test infrastructure only - never imported by the product path).
 
 Score-guided patch ordering of the reference, `MCM.get_ids_shuffle`
-(/root/reference/models/Compression/MCM.py:364-423) and the inverse
+(models/Compression/MCM.py:364-423) and the inverse
 permutation / keep-set of `MCM.random_masking` (MCM.py:548-588).
 
 Two implementations live here:
 
 * `load_reference_get_ids_shuffle()` - pulls the *verbatim* reference function
-  out of /root/reference with `ast` (the function only needs torch, F.softmax
-  and collections.Counter, so it runs without timm/compressai).  Only usable
-  where /root/reference is mounted (the build container); it is what pins the
+  out of the reference checkout (oracle.REFERENCE_ROOT) with `ast` (the function
+  only needs torch, F.softmax and collections.Counter, so it runs without
+  timm/compressai).  Only usable where that checkout exists; it is what pins the
   restatement and what generates tests/golden/mask_*.pt.
 * `ids_shuffle_spec()` - an index-level restatement in torch (same torch
   kernels, same fp32 arithmetic, so it equals the reference wherever torch's
@@ -32,12 +32,14 @@ import numpy as np
 import torch
 import torch.nn.functional as F
 
-REFERENCE_MCM = Path("/root/reference/models/Compression/MCM.py")
+from . import REFERENCE_ROOT, reference_has
+
+REFERENCE_MCM = REFERENCE_ROOT / "models/Compression/MCM.py"
 _HERE = Path(__file__).resolve().parent
 
 
 def reference_available() -> bool:
-    return REFERENCE_MCM.exists()
+    return reference_has("models/Compression/MCM.py")
 
 
 def load_reference_get_ids_shuffle():

@@ -1,8 +1,8 @@
-"""Generates the committed fixtures under tests/golden/.  Run in the build container (needs /root/reference):
+"""Generates the committed fixtures under tests/golden/.  Needs a checkout of the original project (oracle.REFERENCE_ROOT):
 
     python tests/golden/make_golden.py
 
-What comes from REFERENCE CODE executed where it lies (/root/reference, read-only):
+What comes from REFERENCE CODE executed where it lies (the checkout, read-only):
   * kodak_scores.pt   - the reference's score generator (generate_scores_file.py:19-31 calling utils/map.py and
                         utils/distribution.py) on the 24 bundled Kodak PNGs (datasets/kodak).
   * kodak_224.npz     - the 24 Kodak images through the reference's test transform
@@ -25,9 +25,8 @@ import torch
 HERE = Path(__file__).resolve().parent
 ROOT = HERE.parent.parent
 sys.path.insert(0, str(ROOT))
-REF = Path("/root/reference")
 
-from oracle import ref_mask, ref_model  # noqa: E402
+from oracle import REFERENCE_ROOT as REF, SKIP_REASON, ref_mask, ref_model  # noqa: E402
 from textmae_image_compression_b200.config import vit_base  # noqa: E402
 from textmae_image_compression_b200.synthetic import make_state_dict  # noqa: E402
 
@@ -75,7 +74,7 @@ def fuzz_scores(kind: int, L: int, g: torch.Generator) -> torch.Tensor:
 
 
 def main():
-    assert ref_mask.reference_available(), "needs /root/reference"
+    assert ref_mask.reference_available(), SKIP_REASON
     scores, imgs_u8, names = kodak_scores_and_images()
     torch.save(scores, HERE / "kodak_scores.pt")
     np.savez_compressed(HERE / "kodak_224.npz", imgs=imgs_u8, names=np.array(names))

@@ -1,10 +1,11 @@
-"""Generates tests/golden/kodak_gray6.npz and scores_refexec.npz.  Run in the build container (needs /root/reference + cv2):
+"""Generates tests/golden/kodak_gray6.npz and scores_refexec.npz.  Needs a checkout of the original project
+(oracle.REFERENCE_ROOT) and cv2:
 
     python tests/golden/make_scores_golden.py
 
   * kodak_gray6.npz    - cv2.imread(path, IMREAD_GRAYSCALE) (generate_scores_file.py:19) of the first six bundled Kodak PNGs
-                         (kodim04 is portrait): the INPUT of the score generator, which the GPU box cannot decode from
-                         /root/reference.  Their reference scores are rows 0..5 of kodak_scores.pt (make_golden.py).
+                         (kodim04 is portrait): the INPUT of the score generator, for machines without the
+                         reference checkout.  Their reference scores are rows 0..5 of kodak_scores.pt (make_golden.py).
   * scores_refexec.npz - outputs of the REFERENCE functions executed where they lie (utils/map.py Division_Merge_Segmented,
                          laplacian; utils/distribution.py cal_patch_score; the normalisation of generate_scores_file.py:24-31)
                          on seeded synthetic images (oracle.ref_scores.synthetic_gray) at several geometries: s_map, t_map,
@@ -22,9 +23,8 @@ import torch
 HERE = Path(__file__).resolve().parent
 ROOT = HERE.parent.parent
 sys.path.insert(0, str(ROOT))
-REF = Path("/root/reference")
 
-from oracle import ref_scores  # noqa: E402
+from oracle import REFERENCE_ROOT as REF, ref_scores  # noqa: E402
 
 CASES = [(0, 256, 256, 1), (0, 300, 411, 2), (1, 225, 230, 3), (2, 256, 384, 4), (3, 256, 256, 77), (3, 301, 411, 9),
          (4, 512, 768, 5), (4, 333, 500, 6), (0, 768, 512, 7), (2, 230, 226, 8)]

@@ -1,12 +1,12 @@
 """CPU: the host-side side-information coder (csrc/huffman.cpp via textmae_image_compression_b200.huffman.HuffmanCoding)
-against the reference's HuffmanCoding - executed from /root/reference when mounted, committed goldens otherwise - and the
+against the reference's HuffmanCoding - executed from the reference checkout when provided, committed goldens otherwise - and the
 oracle restatement.  Bit strings and code tables must be identical; decode must invert encode."""
 from pathlib import Path
 
 import pytest
 import torch
 
-from oracle import ref_huffman
+from oracle import SKIP_REASON, ref_huffman
 from textmae_image_compression_b200.huffman import HuffmanCoding, side_info_bits
 
 GOLDEN = Path(__file__).resolve().parent / "golden"
@@ -63,7 +63,7 @@ def test_single_symbol_alphabet_behaves_like_the_reference():
         h.decompress(text, shape, dev)
 
 
-@pytest.mark.skipif(not ref_huffman.REF_FILE.exists(), reason="needs /root/reference")
+@pytest.mark.skipif(not ref_huffman.reference_available(), reason=SKIP_REASON)
 def test_matches_reference_class_executed_in_place():
     Ref = ref_huffman.load_reference_class()
     g = torch.Generator().manual_seed(3)

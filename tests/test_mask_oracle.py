@@ -1,6 +1,6 @@
 """CPU: the bit-level C restatement of MCM.get_ids_shuffle (oracle/mask_oracle.c) against
  (a) the committed outputs of the verbatim reference function (tests/golden/mask_golden.pt),
- (b) the verbatim function itself where /root/reference is mounted,
+ (b) the verbatim function itself where the reference checkout is provided,
  (c) the ATen kernels it restates (cascade sum, softmax), bit for bit."""
 import ctypes
 
@@ -8,7 +8,7 @@ import numpy as np
 import pytest
 import torch
 
-from oracle import ref_mask
+from oracle import SKIP_REASON, ref_mask
 
 
 @pytest.fixture(scope="module")
@@ -46,7 +46,7 @@ def test_every_output_is_a_permutation(cases):
         assert torch.equal(srt, torch.arange(L).expand_as(srt))
 
 
-@pytest.mark.skipif(not ref_mask.reference_available(), reason="/root/reference not mounted")
+@pytest.mark.skipif(not ref_mask.reference_available(), reason=SKIP_REASON)
 def test_c_oracle_matches_live_reference_fuzz():
     g = torch.Generator().manual_seed(99)
     for L, K in ((196, 64), (196, 144), (1024, 256)):

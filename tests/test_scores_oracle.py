@@ -1,5 +1,5 @@
 """CPU: the score-generation oracle (oracle/ref_scores.py) against (1) OpenCV itself, (2) the reference's own functions
-executed from /root/reference when it is mounted, (3) the committed reference-generated goldens."""
+executed from the reference checkout when it is provided, (3) the committed reference-generated goldens."""
 import sys
 import types
 from pathlib import Path
@@ -8,10 +8,9 @@ import numpy as np
 import pytest
 import torch
 
-from oracle import ref_scores
+from oracle import REFERENCE_ROOT as REF, SKIP_REASON, ref_scores, reference_has
 
 GOLDEN = Path(__file__).resolve().parent / "golden"
-REF = Path("/root/reference")
 cv2 = pytest.importorskip("cv2")
 
 
@@ -48,7 +47,7 @@ def test_oracle_equals_reference_generated_goldens():
         assert np.array_equal(ref_scores.generate_scores(gray[name]), gold[i]), name
 
 
-@pytest.mark.skipif(not (REF / "utils" / "map.py").exists(), reason="needs /root/reference")
+@pytest.mark.skipif(not reference_has("utils/map.py"), reason=SKIP_REASON)
 def test_oracle_equals_reference_code_executed_in_place():
     sys.path.insert(0, str(GOLDEN))
     import make_scores_golden as mk
