@@ -163,6 +163,27 @@ TMAE_API int  tmae_forward_from_latent_forced(tmae_handle* h, const float* y, co
 TMAE_API int  tmae_forward_encoder(tmae_handle* h, const float* imgs, const float* scores, int N,
                           const tmae_outputs* out, void* stream);
 
+/* Decode (MCM.decompress, MCM.py:896-968, with the range decoder left to the caller) ---------------------------- *
+ * The rate half of the forward with y replaced by the caller's symbols: z_hat -> h_s -> per slice group mu / sigma ->
+ * scale-table indexes -> (caller decodes the group's symbols) -> y_hat = symbols + mu -> lrp_transform.  The range decoder
+ * needs a group's indexes before it can produce that group's symbols, so the decode runs in stages: tmae_decode_begin,
+ * then tmae_decode_step for every slice group in order.  Symbols go in and indexes come out in the range coder's order
+ * (per image, slice by slice, each (c, y, x): the layout of the lists the reference passes to encode_with_indexes /
+ * decode_stream, i.e. NCHW of [Cy, s, s]); z_hat / y_hat / mu / sigma come out channels-last like every other output.
+ * A handle decodes what a handle of the same configuration (flags included) encoded, bit for bit: the same layers run
+ * with the same launch shapes.  Any other call on the handle between begin and the last step, or a step out of order, ends
+ * the decode (that step and the next return TMAE_ESTATE). */
+/* Host-only: the slice groups of the decode (first slice, slice count each); returns their count (7 for 12 slices), or
+ * -TMAE_EINVAL.  first_slice / n_slices may be NULL (count only), else they hold `capacity` entries. */
+TMAE_API int  tmae_decode_groups(int num_slices, int* first_slice, int* n_slices, int capacity);
+/* z_symbols: i32 [N, Cz, s/4, s/4].  Writes out->z_hat (if non-NULL) and the indexes of group 0 into out->y_indexes
+ * (required, i32 [N, Cy*s*s]).  Needs the scale table (tmae_set_scale_table; TMAE_ESTATE without it). */
+TMAE_API int  tmae_decode_begin(tmae_handle* h, const int32_t* z_symbols, int N, const tmae_outputs* out, void* stream);
+/* y_symbols: i32 [N, Cy*s*s] in coder order, of which the region of `group` is read.  Dequantises the group, runs its
+ * lrp_transform and writes the indexes of group + 1 into out->y_indexes; after the last group out->y_hat (and out->mu /
+ * out->sigma when non-NULL) are complete.  Other members of `out` are ignored. */
+TMAE_API int  tmae_decode_step(tmae_handle* h, int group, const int32_t* y_symbols, const tmae_outputs* out, void* stream);
+
 /* Stand-alone operators on the path (each mirrors one reference call) ---------------------------------- */
 /* MCM.get_ids_shuffle + random_masking index work (MCM.py:364-423, 579-583). Outputs may be NULL. */
 TMAE_API int  tmae_mask_select(const float* scores, int N, int L, int K, int softmax_isa,

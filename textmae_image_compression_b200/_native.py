@@ -76,6 +76,9 @@ SIGNATURES = {
     "tmae_forward_from_latent": (C.c_int, [_P, _P, C.c_int, C.POINTER(TmaeOutputs), _P]),
     "tmae_forward_from_latent_forced": (C.c_int, [_P, _P, _P, C.c_int, C.POINTER(TmaeOutputs), _P]),
     "tmae_forward_encoder": (C.c_int, [_P, _P, _P, C.c_int, C.POINTER(TmaeOutputs), _P]),
+    "tmae_decode_groups": (C.c_int, [C.c_int, C.POINTER(C.c_int), C.POINTER(C.c_int), C.c_int]),
+    "tmae_decode_begin": (C.c_int, [_P, _P, C.c_int, C.POINTER(TmaeOutputs), _P]),
+    "tmae_decode_step": (C.c_int, [_P, C.c_int, _P, C.POINTER(TmaeOutputs), _P]),
     "tmae_mask_select": (C.c_int, [_P, C.c_int, C.c_int, C.c_int, C.c_int, _P, _P, _P, _P]),
     "tmae_gaussian_rate": (C.c_int, [_P, _P, _P, C.c_int64, _P, _P, _P, _P]),
     "tmae_bottleneck_rate": (C.c_int, [_P, _P, C.c_int64, _P, _P, _P, _P]),

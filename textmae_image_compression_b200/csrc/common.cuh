@@ -110,6 +110,20 @@ __device__ __forceinline__ void gaussian_elem(float y, float mu, float sigma, fl
     lik = fmaxf(upper - lower, 1e-9f);
 }
 
+// compressai GaussianConditional.build_indexes (MCM.py:839) of four scales: lower-bounded at 0.11, then
+// index = (len - 1) - #{t in table[:-1] : scale <= t}  ==  #{t in table[:-1] : t < scale}.
+// The one definition behind every scale-table index the library emits (encoder and decoder must agree bit for bit).
+__device__ __forceinline__ int4 scale_indexes4(const float* __restrict__ table, int n_table, float4 sv) {
+    const float sc[4] = {fmaxf(sv.x, 0.11f), fmaxf(sv.y, 0.11f), fmaxf(sv.z, 0.11f), fmaxf(sv.w, 0.11f)};
+    int id[4] = {0, 0, 0, 0};
+    for (int t = 0; t < n_table - 1; ++t) {
+        const float tv = __ldg(table + t);
+#pragma unroll
+        for (int e = 0; e < 4; ++e) id[e] += (tv < sc[e]) ? 1 : 0;
+    }
+    return make_int4(id[0], id[1], id[2], id[3]);
+}
+
 // Programmatic dependent launch (PDL): a kernel launched with the programmatic-stream-serialization attribute may start
 // while its predecessor is still running; everything before pdl_wait() (barrier init, TMEM allocation, descriptor
 // prefetch) overlaps the predecessor's tail, pdl_wait() blocks until the predecessor has completed and flushed.

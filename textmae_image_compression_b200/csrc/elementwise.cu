@@ -256,18 +256,7 @@ gaussian_slice_kernel(const float* __restrict__ y, const float* __restrict__ mu,
             s4v.x = sat(sy.x); s4v.y = sat(sy.y); s4v.z = sat(sy.z); s4v.w = sat(sy.w);
             *reinterpret_cast<short4*>(sym16_out + off) = s4v;
         }
-        if (idx_out && scale_table) {
-            // compressai GaussianConditional.build_indexes (MCM.py:839): scales lower-bounded at 0.11, then
-            // index = (len - 1) - #{t in table[:-1] : scale <= t}  ==  #{t in table[:-1] : t < scale}
-            const float sc[4] = {fmaxf(sv.x, 0.11f), fmaxf(sv.y, 0.11f), fmaxf(sv.z, 0.11f), fmaxf(sv.w, 0.11f)};
-            int id[4] = {0, 0, 0, 0};
-            for (int t = 0; t < n_table - 1; ++t) {
-                const float tv = __ldg(scale_table + t);
-#pragma unroll
-                for (int e = 0; e < 4; ++e) id[e] += (tv < sc[e]) ? 1 : 0;
-            }
-            *reinterpret_cast<int4*>(idx_out + off) = make_int4(id[0], id[1], id[2], id[3]);
-        }
+        if (idx_out && scale_table) *reinterpret_cast<int4*>(idx_out + off) = scale_indexes4(scale_table, n_table, sv);
         if (yhat_out) *reinterpret_cast<float4*>(yhat_out + off) = yh;
         const int K = s * s;
         n = (int)(row / K);
@@ -321,7 +310,96 @@ cudaError_t launch_gaussian_flat(const float* y, const float* mu, const float* s
 }
 
 // ---------------------------------------------------------------------------------------------------------
-// Rate finalise: bpp[n] = -sum(log2 lik) / S^2 (rd_loss.py:15-20, per image) and the batch pair
+// Decode side (MCM.decompress, MCM.py:896-968, with the range decoder's symbols given): the symbols arrive in the range
+// coder's order (per image, channel-major (c, y, x)), the latents stay channels-last like everywhere else.  The arithmetic
+// is exactly the encoder's dequantisation - bottleneck_kernel's zh = sym + med and gaussian_elem's yhat = sym + mu - so a
+// decoder of the same configuration reproduces the encoder's latents bit for bit.
+// ---------------------------------------------------------------------------------------------------------
+// z_hat = (float)sym + median (row 60 of eb_tab): fp32 to io->out.z_hat (optional) and the bf16 planes h_s reads.
+__global__ void __launch_bounds__(256)
+z_dequantize_kernel(const float* __restrict__ eb_tab, long long total, int Cz, int hw, __nv_bfloat16* __restrict__ zhat_bf,
+                    long long lo_off, const IoBlock* __restrict__ io) {
+    pdl_wait();
+    pdl_launch_dependents();
+    const long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (idx >= total) return;
+    const long long row = idx / Cz;
+    const int c = (int)(idx - row * Cz);
+    const long long n = row / hw;
+    const int p = (int)(row - n * hw);
+    const float zh = (float)io->z_symbols[(n * Cz + c) * hw + p] + eb_tab[60 * Cz + c];
+    if (io->out.z_hat) io->out.z_hat[idx] = zh;
+    store_bf16_planes(zhat_bf + idx, lo_off, zh);
+}
+cudaError_t launch_z_dequantize(const float* eb_tab, long long rows, int Cz, int hw, __nv_bfloat16* zhat_bf, long long lo_off,
+                                cudaStream_t st, const IoBlock* io) {
+    const long long total = rows * Cz;
+    if (total == 0) return cudaSuccess;
+    TMAE_CARVEOUT_ONCE(z_dequantize_kernel);
+    return launch_k(z_dequantize_kernel, dim3((unsigned)((total + 255) / 256)), dim3(256), 0, st, true, eb_tab, total, Cz, hw, zhat_bf,
+                    lo_off, io);
+}
+
+// Scale-table indexes of `cs` channels from col0 of sigma [rows, ld] (the separate-GEMM path; the fused cc.8 layer emits
+// them in its store phase) into io->out.y_indexes in the range coder's order.  Thread = 4 channels of one pixel.
+__global__ void __launch_bounds__(256)
+slice_indexes_kernel(const float* __restrict__ sigma, long long rows, int ld, int col0, int cs, int hw, const float* __restrict__ scale_table,
+                     int n_table, const IoBlock* __restrict__ io) {
+    pdl_wait();
+    pdl_launch_dependents();
+    const int vec_per_row = cs >> 2;
+    const long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (idx >= rows * vec_per_row) return;
+    const long long row = idx / vec_per_row;
+    const int c = col0 + (int)(idx - row * vec_per_row) * 4;
+    const long long n = row / hw;
+    const int p = (int)(row - n * hw);
+    const int4 id = scale_indexes4(scale_table, n_table, *reinterpret_cast<const float4*>(sigma + (size_t)row * ld + c));
+    int32_t* dst = io->out.y_indexes + (n * ld + c) * hw + p;
+    dst[0] = id.x; dst[hw] = id.y; dst[2 * hw] = id.z; dst[3 * hw] = id.w;
+}
+cudaError_t launch_slice_indexes(const float* sigma, long long rows, int ld, int col0, int cs, int hw, const float* scale_table,
+                                 int n_table, cudaStream_t st, const IoBlock* io) {
+    const long long total = rows * (cs / 4);
+    if (total == 0) return cudaSuccess;
+    TMAE_CARVEOUT_ONCE(slice_indexes_kernel);
+    return launch_k(slice_indexes_kernel, dim3((unsigned)((total + 255) / 256)), dim3(256), 0, st, true, sigma, rows, ld, col0, cs, hw,
+                    scale_table, n_table, io);
+}
+
+// y_hat = (float)sym + mu for `cs` channels from col0: the caller's symbols (io->y_symbols, range-coder order) and this
+// run's mu -> fp32 yhat [rows, ld] and its bf16 planes (support of the later slices; LRP then adds in place, as in the
+// forward).  Thread = 4 channels of one pixel.
+__global__ void __launch_bounds__(256)
+slice_dequantize_kernel(const float* __restrict__ mu, long long rows, int ld, int col0, int cs, int hw, float* __restrict__ yhat,
+                        __nv_bfloat16* __restrict__ yhat_bf, long long lo_off, const IoBlock* __restrict__ io) {
+    pdl_wait();
+    pdl_launch_dependents();
+    const int vec_per_row = cs >> 2;
+    const long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (idx >= rows * vec_per_row) return;
+    const long long row = idx / vec_per_row;
+    const int c = col0 + (int)(idx - row * vec_per_row) * 4;
+    const long long n = row / hw;
+    const int p = (int)(row - n * hw);
+    const int32_t* sym = io->y_symbols + (n * ld + c) * hw + p;
+    const size_t off = (size_t)row * ld + c;
+    const float4 mv = *reinterpret_cast<const float4*>(mu + off);
+    const float4 yh = make_float4((float)sym[0] + mv.x, (float)sym[hw] + mv.y, (float)sym[2 * hw] + mv.z, (float)sym[3 * hw] + mv.w);
+    *reinterpret_cast<float4*>(yhat + off) = yh;
+    store_bf16x4_planes(yhat_bf + off, lo_off, yh.x, yh.y, yh.z, yh.w);
+}
+cudaError_t launch_slice_dequantize(const float* mu, long long rows, int ld, int col0, int cs, int hw, float* yhat,
+                                    __nv_bfloat16* yhat_bf, long long lo_off, cudaStream_t st, const IoBlock* io) {
+    const long long total = rows * (cs / 4);
+    if (total == 0) return cudaSuccess;
+    TMAE_CARVEOUT_ONCE(slice_dequantize_kernel);
+    return launch_k(slice_dequantize_kernel, dim3((unsigned)((total + 255) / 256)), dim3(256), 0, st, true, mu, rows, ld, col0, cs, hw,
+                    yhat, yhat_bf, lo_off, io);
+}
+
+// ---------------------------------------------------------------------------------------------------------
+// Rate finalise:bpp[n] = -sum(log2 lik) / S^2 (rd_loss.py:15-20, per image) and the batch pair
 // {sum log2 lik, N*S*S} that the data-parallel all-reduce combines.
 // ---------------------------------------------------------------------------------------------------------
 __global__ void rate_finalize_kernel(const double* __restrict__ rate_acc, int N, double pixels_per_image,

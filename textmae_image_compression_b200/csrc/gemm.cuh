@@ -110,7 +110,7 @@ struct alignas(64) GemmParams {
     // [32, 64) = sigma of slice i - and the epilogue (thread = pixel) quantises y, evaluates the likelihoods, emits symbols /
     // scale-table indexes / y_hat and adds the pixel's log2-likelihood to its image's rate.  No gaussian_slice_kernel launch, mu
     // and sigma never travel through HBM to be read back.
-    int gc_on;
+    int gc_on;                        // 1 = encoder (EPI_GAUSS), 2 = decoder: mu, sigma and indexes only (EPI_GAUSS_IDX)
     int gc_col0;                      // first channel of the slice in the [rows, gc_ld] tensors
     int gc_ld;                        // Cy
     int gc_pixels;                    // pixels per image (rate accumulator index = row / gc_pixels)

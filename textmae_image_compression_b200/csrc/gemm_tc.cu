@@ -236,7 +236,8 @@ constexpr int kAStageBytes = kBlockM * kBlockK * 2;   // 16 KB
 //                      registers, bf16 boxes of 32 columns staged in smem (64B swizzle) and written by TMA stores
 //   EPI_GAUSS          last layer of cc_transform_mean[i] + cc_transform_scale[i] as one block-diagonal 64-column GEMM: the
 //                      Gaussian conditional (quantise, likelihood, symbols, indexes, y_hat, rate) runs here, thread = pixel
-enum EpiKind : int { EPI_GENERIC = 0, EPI_BF16_SAME = 1, EPI_F32_SAME_RESID = 2, EPI_BF16_TMA = 3, EPI_GAUSS = 4 };
+//   EPI_GAUSS_IDX      the same layer in the decoder (GemmParams::gc_on == 2): mu, sigma and scale-table indexes only
+enum EpiKind : int { EPI_GENERIC = 0, EPI_BF16_SAME = 1, EPI_F32_SAME_RESID = 2, EPI_BF16_TMA = 3, EPI_GAUSS = 4, EPI_GAUSS_IDX = 5 };
 constexpr uint32_t kStoreBoxBytes = kBlockM * 32 * 2;      // one 128 x 32 bf16 box
 
 // ---------------------------------------------------------------------------------------------------------
@@ -384,16 +385,8 @@ __device__ __forceinline__ void epilogue_tile_impl(const EpiCtx& e, int m_tile, 
                         s4v.x = sat(sy.x); s4v.y = sat(sy.y); s4v.z = sat(sy.z); s4v.w = sat(sy.w);
                         *reinterpret_cast<short4*>(sym16_out + o4) = s4v;
                     }
-                    if (idx_out && g.gc_table) {            // GaussianConditional.build_indexes (MCM.py:839), as in gaussian_slice_kernel
-                        const float sc[4] = {fmaxf(sv.x, 0.11f), fmaxf(sv.y, 0.11f), fmaxf(sv.z, 0.11f), fmaxf(sv.w, 0.11f)};
-                        int id[4] = {0, 0, 0, 0};
-                        for (int t = 0; t < g.gc_ntable - 1; ++t) {
-                            const float tv = __ldg(g.gc_table + t);
-#pragma unroll
-                            for (int q = 0; q < 4; ++q) id[q] += (tv < sc[q]) ? 1 : 0;
-                        }
-                        *reinterpret_cast<int4*>(idx_out + o4) = make_int4(id[0], id[1], id[2], id[3]);
-                    }
+                    if (idx_out && g.gc_table)              // GaussianConditional.build_indexes (MCM.py:839)
+                        *reinterpret_cast<int4*>(idx_out + o4) = scale_indexes4(g.gc_table, g.gc_ntable, sv);
                     lg += (log2f(lk.x) + log2f(lk.y)) + (log2f(lk.z) + log2f(lk.w));
                 }
             }
@@ -408,6 +401,51 @@ __device__ __forceinline__ void epilogue_tile_impl(const EpiCtx& e, int m_tile, 
                 if (lane == 0 && sm != 0.f) atomicAdd(g.gc_rate + n_first, (double)sm);
             } else if (r.valid) {
                 atomicAdd(g.gc_rate + r.n, (double)lg);
+            }
+        }
+        return;
+    }
+    if (EPI == EPI_GAUSS_IDX) {
+        // Decoder side of EPI_GAUSS: same column interleave and bias adds, but no y exists yet - the store phase writes mu,
+        // sigma and the scale-table indexes the range decoder needs before it can produce the slice's symbols.  Indexes go
+        // out in the range coder's order: per image, channel-major (c, y, x).
+        const GemmParams& g = *e.gp;
+        const IoBlock* io = reinterpret_cast<const IoBlock*>(g.gc_io);
+        int32_t* idx_out = io->out.y_indexes;
+        const RowCtx r = decode_row(e, m_tile, quarter * 32 + lane);
+        mbar_wait(wait_bar, wait_parity);
+        tc_fence_after();
+        const uint32_t lane_base = tmem_acc + ((uint32_t)(quarter * 32) << 16);
+        const int b = n0 >> 5;
+        uint32_t acc[32];
+        tmem_ld_32x32b_x32(lane_base, acc);
+        tmem_ld_wait();
+        if (r.valid) {
+            const int c0 = g.gc_col0 + b * 16;
+            const size_t off = (size_t)r.lin * g.gc_ld + c0;
+            int32_t* idx_px = idx_out + (size_t)r.n * g.gc_ld * g.gc_pixels + (r.y * e.s + r.x);
+#pragma unroll
+            for (int jj = 0; jj < 2; ++jj) {
+                const int j = half * 2 + jj;
+                const float4 bm = __ldg(reinterpret_cast<const float4*>(e.bias + n0 + 4 * j));
+                const float4 bs = __ldg(reinterpret_cast<const float4*>(e.bias + n0 + 16 + 4 * j));
+                float a[8];
+#pragma unroll
+                for (int q = 0; q < 4; ++q) {
+                    a[q] = __uint_as_float(half == 0 ? acc[4 * jj + q] : acc[8 + 4 * jj + q]);
+                    a[4 + q] = __uint_as_float(half == 0 ? acc[16 + 4 * jj + q] : acc[24 + 4 * jj + q]);
+                }
+                const float4 mv = make_float4(a[0] + bm.x, a[1] + bm.y, a[2] + bm.z, a[3] + bm.w);
+                const float4 sv = make_float4(a[4] + bs.x, a[5] + bs.y, a[6] + bs.z, a[7] + bs.w);
+                const size_t o4 = off + 4 * j;
+                *reinterpret_cast<float4*>(g.gc_mu + o4) = mv;
+                *reinterpret_cast<float4*>(g.gc_sigma + o4) = sv;
+                const int4 id = scale_indexes4(g.gc_table, g.gc_ntable, sv);
+                int32_t* dst = idx_px + (size_t)(c0 + 4 * j) * g.gc_pixels;
+                dst[0] = id.x;
+                dst[g.gc_pixels] = id.y;
+                dst[2 * g.gc_pixels] = id.z;
+                dst[3 * g.gc_pixels] = id.w;
             }
         }
         return;
@@ -1291,6 +1329,7 @@ cudaError_t gemm_tc_configure() {
     if ((e = configure_one<ACT_GELU, EPI_BF16_SAME>()) != cudaSuccess) return e;
     if ((e = configure_one<ACT_NONE, EPI_F32_SAME_RESID>()) != cudaSuccess) return e;
     if ((e = configure_one<ACT_NONE, EPI_GAUSS>()) != cudaSuccess) return e;
+    if ((e = configure_one<ACT_NONE, EPI_GAUSS_IDX>()) != cudaSuccess) return e;
     if ((e = configure_one<ACT_NONE, EPI_BF16_TMA>()) != cudaSuccess) return e;
     if ((e = configure_one<ACT_GELU, EPI_BF16_TMA>()) != cudaSuccess) return e;
     {
@@ -1337,7 +1376,7 @@ bool gemm_use_persistent(int groups, int epi, int act, int tiles, bool share_sm)
 
 // Store-phase specialisation a parameter block qualifies for (every member of a grouped launch must agree).
 int gemm_epi_kind(const GemmParams& p) {
-    if (p.gc_on) return EPI_GAUSS;
+    if (p.gc_on) return p.gc_on == 2 ? EPI_GAUSS_IDX : EPI_GAUSS;
     const bool one_out = p.out[1].dtype == OUT_NONE && p.out[0].map == MAP_SAME;
     static const bool no_tma_store = getenv("TMAE_NO_TMA_STORE") != nullptr;
     if (one_out && p.out[0].dtype == OUT_BF16 && p.resid == nullptr && p.act != ACT_HALF_TANH)
@@ -1455,6 +1494,7 @@ cudaError_t gemm_launch(const GemmParams* d_params, int groups, int max_M, int m
     const int two_prod = two_prod_env >= 0 ? two_prod_env : 0;
     // every member of a grouped launch shares the activation and the store-phase specialisation
     if (epi == EPI_GAUSS) return launch_k(gemm_tc_kernel<ACT_NONE, EPI_GAUSS>, grid, dim3(kGemmThreads), smem, stream, true, d_params, stages, kgroup, d_next, next_groups, two_prod);
+    if (epi == EPI_GAUSS_IDX) return launch_k(gemm_tc_kernel<ACT_NONE, EPI_GAUSS_IDX>, grid, dim3(kGemmThreads), smem, stream, true, d_params, stages, kgroup, d_next, next_groups, two_prod);
     if (epi == EPI_BF16_TMA && act == ACT_GELU) return launch_k(gemm_tc_kernel<ACT_GELU, EPI_BF16_TMA>, grid, dim3(kGemmThreads), smem, stream, true, d_params, stages, kgroup, d_next, next_groups, two_prod);
     else if (epi == EPI_BF16_TMA && act == ACT_NONE) return launch_k(gemm_tc_kernel<ACT_NONE, EPI_BF16_TMA>, grid, dim3(kGemmThreads), smem, stream, true, d_params, stages, kgroup, d_next, next_groups, two_prod);
     else if (epi == EPI_BF16_SAME && act == ACT_GELU) return launch_k(gemm_tc_kernel<ACT_GELU, EPI_BF16_SAME>, grid, dim3(kGemmThreads), smem, stream, true, d_params, stages, kgroup, d_next, next_groups, two_prod);

@@ -15,6 +15,8 @@ struct IoBlock {
     const float* imgs;
     const float* scores;
     tmae_outputs out;
+    const int32_t* z_symbols;        // decode: z symbols [N, Cz, s/4, s/4] (range-coder order)
+    const int32_t* y_symbols;        // decode: y symbols [N, Cy * s * s], per image slice by slice in (c, y, x) order
 };
 
 // gemm_tc.cu
@@ -65,6 +67,13 @@ cudaError_t launch_gaussian_slice(const float* y, const float* mu, const float* 
                                   int cs, float* lik, int32_t* sym, float* yhat, __nv_bfloat16* yhat_bf, long long lo_off,
                                   int ld_bf, int s, double* rate_acc, const float* scale_table, int n_table, int16_t* sym16,
                                   int32_t* idx, cudaStream_t st, const IoBlock* io = nullptr);
+// decode side (the range coder's symbols back to the latents)
+cudaError_t launch_z_dequantize(const float* eb_tab, long long rows, int Cz, int hw, __nv_bfloat16* zhat_bf, long long lo_off,
+                                cudaStream_t st, const IoBlock* io);
+cudaError_t launch_slice_indexes(const float* sigma, long long rows, int ld, int col0, int cs, int hw, const float* scale_table,
+                                 int n_table, cudaStream_t st, const IoBlock* io);
+cudaError_t launch_slice_dequantize(const float* mu, long long rows, int ld, int col0, int cs, int hw, float* yhat,
+                                    __nv_bfloat16* yhat_bf, long long lo_off, cudaStream_t st, const IoBlock* io);
 cudaError_t launch_pack_nchw_i32(const int32_t* src, int32_t* dst, int N, int hw, int C, cudaStream_t st);
 cudaError_t launch_gaussian_flat(const float* y, const float* mu, const float* sigma, long long n, float* lik,
                                  int32_t* sym, float* yhat, cudaStream_t st);

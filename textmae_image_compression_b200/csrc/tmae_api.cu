@@ -51,7 +51,8 @@ struct Bf {
     long long lo = 0;
 };
 
-enum StepKind { ST_MASK, ST_GATHER, ST_GEMM, ST_FORCE, ST_LN, ST_ATTN, ST_EB, ST_GC, ST_RATE, ST_ZERO_RATE };
+enum StepKind { ST_MASK, ST_GATHER, ST_GEMM, ST_FORCE, ST_LN, ST_ATTN, ST_EB, ST_GC, ST_RATE, ST_ZERO_RATE,
+                ST_ZDEQ, ST_IDX, ST_YDEQ, ST_DEC_OUT };     // the last four: decode plans only
 enum Family { FAM_GEMM = 0, FAM_ATTN, FAM_LN, FAM_MASK, FAM_GATHER, FAM_ENTROPY, FAM_MISC, FAM_COUNT };
 const char* kFamilyNames[FAM_COUNT] = {"gemm_tc", "attention", "layernorm", "mask_select", "gather_patches",
                                        "entropy_elementwise", "misc"};
@@ -88,6 +89,10 @@ struct Plan {
     CUtensorMap attn_q, attn_k;
     int first_rate_step = 0;        // index of the first step of the rate half (h_a)
     int encoder_end_step = 0;       // one past the final LayerNorm
+    // decode plans: stage k = steps [stage_begin[k], stage_begin[k + 1]), one CUDA graph per stage
+    std::vector<int> stage_begin;
+    std::vector<cudaGraphExec_t> stage_graph;
+    std::vector<int> stage_calls;
 };
 
 struct Workspace {
@@ -137,6 +142,8 @@ struct tmae_handle {
     bool finalized = false;
     Workspace ws;
     std::map<int, std::unique_ptr<Plan>> plans;
+    std::map<int, std::unique_ptr<Plan>> dec_plans;   // decode plans by batch size (tmae_decode_begin / _step)
+    int dec_N = 0, dec_next = -1;    // decode in progress: batch size and the next group expected (-1 = none)
     PFN_encodeTiled encode = nullptr;
     std::vector<void*> weight_allocs;
     bool use_graph = true;           // TMAE_NO_GRAPH=1 disables CUDA-graph replay
@@ -478,6 +485,7 @@ struct GemmDesc {
     OutSpec out1 = {nullptr, 0, OUT_NONE, MAP_SAME, 0};
     double flops = 0;
     int gc_slice = -1;          // >= 0: fused mean + scale last layer of this slice, Gaussian conditional in the epilogue
+    bool gc_decode = false;     // ... decoder form: mu, sigma and scale-table indexes only (EPI_GAUSS_IDX)
 };
 
 int fill_params(tmae_handle* h, const GemmDesc& d, int groups_for_tiling, GemmParams* p, int force_block_n) {
@@ -581,7 +589,7 @@ int fill_params(tmae_handle* h, const GemmDesc& d, int groups_for_tiling, GemmPa
         const Workspace& w = h->ws;
         if (L.Cout != 2 * h->sc || p->block_n != 32 || (L.Cout & 31) != 0 || L.planes != 1)
             return fail(h, TMAE_EINVAL, "fused Gaussian layer: needs 32-column tiles of a %d-column layer (block_n %d)", L.Cout, p->block_n);
-        p->gc_on = 1;
+        p->gc_on = d.gc_decode ? 2 : 1;
         p->gc_col0 = d.gc_slice * h->sc;
         p->gc_ld = h->Cy;
         p->gc_pixels = h->K;
@@ -595,6 +603,15 @@ int fill_params(tmae_handle* h, const GemmDesc& d, int groups_for_tiling, GemmPa
 }
 
 // ---- workspace -----------------------------------------------------------------------------------------
+void drop_plans(std::map<int, std::unique_ptr<Plan>>& plans) {
+    for (auto& kv : plans) {
+        if (kv.second->d_params) cudaFree(kv.second->d_params);
+        if (kv.second->graph) cudaGraphExecDestroy(kv.second->graph);
+        for (cudaGraphExec_t g : kv.second->stage_graph) if (g) cudaGraphExecDestroy(g);
+    }
+    plans.clear();
+}
+
 void free_pool(std::vector<void*>& pool) {
     for (void* p : pool) cudaFree(p);
     pool.clear();
@@ -604,8 +621,8 @@ int ensure_workspace(tmae_handle* h, int N) {
     Workspace& w = h->ws;
     if (N <= w.cap_N) return TMAE_OK;
     // plans hold pointers into the workspace: drop them
-    for (auto& kv : h->plans) { if (kv.second->d_params) cudaFree(kv.second->d_params); if (kv.second->graph) cudaGraphExecDestroy(kv.second->graph); }
-    h->plans.clear();
+    drop_plans(h->plans);
+    drop_plans(h->dec_plans);
     free_pool(w.allocs);
     w = Workspace();
     size_t tot = 0;
@@ -828,6 +845,165 @@ const Layer* get_layer(tmae_handle* h, const std::string& key) {
     return it == h->layers.end() ? nullptr : &it->second;
 }
 
+// 3x3 conv input over a `side` x `side` grid of all N images (compact rows; the tile grid covers box_y x box_n blocks)
+void conv_input(GemmDesc& d, int side, int N) {
+    ConvGeom cg;
+    conv_geom(side, N, &cg);
+    d.in_mode = IN_CONV; d.side = side; d.n_img = N;
+    d.a_rows = (long long)N * side * side; d.M = cg.m_tiles * kBlockM;
+}
+
+// Pieces of the rate half shared by the forward plan (build_plan) and the decode plan (build_decode_plan): the same
+// layers with the same launch shapes, so that a decoder reproduces the encoder's mu / sigma / y_hat bit for bit.
+// h_s_mean / h_s_scale as a group of two per layer (MCM.py:132-162, 747-748)
+int add_hs_steps(tmae_handle* h, Plan& pl, int N) {
+    Workspace& w = h->ws;
+    const int s = h->s;
+    char tag[96];
+    int rc;
+    auto conv_in = [&](GemmDesc& d, int side) { conv_input(d, side, N); };
+    int ci[5], co[5], up[5];
+    hs_layers(h, ci, co, up);
+    const int sides[5] = {h->s4, h->s4, h->s2, h->s2, s};
+    const char* nets[2] = {"h_s_mean", "h_s_scale"};
+    for (int l = 0; l < 5; ++l) {
+        GemmDesc d[2];
+        for (int net = 0; net < 2; ++net) {
+            const Bf srcs[5] = {w.zhat_bf, w.hs1[net], w.hs2[net], w.hs3[net], w.hs4[net]};
+            const Bf dsts[5] = {w.hs1[net], w.hs2[net], w.hs3[net], w.hs4[net], w.lat[net]};
+            d[net].layer = get_layer(h, std::string(nets[net]) + "." + std::to_string(2 * l));
+            d[net].seg[0] = seg(srcs[l], ci[l], ci[l]);
+            conv_in(d[net], sides[l]);
+            d[net].act = l < 4 ? ACT_GELU : ACT_NONE;
+            d[net].out0 = outspec(dsts[l], co[l], up[l] == 2 ? MAP_SHUF : MAP_SAME);
+            d[net].flops = conv_flops((long long)N * sides[l] * sides[l], ci[l], co[l] * up[l] * up[l], 9);
+        }
+        snprintf(tag, sizeof(tag), "h_s.%d", 2 * l);
+        rc = add_gemm_group(h, pl, d, 2, tag); if (rc) return rc;
+    }
+    return TMAE_OK;
+}
+
+// cc_transform_mean[i] / cc_transform_scale[i] of the slice group [i0, i0 + cnt) (MCM.py:756-768).  decode: the fused last
+// layer stores mu, sigma and the scale-table indexes (EPI_GAUSS_IDX) instead of running the Gaussian conditional.
+int add_cc_steps(tmae_handle* h, Plan& pl, int N, int i0, int cnt, bool decode) {
+    Workspace& w = h->ws;
+    const int s = h->s, Cy = h->Cy;
+    const long long rk = (long long)N * h->K;
+    const int half_sl = h->nsl / 2;
+    const int sup = i0 < half_sl ? i0 : half_sl;
+    char tag[96];
+    int rc;
+    auto conv_in = [&](GemmDesc& d, int side) { conv_input(d, side, N); };
+    int ch[6];
+    cc_channels(h, ch, i0, false);
+    for (int l = 0; l < 5; ++l) {    // cc_transform_mean[i] and cc_transform_scale[i] of every member, grouped
+        if (l == 4 && h->gc_fuse) {
+            // last layers of both nets as ONE block-diagonal GEMM per member (K segments = the two nets' activations);
+            // its epilogue is the Gaussian conditional of the slice (MCM.py:762-776): no mu / sigma round trip, no extra launch
+            std::vector<GemmDesc> d((size_t)cnt);
+            for (int j = 0; j < cnt; ++j) {
+                GemmDesc& g = d[(size_t)j];
+                const int i = i0 + j;
+                g.layer = get_layer(h, "gc." + std::to_string(i));
+                g.seg[0] = seg(w.t[j * 3 + 0][3], ch[4], ch[4]);
+                g.seg[1] = seg(w.t[j * 3 + 1][3], ch[4], ch[4]);
+                g.nseg = 2;
+                conv_in(g, s);
+                g.gc_slice = i;
+                g.gc_decode = decode;
+                g.flops = 2.0 * conv_flops(rk, ch[4], ch[5], 9);      // the two layers as the reference counts them (the zero blocks are not work)
+            }
+            snprintf(tag, sizeof(tag), decode ? "cc.%d.8+idx" : "cc.%d.8+gauss", i0);
+            rc = add_gemm_group(h, pl, d.data(), cnt, tag); if (rc) return rc;
+            continue;
+        }
+        std::vector<GemmDesc> d((size_t)cnt * 2);
+        for (int j = 0; j < cnt; ++j)
+            for (int net = 0; net < 2; ++net) {
+                GemmDesc& g = d[(size_t)j * 2 + net];
+                const int i = i0 + j;
+                const char* nm = net == 0 ? "cc_transform_mean." : "cc_transform_scale.";
+                g.layer = get_layer(h, std::string(nm) + std::to_string(i) + "." + std::to_string(2 * l));
+                if (l == 0) {
+                    g.seg[0] = seg(w.lat[net], Cy, Cy);
+                    g.nseg = 1;
+                    if (sup > 0) { g.seg[1] = seg(w.yhat_bf, h->sc * sup, Cy); g.nseg = 2; }
+                } else {
+                    g.seg[0] = seg(w.t[j * 3 + net][l - 1], ch[l], ch[l]);
+                }
+                conv_in(g, s);
+                if (l < 4) { g.act = ACT_GELU; g.out0 = outspec(w.t[j * 3 + net][l], ch[l + 1], MAP_SAME); }
+                else g.out0 = outspec((net == 0 ? w.mu : w.sigma) + i * h->sc, Cy, OUT_F32, MAP_SAME);
+                g.flops = conv_flops(rk, ch[l], ch[l + 1], 9);
+            }
+        snprintf(tag, sizeof(tag), "cc.%d.%d", i0, 2 * l);
+        rc = add_gemm_group(h, pl, d.data(), cnt * 2, tag); if (rc) return rc;
+    }
+    return TMAE_OK;
+}
+
+// lrp_transform[i] of the slice group (MCM.py:780-783): y_hat += 0.5 tanh(lrp(...)) in place on w.yhat
+int add_lrp_steps(tmae_handle* h, Plan& pl, int N, int i0, int cnt, bool forced) {
+    Workspace& w = h->ws;
+    const int s = h->s, Cy = h->Cy;
+    const long long rk = (long long)N * h->K;
+    const int half_sl = h->nsl / 2;
+    const int sup = i0 < half_sl ? i0 : half_sl;
+    char tag[96];
+    int rc;
+    auto conv_in = [&](GemmDesc& d, int side) { conv_input(d, side, N); };
+    int lch[6];
+    cc_channels(h, lch, i0, true);
+    for (int l = 0; l < 5; ++l) {    // lrp_transform[i] (MCM.py:780-783)
+        std::vector<GemmDesc> d((size_t)cnt);
+        for (int j = 0; j < cnt; ++j) {
+            GemmDesc& g = d[j];
+            const int i = i0 + j;
+            g.layer = get_layer(h, "lrp_transform." + std::to_string(i) + "." + std::to_string(2 * l));
+            if (l == 0) {
+                g.seg[0] = seg(w.lat[0], Cy, Cy);
+                if (i < half_sl) { g.seg[1] = seg(w.yhat_bf, h->sc * (i + 1), Cy); g.nseg = 2; }
+                else { g.seg[1] = seg(w.yhat_bf, h->sc * sup, Cy); g.seg[2] = seg(w.yhat_bf, h->sc, Cy, i * h->sc); g.nseg = 3; }
+            } else {
+                g.seg[0] = seg(w.t[j * 3 + 2][l - 1], lch[l], lch[l]);
+            }
+            conv_in(g, s);
+            if (l < 4) { g.act = ACT_GELU; g.out0 = outspec(w.t[j * 3 + 2][l], lch[l + 1], MAP_SAME); }
+            else {
+                g.act = ACT_HALF_TANH;
+                g.resid = w.yhat + i * h->sc; g.resid_ld = Cy; g.resid_map = MAP_SAME;
+                g.out0 = outspec(w.yhat + i * h->sc, Cy, OUT_F32, MAP_SAME);
+                if (!(forced && i < half_sl)) g.out1 = outspec(w.yhat_bf, Cy, MAP_SAME, i * h->sc);
+            }
+            g.flops = conv_flops(rk, lch[l], lch[l + 1], 9);
+        }
+        snprintf(tag, sizeof(tag), "lrp.%d.%d", i0, 2 * l);
+        rc = add_gemm_group(h, pl, d.data(), cnt, tag); if (rc) return rc;
+    }
+    return TMAE_OK;
+}
+
+// Common tail of every plan: sanity check, weight-prefetch chain, parameter blocks to the device.
+int finish_plan(tmae_handle* h, Plan& pl) {
+    for (const Step& st : pl.steps)
+        if (st.kind == ST_GEMM && pl.host_params[st.param_index].num_segs < 1) return fail(h, TMAE_EINVAL, "bad plan");
+    if (!getenv("TMAE_NO_WEIGHT_PREFETCH")) {      // each GEMM step prefetches the weights of the next one (cyclically)
+        std::vector<int> gemm_steps;
+        for (size_t i = 0; i < pl.steps.size(); ++i) if (pl.steps[i].kind == ST_GEMM) gemm_steps.push_back((int)i);
+        for (size_t k = 0; k < gemm_steps.size(); ++k) {
+            const Step& nx = pl.steps[gemm_steps[(k + 1) % gemm_steps.size()]];
+            pl.steps[gemm_steps[k]].next_index = nx.param_index;
+            pl.steps[gemm_steps[k]].next_groups = nx.groups;
+        }
+    }
+    void* dp = nullptr;
+    CUDA_TRY(h, cudaMalloc(&dp, pl.host_params.size() * sizeof(GemmParams)));
+    pl.d_params = reinterpret_cast<GemmParams*>(dp);
+    CUDA_TRY(h, cudaMemcpy(pl.d_params, pl.host_params.data(), pl.host_params.size() * sizeof(GemmParams), cudaMemcpyHostToDevice));
+    return TMAE_OK;
+}
+
 // forced = slice-wise teacher forcing (tmae_forward_from_latent_forced): after lrp_transform[i] the support columns of
 // slice i are overwritten with the caller's y_hat, so slice j > i never sees a symbol this run decided itself.
 int build_plan(tmae_handle* h, int N, Plan** out, bool forced = false) {
@@ -844,13 +1020,7 @@ int build_plan(tmae_handle* h, int N, Plan** out, bool forced = false) {
     const int C = h->C, T = h->T, K = h->K, s = h->s, Cy = h->Cy, Cz = h->Cz;
     const long long rt = (long long)N * T, rk = (long long)N * K;
     char tag[96];
-    // 3x3 conv input over a `side` x `side` grid of all N images (compact rows; the tile grid covers box_y x box_n blocks)
-    auto conv_in = [&](GemmDesc& d, int side) {
-        ConvGeom cg;
-        conv_geom(side, N, &cg);
-        d.in_mode = IN_CONV; d.side = side; d.n_img = N;
-        d.a_rows = (long long)N * side * side; d.M = cg.m_tiles * kBlockM;
-    };
+    auto conv_in = [&](GemmDesc& d, int side) { conv_input(d, side, N); };
     auto simple = [&](StepKind k, int fam, const char* t) { Step st; st.kind = k; st.family = fam; st.tag = t; pl.steps.push_back(st); };
 
     if (!h->precise_enc && !(h->cfg.flags & TMAE_FLAG_DEBUG_SIMT) && attention_tc_eligible(T)) {
@@ -967,109 +1137,16 @@ int build_plan(tmae_handle* h, int N, Plan** out, bool forced = false) {
         }
     }
     simple(ST_EB, FAM_ENTROPY, "entropy_bottleneck");
-    {   // h_s_mean / h_s_scale as a group of two per layer (MCM.py:132-162, 747-748)
-        int ci[5], co[5], up[5];
-        hs_layers(h, ci, co, up);
-        const int sides[5] = {h->s4, h->s4, h->s2, h->s2, s};
-        const char* nets[2] = {"h_s_mean", "h_s_scale"};
-        for (int l = 0; l < 5; ++l) {
-            GemmDesc d[2];
-            for (int net = 0; net < 2; ++net) {
-                const Bf srcs[5] = {w.zhat_bf, w.hs1[net], w.hs2[net], w.hs3[net], w.hs4[net]};
-                const Bf dsts[5] = {w.hs1[net], w.hs2[net], w.hs3[net], w.hs4[net], w.lat[net]};
-                d[net].layer = get_layer(h, std::string(nets[net]) + "." + std::to_string(2 * l));
-                d[net].seg[0] = seg(srcs[l], ci[l], ci[l]);
-                conv_in(d[net], sides[l]);
-                d[net].act = l < 4 ? ACT_GELU : ACT_NONE;
-                d[net].out0 = outspec(dsts[l], co[l], up[l] == 2 ? MAP_SHUF : MAP_SAME);
-                d[net].flops = conv_flops((long long)N * sides[l] * sides[l], ci[l], co[l] * up[l] * up[l], 9);
-            }
-            snprintf(tag, sizeof(tag), "h_s.%d", 2 * l);
-            rc = add_gemm_group(h, pl, d, 2, tag); if (rc) return rc;
-        }
-    }
+    if ((rc = add_hs_steps(h, pl, N))) return rc;
     const bool skip_dead = (h->cfg.flags & TMAE_FLAG_SKIP_DEAD_LRP) != 0;
     // Slice loop (MCM.py:755-784).  Slice i reads y_hat of slices [0, min(i, 6)): slices 0..5 form a serial chain,
     // slices 6..11 depend only on 0..5 and are mutually independent, so they run as ONE grouped launch per layer.
     const int half_sl = h->nsl / 2;
     for (int i0 = 0; i0 < h->nsl;) {
         const int cnt = i0 < half_sl ? 1 : h->nsl - i0;          // members of this slice group
-        const int sup = i0 < half_sl ? i0 : half_sl;
-        int ch[6];
-        cc_channels(h, ch, i0, false);
-        for (int l = 0; l < 5; ++l) {    // cc_transform_mean[i] and cc_transform_scale[i] of every member, grouped
-            if (l == 4 && h->gc_fuse) {
-                // last layers of both nets as ONE block-diagonal GEMM per member (K segments = the two nets' activations);
-                // its epilogue is the Gaussian conditional of the slice (MCM.py:762-776): no mu / sigma round trip, no extra launch
-                std::vector<GemmDesc> d((size_t)cnt);
-                for (int j = 0; j < cnt; ++j) {
-                    GemmDesc& g = d[(size_t)j];
-                    const int i = i0 + j;
-                    g.layer = get_layer(h, "gc." + std::to_string(i));
-                    g.seg[0] = seg(w.t[j * 3 + 0][3], ch[4], ch[4]);
-                    g.seg[1] = seg(w.t[j * 3 + 1][3], ch[4], ch[4]);
-                    g.nseg = 2;
-                    conv_in(g, s);
-                    g.gc_slice = i;
-                    g.flops = 2.0 * conv_flops(rk, ch[4], ch[5], 9);      // the two layers as the reference counts them (the zero blocks are not work)
-                }
-                snprintf(tag, sizeof(tag), "cc.%d.8+gauss", i0);
-                rc = add_gemm_group(h, pl, d.data(), cnt, tag); if (rc) return rc;
-                continue;
-            }
-            std::vector<GemmDesc> d((size_t)cnt * 2);
-            for (int j = 0; j < cnt; ++j)
-                for (int net = 0; net < 2; ++net) {
-                    GemmDesc& g = d[(size_t)j * 2 + net];
-                    const int i = i0 + j;
-                    const char* nm = net == 0 ? "cc_transform_mean." : "cc_transform_scale.";
-                    g.layer = get_layer(h, std::string(nm) + std::to_string(i) + "." + std::to_string(2 * l));
-                    if (l == 0) {
-                        g.seg[0] = seg(w.lat[net], Cy, Cy);
-                        g.nseg = 1;
-                        if (sup > 0) { g.seg[1] = seg(w.yhat_bf, h->sc * sup, Cy); g.nseg = 2; }
-                    } else {
-                        g.seg[0] = seg(w.t[j * 3 + net][l - 1], ch[l], ch[l]);
-                    }
-                    conv_in(g, s);
-                    if (l < 4) { g.act = ACT_GELU; g.out0 = outspec(w.t[j * 3 + net][l], ch[l + 1], MAP_SAME); }
-                    else g.out0 = outspec((net == 0 ? w.mu : w.sigma) + i * h->sc, Cy, OUT_F32, MAP_SAME);
-                    g.flops = conv_flops(rk, ch[l], ch[l + 1], 9);
-                }
-            snprintf(tag, sizeof(tag), "cc.%d.%d", i0, 2 * l);
-            rc = add_gemm_group(h, pl, d.data(), cnt * 2, tag); if (rc) return rc;
-        }
+        if ((rc = add_cc_steps(h, pl, N, i0, cnt, false))) return rc;
         if (!h->gc_fuse) { Step g; g.kind = ST_GC; g.family = FAM_ENTROPY; g.slice = i0; g.gc_slices = cnt; g.tag = "gaussian." + std::to_string(i0); pl.steps.push_back(g); }
-        if (!(skip_dead && i0 >= half_sl)) {
-            int lch[6];
-            cc_channels(h, lch, i0, true);
-            for (int l = 0; l < 5; ++l) {    // lrp_transform[i] (MCM.py:780-783)
-                std::vector<GemmDesc> d((size_t)cnt);
-                for (int j = 0; j < cnt; ++j) {
-                    GemmDesc& g = d[j];
-                    const int i = i0 + j;
-                    g.layer = get_layer(h, "lrp_transform." + std::to_string(i) + "." + std::to_string(2 * l));
-                    if (l == 0) {
-                        g.seg[0] = seg(w.lat[0], Cy, Cy);
-                        if (i < half_sl) { g.seg[1] = seg(w.yhat_bf, h->sc * (i + 1), Cy); g.nseg = 2; }
-                        else { g.seg[1] = seg(w.yhat_bf, h->sc * sup, Cy); g.seg[2] = seg(w.yhat_bf, h->sc, Cy, i * h->sc); g.nseg = 3; }
-                    } else {
-                        g.seg[0] = seg(w.t[j * 3 + 2][l - 1], lch[l], lch[l]);
-                    }
-                    conv_in(g, s);
-                    if (l < 4) { g.act = ACT_GELU; g.out0 = outspec(w.t[j * 3 + 2][l], lch[l + 1], MAP_SAME); }
-                    else {
-                        g.act = ACT_HALF_TANH;
-                        g.resid = w.yhat + i * h->sc; g.resid_ld = Cy; g.resid_map = MAP_SAME;
-                        g.out0 = outspec(w.yhat + i * h->sc, Cy, OUT_F32, MAP_SAME);
-                        if (!(forced && i < half_sl)) g.out1 = outspec(w.yhat_bf, Cy, MAP_SAME, i * h->sc);
-                    }
-                    g.flops = conv_flops(rk, lch[l], lch[l + 1], 9);
-                }
-                snprintf(tag, sizeof(tag), "lrp.%d.%d", i0, 2 * l);
-                rc = add_gemm_group(h, pl, d.data(), cnt, tag); if (rc) return rc;
-            }
-        }
+        if (!(skip_dead && i0 >= half_sl) && (rc = add_lrp_steps(h, pl, N, i0, cnt, forced))) return rc;
         if (forced && i0 < half_sl) { Step f; f.kind = ST_FORCE; f.family = FAM_MISC; f.slice = i0; f.tag = "force." + std::to_string(i0); pl.steps.push_back(f); }
         i0 += cnt;
     }
@@ -1087,23 +1164,61 @@ int build_plan(tmae_handle* h, int N, Plan** out, bool forced = false) {
             default: break;
         }
     }
-    for (const Step& st : pl.steps)
-        if (st.kind == ST_GEMM && pl.host_params[st.param_index].num_segs < 1) return fail(h, TMAE_EINVAL, "bad plan");
-    if (!getenv("TMAE_NO_WEIGHT_PREFETCH")) {      // each GEMM step prefetches the weights of the next one (cyclically)
-        std::vector<int> gemm_steps;
-        for (size_t i = 0; i < pl.steps.size(); ++i) if (pl.steps[i].kind == ST_GEMM) gemm_steps.push_back((int)i);
-        for (size_t k = 0; k < gemm_steps.size(); ++k) {
-            const Step& nx = pl.steps[gemm_steps[(k + 1) % gemm_steps.size()]];
-            pl.steps[gemm_steps[k]].next_index = nx.param_index;
-            pl.steps[gemm_steps[k]].next_groups = nx.groups;
-        }
-    }
-    void* dp = nullptr;
-    CUDA_TRY(h, cudaMalloc(&dp, pl.host_params.size() * sizeof(GemmParams)));
-    pl.d_params = reinterpret_cast<GemmParams*>(dp);
-    CUDA_TRY(h, cudaMemcpy(pl.d_params, pl.host_params.data(), pl.host_params.size() * sizeof(GemmParams), cudaMemcpyHostToDevice));
+    if ((rc = finish_plan(h, pl))) return rc;
     *out = plp.get();
     h->plans[key] = std::move(plp);
+    return TMAE_OK;
+}
+
+// Slice groups of the chain (MCM.py:755-784): slices 0 .. nsl/2 - 1 one at a time, then nsl/2 .. nsl - 1 together (they read
+// only y_hat of the first half).  The forward plan and the decode stages split the slices the same way.
+void slice_groups(int nsl, std::vector<std::pair<int, int>>& g) {
+    g.clear();
+    const int half_sl = nsl / 2;
+    for (int i0 = 0; i0 < nsl;) {
+        const int cnt = i0 < half_sl ? 1 : nsl - i0;
+        g.push_back({i0, cnt});
+        i0 += cnt;
+    }
+}
+
+// Decode plan (MCM.decompress, MCM.py:896-968, range decoder replaced by the caller's symbols): the rate half of the forward
+// with y replaced by symbols, cut into stages at the slice groups because the range decoder needs the scale-table indexes
+// of a group before it can supply the group's symbols.
+//   stage 0      z dequantise, h_s, cc layers + indexes of group 0
+//   stage g + 1  dequantise group g (symbols + mu), lrp_transform of group g, then cc layers + indexes of group g + 1
+//                (after the last group: y_hat / mu / sigma to the caller's buffers)
+// lrp_transform[6..11] always runs: y_hat is the product here (TMAE_FLAG_SKIP_DEAD_LRP applies to the forward only).
+int build_decode_plan(tmae_handle* h, int N, Plan** out) {
+    auto it = h->dec_plans.find(N);
+    if (it != h->dec_plans.end()) { *out = it->second.get(); return TMAE_OK; }
+    int rc = ensure_workspace(h, N);
+    if (rc) return rc;
+    std::unique_ptr<Plan> plp(new Plan());
+    Plan& pl = *plp;
+    pl.N = N;
+    auto simple = [&](StepKind k, int fam, const std::string& t, int slice = 0, int cnt = 1) {
+        Step st; st.kind = k; st.family = fam; st.tag = t; st.slice = slice; st.gc_slices = cnt; pl.steps.push_back(st);
+    };
+    std::vector<std::pair<int, int>> groups;
+    slice_groups(h->nsl, groups);
+    pl.stage_begin.push_back(0);
+    simple(ST_ZDEQ, FAM_ENTROPY, "z_dequantize");
+    if ((rc = add_hs_steps(h, pl, N))) return rc;
+    for (const auto& g : groups) {
+        if ((rc = add_cc_steps(h, pl, N, g.first, g.second, true))) return rc;
+        if (!h->gc_fuse) simple(ST_IDX, FAM_ENTROPY, "indexes." + std::to_string(g.first), g.first, g.second);
+        pl.stage_begin.push_back((int)pl.steps.size());
+        simple(ST_YDEQ, FAM_ENTROPY, "dequantize." + std::to_string(g.first), g.first, g.second);
+        if ((rc = add_lrp_steps(h, pl, N, g.first, g.second, false))) return rc;
+    }
+    simple(ST_DEC_OUT, FAM_MISC, "decode_outputs");
+    pl.stage_begin.push_back((int)pl.steps.size());
+    pl.stage_graph.assign(pl.stage_begin.size() - 1, nullptr);
+    pl.stage_calls.assign(pl.stage_begin.size() - 1, 0);
+    if ((rc = finish_plan(h, pl))) return rc;
+    *out = plp.get();
+    h->dec_plans[N] = std::move(plp);
     return TMAE_OK;
 }
 
@@ -1226,6 +1341,21 @@ int run_steps(tmae_handle* h, Plan& pl, const RunArgs& a, cudaStream_t st) {
                 CUDA_TRY(h, launch_rate_finalize(w.rate_acc, N, (double)h->cfg.img_size * h->cfg.img_size,
                                                  o.bpp ? o.bpp : w.bpp, o.rate_sums ? o.rate_sums : w.rate_sums, st, a.io));
                 break;
+            case ST_ZDEQ:
+                CUDA_TRY(h, launch_z_dequantize(h->eb_tab, (long long)N * h->s4 * h->s4, h->Cz, h->s4 * h->s4, w.zhat_bf.p, w.zhat_bf.lo, st, a.io));
+                break;
+            case ST_IDX:
+                CUDA_TRY(h, launch_slice_indexes(w.sigma, (long long)N * K, h->Cy, sp.slice * h->sc, h->sc * sp.gc_slices, K, h->scale_table,
+                                                 h->n_scale_table, st, a.io));
+                break;
+            case ST_YDEQ:
+                CUDA_TRY(h, launch_slice_dequantize(w.mu, (long long)N * K, h->Cy, sp.slice * h->sc, h->sc * sp.gc_slices, K, w.yhat, w.yhat_bf.p,
+                                                    w.yhat_bf.lo, st, a.io));
+                break;
+            case ST_DEC_OUT:
+                CUDA_TRY(h, launch_copy_outputs(a.io, w.y, w.z, w.mu, w.sigma, w.yhat, w.ids_keep, (long long)N * K * h->Cy,
+                                                (long long)N * h->s4 * h->s4 * h->Cz, (long long)N * K, st));
+                break;
         }
         if (h->profiling && run_end) CUDA_TRY(h, cudaEventRecord(h->prof_events[h->prof_used - 1].second, st));
     }
@@ -1286,8 +1416,40 @@ int run_full_graph(tmae_handle* h, Plan& pl, const float* imgs, const float* sco
     return TMAE_OK;
 }
 
+// One stage of a decode plan.  The per-call pointers (symbols in; z_hat, indexes, y_hat, mu, sigma out) always travel through
+// the device IoBlock, so the stage's first call runs plain launches and every later one replays a graph captured per
+// (N, stage), exactly as run_full_graph does for the forward.
+int run_decode_stage(tmae_handle* h, Plan& pl, int stage, const int32_t* z_symbols, const int32_t* y_symbols, const tmae_outputs* out,
+                     cudaStream_t st) {
+    Workspace& w = h->ws;
+    IoBlock hio;
+    memset(&hio, 0, sizeof(hio));
+    hio.out.z_hat = out->z_hat; hio.out.y_indexes = out->y_indexes;          // only the outputs a decode produces
+    hio.out.y_hat = out->y_hat; hio.out.mu = out->mu; hio.out.sigma = out->sigma;
+    hio.z_symbols = z_symbols; hio.y_symbols = y_symbols;
+    CUDA_TRY(h, cudaMemcpyAsync(w.io, &hio, sizeof(hio), cudaMemcpyHostToDevice, st));   // pageable source: staged before return
+    RunArgs a;
+    a.begin = pl.stage_begin[stage]; a.end = pl.stage_begin[stage + 1]; a.io = w.io;
+    if (!h->use_graph || h->profiling || pl.stage_calls[stage]++ == 0) return run_steps(h, pl, a, st);
+    if (!pl.stage_graph[stage]) {
+        if (!h->cap_stream) CUDA_TRY(h, cudaStreamCreateWithFlags(&h->cap_stream, cudaStreamNonBlocking));
+        CUDA_TRY(h, cudaStreamBeginCapture(h->cap_stream, cudaStreamCaptureModeThreadLocal));
+        int rc = run_steps(h, pl, a, h->cap_stream);
+        cudaGraph_t g = nullptr;
+        cudaError_t e = cudaStreamEndCapture(h->cap_stream, &g);
+        if (rc != TMAE_OK) { if (g) cudaGraphDestroy(g); return rc; }
+        if (e != cudaSuccess || !g) return fail(h, TMAE_ECUDA, "decode graph capture failed: %s", cudaGetErrorString(e));
+        e = cudaGraphInstantiate(&pl.stage_graph[stage], g, 0);
+        cudaGraphDestroy(g);
+        if (e != cudaSuccess) { pl.stage_graph[stage] = nullptr; return fail(h, TMAE_ECUDA, "decode graph instantiate failed: %s", cudaGetErrorString(e)); }
+    }
+    CUDA_TRY(h, cudaGraphLaunch(pl.stage_graph[stage], st));
+    return TMAE_OK;
+}
+
 int check_ready(tmae_handle* h, int N) {
     if (!h) return TMAE_EINVAL;
+    h->dec_next = -1;                // any other call on the handle ends a decode in progress
     if (!h->finalized) return fail(h, TMAE_ESTATE, "weights not finalized (call tmae_finalize_weights)");
     if (N <= 0) return fail(h, TMAE_EINVAL, "batch size must be positive");
     return TMAE_OK;
@@ -1350,7 +1512,8 @@ void tmae_destroy(tmae_handle* h) {
     if (!h) return;
     cudaDeviceSynchronize();
     for (auto& kv : h->raw) cudaFree(kv.second.ptr);
-    for (auto& kv : h->plans) { if (kv.second->d_params) cudaFree(kv.second->d_params); if (kv.second->graph) cudaGraphExecDestroy(kv.second->graph); }
+    drop_plans(h->plans);
+    drop_plans(h->dec_plans);
     if (h->cap_stream) cudaStreamDestroy(h->cap_stream);
     if (h->scale_table) cudaFree(h->scale_table);
     free_pool(h->ws.allocs);
@@ -1384,8 +1547,9 @@ int tmae_set_weight(tmae_handle* h, const char* name, const void* data, int dtyp
 int tmae_finalize_weights(tmae_handle* h) {
     if (!h) return TMAE_EINVAL;
     // re-finalize: drop previous packs
-    for (auto& kv : h->plans) { if (kv.second->d_params) cudaFree(kv.second->d_params); if (kv.second->graph) cudaGraphExecDestroy(kv.second->graph); }
-    h->plans.clear();
+    drop_plans(h->plans);
+    drop_plans(h->dec_plans);
+    h->dec_next = -1;
     free_pool(h->weight_allocs);
     h->layers.clear();
     h->vecs.clear();
@@ -1650,8 +1814,53 @@ int tmae_set_scale_table(tmae_handle* h, const float* table, int n) {
     CUDA_TRY(h, cudaMemcpy(h->scale_table, table, (size_t)n * sizeof(float), cudaMemcpyDefault));
     h->n_scale_table = n;
     // plans (and their captured graphs) carry the table pointer / length: rebuild them on the next call
-    for (auto& kv : h->plans) { if (kv.second->d_params) cudaFree(kv.second->d_params); if (kv.second->graph) cudaGraphExecDestroy(kv.second->graph); }
-    h->plans.clear();
+    drop_plans(h->plans);
+    drop_plans(h->dec_plans);
+    h->dec_next = -1;
+    return TMAE_OK;
+}
+
+// ---- decode (MCM.decompress without the range coder) ---------------------------------------------------
+int tmae_decode_groups(int num_slices, int* first_slice, int* n_slices, int capacity) {
+    if (num_slices <= 0 || num_slices % 2 != 0) return -TMAE_EINVAL;
+    std::vector<std::pair<int, int>> g;
+    slice_groups(num_slices, g);
+    if ((first_slice || n_slices) && capacity < (int)g.size()) return -TMAE_EINVAL;
+    for (size_t i = 0; i < g.size(); ++i) {
+        if (first_slice) first_slice[i] = g[i].first;
+        if (n_slices) n_slices[i] = g[i].second;
+    }
+    return (int)g.size();
+}
+
+int tmae_decode_begin(tmae_handle* h, const int32_t* z_symbols, int N, const tmae_outputs* out, void* stream) {
+    int rc = check_ready(h, N);
+    if (rc) return rc;
+    if (!z_symbols || !out || !out->y_indexes) return fail(h, TMAE_EINVAL, "z_symbols, out and out->y_indexes must not be null");
+    if (!h->scale_table) return fail(h, TMAE_ESTATE, "decoding needs the scale table (call tmae_set_scale_table first)");
+    Plan* pl = nullptr;
+    if ((rc = build_decode_plan(h, N, &pl))) return rc;
+    if (h->profiling) h->prof_used = 0;
+    if ((rc = run_decode_stage(h, *pl, 0, z_symbols, nullptr, out, reinterpret_cast<cudaStream_t>(stream)))) return rc;
+    h->dec_N = N;
+    h->dec_next = 0;
+    return TMAE_OK;
+}
+
+int tmae_decode_step(tmae_handle* h, int group, const int32_t* y_symbols, const tmae_outputs* out, void* stream) {
+    if (!h) return TMAE_EINVAL;
+    if (!y_symbols || !out || !out->y_indexes) return fail(h, TMAE_EINVAL, "y_symbols, out and out->y_indexes must not be null");
+    const int expected = h->dec_next;
+    auto it = h->dec_plans.find(h->dec_N);
+    h->dec_next = -1;                // an out-of-order step ends the decode as well
+    if (expected < 0 || group != expected || it == h->dec_plans.end())
+        return fail(h, TMAE_ESTATE, "decode step %d out of order (expected %s%d): steps follow tmae_decode_begin in group order, "
+                    "and any other call on the handle in between ends the decode", group, expected < 0 ? "a new tmae_decode_begin, not step " : "step ",
+                    expected < 0 ? group : expected);
+    Plan& pl = *it->second;
+    const int rc = run_decode_stage(h, pl, group + 1, nullptr, y_symbols, out, reinterpret_cast<cudaStream_t>(stream));
+    if (rc) return rc;
+    if (group + 2 < (int)pl.stage_begin.size() - 1) h->dec_next = group + 1;
     return TMAE_OK;
 }
 

@@ -22,11 +22,14 @@ include/tmae.h.  PyTorch is used for device memory, streams and the module plumb
 `compress_symbols` is the front half of `MCM.compress` (MCM.py:805-873): symbols and scale-table indexes of y in the
 order `encode_with_indexes` consumes, z symbols / channel indexes for `entropy_bottleneck.compress` (SURVEY 8f-1);
 the rANS coder itself (compressai C++) stays outside.
+`decompress_symbols` is the decoder side of `MCM.decompress` (MCM.py:896-968) around the range decoder: symbols in (all at
+once, or group by group through a callback that receives the scale-table indexes), y_hat / z_hat / x_hat out, bit-exact
+with the encoder of the same accuracy mode.
 """
 from __future__ import annotations
 
 import ctypes as C
-from typing import Dict, Iterator, Optional, Tuple
+from typing import Callable, Dict, Iterator, Optional, Tuple
 
 import torch
 import torch.nn as nn
@@ -446,6 +449,17 @@ class MCM(nn.Module):
         self._scale_table_dirty = True
         return True
 
+    def _install_scale_table(self):
+        """Hand the GaussianConditional scale table to the handle (the default table if `update()` was never called)."""
+        if self._scale_table is None:
+            self.update()
+        self._ensure_handle()
+        if getattr(self, "_scale_table_dirty", True):
+            tab = self._scale_table
+            with torch.cuda.device(self._handle_device):
+                _native.check(_native.load().tmae_set_scale_table(self._handle, C.c_void_p(tab.data_ptr()), tab.numel()), self._handle)
+            self._scale_table_dirty = False
+
     @torch.no_grad()
     def compress_symbols(self, imgs: torch.Tensor, total_scores: torch.Tensor):
         """Front half of `MCM.compress` (MCM.py:805-873), everything up to the `encode_with_indexes` call:
@@ -456,16 +470,9 @@ class MCM(nn.Module):
                           (:827): quantize(z, "symbols", medians) and the channel index of every element
             "shape": z spatial size (:890), "ids_restore" (:891)
         The range coder itself (compressai's C++ rANS) is not part of this library."""
-        if self._scale_table is None:
-            self.update()
-        self._ensure_handle()
+        self._install_scale_table()
         dev = self._handle_device
         lib = _native.load()
-        if getattr(self, "_scale_table_dirty", True):
-            tab = self._scale_table
-            with torch.cuda.device(dev):
-                _native.check(lib.tmae_set_scale_table(self._handle, C.c_void_p(tab.data_ptr()), tab.numel()), self._handle)
-            self._scale_table_dirty = False
         self._check_inputs(imgs, total_scores)
         imgs = imgs.to(device=dev, dtype=torch.float32).contiguous()
         total_scores = total_scores.to(device=dev, dtype=torch.float32).contiguous()
@@ -485,12 +492,83 @@ class MCM(nn.Module):
         return {"y_symbols": packed[0], "y_indexes": packed[1], "z_symbols": zpacked, "z_indexes": z_idx,
                 "shape": (s4, s4), "ids_restore": t["ids_restore"], "bpp": t["bpp"]}
 
+    @torch.no_grad()
+    def decompress_symbols(self, z_symbols: torch.Tensor, ids_restore: torch.Tensor, y_symbols: Optional[torch.Tensor] = None,
+                           decode_fn: Optional[Callable[[int, torch.Tensor], torch.Tensor]] = None,
+                           need_recon: Optional[bool] = None) -> Dict[str, torch.Tensor]:
+        """`MCM.decompress` (MCM.py:896-968) with the range decoder left to the caller: symbols -> y_hat, z_hat (-> x_hat).
+            z_symbols  i32 [N, Cz, s/4, s/4]  (`compress_symbols()["z_symbols"]`)
+            ids_restore  i64 [N, L]           (the side information; used for x_hat only)
+        and exactly one of
+            y_symbols  i32 [N, Cy*s*s]        every slice's symbols at once (`compress_symbols()["y_symbols"]`): the whole
+                                              decode is enqueued on the current stream without a host synchronisation;
+            decode_fn  callable(first_slice, indexes) -> symbols: called once per slice group (slices 0..5 one by one, then
+                                              6..11 together) with the group's scale-table indexes, i32 [N, n_slices, Cs, s, s]
+                                              on the device - the list the reference hands `decode_stream` for those slices -
+                                              and returning the group's symbols of the same shape (any device).  This is
+                                              where compressai's `RansDecoder.decode_stream` plugs in.
+        The decode runs the encoder's own kernels and launch shapes, so it reproduces the y_hat / z_hat / indexes of a
+        module of the same configuration (same `precise` mode) bit for bit.
+        Returns {"y_hat": f32 [N,Cy,s,s], "z_hat": f32 [N,Cz,s/4,s/4], "y_indexes": i32 [N, Cy*s*s]} and, with `need_recon`
+        (default: whenever the decoder-side weights are loaded), "x_hat": f32 [N,3,S,S] computed exactly as forward's
+        x_hat (recon.synthesize).  No post-processing (e.g. clamping) is applied to x_hat: it is forward's x_hat."""
+        if (y_symbols is None) == (decode_fn is None):
+            raise ValueError("give exactly one of y_symbols and decode_fn")
+        if need_recon is None:
+            need_recon = recon.has_decoder_weights(self._weights)
+        if need_recon and not recon.has_decoder_weights(self._weights):
+            raise RuntimeError("need_recon=True but the loaded state dict has no g_s / decoder tensors")
+        self._install_scale_table()
+        dev = self._handle_device
+        c = self.cfg
+        s, s4, sc, ns = c.side, c.side // 4, c.slice_ch, c.num_slices
+        N = z_symbols.shape[0] if z_symbols.dim() == 4 else -1
+        if z_symbols.dtype != torch.int32 or tuple(z_symbols.shape) != (N, c.hyperprior_depth, s4, s4) or N < 1:
+            raise ValueError(f"z_symbols must be int32 [N, {c.hyperprior_depth}, {s4}, {s4}], got {z_symbols.dtype} {tuple(z_symbols.shape)}")
+        if tuple(ids_restore.shape) != (N, c.num_patches):
+            raise ValueError(f"ids_restore must be [{N}, {c.num_patches}], got {tuple(ids_restore.shape)}")
+        if y_symbols is not None and (y_symbols.dtype != torch.int32 or tuple(y_symbols.shape) != (N, c.latent_depth * s * s)):
+            raise ValueError(f"y_symbols must be int32 [{N}, {c.latent_depth * s * s}], got {y_symbols.dtype} {tuple(y_symbols.shape)}")
+        lib = _native.load()
+        firsts, counts = (C.c_int * ns)(), (C.c_int * ns)()
+        n_groups = lib.tmae_decode_groups(ns, firsts, counts, ns)
+        if n_groups < 1:
+            raise RuntimeError(f"tmae_decode_groups({ns}) failed")
+        groups = [(firsts[g], counts[g]) for g in range(n_groups)]
+        zs = z_symbols.to(dev).contiguous()
+        f32 = torch.float32
+        y_hat = torch.empty((N, s, s, c.latent_depth), dtype=f32, device=dev)
+        z_hat = torch.empty((N, s4, s4, c.hyperprior_depth), dtype=f32, device=dev)
+        y_idx = torch.empty((N, c.latent_depth * s * s), dtype=torch.int32, device=dev)
+        ys = y_symbols.to(dev).contiguous() if y_symbols is not None else torch.empty_like(y_idx)
+        o = _native.TmaeOutputs()
+        o.y_hat, o.z_hat, o.y_indexes = y_hat.data_ptr(), z_hat.data_ptr(), y_idx.data_ptr()
+        by_slice = lambda t: t.view(N, ns, sc, s, s)
+        with torch.cuda.device(dev):
+            cur = self._enter_stream(dev)
+            st = C.c_void_p(cur.cuda_stream)
+            _native.check(lib.tmae_decode_begin(self._handle, C.c_void_p(zs.data_ptr()), N, C.byref(o), st), self._handle, RuntimeError)
+            for g, (first, cnt) in enumerate(groups):
+                if decode_fn is not None:
+                    sym = decode_fn(first, by_slice(y_idx)[:, first:first + cnt])
+                    sym = torch.as_tensor(sym)
+                    if tuple(sym.shape) != (N, cnt, sc, s, s) or sym.is_floating_point() or sym.is_complex():
+                        raise ValueError(f"decode_fn must return integer symbols [{N}, {cnt}, {sc}, {s}, {s}], got {sym.dtype} {tuple(sym.shape)}")
+                    by_slice(ys)[:, first:first + cnt] = sym.to(device=dev, dtype=torch.int32)
+                _native.check(lib.tmae_decode_step(self._handle, g, C.c_void_p(ys.data_ptr()), C.byref(o), st), self._handle, RuntimeError)
+            self._leave_stream(cur)
+        out = {"y_hat": self._nchw(y_hat), "z_hat": self._nchw(z_hat), "y_indexes": y_idx}
+        if need_recon:
+            out["x_hat"] = recon.synthesize(self._weights, c, y_hat.reshape(N, c.num_keep_patches, c.latent_depth), ids_restore.to(dev))
+        return out
+
     def compress(self, *args, **kwargs):
         raise NotImplementedError("bitstream emission (compressai's C++ rANS coder) is outside this library; "
                                   "compress_symbols() returns the symbol / index lists the coder consumes (SURVEY 8f-1)")
 
     def decompress(self, *args, **kwargs):
-        raise NotImplementedError("bitstream decoding is outside this path (SURVEY 8f-1)")
+        raise NotImplementedError("bitstream decoding (compressai's C++ rANS coder) is outside this library; "
+                                  "decompress_symbols() rebuilds y_hat / x_hat from the decoded symbols (SURVEY 8f-1)")
 
     # ------------------------------------------------------------------ profiling hooks (bench.py)
     def profile(self, enable: bool, by_run: bool = False):

@@ -123,10 +123,16 @@ def forward_loss(imgs: torch.Tensor, x_hat: torch.Tensor,
 
 
 @torch.no_grad()
-def reconstruct(w: Dict[str, torch.Tensor], cfg, y_hat_tokens: torch.Tensor, ids_restore: torch.Tensor, imgs: torch.Tensor,
-                feature_loss=None):
-    """MCM.py:789-797: g_s -> forward_decoder -> forward_loss / unpatchify.  Returns (loss 3-tuple, x_hat)."""
+def synthesize(w: Dict[str, torch.Tensor], cfg, y_hat_tokens: torch.Tensor, ids_restore: torch.Tensor) -> torch.Tensor:
+    """MCM.py:789-792 (and the decoder side of MCM.decompress): g_s -> forward_decoder -> unpatchify.  Returns x_hat."""
     tok = g_s(w, y_hat_tokens)
     preds = forward_decoder(w, tok, ids_restore, cfg.decoder_depth, cfg.decoder_num_heads, cfg.ln_eps).float()
-    x_hat = unpatchify(preds, cfg.patch_size)
+    return unpatchify(preds, cfg.patch_size)
+
+
+@torch.no_grad()
+def reconstruct(w: Dict[str, torch.Tensor], cfg, y_hat_tokens: torch.Tensor, ids_restore: torch.Tensor, imgs: torch.Tensor,
+                feature_loss=None):
+    """MCM.py:789-797: synthesize -> forward_loss.  Returns (loss 3-tuple, x_hat)."""
+    x_hat = synthesize(w, cfg, y_hat_tokens, ids_restore)
     return forward_loss(imgs, x_hat, feature_loss), x_hat
