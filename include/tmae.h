@@ -184,6 +184,46 @@ TMAE_API int  tmae_decode_begin(tmae_handle* h, const int32_t* z_symbols, int N,
  * out->sigma when non-NULL) are complete.  Other members of `out` are ignored. */
 TMAE_API int  tmae_decode_step(tmae_handle* h, int group, const int32_t* y_symbols, const tmae_outputs* out, void* stream);
 
+/* Entropy coder: compressai 1.2.4's rANS bitstream (BufferedRansEncoder / RansDecoder *_with_indexes over rans64, precision 16,
+ * 4-bit bypass escapes; DESIGN.md section 7) on the GPU.  A stream is a sequence of 32-bit words, stored little-endian; its
+ * byte length is a multiple of 4 and at least 8.  Streams of a batch are packed back to back: stream i is bytes
+ * [offsets[i], offsets[i + 1]) of `data` (device memory, 4-byte aligned).  Per-stream status: 0 = the stream decoded to its
+ * end exactly (final state equals the encoder's initial state, every word consumed), otherwise TMAE_RANS_* bits.  Input
+ * bytes may be anything: every read is bounded by the stream's length (past the end reads as 0 and sets a bit). */
+#define TMAE_MODEL_GAUSSIAN     0    /* GaussianConditional: one table per scale-table entry, index = build_indexes(sigma) */
+#define TMAE_MODEL_BOTTLENECK   1    /* EntropyBottleneck: one table per channel, index = channel */
+#define TMAE_RANS_OVERRUN       1    /* decode read past the end of the stream */
+#define TMAE_RANS_UNFINISHED    2    /* decode ended in another state than the encoder started from, or left words unread */
+#define TMAE_RANS_BAD_INDEX     4    /* an index outside the table set (coded / decoded with table 0) */
+#define TMAE_RANS_RANGE         8    /* encode: a symbol too far outside its table (escape value >= 2^31; coded as 0) */
+#define TMAE_RANS_OVERFLOW      16   /* encode: the packed streams exceed `capacity` (this stream was not written) */
+#define TMAE_RANS_MALFORMED     32   /* decode: bad byte range, or an escape longer than 8 nibbles */
+/* Host-only: compressai's pmf_to_quantized_cdf at precision 16.  h_pmf [n] -> h_cdf [n + 1] (0 .. 65536, strictly
+ * increasing).  TMAE_EINVAL for a negative / non-finite / all-zero pmf. */
+TMAE_API int  tmae_pmf_to_quantized_cdf(const float* h_pmf, int n, int32_t* h_cdf);
+/* Host-only: bytes that always suffice for one stream of n symbols (10 words per symbol + 2), -1 for n < 0. */
+TMAE_API int64_t tmae_rans_bound(int64_t n_symbols);
+/* Installs one table set: cdf [n_tables, stride] in compressai's padded _quantized_cdf layout, cdf_lengths / offsets [n_tables]
+ * (_cdf_length / _offset); host or device pointers, copied.  Every table must have length >= 3, start at 0, increase strictly
+ * and end at 65536 (TMAE_EINVAL otherwise).  Bottleneck: n_tables must equal hyperprior_depth. */
+TMAE_API int  tmae_set_cdf_tables(tmae_handle* h, int model, const int32_t* cdf, int n_tables, int stride,
+                                  const int32_t* cdf_lengths, const int32_t* offsets);
+/* encode_with_indexes + flush of n_streams streams of n_per_stream symbols each (symbols / indexes i32 [n_streams, n_per_stream]):
+ * packed into out (capacity bytes; n_streams * tmae_rans_bound(n_per_stream) always suffices), offsets i64 [n_streams + 1],
+ * status i32 [n_streams].  Scratch memory is the handle's, grown on the first call of a larger size. */
+TMAE_API int  tmae_rans_encode(tmae_handle* h, int model, const int32_t* symbols, const int32_t* indexes, int n_streams,
+                               int n_per_stream, uint8_t* out, int64_t capacity, int64_t* offsets, int32_t* status, void* stream);
+/* decode_with_indexes of n_streams streams: indexes / symbols i32 [n_streams, n_per_stream], status i32 [n_streams]. */
+TMAE_API int  tmae_rans_decode(tmae_handle* h, int model, const uint8_t* data, const int64_t* offsets, int n_streams,
+                               const int32_t* indexes, int n_per_stream, int32_t* symbols, int32_t* status, void* stream);
+/* The whole decode from bitstreams, enqueued without a host synchronisation: per image one y stream (every slice in order, the
+ * symbols in the order of tmae_decode_step) and one z stream (z symbols in NCHW order, table = channel).  The z streams are
+ * decoded with the bottleneck tables, then each slice group's y symbols with the Gaussian tables and the indexes the decode has
+ * just computed.  Writes out->z_hat / y_hat and, when non-NULL, out->mu / sigma / y_indexes (other members ignored); status
+ * i32 [N].  Needs the scale table and both table sets, the Gaussian set with one table per scale-table entry (TMAE_ESTATE). */
+TMAE_API int  tmae_decompress_streams(tmae_handle* h, const uint8_t* y_data, const int64_t* y_offsets, const uint8_t* z_data,
+                                      const int64_t* z_offsets, int N, const tmae_outputs* out, int32_t* status, void* stream);
+
 /* Stand-alone operators on the path (each mirrors one reference call) ---------------------------------- */
 /* MCM.get_ids_shuffle + random_masking index work (MCM.py:364-423, 579-583). Outputs may be NULL. */
 TMAE_API int  tmae_mask_select(const float* scores, int N, int L, int K, int softmax_isa,

@@ -17,6 +17,7 @@ FLAG_SHARE_SM = 4
 FLAG_PRECISE_RATE = 8
 FLAG_PRECISE_ALL = 16
 FLAG_PRECISE_X6 = 32
+MODEL_GAUSSIAN, MODEL_BOTTLENECK = 0, 1
 
 
 class TmaeConfig(C.Structure):
@@ -79,6 +80,12 @@ SIGNATURES = {
     "tmae_decode_groups": (C.c_int, [C.c_int, C.POINTER(C.c_int), C.POINTER(C.c_int), C.c_int]),
     "tmae_decode_begin": (C.c_int, [_P, _P, C.c_int, C.POINTER(TmaeOutputs), _P]),
     "tmae_decode_step": (C.c_int, [_P, C.c_int, _P, C.POINTER(TmaeOutputs), _P]),
+    "tmae_pmf_to_quantized_cdf": (C.c_int, [_P, C.c_int, _P]),
+    "tmae_rans_bound": (C.c_int64, [C.c_int64]),
+    "tmae_set_cdf_tables": (C.c_int, [_P, C.c_int, _P, C.c_int, C.c_int, _P, _P]),
+    "tmae_rans_encode": (C.c_int, [_P, C.c_int, _P, _P, C.c_int, C.c_int, _P, C.c_int64, _P, _P, _P]),
+    "tmae_rans_decode": (C.c_int, [_P, C.c_int, _P, _P, C.c_int, _P, C.c_int, _P, _P, _P]),
+    "tmae_decompress_streams": (C.c_int, [_P, _P, _P, _P, _P, C.c_int, C.POINTER(TmaeOutputs), _P, _P]),
     "tmae_mask_select": (C.c_int, [_P, C.c_int, C.c_int, C.c_int, C.c_int, _P, _P, _P, _P]),
     "tmae_gaussian_rate": (C.c_int, [_P, _P, _P, C.c_int64, _P, _P, _P, _P]),
     "tmae_bottleneck_rate": (C.c_int, [_P, _P, C.c_int64, _P, _P, _P, _P]),

@@ -23,6 +23,7 @@ SOURCES = {
     "elementwise.cu": [],
     "mask.cu": ["-fmad=false"],
     "scores.cu": ["-fmad=false"],
+    "rans.cu": [],
     "huffman.cpp": [],
     "tmae_api.cu": [],
 }

@@ -17,6 +17,11 @@ struct IoBlock {
     tmae_outputs out;
     const int32_t* z_symbols;        // decode: z symbols [N, Cz, s/4, s/4] (range-coder order)
     const int32_t* y_symbols;        // decode: y symbols [N, Cy * s * s], per image slice by slice in (c, y, x) order
+    const uint8_t* y_data;           // decode from streams (tmae_decompress_streams): image n's y stream is bytes
+    const int64_t* y_offsets;        //   [y_offsets[n], y_offsets[n + 1]) of y_data; likewise z
+    const uint8_t* z_data;
+    const int64_t* z_offsets;
+    int32_t* status;                 //   [N] per-image coder status (RANS_ST_* bits)
 };
 
 // gemm_tc.cu
@@ -93,6 +98,55 @@ cudaError_t launch_permute_bias_shuffle(const float* b, float* out, int Cout, cu
 cudaError_t launch_eb_table(const float* const* ptrs, float* tab, int Cz, cudaStream_t st);
 cudaError_t launch_f32_to_bf16(const float* a, __nv_bfloat16* o, long long n, long long lo_off, cudaStream_t st);
 cudaError_t launch_f32_to_bf16_cols(const float* a, __nv_bfloat16* o, long long rows, int cols, int ld, long long lo_off, cudaStream_t st);
+
+// rans.cu: the entropy coder (compressai's rANS format)
+enum : int32_t {                     // per-stream status bits (include/tmae.h TMAE_RANS_*)
+    RANS_ST_OVERRUN = 1,             // decode read past the end of the stream (those words read as 0)
+    RANS_ST_UNFINISHED = 2,          // decode ended with a state other than the encoder's initial one, or words left over
+    RANS_ST_BAD_INDEX = 4,           // an index outside the table set (coded with table 0)
+    RANS_ST_RANGE = 8,               // encode: a symbol whose escape value does not fit 31 bits (coded as 0)
+    RANS_ST_OVERFLOW = 16,           // encode: the packed output does not fit the capacity (stream not written)
+    RANS_ST_MALFORMED = 32,          // decode: byte range negative / not a multiple of 4, or an escape longer than 8 nibbles
+};
+struct CdfTables {                   // one quantised-CDF table set on the device (tmae_set_cdf_tables)
+    int n = 0;                       // tables
+    int entries = 0;                 // sum of the cdf lengths
+    int* cdf = nullptr;              // [entries] the cdfs back to back, then meta
+    int* meta = nullptr;             // [3 * n]: start in cdf, cdf length, offset of every table
+    uint4* enc = nullptr;            // [entries]: symbol v of table t at start + v: {start | freq << 16, reciprocal shift, reciprocal lo, hi}
+};
+struct RansDecState {                // decoder state of one stream between the stages of a decode plan
+    unsigned long long x;
+    unsigned pos, pad;
+};
+struct RansDecArgs {
+    const int* cdf = nullptr;        // CdfTables::cdf (meta follows the entries)
+    int entries = 0, n_tab = 0;
+    int use_smem = 0, streams_per_block = 1;                 // set by launch_rans_decode
+    const uint8_t* data = nullptr;   // streams: bytes [offsets[s], offsets[s + 1]) of data
+    const int64_t* offsets = nullptr;
+    const int32_t* indexes = nullptr;                        // [s * idx_stride + i]; nullptr: table (i / idx_div)
+    long long idx_stride = 0;
+    int idx_div = 1;
+    int32_t* symbols = nullptr;      // [s * sym_stride + i]
+    long long sym_stride = 0;
+    int n_streams = 0, begin = 0, end = 0;                   // symbols [begin, end) of every stream
+    int init = 1, fin = 1;           // init: read the two head words; fin: check the final state
+    int status_reset = 1;            // init: overwrite status[s] (else OR into it)
+    RansDecState* state = nullptr;   // between stages (init == 0 reads it, fin == 0 writes it)
+    int32_t* status = nullptr;
+    const IoBlock* io = nullptr;     // non-null: data / offsets / status (and, io_stream 1, the indexes io->out.y_indexes)
+    int io_stream = 0;               //   come from the IoBlock: 1 = the y streams, 2 = the z streams
+};
+int pmf_to_quantized_cdf(const float* pmf, int n, int32_t* cdf_out);          // host; cdf_out holds n + 1 entries
+long long rans_bound_bytes(long long n);
+int rans_build_tables(const int32_t* cdf, int n, int stride, const int32_t* len, const int32_t* off, CdfTables* out,
+                      char* err, size_t err_len);                            // host arrays in; uploads (synchronous)
+void rans_free_tables(CdfTables* t);
+cudaError_t launch_rans_encode(const int32_t* sym, const int32_t* idx, int n_streams, int n_per, const CdfTables& tab, uint2* rec,
+                               uint32_t* scratch, long long cap_words, long long* n_words, uint8_t* out, long long capacity,
+                               int64_t* offsets, int32_t* status, cudaStream_t st);
+cudaError_t launch_rans_decode(RansDecArgs a, cudaStream_t st);
 
 // ---- patch-score generation (scores.cu; generate_scores_file.py:19-31, utils/map.py, utils/distribution.py) ----
 constexpr int kScoreMaxLevels = 16;

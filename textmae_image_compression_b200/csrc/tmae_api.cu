@@ -52,10 +52,11 @@ struct Bf {
 };
 
 enum StepKind { ST_MASK, ST_GATHER, ST_GEMM, ST_FORCE, ST_LN, ST_ATTN, ST_EB, ST_GC, ST_RATE, ST_ZERO_RATE,
-                ST_ZDEQ, ST_IDX, ST_YDEQ, ST_DEC_OUT };     // the last four: decode plans only
-enum Family { FAM_GEMM = 0, FAM_ATTN, FAM_LN, FAM_MASK, FAM_GATHER, FAM_ENTROPY, FAM_MISC, FAM_COUNT };
+                ST_ZDEQ, ST_IDX, ST_YDEQ, ST_DEC_OUT,        // decode plans only
+                ST_ZDEC, ST_YDEC };                          // decode-from-streams plans only: the range decoder
+enum Family { FAM_GEMM = 0, FAM_ATTN, FAM_LN, FAM_MASK, FAM_GATHER, FAM_ENTROPY, FAM_MISC, FAM_CODER, FAM_COUNT };
 const char* kFamilyNames[FAM_COUNT] = {"gemm_tc", "attention", "layernorm", "mask_select", "gather_patches",
-                                       "entropy_elementwise", "misc"};
+                                       "entropy_elementwise", "misc", "entropy_coder"};
 
 struct Step {
     StepKind kind;
@@ -125,6 +126,18 @@ struct Workspace {
     IoBlock* io = nullptr;           // per-call pointers for graph replays
 };
 
+// Buffers of the entropy coder, grown on demand apart from the network's workspace (a forward-only handle never needs them).
+struct CoderWorkspace {
+    std::vector<void*> allocs;
+    int cap_N = 0;                   // decode from streams: batch capacity of the four buffers below
+    int32_t* zsym = nullptr;         // [N, Cz, s/4, s/4] decoded z symbols (ST_ZDEC -> ST_ZDEQ)
+    int32_t* ysym = nullptr;         // [N, Cy * K] decoded y symbols (ST_YDEC -> ST_YDEQ)
+    int32_t* idx = nullptr;          // [N, Cy * K] scale-table indexes, when the caller does not ask for them
+    RansDecState* state = nullptr;   // [N] y decoder state between the slice groups
+    size_t enc_bytes = 0;            // tmae_rans_encode scratch: records, per-stream word regions, word counts
+    void* enc = nullptr;
+};
+
 }  // namespace
 
 struct tmae_handle {
@@ -143,6 +156,9 @@ struct tmae_handle {
     Workspace ws;
     std::map<int, std::unique_ptr<Plan>> plans;
     std::map<int, std::unique_ptr<Plan>> dec_plans;   // decode plans by batch size (tmae_decode_begin / _step)
+    std::map<int, std::unique_ptr<Plan>> stream_plans;   // decode-from-streams plans by batch size (tmae_decompress_streams)
+    CdfTables cdf[2];                // quantised CDF tables: [TMAE_MODEL_GAUSSIAN], [TMAE_MODEL_BOTTLENECK]
+    CoderWorkspace cws;
     int dec_N = 0, dec_next = -1;    // decode in progress: batch size and the next group expected (-1 = none)
     PFN_encodeTiled encode = nullptr;
     std::vector<void*> weight_allocs;
@@ -623,6 +639,7 @@ int ensure_workspace(tmae_handle* h, int N) {
     // plans hold pointers into the workspace: drop them
     drop_plans(h->plans);
     drop_plans(h->dec_plans);
+    drop_plans(h->stream_plans);
     free_pool(w.allocs);
     w = Workspace();
     size_t tot = 0;
@@ -1222,6 +1239,60 @@ int build_decode_plan(tmae_handle* h, int N, Plan** out) {
     return TMAE_OK;
 }
 
+int ensure_coder_workspace(tmae_handle* h, int N) {
+    CoderWorkspace& c = h->cws;
+    if (N <= c.cap_N) return TMAE_OK;
+    drop_plans(h->stream_plans);     // they hold pointers into these buffers
+    for (void* p : c.allocs) cudaFree(p);
+    c.allocs.clear();
+    c.cap_N = 0;
+    const size_t ny = (size_t)N * h->Cy * h->K, nz = (size_t)N * h->Cz * h->s4 * h->s4;
+    int rc;
+    if ((rc = dev_alloc(h, c.allocs, &c.zsym, nz)) || (rc = dev_alloc(h, c.allocs, &c.ysym, ny)) ||
+        (rc = dev_alloc(h, c.allocs, &c.idx, ny)) || (rc = dev_alloc(h, c.allocs, &c.state, (size_t)N)))
+        return rc;
+    c.cap_N = N;
+    return TMAE_OK;
+}
+
+// Decode plan fed by the range decoder (tmae_decompress_streams): the decode plan above with the coder in front of the two
+// dequantisations - ST_ZDEC decodes the z streams with the bottleneck tables before ST_ZDEQ, and ST_YDEC decodes slice group g
+// of the y streams, with the indexes the group's cc layers just wrote, before ST_YDEQ.  The y decoder's state stays in the
+// coder workspace between the groups.  One stage: the whole decode replays as one CUDA graph per batch size.
+int build_stream_decode_plan(tmae_handle* h, int N, Plan** out) {
+    auto it = h->stream_plans.find(N);
+    if (it != h->stream_plans.end()) { *out = it->second.get(); return TMAE_OK; }
+    int rc = ensure_workspace(h, N);
+    if (rc || (rc = ensure_coder_workspace(h, N))) return rc;
+    std::unique_ptr<Plan> plp(new Plan());
+    Plan& pl = *plp;
+    pl.N = N;
+    auto simple = [&](StepKind k, int fam, const std::string& t, int slice = 0, int cnt = 1) {
+        Step st; st.kind = k; st.family = fam; st.tag = t; st.slice = slice; st.gc_slices = cnt; pl.steps.push_back(st);
+    };
+    std::vector<std::pair<int, int>> groups;
+    slice_groups(h->nsl, groups);
+    pl.stage_begin.push_back(0);
+    simple(ST_ZDEC, FAM_CODER, "rans_decode.z");
+    simple(ST_ZDEQ, FAM_ENTROPY, "z_dequantize");
+    if ((rc = add_hs_steps(h, pl, N))) return rc;
+    for (const auto& g : groups) {
+        if ((rc = add_cc_steps(h, pl, N, g.first, g.second, true))) return rc;
+        if (!h->gc_fuse) simple(ST_IDX, FAM_ENTROPY, "indexes." + std::to_string(g.first), g.first, g.second);
+        simple(ST_YDEC, FAM_CODER, "rans_decode.y." + std::to_string(g.first), g.first, g.second);
+        simple(ST_YDEQ, FAM_ENTROPY, "dequantize." + std::to_string(g.first), g.first, g.second);
+        if ((rc = add_lrp_steps(h, pl, N, g.first, g.second, false))) return rc;
+    }
+    simple(ST_DEC_OUT, FAM_MISC, "decode_outputs");
+    pl.stage_begin.push_back((int)pl.steps.size());
+    pl.stage_graph.assign(1, nullptr);
+    pl.stage_calls.assign(1, 0);
+    if ((rc = finish_plan(h, pl))) return rc;
+    *out = plp.get();
+    h->stream_plans[N] = std::move(plp);
+    return TMAE_OK;
+}
+
 // ---- execution -----------------------------------------------------------------------------------------
 struct RunArgs {
     const float* imgs = nullptr;
@@ -1356,6 +1427,31 @@ int run_steps(tmae_handle* h, Plan& pl, const RunArgs& a, cudaStream_t st) {
                 CUDA_TRY(h, launch_copy_outputs(a.io, w.y, w.z, w.mu, w.sigma, w.yhat, w.ids_keep, (long long)N * K * h->Cy,
                                                 (long long)N * h->s4 * h->s4 * h->Cz, (long long)N * K, st));
                 break;
+            case ST_ZDEC: {
+                const CdfTables& t = h->cdf[TMAE_MODEL_BOTTLENECK];
+                RansDecArgs d;
+                d.cdf = t.cdf; d.entries = t.entries; d.n_tab = t.n;
+                d.idx_div = h->s4 * h->s4;
+                d.symbols = h->cws.zsym; d.sym_stride = (long long)h->Cz * h->s4 * h->s4;
+                d.n_streams = N; d.begin = 0; d.end = h->Cz * h->s4 * h->s4;
+                d.io = a.io; d.io_stream = 2;
+                CUDA_TRY(h, launch_rans_decode(d, st));
+                break;
+            }
+            case ST_YDEC: {
+                const CdfTables& t = h->cdf[TMAE_MODEL_GAUSSIAN];
+                const int per_slice = h->sc * K;
+                RansDecArgs d;
+                d.cdf = t.cdf; d.entries = t.entries; d.n_tab = t.n;
+                d.idx_stride = (long long)h->Cy * K;
+                d.symbols = h->cws.ysym; d.sym_stride = (long long)h->Cy * K;
+                d.n_streams = N; d.begin = sp.slice * per_slice; d.end = (sp.slice + sp.gc_slices) * per_slice;
+                d.init = sp.slice == 0; d.fin = sp.slice + sp.gc_slices == h->nsl; d.status_reset = 0;
+                d.state = h->cws.state;
+                d.io = a.io; d.io_stream = 1;
+                CUDA_TRY(h, launch_rans_decode(d, st));
+                break;
+            }
         }
         if (h->profiling && run_end) CUDA_TRY(h, cudaEventRecord(h->prof_events[h->prof_used - 1].second, st));
     }
@@ -1419,14 +1515,17 @@ int run_full_graph(tmae_handle* h, Plan& pl, const float* imgs, const float* sco
 // One stage of a decode plan.  The per-call pointers (symbols in; z_hat, indexes, y_hat, mu, sigma out) always travel through
 // the device IoBlock, so the stage's first call runs plain launches and every later one replays a graph captured per
 // (N, stage), exactly as run_full_graph does for the forward.
-int run_decode_stage(tmae_handle* h, Plan& pl, int stage, const int32_t* z_symbols, const int32_t* y_symbols, const tmae_outputs* out,
-                     cudaStream_t st) {
-    Workspace& w = h->ws;
+IoBlock decode_io(const int32_t* z_symbols, const int32_t* y_symbols, const tmae_outputs* out) {
     IoBlock hio;
     memset(&hio, 0, sizeof(hio));
     hio.out.z_hat = out->z_hat; hio.out.y_indexes = out->y_indexes;          // only the outputs a decode produces
     hio.out.y_hat = out->y_hat; hio.out.mu = out->mu; hio.out.sigma = out->sigma;
     hio.z_symbols = z_symbols; hio.y_symbols = y_symbols;
+    return hio;
+}
+
+int run_decode_stage(tmae_handle* h, Plan& pl, int stage, const IoBlock& hio, cudaStream_t st) {
+    Workspace& w = h->ws;
     CUDA_TRY(h, cudaMemcpyAsync(w.io, &hio, sizeof(hio), cudaMemcpyHostToDevice, st));   // pageable source: staged before return
     RunArgs a;
     a.begin = pl.stage_begin[stage]; a.end = pl.stage_begin[stage + 1]; a.io = w.io;
@@ -1514,6 +1613,10 @@ void tmae_destroy(tmae_handle* h) {
     for (auto& kv : h->raw) cudaFree(kv.second.ptr);
     drop_plans(h->plans);
     drop_plans(h->dec_plans);
+    drop_plans(h->stream_plans);
+    for (CdfTables& t : h->cdf) rans_free_tables(&t);
+    free_pool(h->cws.allocs);
+    if (h->cws.enc) cudaFree(h->cws.enc);
     if (h->cap_stream) cudaStreamDestroy(h->cap_stream);
     if (h->scale_table) cudaFree(h->scale_table);
     free_pool(h->ws.allocs);
@@ -1549,6 +1652,7 @@ int tmae_finalize_weights(tmae_handle* h) {
     // re-finalize: drop previous packs
     drop_plans(h->plans);
     drop_plans(h->dec_plans);
+    drop_plans(h->stream_plans);
     h->dec_next = -1;
     free_pool(h->weight_allocs);
     h->layers.clear();
@@ -1816,6 +1920,7 @@ int tmae_set_scale_table(tmae_handle* h, const float* table, int n) {
     // plans (and their captured graphs) carry the table pointer / length: rebuild them on the next call
     drop_plans(h->plans);
     drop_plans(h->dec_plans);
+    drop_plans(h->stream_plans);
     h->dec_next = -1;
     return TMAE_OK;
 }
@@ -1841,7 +1946,7 @@ int tmae_decode_begin(tmae_handle* h, const int32_t* z_symbols, int N, const tma
     Plan* pl = nullptr;
     if ((rc = build_decode_plan(h, N, &pl))) return rc;
     if (h->profiling) h->prof_used = 0;
-    if ((rc = run_decode_stage(h, *pl, 0, z_symbols, nullptr, out, reinterpret_cast<cudaStream_t>(stream)))) return rc;
+    if ((rc = run_decode_stage(h, *pl, 0, decode_io(z_symbols, nullptr, out), reinterpret_cast<cudaStream_t>(stream)))) return rc;
     h->dec_N = N;
     h->dec_next = 0;
     return TMAE_OK;
@@ -1858,10 +1963,124 @@ int tmae_decode_step(tmae_handle* h, int group, const int32_t* y_symbols, const 
                     "and any other call on the handle in between ends the decode", group, expected < 0 ? "a new tmae_decode_begin, not step " : "step ",
                     expected < 0 ? group : expected);
     Plan& pl = *it->second;
-    const int rc = run_decode_stage(h, pl, group + 1, nullptr, y_symbols, out, reinterpret_cast<cudaStream_t>(stream));
+    const int rc = run_decode_stage(h, pl, group + 1, decode_io(nullptr, y_symbols, out), reinterpret_cast<cudaStream_t>(stream));
     if (rc) return rc;
     if (group + 2 < (int)pl.stage_begin.size() - 1) h->dec_next = group + 1;
     return TMAE_OK;
+}
+
+// ---- entropy coder (compressai's rANS format) -----------------------------------------------------------
+int tmae_pmf_to_quantized_cdf(const float* h_pmf, int n, int32_t* h_cdf) {
+    if (!h_pmf || !h_cdf || n < 1) return fail(nullptr, TMAE_EINVAL, "pmf_to_quantized_cdf: null pointer or n < 1");
+    const int rc = pmf_to_quantized_cdf(h_pmf, n, h_cdf);
+    if (rc) return fail(nullptr, rc, "pmf_to_quantized_cdf: the pmf must be finite, non-negative, not all zero, with at most 65536 bins");
+    return TMAE_OK;
+}
+
+int64_t tmae_rans_bound(int64_t n_symbols) { return n_symbols < 0 || n_symbols > ((int64_t)1 << 40) ? -1 : rans_bound_bytes(n_symbols); }
+
+int tmae_set_cdf_tables(tmae_handle* h, int model, const int32_t* cdf, int n_tables, int stride, const int32_t* cdf_lengths,
+                        const int32_t* offsets) {
+    if (!h) return TMAE_EINVAL;
+    h->dec_next = -1;
+    if (model != TMAE_MODEL_GAUSSIAN && model != TMAE_MODEL_BOTTLENECK) return fail(h, TMAE_EINVAL, "unknown entropy model %d", model);
+    if (!cdf || !cdf_lengths || !offsets || n_tables < 1 || stride < 3)
+        return fail(h, TMAE_EINVAL, "cdf tables: null pointer, n_tables < 1 or stride < 3");
+    if ((size_t)n_tables * stride > ((size_t)1 << 30)) return fail(h, TMAE_EINVAL, "cdf tables too large");
+    if (model == TMAE_MODEL_BOTTLENECK && n_tables != h->Cz)
+        return fail(h, TMAE_EINVAL, "bottleneck tables: %d given, one per channel (%d) needed", n_tables, h->Cz);
+    std::vector<int32_t> c((size_t)n_tables * stride), len(n_tables), off(n_tables);
+    CUDA_TRY(h, cudaDeviceSynchronize());           // host or device pointers, possibly written by pending work
+    CUDA_TRY(h, cudaMemcpy(c.data(), cdf, c.size() * 4, cudaMemcpyDefault));
+    CUDA_TRY(h, cudaMemcpy(len.data(), cdf_lengths, len.size() * 4, cudaMemcpyDefault));
+    CUDA_TRY(h, cudaMemcpy(off.data(), offsets, off.size() * 4, cudaMemcpyDefault));
+    CdfTables t;
+    char err[256] = {0};
+    const int rc = rans_build_tables(c.data(), n_tables, stride, len.data(), off.data(), &t, err, sizeof(err));
+    if (rc) return fail(h, rc, "cdf tables: %s", err);
+    drop_plans(h->stream_plans);                     // their graphs captured the previous tables
+    rans_free_tables(&h->cdf[model]);
+    h->cdf[model] = t;
+    return TMAE_OK;
+}
+
+namespace {
+int coder_tables(tmae_handle* h, int model, const CdfTables** out) {
+    if (!h) return TMAE_EINVAL;
+    h->dec_next = -1;                // any other call on the handle ends a decode in progress
+    if (model != TMAE_MODEL_GAUSSIAN && model != TMAE_MODEL_BOTTLENECK) return fail(h, TMAE_EINVAL, "unknown entropy model %d", model);
+    if (!h->cdf[model].n) return fail(h, TMAE_ESTATE, "no cdf tables for model %d (call tmae_set_cdf_tables first)", model);
+    *out = &h->cdf[model];
+    return TMAE_OK;
+}
+}  // namespace
+
+int tmae_rans_encode(tmae_handle* h, int model, const int32_t* symbols, const int32_t* indexes, int n_streams, int n_per_stream,
+                     uint8_t* out, int64_t capacity, int64_t* offsets, int32_t* status, void* stream) {
+    const CdfTables* t = nullptr;
+    int rc = coder_tables(h, model, &t);
+    if (rc) return rc;
+    if (n_streams < 1 || n_per_stream < 0 || (n_per_stream > 0 && (!symbols || !indexes)) || !out || !offsets || !status || capacity < 0)
+        return fail(h, TMAE_EINVAL, "rans_encode: null pointer or bad size");
+    if (reinterpret_cast<uintptr_t>(out) & 3) return fail(h, TMAE_EINVAL, "rans_encode: out must be 4-byte aligned");
+    const long long cap_words = rans_bound_bytes(n_per_stream) / 4;
+    const size_t rec_bytes = ((size_t)n_streams * n_per_stream * sizeof(uint2) + 255) / 256 * 256;
+    const size_t words_bytes = ((size_t)n_streams * cap_words * 4 + 255) / 256 * 256;
+    const size_t need = rec_bytes + words_bytes + (size_t)n_streams * 8;
+    CoderWorkspace& c = h->cws;
+    if (need > c.enc_bytes) {
+        if (c.enc) { cudaFree(c.enc); c.enc = nullptr; c.enc_bytes = 0; }
+        cudaError_t e = cudaMalloc(&c.enc, need);
+        if (e != cudaSuccess) return fail(h, TMAE_ENOMEM, "rans_encode scratch (%zu bytes): %s", need, cudaGetErrorString(e));
+        c.enc_bytes = need;
+    }
+    char* base = static_cast<char*>(c.enc);
+    CUDA_TRY(h, launch_rans_encode(symbols, indexes, n_streams, n_per_stream, *t, reinterpret_cast<uint2*>(base),
+                                   reinterpret_cast<uint32_t*>(base + rec_bytes), cap_words,
+                                   reinterpret_cast<long long*>(base + rec_bytes + words_bytes), out, capacity, offsets, status,
+                                   reinterpret_cast<cudaStream_t>(stream)));
+    return TMAE_OK;
+}
+
+int tmae_rans_decode(tmae_handle* h, int model, const uint8_t* data, const int64_t* offsets, int n_streams, const int32_t* indexes,
+                     int n_per_stream, int32_t* symbols, int32_t* status, void* stream) {
+    const CdfTables* t = nullptr;
+    int rc = coder_tables(h, model, &t);
+    if (rc) return rc;
+    if (n_streams < 1 || n_per_stream < 0 || !data || !offsets || !status || (n_per_stream > 0 && (!indexes || !symbols)))
+        return fail(h, TMAE_EINVAL, "rans_decode: null pointer or bad size");
+    if (reinterpret_cast<uintptr_t>(data) & 3) return fail(h, TMAE_EINVAL, "rans_decode: data must be 4-byte aligned");
+    RansDecArgs d;
+    d.cdf = t->cdf; d.entries = t->entries; d.n_tab = t->n;
+    d.data = data; d.offsets = offsets;
+    d.indexes = indexes; d.idx_stride = n_per_stream;
+    d.symbols = symbols; d.sym_stride = n_per_stream;
+    d.n_streams = n_streams; d.begin = 0; d.end = n_per_stream;
+    d.status = status;
+    CUDA_TRY(h, launch_rans_decode(d, reinterpret_cast<cudaStream_t>(stream)));
+    return TMAE_OK;
+}
+
+int tmae_decompress_streams(tmae_handle* h, const uint8_t* y_data, const int64_t* y_offsets, const uint8_t* z_data,
+                            const int64_t* z_offsets, int N, const tmae_outputs* out, int32_t* status, void* stream) {
+    int rc = check_ready(h, N);
+    if (rc) return rc;
+    if (!y_data || !y_offsets || !z_data || !z_offsets || !out || !status)
+        return fail(h, TMAE_EINVAL, "decompress_streams: stream pointers, out and status must not be null");
+    if ((reinterpret_cast<uintptr_t>(y_data) | reinterpret_cast<uintptr_t>(z_data)) & 3)
+        return fail(h, TMAE_EINVAL, "decompress_streams: stream data must be 4-byte aligned");
+    if (!h->scale_table) return fail(h, TMAE_ESTATE, "decoding needs the scale table (call tmae_set_scale_table first)");
+    if (!h->cdf[TMAE_MODEL_GAUSSIAN].n || !h->cdf[TMAE_MODEL_BOTTLENECK].n)
+        return fail(h, TMAE_ESTATE, "decoding streams needs both cdf table sets (tmae_set_cdf_tables)");
+    if (h->cdf[TMAE_MODEL_GAUSSIAN].n != h->n_scale_table)
+        return fail(h, TMAE_ESTATE, "%d Gaussian cdf tables for a scale table of %d entries", h->cdf[TMAE_MODEL_GAUSSIAN].n, h->n_scale_table);
+    Plan* pl = nullptr;
+    if ((rc = build_stream_decode_plan(h, N, &pl))) return rc;
+    IoBlock hio = decode_io(h->cws.zsym, h->cws.ysym, out);
+    if (!hio.out.y_indexes) hio.out.y_indexes = h->cws.idx;
+    hio.y_data = y_data; hio.y_offsets = y_offsets; hio.z_data = z_data; hio.z_offsets = z_offsets; hio.status = status;
+    if (h->profiling) h->prof_used = 0;
+    return run_decode_stage(h, *pl, 0, hio, reinterpret_cast<cudaStream_t>(stream));
 }
 
 int tmae_pack_nchw_i32(const int32_t* nhwc, int32_t* nchw, int N, int hw, int C, void* stream) {

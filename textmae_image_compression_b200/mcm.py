@@ -20,8 +20,9 @@ include/tmae.h.  PyTorch is used for device memory, streams and the module plumb
                     (tests/test_recon_cpu.py drives both, executed from /root/reference).  The VGG term is a hook
                     (`feature_loss`), 0 when unset: the reference downloads pretrained weights for it.
 `compress_symbols` is the front half of `MCM.compress` (MCM.py:805-873): symbols and scale-table indexes of y in the
-order `encode_with_indexes` consumes, z symbols / channel indexes for `entropy_bottleneck.compress` (SURVEY 8f-1);
-the rANS coder itself (compressai C++) stays outside.
+order `encode_with_indexes` consumes, z symbols / channel indexes for `entropy_bottleneck.compress` (SURVEY 8f-1).
+`compress_bitstream` / `decompress_bitstream` add the GPU rANS coder (entropy.py, csrc/rans.cu) on either side: images to
+compressai-format byte strings and back.
 `decompress_symbols` is the decoder side of `MCM.decompress` (MCM.py:896-968) around the range decoder: symbols in (all at
 once, or group by group through a callback that receives the scale-table indexes), y_hat / z_hat / x_hat out, bit-exact
 with the encoder of the same accuracy mode.
@@ -35,7 +36,7 @@ import torch
 import torch.nn as nn
 import torch.nn.functional as F
 
-from . import _native, recon
+from . import _native, entropy, recon
 from .config import PathConfig
 
 
@@ -81,6 +82,7 @@ class MCM(nn.Module):
         self.softmax_isa = softmax_isa
         self.feature_loss = None                 # optional callable(preds, imgs) -> scalar: the VGG term of forward_loss
         self._scale_table = None                 # GaussianConditional scale table for compress_symbols (update())
+        self._entropy_tables = None              # quantised CDF tables (entropy_tables()), rebuilt after update() / new weights
         self._last_stream = None                 # stream of the previous call on this handle (one workspace per handle)
         self._last_event = None
         self._weights: Dict[str, torch.Tensor] = {}
@@ -102,6 +104,7 @@ class MCM(nn.Module):
         self._weights = {k: v.detach().clone().float() if v.is_floating_point() else v.detach().clone()
                          for k, v in state_dict.items()}
         self._dirty = True
+        self._entropy_tables = None
         return self
 
     @classmethod
@@ -173,6 +176,7 @@ class MCM(nn.Module):
             _native.check(lib.tmae_finalize_weights(hp), hp, RuntimeError)
         self._dirty = False
         self._scale_table_dirty = True           # a fresh handle has no scale table yet
+        self._cdf_dirty = True                   # ... nor cdf tables
         self._last_stream = None
 
     # ------------------------------------------------------------------ helpers
@@ -443,10 +447,11 @@ class MCM(nn.Module):
 
     def update(self, scale_table=None, force: bool = False):
         """The part of `CompressionModel.update(scale_table, force)` that the symbol / index emission needs: install the
-        GaussianConditional scale table (default `get_scale_table()`).  Building the quantised CDF tables for the range
-        coder is compressai's C++ `pmf_to_quantized_cdf` - outside this library (SURVEY 8f-1)."""
+        GaussianConditional scale table (default `get_scale_table()`).  The quantised CDF tables of the range coder
+        (`entropy_tables()`) are rebuilt from it and the weights on their next use."""
         self._scale_table = (self.get_scale_table() if scale_table is None else torch.as_tensor(scale_table)).float().contiguous()
         self._scale_table_dirty = True
+        self._entropy_tables = None
         return True
 
     def _install_scale_table(self):
@@ -469,7 +474,7 @@ class MCM(nn.Module):
             "z_symbols": i32 [N, Cz, s/4, s/4], "z_indexes": i32 [same] - what `entropy_bottleneck.compress(z)` codes
                           (:827): quantize(z, "symbols", medians) and the channel index of every element
             "shape": z spatial size (:890), "ids_restore" (:891)
-        The range coder itself (compressai's C++ rANS) is not part of this library."""
+        `compress_bitstream` runs the range coder on these lists."""
         self._install_scale_table()
         dev = self._handle_device
         lib = _native.load()
@@ -562,13 +567,131 @@ class MCM(nn.Module):
             out["x_hat"] = recon.synthesize(self._weights, c, y_hat.reshape(N, c.num_keep_patches, c.latent_depth), ids_restore.to(dev))
         return out
 
+    # ------------------------------------------------------------------ bitstreams (the GPU rANS coder)
+    def entropy_tables(self) -> Dict[str, torch.Tensor]:
+        """The quantised CDF tables compressai's `update(force=True)` would build for this module's weights and scale table,
+        under compressai's buffer names (CPU int32): gaussian_conditional._quantized_cdf / _cdf_length / _offset (one table
+        per scale-table entry) and entropy_bottleneck._quantized_cdf / _cdf_length / _offset (one per channel)."""
+        if self._entropy_tables is None:
+            if self._scale_table is None:
+                self.update()
+            t = {}
+            for prefix, tabs in (("gaussian_conditional.", entropy.gaussian_tables(self._scale_table)),
+                                 ("entropy_bottleneck.", entropy.bottleneck_tables(self._weights))):
+                t.update({prefix + k: v for k, v in tabs.items()})
+            self._entropy_tables = t
+            self._cdf_dirty = True
+        return self._entropy_tables
+
+    def _install_coder_tables(self):
+        self._install_scale_table()
+        tabs = self.entropy_tables()
+        if self._cdf_dirty:
+            with torch.cuda.device(self._handle_device):
+                for model, prefix in ((_native.MODEL_GAUSSIAN, "gaussian_conditional."), (_native.MODEL_BOTTLENECK, "entropy_bottleneck.")):
+                    entropy.set_tables(self._handle, model, {k: tabs[prefix + k] for k in ("_quantized_cdf", "_cdf_length", "_offset")})
+            self._cdf_dirty = False
+
+    @torch.no_grad()
+    def compress_bitstream(self, imgs: torch.Tensor, total_scores: torch.Tensor):
+        """`MCM.compress` (MCM.py:805-893) on the GPU: {"strings": [y_strings, z_strings], "shape", "ids_restore"} with one
+        `bytes` per image in each list (compressai's rANS format: the y stream codes every slice in order with the Gaussian
+        tables, the z stream the z symbols with the bottleneck tables), plus "bpp" [N], the likelihood estimate of the rate.
+        compress_symbols, one encode call per stream kind, then two reads to the host: the stream offsets and status (a few
+        hundred bytes, which size the second read), then exactly the packed bytes.  Each encode call writes into an output of
+        n_streams * tmae_rans_bound(n) bytes (the worst case, ~63 MB for the y streams at batch 64 and K=64), and the handle
+        keeps an encode scratch of about the same size."""
+        self._ensure_handle()
+        self._install_coder_tables()
+        sym = self.compress_symbols(imgs, total_scores)
+        N = sym["y_symbols"].shape[0]
+        lib_h = self._handle
+        with torch.cuda.device(self._handle_device):
+            cur = self._enter_stream(self._handle_device)
+            y_out, y_off, y_st = entropy.encode(lib_h, _native.MODEL_GAUSSIAN, sym["y_symbols"], sym["y_indexes"])
+            z_out, z_off, z_st = entropy.encode(lib_h, _native.MODEL_BOTTLENECK, sym["z_symbols"].reshape(N, -1),
+                                                sym["z_indexes"].reshape(N, -1))
+            self._leave_stream(cur)
+            meta = torch.cat([y_off, z_off, y_st.long(), z_st.long()]).cpu()
+            y_off, z_off = meta[: N + 1].tolist(), meta[N + 1: 2 * N + 2].tolist()
+            bad = [i for i in range(N) if meta[2 * N + 2 + i] or meta[3 * N + 2 + i]]
+            if bad:
+                raise RuntimeError(f"rANS encode failed for images {bad} (status {meta[2 * N + 2:].tolist()})")
+            host = torch.cat([y_out[: y_off[-1]], z_out[: z_off[-1]]]).cpu().numpy().tobytes()
+        zb = y_off[-1]
+        y_strings = [host[y_off[i]: y_off[i + 1]] for i in range(N)]
+        z_strings = [host[zb + z_off[i]: zb + z_off[i + 1]] for i in range(N)]
+        return {"strings": [y_strings, z_strings], "shape": sym["shape"], "ids_restore": sym["ids_restore"], "bpp": sym["bpp"]}
+
+    @torch.no_grad()
+    def decompress_bitstream(self, strings, shape, ids_restore: torch.Tensor, need_recon: Optional[bool] = None) -> Dict[str, torch.Tensor]:
+        """`MCM.decompress` (MCM.py:896-968) on the GPU from `compress_bitstream`'s strings: one copy of the concatenated bytes
+        to the device, then the range decoder and the network in one enqueued decode (no host round trip in between).
+        Returns {"y_hat": f32 [N,Cy,s,s], "z_hat": f32 [N,Cz,s/4,s/4]} and, with `need_recon` (default: whenever the
+        decoder-side weights are loaded), "x_hat" exactly as forward computes it.  Raises ValueError for malformed arguments,
+        and for images whose streams do not decode exactly to their end (naming them)."""
+        if need_recon is None:
+            need_recon = recon.has_decoder_weights(self._weights)
+        if need_recon and not recon.has_decoder_weights(self._weights):
+            raise RuntimeError("need_recon=True but the loaded state dict has no g_s / decoder tensors")
+        self._ensure_handle()
+        c = self.cfg
+        s, s4 = c.side, c.side // 4
+        if not isinstance(strings, (list, tuple)) or len(strings) != 2:
+            raise ValueError("strings must be [y_strings, z_strings]")
+        y_strings, z_strings = list(strings[0]), list(strings[1])
+        N = len(y_strings)
+        if N < 1 or len(z_strings) != N:
+            raise ValueError(f"need as many z strings as y strings (>= 1), got {N} and {len(z_strings)}")
+        for kind, lst in (("y", y_strings), ("z", z_strings)):
+            for i, b in enumerate(lst):
+                if not isinstance(b, (bytes, bytearray, memoryview)) or len(b) % 4 or len(b) < 8:
+                    raise ValueError(f"{kind} string of image {i}: need bytes of a length that is a multiple of 4 and >= 8")
+        if tuple(shape) != (s4, s4):
+            raise ValueError(f"shape must be ({s4}, {s4}) for this model, got {tuple(shape)}")
+        if tuple(ids_restore.shape) != (N, c.num_patches):
+            raise ValueError(f"ids_restore must be [{N}, {c.num_patches}], got {tuple(ids_restore.shape)}")
+        self._install_coder_tables()
+        dev = self._handle_device
+        # one host buffer: y offsets | z offsets (int64 [N + 1] each) | y bytes | z bytes
+        y_data, y_off = entropy.pack_strings([bytes(b) for b in y_strings])
+        z_data, z_off = entropy.pack_strings([bytes(b) for b in z_strings])
+        host = torch.cat([y_off.view(torch.uint8), z_off.view(torch.uint8), y_data, z_data])
+        f32 = torch.float32
+        y_hat = torch.empty((N, s, s, c.latent_depth), dtype=f32, device=dev)
+        z_hat = torch.empty((N, s4, s4, c.hyperprior_depth), dtype=f32, device=dev)
+        status = torch.empty(N, dtype=torch.int32, device=dev)
+        o = _native.TmaeOutputs()
+        o.y_hat, o.z_hat = y_hat.data_ptr(), z_hat.data_ptr()
+        lib = _native.load()
+        with torch.cuda.device(dev):
+            cur = self._enter_stream(dev)
+            buf = host.pin_memory().to(dev, non_blocking=True)
+            b0 = buf.data_ptr()
+            no = 8 * (N + 1)
+            _native.check(lib.tmae_decompress_streams(self._handle, C.c_void_p(b0 + 2 * no), C.c_void_p(b0),
+                                                      C.c_void_p(b0 + 2 * no + y_data.numel()), C.c_void_p(b0 + no), N,
+                                                      C.byref(o), C.c_void_p(status.data_ptr()), C.c_void_p(cur.cuda_stream)),
+                          self._handle, RuntimeError)
+            self._leave_stream(cur)
+        st = status.cpu()
+        bad = [i for i in range(N) if st[i]]
+        if bad:
+            raise ValueError(f"the streams of images {bad} do not decode (status {[int(st[i]) for i in bad]}: truncated or corrupt)")
+        out = {"y_hat": self._nchw(y_hat), "z_hat": self._nchw(z_hat)}
+        if need_recon:
+            out["x_hat"] = recon.synthesize(self._weights, c, y_hat.reshape(N, c.num_keep_patches, c.latent_depth), ids_restore.to(dev))
+        return out
+
     def compress(self, *args, **kwargs):
-        raise NotImplementedError("bitstream emission (compressai's C++ rANS coder) is outside this library; "
-                                  "compress_symbols() returns the symbol / index lists the coder consumes (SURVEY 8f-1)")
+        raise NotImplementedError("MCM.compress is not provided under the reference's name until the bitstream format has been "
+                                  "checked against compressai itself; compress_bitstream() returns the reference's compress dict "
+                                  "(rANS strings coded on the GPU), compress_symbols() the symbol / index lists")
 
     def decompress(self, *args, **kwargs):
-        raise NotImplementedError("bitstream decoding (compressai's C++ rANS coder) is outside this library; "
-                                  "decompress_symbols() rebuilds y_hat / x_hat from the decoded symbols (SURVEY 8f-1)")
+        raise NotImplementedError("MCM.decompress is not provided under the reference's name until the bitstream format has been "
+                                  "checked against compressai itself; decompress_bitstream() decodes compress_bitstream()'s "
+                                  "strings on the GPU, decompress_symbols() rebuilds y_hat / x_hat from decoded symbols")
 
     # ------------------------------------------------------------------ profiling hooks (bench.py)
     def profile(self, enable: bool, by_run: bool = False):
