@@ -224,6 +224,31 @@ TMAE_API int  tmae_rans_decode(tmae_handle* h, int model, const uint8_t* data, c
 TMAE_API int  tmae_decompress_streams(tmae_handle* h, const uint8_t* y_data, const int64_t* y_offsets, const uint8_t* z_data,
                                       const int64_t* z_offsets, int N, const tmae_outputs* out, int32_t* status, void* stream);
 
+/* Laned rANS format (DESIGN.md section 7): a stream of n symbols with W lanes (1 <= W <= 32) is, as little-endian 32-bit words,
+ * {W, len[0..W), lane 0 .. lane W-1}: lane l holds the compressai stream (as above) of the symbols l, l + W, l + 2W, ... with their
+ * indexes, len[l] its byte length (a multiple of 4, at least 8; a lane without symbols is the 8 flush bytes).  The stream is
+ * 4 (1 + W) + sum len bytes.  The lanes decode in parallel (one thread each), so a stream's decode chain is W times shorter.
+ * Decode status per stream: TMAE_RANS_MALFORMED for a header with another W or lengths that do not add up; every read is
+ * bounded by its own lane (TMAE_RANS_OVERRUN); every lane must end in the encoder's initial state with all its words read
+ * (TMAE_RANS_UNFINISHED); the stream's status is the OR over its lanes.  The calls below take lanes in 1..32 and reject it, and
+ * null pointers, with TMAE_EINVAL (a null handle included); without the needed tables they return TMAE_ESTATE. */
+/* Host-only: bytes that always suffice for one laned stream of n symbols (4 (1 + W) + 4 (10 n + 2 W)); -1 for n < 0 or W outside
+ * 1..32. */
+TMAE_API int64_t tmae_rans_bound_lanes(int64_t n_symbols, int lanes);
+/* tmae_rans_encode in the laned format: n_streams * tmae_rans_bound_lanes(n_per_stream, lanes) bytes of `out` always suffice. */
+TMAE_API int  tmae_rans_encode_lanes(tmae_handle* h, int model, const int32_t* symbols, const int32_t* indexes, int n_streams,
+                                     int n_per_stream, int lanes, uint8_t* out, int64_t capacity, int64_t* offsets, int32_t* status,
+                                     void* stream);
+/* tmae_rans_decode of laned streams. */
+TMAE_API int  tmae_rans_decode_lanes(tmae_handle* h, int model, const uint8_t* data, const int64_t* offsets, int n_streams,
+                                     const int32_t* indexes, int n_per_stream, int lanes, int32_t* symbols, int32_t* status, void* stream);
+/* tmae_decompress_streams of laned streams: y streams of y_lanes lanes (lanes assigned on the symbol's position in the image's
+ * whole y stream, so a lane's state carries across the slice groups), z streams of z_lanes lanes.  Replays as one CUDA graph per
+ * (N, y_lanes, z_lanes). */
+TMAE_API int  tmae_decompress_streams_lanes(tmae_handle* h, const uint8_t* y_data, const int64_t* y_offsets, int y_lanes,
+                                            const uint8_t* z_data, const int64_t* z_offsets, int z_lanes, int N,
+                                            const tmae_outputs* out, int32_t* status, void* stream);
+
 /* Stand-alone operators on the path (each mirrors one reference call) ---------------------------------- */
 /* MCM.get_ids_shuffle + random_masking index work (MCM.py:364-423, 579-583). Outputs may be NULL. */
 TMAE_API int  tmae_mask_select(const float* scores, int N, int L, int K, int softmax_isa,

@@ -86,6 +86,10 @@ SIGNATURES = {
     "tmae_rans_encode": (C.c_int, [_P, C.c_int, _P, _P, C.c_int, C.c_int, _P, C.c_int64, _P, _P, _P]),
     "tmae_rans_decode": (C.c_int, [_P, C.c_int, _P, _P, C.c_int, _P, C.c_int, _P, _P, _P]),
     "tmae_decompress_streams": (C.c_int, [_P, _P, _P, _P, _P, C.c_int, C.POINTER(TmaeOutputs), _P, _P]),
+    "tmae_rans_bound_lanes": (C.c_int64, [C.c_int64, C.c_int]),
+    "tmae_rans_encode_lanes": (C.c_int, [_P, C.c_int, _P, _P, C.c_int, C.c_int, C.c_int, _P, C.c_int64, _P, _P, _P]),
+    "tmae_rans_decode_lanes": (C.c_int, [_P, C.c_int, _P, _P, C.c_int, _P, C.c_int, C.c_int, _P, _P, _P]),
+    "tmae_decompress_streams_lanes": (C.c_int, [_P, _P, _P, C.c_int, _P, _P, C.c_int, C.c_int, C.POINTER(TmaeOutputs), _P, _P]),
     "tmae_mask_select": (C.c_int, [_P, C.c_int, C.c_int, C.c_int, C.c_int, _P, _P, _P, _P]),
     "tmae_gaussian_rate": (C.c_int, [_P, _P, _P, C.c_int64, _P, _P, _P, _P]),
     "tmae_bottleneck_rate": (C.c_int, [_P, _P, C.c_int64, _P, _P, _P, _P]),

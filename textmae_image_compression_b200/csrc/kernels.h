@@ -115,13 +115,14 @@ struct CdfTables {                   // one quantised-CDF table set on the devic
     int* meta = nullptr;             // [3 * n]: start in cdf, cdf length, offset of every table
     uint4* enc = nullptr;            // [entries]: symbol v of table t at start + v: {start | freq << 16, reciprocal shift, reciprocal lo, hi}
 };
-struct RansDecState {                // decoder state of one stream between the stages of a decode plan
+struct RansDecState {                // decoder state of one stream (laned format: one lane) between the stages of a decode plan
     unsigned long long x;
-    unsigned pos, pad;
+    unsigned pos, pad;               // next word; laned format: pad = the lane's end word
 };
 struct RansDecArgs {
     const int* cdf = nullptr;        // CdfTables::cdf (meta follows the entries)
     int entries = 0, n_tab = 0;
+    int lanes = 0;                   // 0: compressai's format (warp per stream); 1..32: laned format (thread per lane), state [s * lanes + l]
     int use_smem = 0, streams_per_block = 1;                 // set by launch_rans_decode
     const uint8_t* data = nullptr;   // streams: bytes [offsets[s], offsets[s + 1]) of data
     const int64_t* offsets = nullptr;
@@ -143,8 +144,10 @@ long long rans_bound_bytes(long long n);
 int rans_build_tables(const int32_t* cdf, int n, int stride, const int32_t* len, const int32_t* off, CdfTables* out,
                       char* err, size_t err_len);                            // host arrays in; uploads (synchronous)
 void rans_free_tables(CdfTables* t);
-cudaError_t launch_rans_encode(const int32_t* sym, const int32_t* idx, int n_streams, int n_per, const CdfTables& tab, uint2* rec,
-                               uint32_t* scratch, long long cap_words, long long* n_words, uint8_t* out, long long capacity,
+long long rans_bound_lanes_bytes(long long n, int lanes);                    // laned format; -1 for n < 0 or lanes outside 1..32
+// lanes = 0: compressai's format; 1..32: the laned format (scratch: n_streams * lanes regions of cap_words)
+cudaError_t launch_rans_encode(const int32_t* sym, const int32_t* idx, int n_streams, int n_per, int lanes, const CdfTables& tab,
+                               uint2* rec, uint32_t* scratch, long long cap_words, long long* n_words, uint8_t* out, long long capacity,
                                int64_t* offsets, int32_t* status, cudaStream_t st);
 cudaError_t launch_rans_decode(RansDecArgs a, cudaStream_t st);
 

@@ -9,6 +9,9 @@
 // ballot, indexes and words are read 32 at a time.  Every read of a stream is bounded by its length: words past the end
 // read as 0 and set a status bit, so a truncated or corrupt stream decodes to garbage with a nonzero status, never out of
 // bounds.
+// Laned format (DESIGN.md section 7): a stream of W lanes is {W, byte length of every lane, the lanes}, lane l being the compressai
+// stream of the symbols l, l + W, ...  The encode recurrence runs per (stream, lane) and a second compaction writes the header;
+// the decode is one thread per (stream, lane), each with its own binary search and every read bounded by its lane.
 #include <math.h>
 
 #include <algorithm>
@@ -66,6 +69,11 @@ int pmf_to_quantized_cdf(const float* pmf, int n, int32_t* cdf_out) {
 long long rans_bound_bytes(long long n) {
     // per symbol at most 1 put + 1 bypass-count put + 8 nibble puts (raw < 2^32), each emitting at most one word; + 2 flush words
     return n < 0 ? -1 : 4 * (10 * n + 2);
+}
+
+long long rans_bound_lanes_bytes(long long n, int lanes) {
+    // the header, then per lane the bound of its ceil((n - l) / lanes) symbols: 4 (1 + lanes) + 4 (10 n + 2 lanes)
+    return n < 0 || lanes < 1 || lanes > 32 ? -1 : 4 * (1 + lanes) + 4 * (10 * n + 2 * lanes);
 }
 
 namespace {
@@ -172,18 +180,20 @@ __device__ __forceinline__ void enc_put_bits(uint64_t& x, uint32_t v, uint32_t* 
     x = (x << 4) | v;
 }
 
-// Pass 2, thread per stream: the reverse recurrence from x = L over the stream's entries, words written backwards from the end
-// of the stream's region [s * cap_words, (s + 1) * cap_words); then the two flush words (low word first).
+// Pass 2, thread per (stream, lane): the reverse recurrence from x = L over the lane's entries (entries lane, lane + lanes, ...
+// of the stream), words written backwards from the end of region r = s * lanes + lane, [r * cap_words, (r + 1) * cap_words);
+// then the two flush words (low word first).  lanes = 1: one chain per stream, compressai's format.
 __global__ void __launch_bounds__(32)
-rans_encode_kernel(const uint2* __restrict__ rec, const uint4* __restrict__ enc, int n_streams, int n_per, uint32_t* __restrict__ scratch,
-                   long long cap_words, long long* __restrict__ n_words) {
-    const int s = blockIdx.x * blockDim.x + threadIdx.x;
-    if (s >= n_streams) return;
-    uint32_t* base = scratch + (size_t)s * cap_words;
+rans_encode_kernel(const uint2* __restrict__ rec, const uint4* __restrict__ enc, int n_streams, int n_per, int lanes,
+                   uint32_t* __restrict__ scratch, long long cap_words, long long* __restrict__ n_words) {
+    const int rg = blockIdx.x * blockDim.x + threadIdx.x;
+    if (rg >= n_streams * lanes) return;
+    const int s = rg / lanes, lane = rg - s * lanes;
+    uint32_t* base = scratch + (size_t)rg * cap_words;
     long long wp = cap_words;
     uint64_t x = kRansL;
     const uint2* r = rec + (size_t)s * n_per;
-    for (int i = n_per - 1; i >= 0; --i) {
+    for (int i = n_per > lane ? lane + (n_per - 1 - lane) / lanes * lanes : -1; i >= 0; i -= lanes) {
         const uint2 e = r[i];
         if (e.y) {
             const uint32_t raw = e.y & 0x7fffffffu;
@@ -202,23 +212,28 @@ rans_encode_kernel(const uint2* __restrict__ rec, const uint4* __restrict__ enc,
     }
     base[--wp] = (uint32_t)(x >> 32);
     base[--wp] = (uint32_t)x;
-    n_words[s] = cap_words - wp;
+    n_words[rg] = cap_words - wp;
+}
+
+// sum of v[0, n) over a block of 256 threads
+__device__ __forceinline__ long long block_sum256(const long long* __restrict__ v, long long n) {
+    __shared__ long long part[8];
+    long long acc = 0;
+    for (long long j = threadIdx.x; j < n; j += blockDim.x) acc += v[j];
+    for (int o = 16; o; o >>= 1) acc += __shfl_xor_sync(kFull, acc, o);
+    if ((threadIdx.x & 31) == 0) part[threadIdx.x >> 5] = acc;
+    __syncthreads();
+    long long sum = 0;
+    for (int w = 0; w < 8; ++w) sum += part[w];
+    return sum;
 }
 
 // Pass 3, block per stream: byte offset = sum of the earlier streams' sizes; copy the words to the packed output.
 __global__ void __launch_bounds__(256)
 rans_compact_kernel(const uint32_t* __restrict__ scratch, long long cap_words, const long long* __restrict__ n_words, int n_streams,
                     uint8_t* __restrict__ out, long long capacity, int64_t* __restrict__ offsets, int32_t* __restrict__ status) {
-    __shared__ long long part[8];
     const int s = blockIdx.x;
-    long long acc = 0;
-    for (int j = threadIdx.x; j < s; j += blockDim.x) acc += n_words[j];
-    for (int o = 16; o; o >>= 1) acc += __shfl_xor_sync(kFull, acc, o);
-    if ((threadIdx.x & 31) == 0) part[threadIdx.x >> 5] = acc;
-    __syncthreads();
-    long long off = 0;
-    for (int w = 0; w < 8; ++w) off += part[w];
-    off *= 4;
+    const long long off = block_sum256(n_words, s) * 4;
     const long long nw = n_words[s];
     if (threadIdx.x == 0) {
         offsets[s] = off;
@@ -231,8 +246,36 @@ rans_compact_kernel(const uint32_t* __restrict__ scratch, long long cap_words, c
     for (long long j = threadIdx.x; j < nw; j += blockDim.x) dst[j] = src[j];
 }
 
-cudaError_t launch_rans_encode(const int32_t* sym, const int32_t* idx, int n_streams, int n_per, const CdfTables& tab, uint2* rec,
-                               uint32_t* scratch, long long cap_words, long long* n_words, uint8_t* out, long long capacity,
+// Pass 3 of the laned format, block per stream: the stream is the words {lanes, byte length of every lane, the lanes in order};
+// its byte offset is the sum of the earlier streams' sizes.
+__global__ void __launch_bounds__(256)
+rans_compact_lanes_kernel(const uint32_t* __restrict__ scratch, long long cap_words, const long long* __restrict__ n_words, int n_streams,
+                          int lanes, uint8_t* __restrict__ out, long long capacity, int64_t* __restrict__ offsets,
+                          int32_t* __restrict__ status) {
+    const int s = blockIdx.x;
+    const long long off = (block_sum256(n_words, (long long)s * lanes) + (long long)s * (1 + lanes)) * 4;
+    const long long* nw = n_words + (size_t)s * lanes;
+    long long total = 1 + lanes;
+    for (int l = 0; l < lanes; ++l) total += nw[l];
+    if (threadIdx.x == 0) {
+        offsets[s] = off;
+        if (s == n_streams - 1) offsets[n_streams] = off + total * 4;
+        if (off + total * 4 > capacity) atomicOr(status + s, RANS_ST_OVERFLOW);
+    }
+    if (off + total * 4 > capacity) return;
+    uint32_t* dst = reinterpret_cast<uint32_t*>(out + off);
+    if (threadIdx.x == 0) dst[0] = (uint32_t)lanes;
+    if ((int)threadIdx.x < lanes) dst[1 + threadIdx.x] = (uint32_t)(nw[threadIdx.x] * 4);
+    dst += 1 + lanes;
+    for (int l = 0; l < lanes; ++l) {
+        const uint32_t* src = scratch + ((size_t)s * lanes + l + 1) * cap_words - nw[l];
+        for (long long j = threadIdx.x; j < nw[l]; j += blockDim.x) dst[j] = src[j];
+        dst += nw[l];
+    }
+}
+
+cudaError_t launch_rans_encode(const int32_t* sym, const int32_t* idx, int n_streams, int n_per, int lanes, const CdfTables& tab,
+                               uint2* rec, uint32_t* scratch, long long cap_words, long long* n_words, uint8_t* out, long long capacity,
                                int64_t* offsets, int32_t* status, cudaStream_t st) {
     cudaError_t e = cudaMemsetAsync(status, 0, sizeof(int32_t) * n_streams, st);
     if (e != cudaSuccess) return e;
@@ -241,9 +284,13 @@ cudaError_t launch_rans_encode(const int32_t* sym, const int32_t* idx, int n_str
         rans_map_kernel<<<(unsigned)((total + 255) / 256), 256, 0, st>>>(sym, idx, total, n_per, tab.meta, tab.n, rec, status);
         if ((e = cudaGetLastError()) != cudaSuccess) return e;
     }
-    rans_encode_kernel<<<(n_streams + 31) / 32, 32, 0, st>>>(rec, tab.enc, n_streams, n_per, scratch, cap_words, n_words);
+    const int chains = n_streams * std::max(lanes, 1);
+    rans_encode_kernel<<<(chains + 31) / 32, 32, 0, st>>>(rec, tab.enc, n_streams, n_per, std::max(lanes, 1), scratch, cap_words, n_words);
     if ((e = cudaGetLastError()) != cudaSuccess) return e;
-    rans_compact_kernel<<<n_streams, 256, 0, st>>>(scratch, cap_words, n_words, n_streams, out, capacity, offsets, status);
+    if (lanes == 0)
+        rans_compact_kernel<<<n_streams, 256, 0, st>>>(scratch, cap_words, n_words, n_streams, out, capacity, offsets, status);
+    else
+        rans_compact_lanes_kernel<<<n_streams, 256, 0, st>>>(scratch, cap_words, n_words, n_streams, lanes, out, capacity, offsets, status);
     return cudaGetLastError();
 }
 
@@ -270,32 +317,83 @@ struct WordReader {
         return v;
     }
 };
-}  // namespace
 
-// Warp per stream: decodes symbols [a.begin, a.end) of every stream, continuing from (and leaving) the state in a.state unless
-// a.init / a.fin.  Table set: [cdf entries | meta 3 per table], in shared memory when it fits.
-__global__ void __launch_bounds__(256)
-rans_decode_kernel(RansDecArgs a) {
-    extern __shared__ int smem_tab[];
-    const int n_words_tab = a.entries + 3 * a.n_tab;
+// one lane's reader (laned format): words [pos, end) of the stream, the next word already in flight
+struct LaneReader {
+    const uint32_t* w;
+    unsigned pos, end;
+    uint32_t nxt;
+    int bad;
+    __device__ __forceinline__ uint32_t fetch(unsigned j) const { return j < end ? __ldg(w + j) : 0u; }
+    __device__ __forceinline__ uint32_t next() {
+        const uint32_t v = nxt;
+        if (pos >= end) bad |= RANS_ST_OVERRUN;
+        nxt = fetch(++pos);
+        return v;
+    }
+};
+
+// The table set, [cdf entries | meta 3 per table], staged in shared memory when a.use_smem (the tables are constant: staged
+// while the predecessor finishes); then the per-call pointers, from the IoBlock in a decode-plan replay.
+__device__ __forceinline__ const int* dec_prologue(const RansDecArgs& a, int* smem_tab, const uint8_t*& data, const int64_t*& offsets,
+                                                   const int32_t*& indexes, int32_t*& status) {
     const int* tab = a.cdf;
-    if (a.use_smem) {                             // the tables are constant: staged while the predecessor finishes
+    if (a.use_smem) {
+        const int n_words_tab = a.entries + 3 * a.n_tab;
         for (int j = threadIdx.x; j < n_words_tab; j += blockDim.x) smem_tab[j] = __ldg(a.cdf + j);
         __syncthreads();
         tab = smem_tab;
     }
     pdl_wait();
-    const uint8_t* data = a.data;
-    const int64_t* offsets = a.offsets;
-    const int32_t* indexes = a.indexes;
-    int32_t* status = a.status;
-    if (a.io) {                                   // per-call pointers of a decode-plan replay
+    data = a.data;
+    offsets = a.offsets;
+    indexes = a.indexes;
+    status = a.status;
+    if (a.io) {
         const bool y = a.io_stream == 1;
         data = y ? a.io->y_data : a.io->z_data;
         offsets = y ? a.io->y_offsets : a.io->z_offsets;
         status = a.io->status;
         if (y) indexes = a.io->out.y_indexes;
     }
+    return tab;
+}
+
+// Decodes past symbol sv = [start, start + freq) of a table of length L and renormalises; for the escape symbol (sv = L - 2) then
+// the bypass count and the raw value's nibbles.  Returns the value before the table's offset.  next() yields the stream's next word.
+template <class Next>
+__device__ __forceinline__ int dec_symbol(uint64_t& x, int sv, int L, uint32_t start, uint32_t freq, Next&& next, int& bad) {
+    x = freq * (x >> kPrec) + (x & 0xffff) - start;
+    if (x < kRansL) x = (x << 32) | next();
+    if (sv != L - 2) return sv;
+    auto get4 = [&]() -> uint32_t {
+        const uint32_t v = (uint32_t)(x & kBypassMax);
+        x >>= 4;
+        if (x < kRansL) x = (x << 32) | next();
+        return v;
+    };
+    uint32_t v = get4();
+    int nb = (int)v;
+    while (v == kBypassMax && nb <= 8) { v = get4(); nb += (int)v; }
+    if (nb > 8) { bad |= RANS_ST_MALFORMED; nb = 8; }      // our encoder never writes more than 8 nibbles
+    uint32_t raw = 0;
+    for (int j = 0; j < nb; ++j) raw |= get4() << (4 * j);
+    const int r = (int)raw;                   // int32 arithmetic as compressai's decoder
+    const int value = r >> 1;
+    return (r & 1) ? -value - 1 : value + (L - 2);
+}
+}  // namespace
+
+// Warp per stream: decodes symbols [a.begin, a.end) of every stream, continuing from (and leaving) the state in a.state unless
+// a.init / a.fin.
+__global__ void __launch_bounds__(256)
+rans_decode_kernel(RansDecArgs a) {
+    extern __shared__ int smem_tab[];
+    const uint8_t* data;
+    const int64_t* offsets;
+    const int32_t* indexes;
+    int32_t* status;
+    const int* tab = dec_prologue(a, smem_tab, data, offsets, indexes, status);
     const int* meta = tab + a.entries;
     const int lane = threadIdx.x & 31;
     const int s = blockIdx.x * a.streams_per_block + (threadIdx.x >> 5);
@@ -348,26 +446,7 @@ rans_decode_kernel(RansDecArgs a) {
             const int p = lo + lane;
             const int sv = lo + __popc(__ballot_sync(kFull, p < hi && c[p] <= cf)) - 1;
             const uint32_t start = (uint32_t)c[sv], freq = (uint32_t)(c[sv + 1] - c[sv]);
-            x = freq * (x >> kPrec) + (x & 0xffff) - start;
-            if (x < kRansL) x = (x << 32) | rd.next(lane);
-            int value = sv;
-            if (sv == L - 2) {                            // escape: bypass count, then the raw value's nibbles
-                auto get4 = [&]() -> uint32_t {
-                    const uint32_t v = (uint32_t)(x & kBypassMax);
-                    x >>= 4;
-                    if (x < kRansL) x = (x << 32) | rd.next(lane);
-                    return v;
-                };
-                uint32_t v = get4();
-                int nb = (int)v;
-                while (v == kBypassMax && nb <= 8) { v = get4(); nb += (int)v; }
-                if (nb > 8) { rd.bad |= RANS_ST_MALFORMED; nb = 8; }      // our encoder never writes more than 8 nibbles
-                uint32_t raw = 0;
-                for (int j = 0; j < nb; ++j) raw |= get4() << (4 * j);
-                const int r = (int)raw;                   // int32 arithmetic as compressai's decoder
-                value = r >> 1;
-                value = (r & 1) ? -value - 1 : value + (L - 2);
-            }
+            const int value = dec_symbol(x, sv, L, start, freq, [&]() { return rd.next(lane); }, rd.bad);
             if (lane == k) my_sym = value + offset;
         }
         if (lane < cnt) out[i0 + lane] = my_sym;
@@ -381,6 +460,104 @@ rans_decode_kernel(RansDecArgs a) {
     }
 }
 
+// Laned format, thread per (stream, lane): lane l of a stream decodes its symbols l, l + lanes, ... within [a.begin, a.end), with
+// its own binary search of the table; consecutive lanes read consecutive indexes and write consecutive symbols.  A block holds
+// a.streams_per_block whole streams, whose status bits are gathered in shared memory.  State between stages: a.state[s * lanes
+// + l] = {x, next word, end word}, word positions relative to the stream's first byte.
+__global__ void __launch_bounds__(256)
+rans_decode_lanes_kernel(RansDecArgs a) {
+    extern __shared__ int smem_tab[];
+    __shared__ int st_img[256];
+    const uint8_t* data;
+    const int64_t* offsets;
+    const int32_t* indexes;
+    int32_t* status;
+    const int* tab = dec_prologue(a, smem_tab, data, offsets, indexes, status);
+    const int* meta = tab + a.entries;
+    const int W = a.lanes;
+    const int j = threadIdx.x / W, l = threadIdx.x - j * W;
+    const int s = blockIdx.x * a.streams_per_block + j;
+    if ((int)threadIdx.x < a.streams_per_block) st_img[threadIdx.x] = 0;
+    __syncthreads();
+    if (j < a.streams_per_block && s < a.n_streams) {
+        const long long b0 = offsets[s], b1 = offsets[s + 1];
+        const bool range_ok = !(b0 < 0 || b1 < b0 || (b0 & 3) || ((b1 - b0) & 3) || (b1 - b0) / 4 > 0xffffffffll);
+        LaneReader rd;
+        rd.w = reinterpret_cast<const uint32_t*>(data + (range_ok ? b0 : 0));
+        rd.bad = 0;
+        uint64_t x;
+        if (a.init) {
+            // header: {W, byte length of every lane (a multiple of 4, >= 8)}, lengths adding up to the stream
+            const unsigned n = range_ok ? (unsigned)((b1 - b0) / 4) : 0u;
+            bool ok = range_ok && n >= 1u + W && __ldg(rd.w) == (unsigned)W;
+            unsigned long long sum = 1 + W, begin = 0;
+            for (int k = 0; ok && k < W; ++k) {
+                const uint32_t len = __ldg(rd.w + 1 + k);
+                if ((len & 3) || len < 8) ok = false;
+                if (k == l) begin = sum;
+                sum += len / 4;
+            }
+            if (ok && sum == n) {
+                rd.pos = (unsigned)begin;
+                rd.end = (unsigned)begin + __ldg(rd.w + 1 + l) / 4;
+            } else {
+                rd.bad = RANS_ST_MALFORMED;
+                rd.pos = rd.end = 0;
+            }
+            rd.nxt = rd.fetch(rd.pos);
+            const uint32_t lo = rd.next(), hi = rd.next();
+            x = ((uint64_t)hi << 32) | lo;
+        } else {
+            const RansDecState q = a.state[(size_t)s * W + l];
+            x = q.x; rd.pos = q.pos; rd.end = q.pad;
+            rd.nxt = rd.fetch(rd.pos);
+        }
+        const int32_t* ix = indexes ? indexes + (size_t)s * a.idx_stride : nullptr;
+        int32_t* out = a.symbols + (size_t)s * a.sym_stride;
+        // the index loads take longer than a symbol's decode: kAhead of them stay in flight, each in a fixed register slot (the
+        // loop body is unrolled over the slots, so no register move waits on a pending load)
+        constexpr int kAhead = 4;
+        auto index_at = [&](int k) { return k < a.end ? (ix ? ix[k] : k / a.idx_div) : 0; };
+        int i = a.begin + ((l - a.begin) % W + W) % W;              // first symbol of this lane in [begin, end)
+        int tq[kAhead];
+#pragma unroll
+        for (int k = 0; k < kAhead; ++k) tq[k] = index_at(i + k * W);
+        for (; i < a.end; i += kAhead * W) {
+#pragma unroll
+            for (int k = 0; k < kAhead; ++k) {
+                const int ik = i + k * W;
+                if (ik >= a.end) break;
+                int t = tq[k];
+                tq[k] = index_at(ik + kAhead * W);
+                if (t < 0 || t >= a.n_tab) { rd.bad |= RANS_ST_BAD_INDEX; t = 0; }
+                const int ts = meta[3 * t], L = meta[3 * t + 1], offset = meta[3 * t + 2];
+                const int* c = tab + ts;
+                const int cf = (int)(x & 0xffff);
+                int lo = 0, hi = L - 1;                              // c[lo] <= cf < c[hi]
+                while (hi - lo > 1) {
+                    const int mid = (lo + hi) >> 1;
+                    if (c[mid] <= cf) lo = mid; else hi = mid;
+                }
+                const uint32_t start = (uint32_t)c[lo], freq = (uint32_t)(c[lo + 1] - c[lo]);
+                int esc_bad = 0;         // not rd.bad itself: aliasing the reader's member makes ptxas keep it on the stack
+                out[ik] = dec_symbol(x, lo, L, start, freq, [&]() { return rd.next(); }, esc_bad) + offset;
+                rd.bad |= esc_bad;
+            }
+        }
+        int stv = rd.bad;
+        if (a.fin && (x != kRansL || rd.pos != rd.end)) stv |= RANS_ST_UNFINISHED;
+        if (!a.fin) { RansDecState q; q.x = x; q.pos = rd.pos; q.pad = rd.end; a.state[(size_t)s * W + l] = q; }
+        if (stv) atomicOr(st_img + j, stv);
+    }
+    __syncthreads();
+    const int si = blockIdx.x * a.streams_per_block + threadIdx.x;
+    if ((int)threadIdx.x < a.streams_per_block && si < a.n_streams) {
+        const int v = st_img[threadIdx.x];
+        if (a.init && a.status_reset) status[si] = v;
+        else if (v) atomicOr(status + si, v);
+    }
+}
+
 cudaError_t launch_rans_decode(RansDecArgs a, cudaStream_t st) {
     if (a.n_streams <= 0) return cudaSuccess;
     const size_t tab_bytes = (size_t)(a.entries + 3 * a.n_tab) * 4;
@@ -388,15 +565,23 @@ cudaError_t launch_rans_decode(RansDecArgs a, cudaStream_t st) {
     static bool configured = false;
     if (!configured) {
         cudaError_t e = cudaFuncSetAttribute(rans_decode_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kDecSmemMax);
+        if (e == cudaSuccess)
+            e = cudaFuncSetAttribute(rans_decode_lanes_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kDecSmemMax);
         if (e != cudaSuccess) return e;
         configured = true;
     }
-    // spread the streams over the SMs (each warp's loop is latency-bound), at most 8 per block
+    // spread the streams over the SMs (every warp's / thread's loop is latency-bound)
     int dev = 0, sms = 0;
     cudaError_t e = cudaGetDevice(&dev);
     if (e == cudaSuccess) e = cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
     if (e != cudaSuccess) return e;
-    a.streams_per_block = std::min(8, std::max(1, (a.n_streams + sms - 1) / sms));
+    const int spread = std::max(1, (a.n_streams + sms - 1) / sms);
+    if (a.lanes > 0) {           // whole streams per block; 256 threads however few lanes, so that the table staging is as fast
+        a.streams_per_block = std::min(256 / a.lanes, spread);      // as the warp kernel's
+        const int blocks = (a.n_streams + a.streams_per_block - 1) / a.streams_per_block;
+        return launch_k(rans_decode_lanes_kernel, dim3(blocks), dim3(256), a.use_smem ? tab_bytes : 0, st, true, a);
+    }
+    a.streams_per_block = std::min(8, spread);     // warp per stream, at most 8 per block
     const int blocks = (a.n_streams + a.streams_per_block - 1) / a.streams_per_block;
     return launch_k(rans_decode_kernel, dim3(blocks), dim3(256), a.use_smem ? tab_bytes : 0, st, true, a);
 }

@@ -13,6 +13,7 @@
 #include <map>
 #include <memory>
 #include <string>
+#include <tuple>
 #include <vector>
 
 #include "../../include/tmae.h"
@@ -75,6 +76,8 @@ struct Step {
     int ln_final = 0;
     // GC
     int slice = 0, gc_slices = 1;
+    // ST_ZDEC / ST_YDEC: lanes per stream (0 = compressai's format)
+    int lanes = 0;
     std::string tag;
 };
 
@@ -133,7 +136,7 @@ struct CoderWorkspace {
     int32_t* zsym = nullptr;         // [N, Cz, s/4, s/4] decoded z symbols (ST_ZDEC -> ST_ZDEQ)
     int32_t* ysym = nullptr;         // [N, Cy * K] decoded y symbols (ST_YDEC -> ST_YDEQ)
     int32_t* idx = nullptr;          // [N, Cy * K] scale-table indexes, when the caller does not ask for them
-    RansDecState* state = nullptr;   // [N] y decoder state between the slice groups
+    RansDecState* state = nullptr;   // [N * 32] y decoder state between the slice groups (per image, or per image and lane)
     size_t enc_bytes = 0;            // tmae_rans_encode scratch: records, per-stream word regions, word counts
     void* enc = nullptr;
 };
@@ -156,7 +159,8 @@ struct tmae_handle {
     Workspace ws;
     std::map<int, std::unique_ptr<Plan>> plans;
     std::map<int, std::unique_ptr<Plan>> dec_plans;   // decode plans by batch size (tmae_decode_begin / _step)
-    std::map<int, std::unique_ptr<Plan>> stream_plans;   // decode-from-streams plans by batch size (tmae_decompress_streams)
+    // decode-from-streams plans by (batch size, y lanes, z lanes); lanes (0, 0) = compressai's format (tmae_decompress_streams)
+    std::map<std::tuple<int, int, int>, std::unique_ptr<Plan>> stream_plans;
     CdfTables cdf[2];                // quantised CDF tables: [TMAE_MODEL_GAUSSIAN], [TMAE_MODEL_BOTTLENECK]
     CoderWorkspace cws;
     int dec_N = 0, dec_next = -1;    // decode in progress: batch size and the next group expected (-1 = none)
@@ -619,7 +623,8 @@ int fill_params(tmae_handle* h, const GemmDesc& d, int groups_for_tiling, GemmPa
 }
 
 // ---- workspace -----------------------------------------------------------------------------------------
-void drop_plans(std::map<int, std::unique_ptr<Plan>>& plans) {
+template <typename Key>
+void drop_plans(std::map<Key, std::unique_ptr<Plan>>& plans) {
     for (auto& kv : plans) {
         if (kv.second->d_params) cudaFree(kv.second->d_params);
         if (kv.second->graph) cudaGraphExecDestroy(kv.second->graph);
@@ -1249,7 +1254,7 @@ int ensure_coder_workspace(tmae_handle* h, int N) {
     const size_t ny = (size_t)N * h->Cy * h->K, nz = (size_t)N * h->Cz * h->s4 * h->s4;
     int rc;
     if ((rc = dev_alloc(h, c.allocs, &c.zsym, nz)) || (rc = dev_alloc(h, c.allocs, &c.ysym, ny)) ||
-        (rc = dev_alloc(h, c.allocs, &c.idx, ny)) || (rc = dev_alloc(h, c.allocs, &c.state, (size_t)N)))
+        (rc = dev_alloc(h, c.allocs, &c.idx, ny)) || (rc = dev_alloc(h, c.allocs, &c.state, (size_t)N * 32)))
         return rc;
     c.cap_N = N;
     return TMAE_OK;
@@ -1258,9 +1263,11 @@ int ensure_coder_workspace(tmae_handle* h, int N) {
 // Decode plan fed by the range decoder (tmae_decompress_streams): the decode plan above with the coder in front of the two
 // dequantisations - ST_ZDEC decodes the z streams with the bottleneck tables before ST_ZDEQ, and ST_YDEC decodes slice group g
 // of the y streams, with the indexes the group's cc layers just wrote, before ST_YDEQ.  The y decoder's state stays in the
-// coder workspace between the groups.  One stage: the whole decode replays as one CUDA graph per batch size.
-int build_stream_decode_plan(tmae_handle* h, int N, Plan** out) {
-    auto it = h->stream_plans.find(N);
+// coder workspace between the groups.  One stage: the whole decode replays as one CUDA graph per (batch size, lanes).
+// lanes_y / lanes_z = 0: compressai's format; else the laned format with that many lanes per y / z stream.
+int build_stream_decode_plan(tmae_handle* h, int N, int lanes_y, int lanes_z, Plan** out) {
+    const auto key = std::make_tuple(N, lanes_y, lanes_z);
+    auto it = h->stream_plans.find(key);
     if (it != h->stream_plans.end()) { *out = it->second.get(); return TMAE_OK; }
     int rc = ensure_workspace(h, N);
     if (rc || (rc = ensure_coder_workspace(h, N))) return rc;
@@ -1274,12 +1281,14 @@ int build_stream_decode_plan(tmae_handle* h, int N, Plan** out) {
     slice_groups(h->nsl, groups);
     pl.stage_begin.push_back(0);
     simple(ST_ZDEC, FAM_CODER, "rans_decode.z");
+    pl.steps.back().lanes = lanes_z;
     simple(ST_ZDEQ, FAM_ENTROPY, "z_dequantize");
     if ((rc = add_hs_steps(h, pl, N))) return rc;
     for (const auto& g : groups) {
         if ((rc = add_cc_steps(h, pl, N, g.first, g.second, true))) return rc;
         if (!h->gc_fuse) simple(ST_IDX, FAM_ENTROPY, "indexes." + std::to_string(g.first), g.first, g.second);
         simple(ST_YDEC, FAM_CODER, "rans_decode.y." + std::to_string(g.first), g.first, g.second);
+        pl.steps.back().lanes = lanes_y;
         simple(ST_YDEQ, FAM_ENTROPY, "dequantize." + std::to_string(g.first), g.first, g.second);
         if ((rc = add_lrp_steps(h, pl, N, g.first, g.second, false))) return rc;
     }
@@ -1289,7 +1298,7 @@ int build_stream_decode_plan(tmae_handle* h, int N, Plan** out) {
     pl.stage_calls.assign(1, 0);
     if ((rc = finish_plan(h, pl))) return rc;
     *out = plp.get();
-    h->stream_plans[N] = std::move(plp);
+    h->stream_plans[key] = std::move(plp);
     return TMAE_OK;
 }
 
@@ -1434,6 +1443,7 @@ int run_steps(tmae_handle* h, Plan& pl, const RunArgs& a, cudaStream_t st) {
                 d.idx_div = h->s4 * h->s4;
                 d.symbols = h->cws.zsym; d.sym_stride = (long long)h->Cz * h->s4 * h->s4;
                 d.n_streams = N; d.begin = 0; d.end = h->Cz * h->s4 * h->s4;
+                d.lanes = sp.lanes;
                 d.io = a.io; d.io_stream = 2;
                 CUDA_TRY(h, launch_rans_decode(d, st));
                 break;
@@ -1448,6 +1458,7 @@ int run_steps(tmae_handle* h, Plan& pl, const RunArgs& a, cudaStream_t st) {
                 d.n_streams = N; d.begin = sp.slice * per_slice; d.end = (sp.slice + sp.gc_slices) * per_slice;
                 d.init = sp.slice == 0; d.fin = sp.slice + sp.gc_slices == h->nsl; d.status_reset = 0;
                 d.state = h->cws.state;
+                d.lanes = sp.lanes;
                 d.io = a.io; d.io_stream = 1;
                 CUDA_TRY(h, launch_rans_decode(d, st));
                 break;
@@ -2015,18 +2026,23 @@ int coder_tables(tmae_handle* h, int model, const CdfTables** out) {
 }
 }  // namespace
 
-int tmae_rans_encode(tmae_handle* h, int model, const int32_t* symbols, const int32_t* indexes, int n_streams, int n_per_stream,
-                     uint8_t* out, int64_t capacity, int64_t* offsets, int32_t* status, void* stream) {
+namespace {
+bool bad_lanes(int lanes) { return lanes < 1 || lanes > 32; }
+
+// lanes = 0: compressai's format, else the laned format
+int rans_encode_impl(tmae_handle* h, int model, const int32_t* symbols, const int32_t* indexes, int n_streams, int n_per_stream,
+                     int lanes, uint8_t* out, int64_t capacity, int64_t* offsets, int32_t* status, void* stream) {
     const CdfTables* t = nullptr;
     int rc = coder_tables(h, model, &t);
     if (rc) return rc;
     if (n_streams < 1 || n_per_stream < 0 || (n_per_stream > 0 && (!symbols || !indexes)) || !out || !offsets || !status || capacity < 0)
         return fail(h, TMAE_EINVAL, "rans_encode: null pointer or bad size");
     if (reinterpret_cast<uintptr_t>(out) & 3) return fail(h, TMAE_EINVAL, "rans_encode: out must be 4-byte aligned");
-    const long long cap_words = rans_bound_bytes(n_per_stream) / 4;
+    const int chains = lanes ? lanes : 1;           // scratch: one region per (stream, lane), sized for the longest lane
+    const long long cap_words = rans_bound_bytes((n_per_stream + chains - 1) / chains) / 4;
     const size_t rec_bytes = ((size_t)n_streams * n_per_stream * sizeof(uint2) + 255) / 256 * 256;
-    const size_t words_bytes = ((size_t)n_streams * cap_words * 4 + 255) / 256 * 256;
-    const size_t need = rec_bytes + words_bytes + (size_t)n_streams * 8;
+    const size_t words_bytes = ((size_t)n_streams * chains * cap_words * 4 + 255) / 256 * 256;
+    const size_t need = rec_bytes + words_bytes + (size_t)n_streams * chains * 8;
     CoderWorkspace& c = h->cws;
     if (need > c.enc_bytes) {
         if (c.enc) { cudaFree(c.enc); c.enc = nullptr; c.enc_bytes = 0; }
@@ -2035,15 +2051,15 @@ int tmae_rans_encode(tmae_handle* h, int model, const int32_t* symbols, const in
         c.enc_bytes = need;
     }
     char* base = static_cast<char*>(c.enc);
-    CUDA_TRY(h, launch_rans_encode(symbols, indexes, n_streams, n_per_stream, *t, reinterpret_cast<uint2*>(base),
+    CUDA_TRY(h, launch_rans_encode(symbols, indexes, n_streams, n_per_stream, lanes, *t, reinterpret_cast<uint2*>(base),
                                    reinterpret_cast<uint32_t*>(base + rec_bytes), cap_words,
                                    reinterpret_cast<long long*>(base + rec_bytes + words_bytes), out, capacity, offsets, status,
                                    reinterpret_cast<cudaStream_t>(stream)));
     return TMAE_OK;
 }
 
-int tmae_rans_decode(tmae_handle* h, int model, const uint8_t* data, const int64_t* offsets, int n_streams, const int32_t* indexes,
-                     int n_per_stream, int32_t* symbols, int32_t* status, void* stream) {
+int rans_decode_impl(tmae_handle* h, int model, const uint8_t* data, const int64_t* offsets, int n_streams, const int32_t* indexes,
+                     int n_per_stream, int lanes, int32_t* symbols, int32_t* status, void* stream) {
     const CdfTables* t = nullptr;
     int rc = coder_tables(h, model, &t);
     if (rc) return rc;
@@ -2052,6 +2068,7 @@ int tmae_rans_decode(tmae_handle* h, int model, const uint8_t* data, const int64
     if (reinterpret_cast<uintptr_t>(data) & 3) return fail(h, TMAE_EINVAL, "rans_decode: data must be 4-byte aligned");
     RansDecArgs d;
     d.cdf = t->cdf; d.entries = t->entries; d.n_tab = t->n;
+    d.lanes = lanes;
     d.data = data; d.offsets = offsets;
     d.indexes = indexes; d.idx_stride = n_per_stream;
     d.symbols = symbols; d.sym_stride = n_per_stream;
@@ -2061,8 +2078,8 @@ int tmae_rans_decode(tmae_handle* h, int model, const uint8_t* data, const int64
     return TMAE_OK;
 }
 
-int tmae_decompress_streams(tmae_handle* h, const uint8_t* y_data, const int64_t* y_offsets, const uint8_t* z_data,
-                            const int64_t* z_offsets, int N, const tmae_outputs* out, int32_t* status, void* stream) {
+int decompress_streams_impl(tmae_handle* h, const uint8_t* y_data, const int64_t* y_offsets, int y_lanes, const uint8_t* z_data,
+                            const int64_t* z_offsets, int z_lanes, int N, const tmae_outputs* out, int32_t* status, void* stream) {
     int rc = check_ready(h, N);
     if (rc) return rc;
     if (!y_data || !y_offsets || !z_data || !z_offsets || !out || !status)
@@ -2075,12 +2092,53 @@ int tmae_decompress_streams(tmae_handle* h, const uint8_t* y_data, const int64_t
     if (h->cdf[TMAE_MODEL_GAUSSIAN].n != h->n_scale_table)
         return fail(h, TMAE_ESTATE, "%d Gaussian cdf tables for a scale table of %d entries", h->cdf[TMAE_MODEL_GAUSSIAN].n, h->n_scale_table);
     Plan* pl = nullptr;
-    if ((rc = build_stream_decode_plan(h, N, &pl))) return rc;
+    if ((rc = build_stream_decode_plan(h, N, y_lanes, z_lanes, &pl))) return rc;
     IoBlock hio = decode_io(h->cws.zsym, h->cws.ysym, out);
     if (!hio.out.y_indexes) hio.out.y_indexes = h->cws.idx;
     hio.y_data = y_data; hio.y_offsets = y_offsets; hio.z_data = z_data; hio.z_offsets = z_offsets; hio.status = status;
     if (h->profiling) h->prof_used = 0;
     return run_decode_stage(h, *pl, 0, hio, reinterpret_cast<cudaStream_t>(stream));
+}
+}  // namespace
+
+int tmae_rans_encode(tmae_handle* h, int model, const int32_t* symbols, const int32_t* indexes, int n_streams, int n_per_stream,
+                     uint8_t* out, int64_t capacity, int64_t* offsets, int32_t* status, void* stream) {
+    return rans_encode_impl(h, model, symbols, indexes, n_streams, n_per_stream, 0, out, capacity, offsets, status, stream);
+}
+
+int tmae_rans_decode(tmae_handle* h, int model, const uint8_t* data, const int64_t* offsets, int n_streams, const int32_t* indexes,
+                     int n_per_stream, int32_t* symbols, int32_t* status, void* stream) {
+    return rans_decode_impl(h, model, data, offsets, n_streams, indexes, n_per_stream, 0, symbols, status, stream);
+}
+
+int tmae_decompress_streams(tmae_handle* h, const uint8_t* y_data, const int64_t* y_offsets, const uint8_t* z_data,
+                            const int64_t* z_offsets, int N, const tmae_outputs* out, int32_t* status, void* stream) {
+    return decompress_streams_impl(h, y_data, y_offsets, 0, z_data, z_offsets, 0, N, out, status, stream);
+}
+
+int64_t tmae_rans_bound_lanes(int64_t n_symbols, int lanes) {
+    return n_symbols > ((int64_t)1 << 40) ? -1 : rans_bound_lanes_bytes(n_symbols, lanes);
+}
+
+int tmae_rans_encode_lanes(tmae_handle* h, int model, const int32_t* symbols, const int32_t* indexes, int n_streams, int n_per_stream,
+                           int lanes, uint8_t* out, int64_t capacity, int64_t* offsets, int32_t* status, void* stream) {
+    if (!h || bad_lanes(lanes) || !out || !offsets || !status || (n_per_stream > 0 && (!symbols || !indexes)))
+        return fail(h, TMAE_EINVAL, "rans_encode_lanes: null pointer, or lanes %d outside 1..32", lanes);
+    return rans_encode_impl(h, model, symbols, indexes, n_streams, n_per_stream, lanes, out, capacity, offsets, status, stream);
+}
+
+int tmae_rans_decode_lanes(tmae_handle* h, int model, const uint8_t* data, const int64_t* offsets, int n_streams,
+                           const int32_t* indexes, int n_per_stream, int lanes, int32_t* symbols, int32_t* status, void* stream) {
+    if (!h || bad_lanes(lanes) || !data || !offsets || !status || (n_per_stream > 0 && (!indexes || !symbols)))
+        return fail(h, TMAE_EINVAL, "rans_decode_lanes: null pointer, or lanes %d outside 1..32", lanes);
+    return rans_decode_impl(h, model, data, offsets, n_streams, indexes, n_per_stream, lanes, symbols, status, stream);
+}
+
+int tmae_decompress_streams_lanes(tmae_handle* h, const uint8_t* y_data, const int64_t* y_offsets, int y_lanes, const uint8_t* z_data,
+                                  const int64_t* z_offsets, int z_lanes, int N, const tmae_outputs* out, int32_t* status, void* stream) {
+    if (!h || bad_lanes(y_lanes) || bad_lanes(z_lanes) || !y_data || !y_offsets || !z_data || !z_offsets || !out || !status)
+        return fail(h, TMAE_EINVAL, "decompress_streams_lanes: null pointer, or lanes (%d, %d) outside 1..32", y_lanes, z_lanes);
+    return decompress_streams_impl(h, y_data, y_offsets, y_lanes, z_data, z_offsets, z_lanes, N, out, status, stream);
 }
 
 int tmae_pack_nchw_i32(const int32_t* nhwc, int32_t* nchw, int N, int hw, int C, void* stream) {

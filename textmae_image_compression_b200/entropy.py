@@ -134,6 +134,45 @@ def decode(handle, model: int, data: torch.Tensor, offsets: torch.Tensor, indexe
     return sym, status
 
 
+def rans_bound_lanes(n_symbols: int, lanes: int) -> int:
+    return int(_native.load().tmae_rans_bound_lanes(n_symbols, lanes))
+
+
+def encode_lanes(handle, model: int, symbols: torch.Tensor, indexes: torch.Tensor, lanes: int
+                 ) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor]:
+    """`encode` in the laned format: every row becomes {lanes, lane byte lengths, lanes}, lane l being the compressai stream of the
+    row's symbols l, l + lanes, ... (DESIGN.md section 7)."""
+    n_streams, n = symbols.shape
+    sym = symbols.to(torch.int32).contiguous()
+    idx = indexes.to(torch.int32).contiguous()
+    cap = n_streams * max(rans_bound_lanes(n, lanes), 0)
+    out = torch.empty(max(cap, 4), dtype=torch.uint8, device=sym.device)
+    offsets = torch.empty(n_streams + 1, dtype=torch.int64, device=sym.device)
+    status = torch.empty(n_streams, dtype=torch.int32, device=sym.device)
+    _native.check(_native.load().tmae_rans_encode_lanes(handle, model, C.c_void_p(sym.data_ptr()), C.c_void_p(idx.data_ptr()),
+                                                        n_streams, n, lanes, C.c_void_p(out.data_ptr()), cap,
+                                                        C.c_void_p(offsets.data_ptr()), C.c_void_p(status.data_ptr()), _stream()),
+                  handle)
+    return out, offsets, status
+
+
+def decode_lanes(handle, model: int, data: torch.Tensor, offsets: torch.Tensor, indexes: torch.Tensor, lanes: int
+                 ) -> Tuple[torch.Tensor, torch.Tensor]:
+    """`decode` of laned streams."""
+    n_streams, n = indexes.shape
+    idx = indexes.to(torch.int32).contiguous()
+    data = data.contiguous()
+    offsets = offsets.to(torch.int64).contiguous()
+    if data.numel() == 0:
+        data = torch.zeros(4, dtype=torch.uint8, device=idx.device)
+    sym = torch.empty((n_streams, n), dtype=torch.int32, device=idx.device)
+    status = torch.empty(n_streams, dtype=torch.int32, device=idx.device)
+    _native.check(_native.load().tmae_rans_decode_lanes(handle, model, C.c_void_p(data.data_ptr()), C.c_void_p(offsets.data_ptr()),
+                                                        n_streams, C.c_void_p(idx.data_ptr()), n, lanes, C.c_void_p(sym.data_ptr()),
+                                                        C.c_void_p(status.data_ptr()), _stream()), handle)
+    return sym, status
+
+
 def pack_strings(strings) -> Tuple[torch.Tensor, torch.Tensor]:
     """list of bytes -> (uint8 [total] host tensor, int64 [n + 1] byte offsets)."""
     lens = [len(s) for s in strings]

@@ -592,15 +592,28 @@ class MCM(nn.Module):
                     entropy.set_tables(self._handle, model, {k: tabs[prefix + k] for k in ("_quantized_cdf", "_cdf_length", "_offset")})
             self._cdf_dirty = False
 
+    @staticmethod
+    def _check_lanes(lanes):
+        """None (compressai's format) or (W_y, W_z), each in 1..32 (the laned format, DESIGN.md section 7)."""
+        if lanes is None:
+            return None
+        if (not isinstance(lanes, (tuple, list)) or len(lanes) != 2
+                or not all(isinstance(w, int) and not isinstance(w, bool) and 1 <= w <= 32 for w in lanes)):
+            raise ValueError(f"lanes must be None or (W_y, W_z) with integers in 1..32, got {lanes!r}")
+        return int(lanes[0]), int(lanes[1])
+
     @torch.no_grad()
-    def compress_bitstream(self, imgs: torch.Tensor, total_scores: torch.Tensor):
+    def compress_bitstream(self, imgs: torch.Tensor, total_scores: torch.Tensor, lanes=None):
         """`MCM.compress` (MCM.py:805-893) on the GPU: {"strings": [y_strings, z_strings], "shape", "ids_restore"} with one
         `bytes` per image in each list (compressai's rANS format: the y stream codes every slice in order with the Gaussian
         tables, the z stream the z symbols with the bottleneck tables), plus "bpp" [N], the likelihood estimate of the rate.
         compress_symbols, one encode call per stream kind, then two reads to the host: the stream offsets and status (a few
         hundred bytes, which size the second read), then exactly the packed bytes.  Each encode call writes into an output of
         n_streams * tmae_rans_bound(n) bytes (the worst case, ~63 MB for the y streams at batch 64 and K=64), and the handle
-        keeps an encode scratch of about the same size."""
+        keeps an encode scratch of about the same size.
+        lanes=(W_y, W_z) writes the laned format instead (every y stream in W_y lanes, every z stream in W_z, each lane a
+        compressai stream; they decode in parallel) and adds "lanes": (W_y, W_z) to the dict."""
+        lanes = self._check_lanes(lanes)
         self._ensure_handle()
         self._install_coder_tables()
         sym = self.compress_symbols(imgs, total_scores)
@@ -608,9 +621,14 @@ class MCM(nn.Module):
         lib_h = self._handle
         with torch.cuda.device(self._handle_device):
             cur = self._enter_stream(self._handle_device)
-            y_out, y_off, y_st = entropy.encode(lib_h, _native.MODEL_GAUSSIAN, sym["y_symbols"], sym["y_indexes"])
-            z_out, z_off, z_st = entropy.encode(lib_h, _native.MODEL_BOTTLENECK, sym["z_symbols"].reshape(N, -1),
-                                                sym["z_indexes"].reshape(N, -1))
+            if lanes is None:
+                y_out, y_off, y_st = entropy.encode(lib_h, _native.MODEL_GAUSSIAN, sym["y_symbols"], sym["y_indexes"])
+                z_out, z_off, z_st = entropy.encode(lib_h, _native.MODEL_BOTTLENECK, sym["z_symbols"].reshape(N, -1),
+                                                    sym["z_indexes"].reshape(N, -1))
+            else:
+                y_out, y_off, y_st = entropy.encode_lanes(lib_h, _native.MODEL_GAUSSIAN, sym["y_symbols"], sym["y_indexes"], lanes[0])
+                z_out, z_off, z_st = entropy.encode_lanes(lib_h, _native.MODEL_BOTTLENECK, sym["z_symbols"].reshape(N, -1),
+                                                          sym["z_indexes"].reshape(N, -1), lanes[1])
             self._leave_stream(cur)
             meta = torch.cat([y_off, z_off, y_st.long(), z_st.long()]).cpu()
             y_off, z_off = meta[: N + 1].tolist(), meta[N + 1: 2 * N + 2].tolist()
@@ -621,15 +639,22 @@ class MCM(nn.Module):
         zb = y_off[-1]
         y_strings = [host[y_off[i]: y_off[i + 1]] for i in range(N)]
         z_strings = [host[zb + z_off[i]: zb + z_off[i + 1]] for i in range(N)]
-        return {"strings": [y_strings, z_strings], "shape": sym["shape"], "ids_restore": sym["ids_restore"], "bpp": sym["bpp"]}
+        out = {"strings": [y_strings, z_strings], "shape": sym["shape"], "ids_restore": sym["ids_restore"], "bpp": sym["bpp"]}
+        if lanes is not None:
+            out["lanes"] = lanes
+        return out
 
     @torch.no_grad()
-    def decompress_bitstream(self, strings, shape, ids_restore: torch.Tensor, need_recon: Optional[bool] = None) -> Dict[str, torch.Tensor]:
+    def decompress_bitstream(self, strings, shape, ids_restore: torch.Tensor, need_recon: Optional[bool] = None,
+                             lanes=None) -> Dict[str, torch.Tensor]:
         """`MCM.decompress` (MCM.py:896-968) on the GPU from `compress_bitstream`'s strings: one copy of the concatenated bytes
         to the device, then the range decoder and the network in one enqueued decode (no host round trip in between).
         Returns {"y_hat": f32 [N,Cy,s,s], "z_hat": f32 [N,Cz,s/4,s/4]} and, with `need_recon` (default: whenever the
         decoder-side weights are loaded), "x_hat" exactly as forward computes it.  Raises ValueError for malformed arguments,
-        and for images whose streams do not decode exactly to their end (naming them)."""
+        and for images whose streams do not decode exactly to their end (naming them).  lanes=(W_y, W_z): the strings are in
+        the laned format of `compress_bitstream(..., lanes=(W_y, W_z))`; a header with another lane count, or lane lengths
+        that do not add up, is a stream that does not decode."""
+        lanes = self._check_lanes(lanes)
         if need_recon is None:
             need_recon = recon.has_decoder_weights(self._weights)
         if need_recon and not recon.has_decoder_weights(self._weights):
@@ -643,10 +668,12 @@ class MCM(nn.Module):
         N = len(y_strings)
         if N < 1 or len(z_strings) != N:
             raise ValueError(f"need as many z strings as y strings (>= 1), got {N} and {len(z_strings)}")
-        for kind, lst in (("y", y_strings), ("z", z_strings)):
+        for k, (kind, lst) in enumerate((("y", y_strings), ("z", z_strings))):
+            # shortest stream: 8 bytes, or with W lanes the header and W empty lanes, 4 (1 + W) + 8 W
+            least = 8 if lanes is None else 4 * (1 + lanes[k]) + 8 * lanes[k]
             for i, b in enumerate(lst):
-                if not isinstance(b, (bytes, bytearray, memoryview)) or len(b) % 4 or len(b) < 8:
-                    raise ValueError(f"{kind} string of image {i}: need bytes of a length that is a multiple of 4 and >= 8")
+                if not isinstance(b, (bytes, bytearray, memoryview)) or len(b) % 4 or len(b) < least:
+                    raise ValueError(f"{kind} string of image {i}: need bytes of a length that is a multiple of 4 and >= {least}")
         if tuple(shape) != (s4, s4):
             raise ValueError(f"shape must be ({s4}, {s4}) for this model, got {tuple(shape)}")
         if tuple(ids_restore.shape) != (N, c.num_patches):
@@ -669,10 +696,14 @@ class MCM(nn.Module):
             buf = host.pin_memory().to(dev, non_blocking=True)
             b0 = buf.data_ptr()
             no = 8 * (N + 1)
-            _native.check(lib.tmae_decompress_streams(self._handle, C.c_void_p(b0 + 2 * no), C.c_void_p(b0),
-                                                      C.c_void_p(b0 + 2 * no + y_data.numel()), C.c_void_p(b0 + no), N,
-                                                      C.byref(o), C.c_void_p(status.data_ptr()), C.c_void_p(cur.cuda_stream)),
-                          self._handle, RuntimeError)
+            yp, yo, zp, zo = (C.c_void_p(b0 + 2 * no), C.c_void_p(b0), C.c_void_p(b0 + 2 * no + y_data.numel()), C.c_void_p(b0 + no))
+            if lanes is None:
+                rc = lib.tmae_decompress_streams(self._handle, yp, yo, zp, zo, N, C.byref(o), C.c_void_p(status.data_ptr()),
+                                                 C.c_void_p(cur.cuda_stream))
+            else:
+                rc = lib.tmae_decompress_streams_lanes(self._handle, yp, yo, lanes[0], zp, zo, lanes[1], N, C.byref(o),
+                                                       C.c_void_p(status.data_ptr()), C.c_void_p(cur.cuda_stream))
+            _native.check(rc, self._handle, RuntimeError)
             self._leave_stream(cur)
         st = status.cpu()
         bad = [i for i in range(N) if st[i]]
