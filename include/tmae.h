@@ -125,13 +125,29 @@ TMAE_API const char* tmae_last_error(const tmae_handle* h);   /* h may be NULL: 
 
 /* Weights: one call per state-dict entry, names exactly as in MCM.state_dict() (SURVEY 8b), e.g.
  * "encoder_blocks.3.attn.qkv.weight".  `data` may be a device or host pointer (cudaMemcpyDefault); the library
- * copies it, so the caller may free it on return.  Unknown names (decoder, g_s, buffers) are ignored and
- * reported through *ignored when non-NULL. */
+ * copies it, so the caller may free it on return.  Unknown names (buffers; the decoder side - g_s, decoder_*,
+ * mask_token - unless tmae_enable_synthesis was called) are ignored and reported through *ignored when non-NULL. */
 TMAE_API int  tmae_set_weight(tmae_handle* h, const char* name, const void* data, int dtype, int ndim,
                      const int64_t* shape, int* ignored);
 /* Checks that every tensor the path needs is present, prepacks to bf16 tensor-core layouts, precomputes
  * softplus/tanh of the factorized-prior parameters.  Synchronises the device. */
 TMAE_API int  tmae_finalize_weights(tmae_handle* h);
+
+/* Synthesis: x_hat from y_hat on the engine (g_s, the MAE decoder and unpatchify; the reference's MCM.py:789-792).
+ * tmae_enable_synthesis, before tmae_finalize_weights (after it, it marks the weights unfinalized as tmae_set_weight does),
+ * makes tmae_set_weight accept the decoder-side tensors (g_s.*, decoder_embed.*, mask_token, decoder_pos_embed,
+ * decoder_blocks.*, decoder_norm.*, decoder_pred.*) and tmae_finalize_weights require them (TMAE_ESTATE naming a missing one;
+ * TMAE_EINVAL for a wrong shape: g_s.{0,2,4,6}.weight are ConvTranspose2d [cin, cout, 1, 1], mask_token [1, 1, Dd],
+ * decoder_pos_embed [1, L + 1, Dd]).  TMAE_EINVAL for depth < 1, a head count that does not divide decoder_embed_dim, a
+ * head dim other than 32, or a TMAE_FLAG_DEBUG_SIMT handle (or TMAE_NO_TMA_STORE set).  Synthesis runs bf16 operands with fp32 accumulation, residual
+ * stream, LayerNorm statistics and softmax in every accuracy mode (the TMAE_FLAG_PRECISE_* flags govern the rate path). */
+TMAE_API int  tmae_enable_synthesis(tmae_handle* h, int decoder_depth, int decoder_num_heads);
+/* x_hat f32 [N, 3, S, S] (NCHW) from y_hat f32 [N, s, s, Cy] (channels-last, as the forward and the decodes write it) and
+ * ids_restore i64 [N, L]: recon.synthesize computed on the engine.  y_hat and x_hat 16-byte aligned.  Asynchronous: no host
+ * synchronisation and, once the plan of this N exists, no allocation; replays as one CUDA graph per N.  An ids_restore value
+ * outside [0, L) is clamped (never read out of bounds); the pixels are then unspecified.  TMAE_ESTATE unless synthesis is
+ * enabled and the weights are finalized. */
+TMAE_API int  tmae_synthesize(tmae_handle* h, const float* y_hat, const int64_t* ids_restore, int N, float* x_hat, void* stream);
 
 /* Scale table of the reference's GaussianConditional (testing.py:223 model.update(force=True) builds it with
  * compressai's get_scale_table(): 64 log-spaced scales 0.11..256): enables out->y_indexes.  Host or device pointer,
@@ -320,6 +336,9 @@ TMAE_API int  tmae_conv3x3_bf16(const void* x, const float* w, const float* bias
  * multi-stream form (one softmax group per CTA, two CTAs per SM; T <= 96, else the same as 1), 3 = two heads per tile
  * (T = 65 and H even, else the same as 1; measured slower, kept as an experiment). */
 TMAE_API int  tmae_attention_bf16(const void* qkv, void* out, int N, int T, int H, int impl, void* stream);
+/* The synthesis plan's attention (head dim 32, mma.sync, T up to 1025 and beyond): softmax(q k^T / sqrt(32)) v over qkv bf16
+ * [N*T, 3*H*32] with columns [3][H][32] -> out bf16 [N*T, H*32].  Synchronises the stream. */
+TMAE_API int  tmae_attention_hd32_bf16(const void* qkv, void* out, int N, int T, int H, void* stream);
 /* C = resid + A B^T + bias (fp32 residual in, fp32 out; the proj / fc2 store phase).  pair = 1: the CTA-pair kernel
  * (tcgen05.mma.cta_group::2, 256-row tiles over two SMs; needs block_n % 32 == 0), 0: the one-CTA kernel. */
 TMAE_API int  tmae_gemm_bf16_resid(const void* A, const void* B, const float* bias, const float* resid, float* C,

@@ -68,6 +68,8 @@ SIGNATURES = {
     "tmae_last_error": (C.c_char_p, [_P]),
     "tmae_set_weight": (C.c_int, [_P, C.c_char_p, _P, C.c_int, C.c_int, C.POINTER(C.c_int64), C.POINTER(C.c_int)]),
     "tmae_finalize_weights": (C.c_int, [_P]),
+    "tmae_enable_synthesis": (C.c_int, [_P, C.c_int, C.c_int]),
+    "tmae_synthesize": (C.c_int, [_P, _P, _P, C.c_int, _P, _P]),
     "tmae_workspace_bytes": (C.c_size_t, [_P, C.c_int]),
     "tmae_reserve": (C.c_int, [_P, C.c_int]),
     "tmae_forward": (C.c_int, [_P, _P, _P, C.c_int, C.POINTER(TmaeOutputs), _P]),
@@ -107,6 +109,7 @@ SIGNATURES = {
     "tmae_gemm_bf16_out": (C.c_int, [_P, _P, _P, _P, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, _P]),
     "tmae_conv3x3_bf16": (C.c_int, [_P, _P, _P, _P, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, _P]),
     "tmae_attention_bf16": (C.c_int, [_P, _P, C.c_int, C.c_int, C.c_int, C.c_int, _P]),
+    "tmae_attention_hd32_bf16": (C.c_int, [_P, _P, C.c_int, C.c_int, C.c_int, _P]),
     "tmae_gemm_bf16_resid": (C.c_int, [_P, _P, _P, _P, _P, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, _P]),
     "tmae_gemm_split": (C.c_int, [_P, _P, _P, _P, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, _P]),
     "tmae_conv3x3_split": (C.c_int, [_P, _P, _P, _P, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, _P]),

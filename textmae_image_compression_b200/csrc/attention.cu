@@ -21,6 +21,10 @@ constexpr int HD = 64;
 constexpr int KPITCH = HD + 8;        // bf16 elements per K row in smem: 36 words -> conflict-free B-fragment loads
 constexpr int kAttnWarps = 5;          // T = 65 (K = 64 kept patches + cls) is 5 query tiles of 16: one per warp, one round
 constexpr int kAttnThreads = 32 * kAttnWarps;
+// head dim 32 (the MAE decoder blocks, T = L + 1 up to 1025): pitch 40 elements (20 words: the 8 rows of an ldmatrix tile
+// still fall in distinct bank groups), 8 warps and <= 64 registers (4 CTAs per SM at T = 197; a CTA holds all keys and its
+// warps' Q tiles, (2 * 1040 + 8 * 16) * 40 * 2 B = 172.5 KiB at T = 1025, so there one CTA fills an SM's shared memory)
+constexpr int kAttn32Warps = 8;
 
 __device__ __forceinline__ void mma_bf16_16816(float (&c)[4], const uint32_t (&a)[4], uint32_t b0, uint32_t b1) {
     asm volatile(
@@ -44,9 +48,13 @@ __device__ __forceinline__ void ldmatrix_x4_trans(uint32_t (&r)[4], uint32_t add
 // fragment then comes from ldmatrix (Q, K plain; V .trans): no transposed copy of V, no scalar shared-memory traffic
 // and no Q registers held across the key loop (<= 64 registers -> 6 CTAs / 30 warps per SM, 888 slots >= the 768
 // (image, head) CTAs of batch 64: one wave, one query tile per warp).
-__global__ void __launch_bounds__(kAttnThreads, 6)
+// Templated on the head dim D (64: the encoder, 32: the MAE decoder of the synthesis plan) and the warp count W; the D = 64,
+// W = 5 instance is the encoder's kernel.
+template <int D, int W, int MINB>
+__global__ void __launch_bounds__(32 * W, MINB)
 attention_kernel(const __nv_bfloat16* __restrict__ qkv, __nv_bfloat16* __restrict__ out, int T, int Tp, int H, int C,
                  float scale_log2e) {
+    constexpr int HD = D, KPITCH = D + 8, kAttnWarps = W, kAttnThreads = 32 * W;
     pdl_wait();
     pdl_launch_dependents();
     extern __shared__ __align__(16) uint8_t smem_attn[];
@@ -60,11 +68,11 @@ attention_kernel(const __nv_bfloat16* __restrict__ qkv, __nv_bfloat16* __restric
     const __nv_bfloat16* base = qkv + (size_t)n * T * ld + (size_t)h * HD;
     __nv_bfloat16* myQ = sQ + (size_t)warp * 16 * KPITCH;
 
-    // this warp's Q tile: 16 rows x 64 dims = 128 16-byte chunks, 4 per lane (rows >= T are zero)
+    // this warp's Q tile: 16 rows x HD dims = 2 HD 16-byte chunks, HD / 16 per lane (rows >= T are zero)
     auto stage_q = [&](int q0) {
 #pragma unroll
-        for (int i = 0; i < 4; ++i) {
-            const int e = i * 32 + lane, r = e >> 3, c8 = (e & 7) * 8;
+        for (int i = 0; i < HD / 16; ++i) {
+            const int e = i * 32 + lane, r = e / (HD / 8), c8 = (e % (HD / 8)) * 8;
             uint4 qv = make_uint4(0, 0, 0, 0);
             if (q0 + r < T) qv = *reinterpret_cast<const uint4*>(base + (size_t)(q0 + r) * ld + c8);
             *reinterpret_cast<uint4*>(myQ + r * KPITCH + c8) = qv;
@@ -101,9 +109,9 @@ attention_kernel(const __nv_bfloat16* __restrict__ qkv, __nv_bfloat16* __restric
             stage_q(q0);
             __syncwarp();
         }
-        float o[8][4];
+        float o[HD / 8][4];
 #pragma unroll
-        for (int i = 0; i < 8; ++i) { o[i][0] = o[i][1] = o[i][2] = o[i][3] = 0.f; }
+        for (int i = 0; i < HD / 8; ++i) { o[i][0] = o[i][1] = o[i][2] = o[i][3] = 0.f; }
         float m0 = -INFINITY, m1 = -INFINITY, l0 = 0.f, l1 = 0.f;     // rows g and g+8
 
         for (int k0 = 0; k0 < Tp; k0 += 16) {
@@ -113,7 +121,7 @@ attention_kernel(const __nv_bfloat16* __restrict__ qkv, __nv_bfloat16* __restric
             sacc[1][0] = sacc[1][1] = sacc[1][2] = sacc[1][3] = 0.f;
             const uint32_t ka = sK_a + (uint32_t)(k0 * KPITCH * 2) + k_lane;
 #pragma unroll
-            for (int hk = 0; hk < 2; ++hk) {       // d 0..31 (k-steps 0, 1), then d 32..63 (k-steps 2, 3)
+            for (int hk = 0; hk < HD / 32; ++hk) {  // d 0..31 (k-steps 0, 1), then d 32..63 (k-steps 2, 3)
                 uint32_t kb0[4], kb1[4], qa[4];
                 ldmatrix_x4(kb0, ka + (uint32_t)(hk * 64));                               // keys k0 .. k0+7
                 ldmatrix_x4(kb1, ka + (uint32_t)(8 * KPITCH * 2 + hk * 64));              // keys k0+8 .. k0+15
@@ -158,13 +166,13 @@ attention_kernel(const __nv_bfloat16* __restrict__ qkv, __nv_bfloat16* __restric
             l0 = l0 * corr0 + rs0;
             l1 = l1 * corr1 + rs1;
 #pragma unroll
-            for (int dt = 0; dt < 8; ++dt) {
+            for (int dt = 0; dt < HD / 8; ++dt) {
                 o[dt][0] *= corr0; o[dt][1] *= corr0; o[dt][2] *= corr1; o[dt][3] *= corr1;
             }
-            // O += P (16 x 16 keys) * V[k0..k0+16) (16 keys x 64): one transposing ldmatrix per pair of 8-wide d tiles
+            // O += P (16 x 16 keys) * V[k0..k0+16) (16 keys x HD): one transposing ldmatrix per pair of 8-wide d tiles
             const uint32_t va = sV_a + (uint32_t)(k0 * KPITCH * 2) + v_lane;
 #pragma unroll
-            for (int dp = 0; dp < 4; ++dp) {
+            for (int dp = 0; dp < HD / 16; ++dp) {
                 uint32_t vb[4];
                 ldmatrix_x4_trans(vb, va + (uint32_t)(dp * 32));
                 mma_bf16_16816(o[2 * dp], pa, vb[0], vb[1]);
@@ -180,7 +188,7 @@ attention_kernel(const __nv_bfloat16* __restrict__ qkv, __nv_bfloat16* __restric
         const int r0 = q0 + g, r1 = q0 + g + 8;
         __nv_bfloat16* obase = out + (size_t)n * T * C + (size_t)h * HD;
 #pragma unroll
-        for (int dt = 0; dt < 8; ++dt) {
+        for (int dt = 0; dt < HD / 8; ++dt) {
             const int c = dt * 8 + 2 * t;
             if (r0 < T) *reinterpret_cast<uint32_t*>(obase + (size_t)r0 * C + c) = pack_bf16x2(o[dt][0] * inv0, o[dt][1] * inv0);
             if (r1 < T) *reinterpret_cast<uint32_t*>(obase + (size_t)r1 * C + c) = pack_bf16x2(o[dt][2] * inv1, o[dt][3] * inv1);
@@ -189,10 +197,12 @@ attention_kernel(const __nv_bfloat16* __restrict__ qkv, __nv_bfloat16* __restric
 }
 
 inline int attn_tp(int T) { return (T + 15) / 16 * 16; }
-inline size_t attn_smem(int T) {
+inline size_t attn_smem(int T, int hd = HD, int warps = kAttnWarps) {
     const int Tp = attn_tp(T);
-    return ((size_t)2 * Tp + (size_t)kAttnWarps * 16) * KPITCH * sizeof(__nv_bfloat16);
+    return ((size_t)2 * Tp + (size_t)warps * 16) * (hd + 8) * sizeof(__nv_bfloat16);
 }
+#define ATTN64 attention_kernel<64, kAttnWarps, 6>
+#define ATTN32 attention_kernel<32, kAttn32Warps, 4>
 
 // ---------------------------------------------------------------------------------------------------------
 // Precise mode (TMAE_FLAG_PRECISE_ALL): fp32 softmax attention on CUDA cores.  q, k, v arrive as split-bf16 plane pairs
@@ -781,7 +791,7 @@ inline bool attn_tc_plan(int T, int H, int C, int N, float scale, AttnTcParams* 
 cudaError_t attention_configure(int T) {
     if (attn_smem(T) > 227 * 1024) return cudaErrorInvalidValue;
     static cudaError_t once = [] {
-        cudaError_t e = cudaFuncSetAttribute(attention_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
+        cudaError_t e = cudaFuncSetAttribute(ATTN64, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
         if (e != cudaSuccess) return e;
         e = cudaFuncSetAttribute(attention_tc_kernel<3, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
         if (e != cudaSuccess) return e;
@@ -800,8 +810,20 @@ cudaError_t launch_attention(const __nv_bfloat16* qkv, __nv_bfloat16* out, int N
                              cudaStream_t st) {
     if (C != H * HD) return cudaErrorInvalidValue;
     const int Tp = attn_tp(T);
-    TMAE_CARVEOUT_ONCE(attention_kernel);
-    return launch_k(attention_kernel, dim3(N * H), dim3(kAttnThreads), attn_smem(T), st, true, qkv, out, T, Tp, H, C,
+    TMAE_CARVEOUT_ONCE(ATTN64);
+    return launch_k(ATTN64, dim3(N * H), dim3(kAttnThreads), attn_smem(T), st, true, qkv, out, T, Tp, H, C,
+                    scale * 1.4426950408889634f);
+}
+
+bool attention_hd32_supported(int T) { return T >= 1 && attn_smem(T, 32, kAttn32Warps) <= 227 * 1024; }
+
+cudaError_t launch_attention_hd32(const __nv_bfloat16* qkv, __nv_bfloat16* out, int N, int T, int H, float scale, cudaStream_t st) {
+    if (!attention_hd32_supported(T)) return cudaErrorInvalidValue;
+    static const cudaError_t configured = cudaFuncSetAttribute(ATTN32, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
+    if (configured != cudaSuccess) return configured;
+    const int Tp = attn_tp(T);
+    TMAE_CARVEOUT_ONCE(ATTN32);
+    return launch_k(ATTN32, dim3(N * H), dim3(32 * kAttn32Warps), attn_smem(T, 32, kAttn32Warps), st, true, qkv, out, T, Tp, H, H * 32,
                     scale * 1.4426950408889634f);
 }
 

@@ -673,4 +673,117 @@ cudaError_t launch_f32_to_bf16_cols(const float* a, __nv_bfloat16* o, long long 
     return cudaGetLastError();
 }
 
+// ---------------------------------------------------------------------------------------------------------
+// Synthesis (tmae_synthesize: recon.synthesize on the engine).  The per-call pointers come from the IoBlock.
+// ---------------------------------------------------------------------------------------------------------
+// io->syn_y_hat (f32 [rows, Cy], the caller's channels-last y_hat) -> bf16, the A operand of g_s.0.  n4 = elements / 4.
+__global__ void __launch_bounds__(256)
+synth_input_kernel(__nv_bfloat16* __restrict__ out, long long n4, const IoBlock* __restrict__ io) {
+    pdl_wait();
+    pdl_launch_dependents();
+    const float4* a = reinterpret_cast<const float4*>(io->syn_y_hat);
+    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n4; i += (long long)gridDim.x * blockDim.x) {
+        const float4 v = a[i];
+        uint2 pk;
+        pk.x = pack_bf16x2(v.x, v.y);
+        pk.y = pack_bf16x2(v.z, v.w);
+        reinterpret_cast<uint2*>(out)[i] = pk;
+    }
+}
+
+cudaError_t launch_synth_input(__nv_bfloat16* out, long long n, cudaStream_t st, const IoBlock* io) {
+    if (n % 4 != 0) return cudaErrorInvalidValue;
+    const long long n4 = n / 4;
+    const unsigned blocks = (unsigned)((n4 + 255) / 256 < 1184 ? (n4 + 255) / 256 : 1184);
+    TMAE_CARVEOUT_ONCE(synth_input_kernel);
+    return launch_k(synth_input_kernel, dim3(blocks > 0 ? blocks : 1), dim3(256), 0, st, true, out, n4, io);
+}
+
+// MAE decoder input (recon.forward_decoder, MCM.py:636-665, with its quirk reproduced): decoder_embed's output emb f32
+// [N*K, D] -> residual stream x f32 [N*T, D], T = L + 1.  Row 0 of an image is its token 0; row t >= 1 takes
+// j = ids_restore[t - 1], clamped to [0, L) so that no id can read out of bounds: token j + 1 if j < K - 1, else mask_token.
+// Every row then adds decoder_pos_embed[t].  Also writes the bf16 copy of x and one (sum, sum of squares) partial per row and
+// 32-column chunk - the statistics block 0's LayerNorm-folded QKV reads, in the layout the proj / fc2 store phases write.
+// Thread = 4 columns of one row, 8 threads = one chunk.
+__global__ void __launch_bounds__(256)
+synth_unshuffle_kernel(const float* __restrict__ emb, const float* __restrict__ mask_token, const float* __restrict__ pos,
+                       float* __restrict__ x, __nv_bfloat16* __restrict__ x_bf, float* __restrict__ stats, int N, int K, int L, int D,
+                       const IoBlock* __restrict__ io) {
+    pdl_wait();
+    pdl_launch_dependents();
+    const int T = L + 1, q = D / 4;
+    const long long total = (long long)N * T * q;
+    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    const bool ok = i < total;                       // every lane takes part in the chunk reduction below
+    float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
+    long long row = 0;
+    int c = 0;
+    if (ok) {
+        row = i / q;
+        c = (int)(i - row * q) * 4;
+        const int n = (int)(row / T), t = (int)(row - (long long)n * T);
+        const float* src = emb + (size_t)n * K * D;
+        if (t > 0) {
+            long long j = io->syn_ids[(size_t)n * L + (t - 1)];
+            j = j < 0 ? 0 : (j >= L ? L - 1 : j);
+            src = j < K - 1 ? emb + ((size_t)n * K + (size_t)j + 1) * D : mask_token;
+        }
+        const float4 a = *reinterpret_cast<const float4*>(src + c);
+        const float4 p = __ldg(reinterpret_cast<const float4*>(pos + (size_t)t * D + c));
+        v = make_float4(a.x + p.x, a.y + p.y, a.z + p.z, a.w + p.w);
+        *reinterpret_cast<float4*>(x + (size_t)row * D + c) = v;
+        uint2 pk;
+        pk.x = pack_bf16x2(v.x, v.y);
+        pk.y = pack_bf16x2(v.z, v.w);
+        *reinterpret_cast<uint2*>(x_bf + (size_t)row * D + c) = pk;
+    }
+    float s1 = (v.x + v.y) + (v.z + v.w);
+    float s2 = fmaf(v.x, v.x, v.y * v.y) + fmaf(v.z, v.z, v.w * v.w);
+#pragma unroll
+    for (int sh = 1; sh < 8; sh <<= 1) {
+        s1 += __shfl_xor_sync(0xffffffffu, s1, sh);
+        s2 += __shfl_xor_sync(0xffffffffu, s2, sh);
+    }
+    if (ok && (threadIdx.x & 7) == 0) reinterpret_cast<float2*>(stats)[row * (D / 32) + c / 32] = make_float2(s1, s2);
+}
+
+cudaError_t launch_synth_unshuffle(const float* emb, const float* mask_token, const float* pos, float* x, __nv_bfloat16* x_bf, float* stats,
+                                   int N, int K, int L, int D, cudaStream_t st, const IoBlock* io) {
+    if (D % 32 != 0 || K < 1 || K > L) return cudaErrorInvalidValue;
+    const long long total = (long long)N * (L + 1) * (D / 4);
+    TMAE_CARVEOUT_ONCE(synth_unshuffle_kernel);
+    return launch_k(synth_unshuffle_kernel, dim3((unsigned)((total + 255) / 256)), dim3(256), 0, st, true, emb, mask_token, pos, x, x_bf,
+                    stats, N, K, L, D, io);
+}
+
+// decoder_pred's output preds bf16 [N*T, P*P*3] -> io->syn_x_hat f32 [N, 3, S, S] (recon.unpatchify, MCM.py:524-546: (p, q, c)
+// order within a patch); row 0 of every image is dropped.  Thread = 4 consecutive pixels of one row of one channel.
+__global__ void __launch_bounds__(256)
+synth_unpatchify_kernel(const __nv_bfloat16* __restrict__ preds, int N, int P, int gw, const IoBlock* __restrict__ io) {
+    pdl_wait();
+    pdl_launch_dependents();
+    float* __restrict__ xh = io->syn_x_hat;
+    const int S = gw * P, S4 = S / 4, T = gw * gw + 1, ld = P * P * 3;
+    const long long total = (long long)N * 3 * S * S4;
+    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
+        const int X = (int)(i % S4) * 4;
+        long long r = i / S4;
+        const int y = (int)(r % S);
+        r /= S;
+        const int ch = (int)(r % 3), n = (int)(r / 3);
+        const int hh = y / P, p = y - hh * P, ww = X / P, qq = X - ww * P;
+        const __nv_bfloat16* src = preds + ((size_t)n * T + 1 + hh * gw + ww) * ld + (p * P + qq) * 3 + ch;
+        const float4 o = make_float4(__bfloat162float(src[0]), __bfloat162float(src[3]), __bfloat162float(src[6]), __bfloat162float(src[9]));
+        *reinterpret_cast<float4*>(xh + (((size_t)n * 3 + ch) * S + y) * S + X) = o;
+    }
+}
+
+cudaError_t launch_synth_unpatchify(const __nv_bfloat16* preds, int N, int P, int gw, cudaStream_t st, const IoBlock* io) {
+    if (P % 4 != 0) return cudaErrorInvalidValue;
+    const long long total = (long long)N * 3 * gw * P * gw * P / 4;
+    const long long want = (total + 255) / 256;
+    TMAE_CARVEOUT_ONCE(synth_unpatchify_kernel);
+    return launch_k(synth_unpatchify_kernel, dim3((unsigned)(want < 2368 ? want : 2368)), dim3(256), 0, st, true, preds, N, P, gw, io);
+}
+
 }  // namespace tmae

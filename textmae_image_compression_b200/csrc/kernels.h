@@ -22,6 +22,9 @@ struct IoBlock {
     const uint8_t* z_data;
     const int64_t* z_offsets;
     int32_t* status;                 //   [N] per-image coder status (RANS_ST_* bits)
+    const float* syn_y_hat;          // synthesis (tmae_synthesize): y_hat f32 [N, s, s, Cy] in,
+    const int64_t* syn_ids;          //   ids_restore [N, L] in,
+    float* syn_x_hat;                //   x_hat f32 [N, 3, S, S] out
 };
 
 // gemm_tc.cu
@@ -52,6 +55,9 @@ bool attention_tc_describe(int T, int H, int N, int mode, int* out12);        //
 void attention_tc_boxes(int T, int H, int mode, int* q_rows, int* kv_rows);   // TMA box rows of the Q map and of the K / V map
 cudaError_t launch_attention_tc(const CUtensorMap* map_q, const CUtensorMap* map_kv, const __nv_bfloat16* qkv, __nv_bfloat16* out, int N,
                                 int T, int H, int C, float scale, cudaStream_t st, long long* dbg = nullptr, int mode = 1);
+// head dim 32 (the MAE decoder of the synthesis plan): the mma.sync kernel above with 32-column heads, qkv columns [3][H][32]
+bool attention_hd32_supported(int T);     // K and V of all T keys fit shared memory (T <= ~1300)
+cudaError_t launch_attention_hd32(const __nv_bfloat16* qkv, __nv_bfloat16* out, int N, int T, int H, float scale, cudaStream_t st);
 // precise mode: fp32 softmax attention on CUDA cores over split-bf16 (hi + lo plane) q, k, v; writes both planes
 cudaError_t launch_attention_f32(const __nv_bfloat16* qkv, long long qkv_lo, __nv_bfloat16* out, long long out_lo, int N,
                                  int T, int H, int C, float scale, cudaStream_t st);
@@ -96,6 +102,11 @@ cudaError_t launch_build_blockdiag2(const float* wa, const float* wb, const floa
                                     int half, int Cin, int taps, cudaStream_t st);
 cudaError_t launch_permute_bias_shuffle(const float* b, float* out, int Cout, cudaStream_t st);
 cudaError_t launch_eb_table(const float* const* ptrs, float* tab, int Cz, cudaStream_t st);
+// synthesis (tmae_synthesize): y_hat in, the MAE decoder's input rows, x_hat out (per-call pointers from the IoBlock)
+cudaError_t launch_synth_input(__nv_bfloat16* out, long long n, cudaStream_t st, const IoBlock* io);
+cudaError_t launch_synth_unshuffle(const float* emb, const float* mask_token, const float* pos, float* x, __nv_bfloat16* x_bf, float* stats,
+                                   int N, int K, int L, int D, cudaStream_t st, const IoBlock* io);
+cudaError_t launch_synth_unpatchify(const __nv_bfloat16* preds, int N, int P, int gw, cudaStream_t st, const IoBlock* io);
 cudaError_t launch_f32_to_bf16(const float* a, __nv_bfloat16* o, long long n, long long lo_off, cudaStream_t st);
 cudaError_t launch_f32_to_bf16_cols(const float* a, __nv_bfloat16* o, long long rows, int cols, int ld, long long lo_off, cudaStream_t st);
 

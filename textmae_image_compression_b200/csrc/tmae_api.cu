@@ -54,7 +54,8 @@ struct Bf {
 
 enum StepKind { ST_MASK, ST_GATHER, ST_GEMM, ST_FORCE, ST_LN, ST_ATTN, ST_EB, ST_GC, ST_RATE, ST_ZERO_RATE,
                 ST_ZDEQ, ST_IDX, ST_YDEQ, ST_DEC_OUT,        // decode plans only
-                ST_ZDEC, ST_YDEC };                          // decode-from-streams plans only: the range decoder
+                ST_ZDEC, ST_YDEC,                            // decode-from-streams plans only: the range decoder
+                ST_SYN_IN, ST_UNSHUF, ST_ATTN32, ST_UNPATCH };  // synthesis plans only
 enum Family { FAM_GEMM = 0, FAM_ATTN, FAM_LN, FAM_MASK, FAM_GATHER, FAM_ENTROPY, FAM_MISC, FAM_CODER, FAM_COUNT };
 const char* kFamilyNames[FAM_COUNT] = {"gemm_tc", "attention", "layernorm", "mask_select", "gather_patches",
                                        "entropy_elementwise", "misc", "entropy_coder"};
@@ -141,6 +142,20 @@ struct CoderWorkspace {
     void* enc = nullptr;
 };
 
+// Buffers of the synthesis plans (tmae_synthesize), allocated only on handles with synthesis enabled.  All bf16 buffers hold
+// one plane: synthesis runs bf16 operands in every accuracy mode.
+struct SynthWorkspace {
+    std::vector<void*> allocs;
+    int cap_N = 0;
+    Bf y_bf;                         // [N*K, Cy] the caller's y_hat in bf16 (A operand of g_s.0)
+    Bf gs[3], tok;                   // g_s.0 / .2 / .4 outputs, g_s.6 output [N*K, E]
+    float* emb = nullptr;            // decoder_embed output [N*K, Dd]
+    float* x = nullptr;              // residual stream of the MAE decoder [N*T, Dd], T = L + 1
+    Bf x_bf, qkv, attn, h1, pred;    // pred: decoder_pred output [N*T, p*p*3]
+    float* ln_stats = nullptr;       // [2 * depth + 1][N * T][Dd / 32][2]: norm1 / norm2 of every block, then decoder_norm
+    IoBlock* io = nullptr;           // per-call pointers (y_hat, ids_restore, x_hat)
+};
+
 }  // namespace
 
 struct tmae_handle {
@@ -161,6 +176,11 @@ struct tmae_handle {
     std::map<int, std::unique_ptr<Plan>> dec_plans;   // decode plans by batch size (tmae_decode_begin / _step)
     // decode-from-streams plans by (batch size, y lanes, z lanes); lanes (0, 0) = compressai's format (tmae_decompress_streams)
     std::map<std::tuple<int, int, int>, std::unique_ptr<Plan>> stream_plans;
+    // synthesis (tmae_enable_synthesis): g_s, the MAE decoder and unpatchify on the engine, one plan per batch size
+    int syn_depth = 0, syn_heads = 0;    // 0: synthesis disabled (the decoder-side weights are ignored)
+    int Dd = 0, syn_mlp = 0, syn_out = 0; // decoder width, its MLP width, decoder_pred outputs (p * p * in_chans)
+    SynthWorkspace sws;
+    std::map<int, std::unique_ptr<Plan>> syn_plans;
     CdfTables cdf[2];                // quantised CDF tables: [TMAE_MODEL_GAUSSIAN], [TMAE_MODEL_BOTTLENECK]
     CoderWorkspace cws;
     int dec_N = 0, dec_next = -1;    // decode in progress: batch size and the next group expected (-1 = none)
@@ -296,9 +316,13 @@ bool name_is_needed(const tmae_handle* h, const std::string& n) {
                                      "cc_transform_scale.", "lrp_transform.", "entropy_bottleneck._matrix",
                                      "entropy_bottleneck._bias", "entropy_bottleneck._factor",
                                      "entropy_bottleneck.quantiles"};
+    static const char* decoder_prefixes[] = {"g_s.", "decoder_embed.", "mask_token", "decoder_pos_embed", "decoder_blocks.",
+                                             "decoder_norm.", "decoder_pred."};
     for (const char* p : prefixes)
         if (n.compare(0, strlen(p), p) == 0) return true;
-    (void)h;
+    if (h->syn_depth > 0)                    // synthesis enabled: the decoder side is needed as well
+        for (const char* p : decoder_prefixes)
+            if (n.compare(0, strlen(p), p) == 0) return true;
     return false;
 }
 
@@ -372,6 +396,58 @@ int keep_vec(tmae_handle* h, const std::string& name, size_t numel) {
     CUDA_TRY(h, cudaMemcpyAsync(p, r->ptr, numel * sizeof(float), cudaMemcpyDeviceToDevice, 0));
     h->vecs[name] = p;
     return TMAE_OK;
+}
+
+// Decoder side of the weights (tmae_enable_synthesis), bf16 in every accuracy mode.  g_s.<l> are ConvTranspose2d 1x1 weights
+// [cin, cout, 1, 1]: transposed to [cout, cin] here, then packed like every linear.  The block LayerNorms and decoder_norm are
+// folded into the layers that read them (QKV, fc1, decoder_pred).
+int pack_synthesis(tmae_handle* h) {
+    const int Dd = h->Dd, T = h->L + 1;
+    int rc;
+    const int ch[5] = {h->Cy, h->ga_ch[3], h->ga_ch[2], h->ga_ch[1], h->C};
+    for (int l = 0; l < 4; ++l) {
+        const std::string nm = "g_s." + std::to_string(2 * l);
+        const RawTensor *w = nullptr, *b = nullptr;
+        if ((rc = need_raw(h, nm + ".weight", (size_t)ch[l] * ch[l + 1], &w)) || (rc = need_raw(h, nm + ".bias", (size_t)ch[l + 1], &b))) return rc;
+        if (w->shape.size() != 4 || w->shape[0] != ch[l] || w->shape[1] != ch[l + 1] || w->shape[2] != 1 || w->shape[3] != 1)
+            return fail(h, TMAE_EINVAL, "weight '%s.weight' has the wrong shape (expected ConvTranspose2d [%d, %d, 1, 1])", nm.c_str(), ch[l], ch[l + 1]);
+        std::vector<float> src(w->numel), dst(w->numel), bias(b->numel);
+        CUDA_TRY(h, cudaMemcpy(src.data(), w->ptr, w->numel * sizeof(float), cudaMemcpyDeviceToHost));
+        CUDA_TRY(h, cudaMemcpy(bias.data(), b->ptr, b->numel * sizeof(float), cudaMemcpyDeviceToHost));
+        for (int i = 0; i < ch[l]; ++i)
+            for (int o = 0; o < ch[l + 1]; ++o) dst[(size_t)o * ch[l] + i] = src[(size_t)i * ch[l + 1] + o];
+        RawTensor wt, bt;
+        wt.numel = w->numel; wt.shape = {ch[l + 1], ch[l]};
+        bt.numel = b->numel; bt.shape = {ch[l + 1]};
+        CUDA_TRY(h, cudaMalloc(reinterpret_cast<void**>(&wt.ptr), wt.numel * sizeof(float)));
+        h->raw[nm + ".T.weight"] = wt;          // freed with the other raw tensors at the end of finalize
+        CUDA_TRY(h, cudaMalloc(reinterpret_cast<void**>(&bt.ptr), bt.numel * sizeof(float)));
+        h->raw[nm + ".T.bias"] = bt;
+        CUDA_TRY(h, cudaMemcpy(wt.ptr, dst.data(), wt.numel * sizeof(float), cudaMemcpyHostToDevice));
+        CUDA_TRY(h, cudaMemcpy(bt.ptr, bias.data(), bt.numel * sizeof(float), cudaMemcpyHostToDevice));
+        int sg[1] = {ch[l]};
+        if ((rc = pack_layer(h, nm, nm + ".T", ch[l + 1], ch[l], 1, 1, sg, 0, false))) return rc;
+    }
+    { int sg[1] = {h->C}; if ((rc = pack_layer(h, "decoder_embed", "decoder_embed", Dd, h->C, 1, 1, sg, 0, false))) return rc; }
+    const RawTensor* r = nullptr;
+    if ((rc = need_raw(h, "mask_token", (size_t)Dd, &r))) return rc;
+    if (r->shape.size() != 3 || r->shape[0] != 1 || r->shape[1] != 1)
+        return fail(h, TMAE_EINVAL, "weight 'mask_token' has the wrong shape (expected [1, 1, %d])", Dd);
+    if ((rc = need_raw(h, "decoder_pos_embed", (size_t)T * Dd, &r))) return rc;
+    if (r->shape.size() != 3 || r->shape[0] != 1 || r->shape[1] != T || r->shape[2] != Dd)
+        return fail(h, TMAE_EINVAL, "weight 'decoder_pos_embed' has the wrong shape (expected [1, %d, %d])", T, Dd);
+    if ((rc = keep_vec(h, "mask_token", Dd)) || (rc = keep_vec(h, "decoder_pos_embed", (size_t)T * Dd))) return rc;
+    for (int i = 0; i < h->syn_depth; ++i) {
+        const std::string pre = "decoder_blocks." + std::to_string(i);
+        int sgD[1] = {Dd}, sgM[1] = {h->syn_mlp};
+        if ((rc = pack_layer(h, pre + ".attn.qkv", pre + ".attn.qkv", 3 * Dd, Dd, 1, 1, sgD, 0, false, pre + ".norm1")) ||
+            (rc = pack_layer(h, pre + ".attn.proj", pre + ".attn.proj", Dd, Dd, 1, 1, sgD, 0, false)) ||
+            (rc = pack_layer(h, pre + ".mlp.fc1", pre + ".mlp.fc1", h->syn_mlp, Dd, 1, 1, sgD, 0, false, pre + ".norm2")) ||
+            (rc = pack_layer(h, pre + ".mlp.fc2", pre + ".mlp.fc2", Dd, h->syn_mlp, 1, 1, sgM, 0, false)))
+            return rc;
+    }
+    int sg[1] = {Dd};
+    return pack_layer(h, "decoder_pred", "decoder_pred", h->syn_out, Dd, 1, 1, sg, 0, false, "decoder_norm");
 }
 
 // ---- tensor maps ---------------------------------------------------------------------------------------
@@ -730,6 +806,12 @@ size_t workspace_bytes_estimate(const tmae_handle* h, int N) {
     if (h->precise_rate) b += b / 2;            // second bf16 plane of the activations (upper bound)
     if (h->precise_enc) b += b / 3;
     b += (size_t)N * h->cfg.in_chans * h->cfg.img_size * h->cfg.img_size * 4 + (size_t)N * h->L * 4;
+    if (h->syn_depth > 0) {          // synthesis buffers (ensure_synth_workspace)
+        const size_t sk = (size_t)N * h->K, st = (size_t)N * (h->L + 1), Dd = h->Dd;
+        b += sk * (h->Cy + h->ga_ch[3] + h->ga_ch[2] + h->ga_ch[1] + h->C) * 2 + sk * Dd * 4;
+        b += st * Dd * (4 + 2 + 3 * 2 + 2) + st * h->syn_mlp * 2 + st * h->syn_out * 2;
+        b += (size_t)(2 * h->syn_depth + 1) * st * (Dd / 32) * 8;
+    }
     return b;
 }
 
@@ -1026,6 +1108,85 @@ int finish_plan(tmae_handle* h, Plan& pl) {
     return TMAE_OK;
 }
 
+// Pre-norm ViT blocks (timm 0.4.5 Block, eval): QKV -> attention -> proj (+ residual) -> fc1 (GELU) -> fc2 (+ residual) over
+// the fp32 residual stream `x`.  The encoder (build_plan) and the MAE decoder of the synthesis plan (build_synth_plan) use it.
+struct BlockSet {
+    const char* prefix = nullptr;    // weight names "<prefix>.<i>.attn.qkv" ...
+    const char* tag = nullptr;       // step tags "<tag><i>.qkv" ...
+    int depth = 0, C = 0, mlp = 0, T = 0, N = 0;
+    bool fold = false;               // LayerNorm fold: proj / fc2 emit row statistics + a bf16 copy of x, QKV / fc1 apply them
+    bool stats_in = false;           // fold: the statistics for block 0's norm1 arrive with the input rows (else a LayerNorm kernel)
+    bool stats_out = false;          // fold: the last fc2 emits statistics as well (slot 2 * depth), for a LayerNorm folded after the blocks
+    StepKind attn = ST_ATTN;
+    float* x = nullptr;
+    Bf xn, x_bf, qkv, attn_out, h1;
+    float* ln_stats = nullptr;       // [2 * depth (+ 1)][N * T][C / 32][2]
+};
+
+int add_blocks(tmae_handle* h, Plan& pl, const BlockSet& b) {
+    const int C = b.C, T = b.T, N = b.N;
+    const long long rt = (long long)N * T;
+    char tag[96];
+    int rc;
+    if (!b.fold && b.x != h->ws.x) return fail(h, TMAE_EINVAL, "%s: LayerNorm kernels run on the encoder's buffers only", b.prefix);
+    for (int i = 0; i < b.depth; ++i) {
+        const std::string pre = std::string(b.prefix) + "." + std::to_string(i);
+        // LayerNorm fold: in the encoder, norm1 of block 0 follows the patch embed + cls rows and stays a kernel; every other
+        // block LayerNorm lives in the GEMMs around it - proj / fc2 emit row statistics + a bf16 copy of x, QKV / fc1 apply them
+        const bool fold1 = b.fold && (i > 0 || b.stats_in), fold2 = b.fold;
+        const size_t stat_stride = (size_t)rt * (C / 32) * 2;
+        float* stats1 = b.ln_stats + (size_t)(2 * i) * stat_stride;          // statistics of x entering norm1 / norm2 of block i
+        float* stats2 = b.ln_stats + (size_t)(2 * i + 1) * stat_stride;
+        if (!fold1) {
+            Step ln; ln.kind = ST_LN; ln.family = FAM_LN; ln.ln_gamma = h->vecs[pre + ".norm1.weight"]; ln.ln_beta = h->vecs[pre + ".norm1.bias"]; ln.tag = pre + ".norm1";
+            pl.steps.push_back(ln);
+        }
+        GemmDesc d;
+        d.layer = get_layer(h, pre + ".attn.qkv");
+        d.seg[0] = fold1 ? seg(b.x_bf, C, C) : seg(b.xn, C, C); d.a_rows = rt; d.M = (int)rt;
+        if (fold1) d.ln_stats_in = stats1;
+        d.out0 = outspec(b.qkv, 3 * C, MAP_SAME);
+        d.flops = 2.0 * rt * C * 3.0 * C;
+        snprintf(tag, sizeof(tag), "%s%d.qkv", b.tag, i);
+        rc = add_gemm_group(h, pl, &d, 1, tag); if (rc) return rc;
+        Step at; at.kind = b.attn; at.family = FAM_ATTN; at.flops = 4.0 * (double)N * T * T * C; at.tag = pre + ".attn";
+        pl.steps.push_back(at);
+        GemmDesc p2;
+        p2.layer = get_layer(h, pre + ".attn.proj");
+        p2.seg[0] = seg(b.attn_out, C, C); p2.a_rows = rt; p2.M = (int)rt;
+        p2.resid = b.x; p2.resid_ld = C; p2.resid_map = MAP_SAME;
+        p2.out0 = outspec(b.x, C, OUT_F32, MAP_SAME);
+        if (fold2) { p2.ln_stats_out = stats2; p2.xbf_out = b.x_bf.p; }
+        p2.flops = 2.0 * rt * C * (double)C;
+        snprintf(tag, sizeof(tag), "%s%d.proj", b.tag, i);
+        rc = add_gemm_group(h, pl, &p2, 1, tag); if (rc) return rc;
+        if (!fold2) {
+            Step ln2; ln2.kind = ST_LN; ln2.family = FAM_LN; ln2.ln_gamma = h->vecs[pre + ".norm2.weight"]; ln2.ln_beta = h->vecs[pre + ".norm2.bias"]; ln2.tag = pre + ".norm2";
+            pl.steps.push_back(ln2);
+        }
+        GemmDesc f1;
+        f1.layer = get_layer(h, pre + ".mlp.fc1");
+        f1.seg[0] = fold2 ? seg(b.x_bf, C, C) : seg(b.xn, C, C); f1.a_rows = rt; f1.M = (int)rt; f1.act = ACT_GELU;
+        if (fold2) f1.ln_stats_in = stats2;
+        f1.out0 = outspec(b.h1, b.mlp, MAP_SAME);
+        f1.flops = 2.0 * rt * C * (double)b.mlp;
+        snprintf(tag, sizeof(tag), "%s%d.fc1", b.tag, i);
+        rc = add_gemm_group(h, pl, &f1, 1, tag); if (rc) return rc;
+        GemmDesc f2;
+        f2.layer = get_layer(h, pre + ".mlp.fc2");
+        f2.seg[0] = seg(b.h1, b.mlp, b.mlp); f2.a_rows = rt; f2.M = (int)rt;
+        f2.resid = b.x; f2.resid_ld = C; f2.resid_map = MAP_SAME;
+        f2.out0 = outspec(b.x, C, OUT_F32, MAP_SAME);
+        if (b.fold && (i + 1 < b.depth || b.stats_out)) {                    // statistics for norm1 of the next block
+            f2.ln_stats_out = b.ln_stats + (size_t)(2 * i + 2) * stat_stride; f2.xbf_out = b.x_bf.p;
+        }
+        f2.flops = 2.0 * rt * C * (double)b.mlp;
+        snprintf(tag, sizeof(tag), "%s%d.fc2", b.tag, i);
+        rc = add_gemm_group(h, pl, &f2, 1, tag); if (rc) return rc;
+    }
+    return TMAE_OK;
+}
+
 // forced = slice-wise teacher forcing (tmae_forward_from_latent_forced): after lrp_transform[i] the support columns of
 // slice i are overwritten with the caller's y_hat, so slice j > i never sees a symbol this run decided itself.
 int build_plan(tmae_handle* h, int N, Plan** out, bool forced = false) {
@@ -1063,60 +1224,13 @@ int build_plan(tmae_handle* h, int N, Plan** out, bool forced = false) {
         rc = add_gemm_group(h, pl, &d, 1, "patch_embed");
         if (rc) return rc;
     }
-    for (int i = 0; i < h->cfg.encoder_depth; ++i) {
-        const std::string pre = "encoder_blocks." + std::to_string(i);
-        // LayerNorm fold (bf16 encoder): norm1 of block 0 follows the patch embed + cls rows and stays a kernel; every other
-        // block LayerNorm lives in the GEMMs around it - proj / fc2 emit row statistics + a bf16 copy of x, QKV / fc1 apply them
-        const bool fold1 = h->ln_fold && i > 0, fold2 = h->ln_fold;
-        const size_t stat_stride = (size_t)rt * (C / 32) * 2;
-        float* stats1 = w.ln_stats + (size_t)(2 * i) * stat_stride;          // statistics of x entering norm1 / norm2 of block i
-        float* stats2 = w.ln_stats + (size_t)(2 * i + 1) * stat_stride;
-        if (!fold1) {
-            Step ln; ln.kind = ST_LN; ln.family = FAM_LN; ln.ln_gamma = h->vecs[pre + ".norm1.weight"]; ln.ln_beta = h->vecs[pre + ".norm1.bias"]; ln.tag = pre + ".norm1";
-            pl.steps.push_back(ln);
-        }
-        GemmDesc d;
-        d.layer = get_layer(h, pre + ".attn.qkv");
-        d.seg[0] = fold1 ? seg(w.x_bf, C, C) : seg(w.xn, C, C); d.a_rows = rt; d.M = (int)rt;
-        if (fold1) d.ln_stats_in = stats1;
-        d.out0 = outspec(w.qkv, 3 * C, MAP_SAME);
-        d.flops = 2.0 * rt * C * 3.0 * C;
-        snprintf(tag, sizeof(tag), "blk%d.qkv", i);
-        rc = add_gemm_group(h, pl, &d, 1, tag); if (rc) return rc;
-        Step at; at.kind = ST_ATTN; at.family = FAM_ATTN; at.flops = 4.0 * (double)N * T * T * C; at.tag = pre + ".attn";
-        pl.steps.push_back(at);
-        GemmDesc p2;
-        p2.layer = get_layer(h, pre + ".attn.proj");
-        p2.seg[0] = seg(w.attn, C, C); p2.a_rows = rt; p2.M = (int)rt;
-        p2.resid = w.x; p2.resid_ld = C; p2.resid_map = MAP_SAME;
-        p2.out0 = outspec(w.x, C, OUT_F32, MAP_SAME);
-        if (fold2) { p2.ln_stats_out = stats2; p2.xbf_out = w.x_bf.p; }
-        p2.flops = 2.0 * rt * C * (double)C;
-        snprintf(tag, sizeof(tag), "blk%d.proj", i);
-        rc = add_gemm_group(h, pl, &p2, 1, tag); if (rc) return rc;
-        if (!fold2) {
-            Step ln2; ln2.kind = ST_LN; ln2.family = FAM_LN; ln2.ln_gamma = h->vecs[pre + ".norm2.weight"]; ln2.ln_beta = h->vecs[pre + ".norm2.bias"]; ln2.tag = pre + ".norm2";
-            pl.steps.push_back(ln2);
-        }
-        GemmDesc f1;
-        f1.layer = get_layer(h, pre + ".mlp.fc1");
-        f1.seg[0] = fold2 ? seg(w.x_bf, C, C) : seg(w.xn, C, C); f1.a_rows = rt; f1.M = (int)rt; f1.act = ACT_GELU;
-        if (fold2) f1.ln_stats_in = stats2;
-        f1.out0 = outspec(w.h1, h->mlp, MAP_SAME);
-        f1.flops = 2.0 * rt * C * (double)h->mlp;
-        snprintf(tag, sizeof(tag), "blk%d.fc1", i);
-        rc = add_gemm_group(h, pl, &f1, 1, tag); if (rc) return rc;
-        GemmDesc f2;
-        f2.layer = get_layer(h, pre + ".mlp.fc2");
-        f2.seg[0] = seg(w.h1, h->mlp, h->mlp); f2.a_rows = rt; f2.M = (int)rt;
-        f2.resid = w.x; f2.resid_ld = C; f2.resid_map = MAP_SAME;
-        f2.out0 = outspec(w.x, C, OUT_F32, MAP_SAME);
-        if (h->ln_fold && i + 1 < h->cfg.encoder_depth) {                    // statistics for norm1 of the next block
-            f2.ln_stats_out = w.ln_stats + (size_t)(2 * i + 2) * stat_stride; f2.xbf_out = w.x_bf.p;
-        }
-        f2.flops = 2.0 * rt * C * (double)h->mlp;
-        snprintf(tag, sizeof(tag), "blk%d.fc2", i);
-        rc = add_gemm_group(h, pl, &f2, 1, tag); if (rc) return rc;
+    {
+        BlockSet b;
+        b.prefix = "encoder_blocks"; b.tag = "blk";
+        b.depth = h->cfg.encoder_depth; b.C = C; b.mlp = h->mlp; b.T = T; b.N = N;
+        b.fold = h->ln_fold; b.attn = ST_ATTN;
+        b.x = w.x; b.xn = w.xn; b.x_bf = w.x_bf; b.qkv = w.qkv; b.attn_out = w.attn; b.h1 = w.h1; b.ln_stats = w.ln_stats;
+        if ((rc = add_blocks(h, pl, b))) return rc;
     }
     {
         Step ln; ln.kind = ST_LN; ln.family = FAM_LN; ln.ln_gamma = h->vecs["encoder_norm.weight"]; ln.ln_beta = h->vecs["encoder_norm.bias"]; ln.ln_final = 1; ln.tag = "encoder_norm";
@@ -1302,6 +1416,102 @@ int build_stream_decode_plan(tmae_handle* h, int N, int lanes_y, int lanes_z, Pl
     return TMAE_OK;
 }
 
+int ensure_synth_workspace(tmae_handle* h, int N) {
+    SynthWorkspace& w = h->sws;
+    if (N <= w.cap_N) return TMAE_OK;
+    drop_plans(h->syn_plans);        // they hold pointers into these buffers
+    free_pool(w.allocs);
+    w = SynthWorkspace();
+    const size_t rk = (size_t)N * h->K, rt = (size_t)N * (h->L + 1), Dd = h->Dd;
+    int rc;
+    auto bf = [&](Bf& b, size_t count) { return dev_alloc(h, w.allocs, &b.p, (count + 63) / 64 * 64); };
+    if ((rc = bf(w.y_bf, rk * h->Cy)) || (rc = bf(w.gs[0], rk * h->ga_ch[3])) || (rc = bf(w.gs[1], rk * h->ga_ch[2])) ||
+        (rc = bf(w.gs[2], rk * h->ga_ch[1])) || (rc = bf(w.tok, rk * h->C)) || (rc = dev_alloc(h, w.allocs, &w.emb, rk * Dd)) ||
+        (rc = dev_alloc(h, w.allocs, &w.x, rt * Dd)) || (rc = bf(w.x_bf, rt * Dd)) || (rc = bf(w.qkv, rt * 3 * Dd)) ||
+        (rc = bf(w.attn, rt * Dd)) || (rc = bf(w.h1, rt * h->syn_mlp)) || (rc = bf(w.pred, rt * h->syn_out)) ||
+        (rc = dev_alloc(h, w.allocs, &w.ln_stats, (size_t)(2 * h->syn_depth + 1) * rt * (Dd / 32) * 2)) ||
+        (rc = dev_alloc(h, w.allocs, &w.io, (size_t)1)))
+        return rc;
+    w.cap_N = N;
+    return TMAE_OK;
+}
+
+// Synthesis plan (recon.synthesize, MCM.py:789-792 and 636-688, on the engine): x_hat from y_hat and ids_restore.  bf16 operands,
+// fp32 accumulation, fp32 residual stream / LayerNorm statistics / softmax, in every accuracy mode (the precise flags govern the
+// rate path; no symbol depends on x_hat).  Every LayerNorm is folded: block 0's norm1 into its QKV with the statistics the
+// unshuffle writes, decoder_norm into decoder_pred with the statistics of the last fc2.  One stage: one CUDA graph per N.
+int build_synth_plan(tmae_handle* h, int N, Plan** out) {
+    auto it = h->syn_plans.find(N);
+    if (it != h->syn_plans.end()) { *out = it->second.get(); return TMAE_OK; }
+    int rc = ensure_synth_workspace(h, N);
+    if (rc) return rc;
+    std::unique_ptr<Plan> plp(new Plan());
+    Plan& pl = *plp;
+    pl.N = N;
+    SynthWorkspace& w = h->sws;
+    const int Dd = h->Dd, T = h->L + 1, Cy = h->Cy;
+    const long long rk = (long long)N * h->K, rt = (long long)N * T;
+    auto simple = [&](StepKind k, int fam, const char* t) { Step st; st.kind = k; st.family = fam; st.tag = t; pl.steps.push_back(st); };
+    simple(ST_SYN_IN, FAM_MISC, "synth_input");
+    {   // g_s: four 1x1 ConvTranspose2d == per-token linears, GELU after the first three (MCM.py:96-112, 790)
+        const int ch[5] = {Cy, h->ga_ch[3], h->ga_ch[2], h->ga_ch[1], h->C};
+        const Bf srcs[4] = {w.y_bf, w.gs[0], w.gs[1], w.gs[2]}, dsts[4] = {w.gs[0], w.gs[1], w.gs[2], w.tok};
+        char tag[32];
+        for (int l = 0; l < 4; ++l) {
+            GemmDesc d;
+            d.layer = get_layer(h, "g_s." + std::to_string(2 * l));
+            d.seg[0] = seg(srcs[l], ch[l], ch[l]); d.a_rows = rk; d.M = (int)rk;
+            d.act = l < 3 ? ACT_GELU : ACT_NONE;
+            d.out0 = outspec(dsts[l], ch[l + 1], MAP_SAME);
+            d.flops = 2.0 * rk * ch[l] * (double)ch[l + 1];
+            snprintf(tag, sizeof(tag), "g_s.%d", 2 * l);
+            if ((rc = add_gemm_group(h, pl, &d, 1, tag))) return rc;
+        }
+    }
+    {   // decoder_embed (MCM.py:638), fp32 out: the unshuffle builds the residual stream from it
+        GemmDesc d;
+        d.layer = get_layer(h, "decoder_embed");
+        d.seg[0] = seg(w.tok, h->C, h->C); d.a_rows = rk; d.M = (int)rk;
+        d.out0 = outspec(w.emb, Dd, OUT_F32, MAP_SAME);
+        d.flops = 2.0 * rk * h->C * (double)Dd;
+        if ((rc = add_gemm_group(h, pl, &d, 1, "decoder_embed"))) return rc;
+    }
+    simple(ST_UNSHUF, FAM_GATHER, "unshuffle");
+    {
+        BlockSet b;
+        b.prefix = "decoder_blocks"; b.tag = "dec_blk";
+        b.depth = h->syn_depth; b.C = Dd; b.mlp = h->syn_mlp; b.T = T; b.N = N;
+        b.fold = true; b.stats_in = true; b.stats_out = true; b.attn = ST_ATTN32;
+        b.x = w.x; b.x_bf = w.x_bf; b.qkv = w.qkv; b.attn_out = w.attn; b.h1 = w.h1; b.ln_stats = w.ln_stats;
+        if ((rc = add_blocks(h, pl, b))) return rc;
+    }
+    {   // decoder_norm folded into decoder_pred (MCM.py:684-686); every row, row 0 is dropped by the unpatchify
+        GemmDesc d;
+        d.layer = get_layer(h, "decoder_pred");
+        d.seg[0] = seg(w.x_bf, Dd, Dd); d.a_rows = rt; d.M = (int)rt;
+        d.ln_stats_in = w.ln_stats + (size_t)(2 * h->syn_depth) * rt * (Dd / 32) * 2;
+        d.out0 = outspec(w.pred, h->syn_out, MAP_SAME);
+        d.flops = 2.0 * rt * Dd * (double)h->syn_out;
+        if ((rc = add_gemm_group(h, pl, &d, 1, "decoder_pred"))) return rc;
+    }
+    simple(ST_UNPATCH, FAM_MISC, "unpatchify");
+    for (Step& st : pl.steps) {      // algorithmic HBM bytes of the elementwise steps
+        switch (st.kind) {
+            case ST_SYN_IN: st.bytes = (double)rk * Cy * (4 + 2); break;
+            case ST_UNSHUF: st.bytes = (double)rt * Dd * (4 + 4 + 2) + (double)rt * (Dd / 32) * 8 + (double)N * h->L * 8; break;
+            case ST_UNPATCH: st.bytes = (double)N * h->L * h->syn_out * (2 + 4); break;
+            default: break;
+        }
+    }
+    pl.stage_begin = {0, (int)pl.steps.size()};
+    pl.stage_graph.assign(1, nullptr);
+    pl.stage_calls.assign(1, 0);
+    if ((rc = finish_plan(h, pl))) return rc;
+    *out = plp.get();
+    h->syn_plans[N] = std::move(plp);
+    return TMAE_OK;
+}
+
 // ---- execution -----------------------------------------------------------------------------------------
 struct RunArgs {
     const float* imgs = nullptr;
@@ -1448,6 +1658,19 @@ int run_steps(tmae_handle* h, Plan& pl, const RunArgs& a, cudaStream_t st) {
                 CUDA_TRY(h, launch_rans_decode(d, st));
                 break;
             }
+            case ST_SYN_IN:
+                CUDA_TRY(h, launch_synth_input(h->sws.y_bf.p, (long long)N * K * h->Cy, st, a.io));
+                break;
+            case ST_UNSHUF:
+                CUDA_TRY(h, launch_synth_unshuffle(h->sws.emb, h->vecs["mask_token"], h->vecs["decoder_pos_embed"], h->sws.x, h->sws.x_bf.p,
+                                                   h->sws.ln_stats, N, K, h->L, h->Dd, st, a.io));
+                break;
+            case ST_ATTN32:
+                CUDA_TRY(h, launch_attention_hd32(h->sws.qkv.p, h->sws.attn.p, N, h->L + 1, h->syn_heads, 1.0f / sqrtf(32.0f), st));
+                break;
+            case ST_UNPATCH:
+                CUDA_TRY(h, launch_synth_unpatchify(h->sws.pred.p, N, h->cfg.patch_size, h->grid_w, st, a.io));
+                break;
             case ST_YDEC: {
                 const CdfTables& t = h->cdf[TMAE_MODEL_GAUSSIAN];
                 const int per_slice = h->sc * K;
@@ -1535,11 +1758,12 @@ IoBlock decode_io(const int32_t* z_symbols, const int32_t* y_symbols, const tmae
     return hio;
 }
 
-int run_decode_stage(tmae_handle* h, Plan& pl, int stage, const IoBlock& hio, cudaStream_t st) {
-    Workspace& w = h->ws;
-    CUDA_TRY(h, cudaMemcpyAsync(w.io, &hio, sizeof(hio), cudaMemcpyHostToDevice, st));   // pageable source: staged before return
+// dev_io: the device IoBlock the stage reads (default: the workspace's; synthesis plans have their own)
+int run_decode_stage(tmae_handle* h, Plan& pl, int stage, const IoBlock& hio, cudaStream_t st, IoBlock* dev_io = nullptr) {
+    IoBlock* io = dev_io ? dev_io : h->ws.io;
+    CUDA_TRY(h, cudaMemcpyAsync(io, &hio, sizeof(hio), cudaMemcpyHostToDevice, st));   // pageable source: staged before return
     RunArgs a;
-    a.begin = pl.stage_begin[stage]; a.end = pl.stage_begin[stage + 1]; a.io = w.io;
+    a.begin = pl.stage_begin[stage]; a.end = pl.stage_begin[stage + 1]; a.io = io;
     if (!h->use_graph || h->profiling || pl.stage_calls[stage]++ == 0) return run_steps(h, pl, a, st);
     if (!pl.stage_graph[stage]) {
         if (!h->cap_stream) CUDA_TRY(h, cudaStreamCreateWithFlags(&h->cap_stream, cudaStreamNonBlocking));
@@ -1625,8 +1849,10 @@ void tmae_destroy(tmae_handle* h) {
     drop_plans(h->plans);
     drop_plans(h->dec_plans);
     drop_plans(h->stream_plans);
+    drop_plans(h->syn_plans);
     for (CdfTables& t : h->cdf) rans_free_tables(&t);
     free_pool(h->cws.allocs);
+    free_pool(h->sws.allocs);
     if (h->cws.enc) cudaFree(h->cws.enc);
     if (h->cap_stream) cudaStreamDestroy(h->cap_stream);
     if (h->scale_table) cudaFree(h->scale_table);
@@ -1664,6 +1890,7 @@ int tmae_finalize_weights(tmae_handle* h) {
     drop_plans(h->plans);
     drop_plans(h->dec_plans);
     drop_plans(h->stream_plans);
+    drop_plans(h->syn_plans);
     h->dec_next = -1;
     free_pool(h->weight_allocs);
     h->layers.clear();
@@ -1768,6 +1995,7 @@ int tmae_finalize_weights(tmae_handle* h) {
         if ((rc = dev_alloc(h, h->weight_allocs, &h->eb_tab, (size_t)Cz * 64))) return rc;
         CUDA_TRY(h, launch_eb_table(ptrs, h->eb_tab, Cz, 0));
     }
+    if (h->syn_depth > 0 && (rc = pack_synthesis(h))) return rc;
     CUDA_TRY(h, cudaDeviceSynchronize());
     for (auto& kv : h->raw) cudaFree(kv.second.ptr);
     h->raw.clear();
@@ -1978,6 +2206,56 @@ int tmae_decode_step(tmae_handle* h, int group, const int32_t* y_symbols, const 
     if (rc) return rc;
     if (group + 2 < (int)pl.stage_begin.size() - 1) h->dec_next = group + 1;
     return TMAE_OK;
+}
+
+// ---- synthesis (recon.synthesize on the engine) ---------------------------------------------------------
+int tmae_enable_synthesis(tmae_handle* h, int decoder_depth, int decoder_num_heads) {
+    if (!h) return TMAE_EINVAL;
+    const int Dd = h->cfg.decoder_embed_dim;
+    if (decoder_depth < 1) return fail(h, TMAE_EINVAL, "decoder_depth must be >= 1 (got %d)", decoder_depth);
+    if (decoder_num_heads < 1 || Dd % decoder_num_heads != 0)
+        return fail(h, TMAE_EINVAL, "decoder_num_heads %d does not divide decoder_embed_dim %d", decoder_num_heads, Dd);
+    if (Dd / decoder_num_heads != 32)
+        return fail(h, TMAE_EINVAL, "synthesis supports a decoder head dim of 32 only (decoder_embed_dim %d / %d heads = %d)", Dd,
+                    decoder_num_heads, Dd / decoder_num_heads);
+    if ((h->cfg.flags & TMAE_FLAG_DEBUG_SIMT) || getenv("TMAE_NO_TMA_STORE"))
+        return fail(h, TMAE_EINVAL, "synthesis folds its LayerNorms into the TMA-store phase of the tensor-core GEMMs: not available with "
+                    "TMAE_FLAG_DEBUG_SIMT or TMAE_NO_TMA_STORE");
+    const int mlp = (int)(Dd * h->cfg.mlp_ratio);
+    if (mlp <= 0 || mlp % 32 != 0) return fail(h, TMAE_EINVAL, "decoder MLP width %d must be a positive multiple of 32", mlp);
+    if (!attention_hd32_supported(h->L + 1))
+        return fail(h, TMAE_EINVAL, "synthesis attention over %d tokens does not fit shared memory", h->L + 1);
+    h->dec_next = -1;
+    drop_plans(h->syn_plans);
+    if (decoder_depth != h->syn_depth || Dd != h->Dd || mlp != h->syn_mlp) {   // buffers sized for another decoder
+        free_pool(h->sws.allocs);
+        h->sws = SynthWorkspace();
+    }
+    h->syn_depth = decoder_depth;
+    h->syn_heads = decoder_num_heads;
+    h->Dd = Dd;
+    h->syn_mlp = mlp;
+    h->syn_out = h->cfg.patch_size * h->cfg.patch_size * h->cfg.in_chans;
+    h->finalized = false;            // the decoder-side tensors must be packed
+    return TMAE_OK;
+}
+
+int tmae_synthesize(tmae_handle* h, const float* y_hat, const int64_t* ids_restore, int N, float* x_hat, void* stream) {
+    if (!h) return TMAE_EINVAL;
+    if (h->syn_depth == 0) { h->dec_next = -1; return fail(h, TMAE_ESTATE, "synthesis is not enabled (call tmae_enable_synthesis)"); }
+    int rc = check_ready(h, N);
+    if (rc) return rc;
+    if (!y_hat || !ids_restore || !x_hat) return fail(h, TMAE_EINVAL, "y_hat, ids_restore and x_hat must not be null");
+    if (((reinterpret_cast<uintptr_t>(y_hat) | reinterpret_cast<uintptr_t>(x_hat)) & 15) != 0)
+        return fail(h, TMAE_EINVAL, "y_hat and x_hat must be 16-byte aligned");
+    if (h->cfg.in_chans != 3) return fail(h, TMAE_EINVAL, "synthesis writes 3-channel images (in_chans %d)", h->cfg.in_chans);
+    Plan* pl = nullptr;
+    if ((rc = build_synth_plan(h, N, &pl))) return rc;
+    IoBlock hio;
+    memset(&hio, 0, sizeof(hio));
+    hio.syn_y_hat = y_hat; hio.syn_ids = ids_restore; hio.syn_x_hat = x_hat;
+    if (h->profiling) h->prof_used = 0;
+    return run_decode_stage(h, *pl, 0, hio, reinterpret_cast<cudaStream_t>(stream), h->sws.io);
 }
 
 // ---- entropy coder (compressai's rANS format) -----------------------------------------------------------
@@ -2491,6 +2769,19 @@ int tmae_attention_bf16(const void* qkv, void* out, int N, int T, int H, int imp
     } else {
         e = launch_attention(reinterpret_cast<const __nv_bfloat16*>(qkv), reinterpret_cast<__nv_bfloat16*>(out), N, T, H, C, 0.125f, st);
     }
+    cudaError_t e2 = cudaStreamSynchronize(st);
+    if (e != cudaSuccess || e2 != cudaSuccess) return fail(nullptr, TMAE_ECUDA, "attention launch: %s / %s", cudaGetErrorString(e), cudaGetErrorString(e2));
+    return TMAE_OK;
+}
+
+// softmax(q k^T / sqrt(32)) v for qkv bf16 [N*T, 3*H*32] (columns [3][H][32]) -> out bf16 [N*T, H*32]: the attention kernel of the
+// synthesis plan's decoder blocks stand-alone.
+int tmae_attention_hd32_bf16(const void* qkv, void* out, int N, int T, int H, void* stream) {
+    if (!qkv || !out || N <= 0 || T <= 0 || H <= 0) return fail(nullptr, TMAE_EINVAL, "tmae_attention_hd32_bf16: invalid argument");
+    if (!attention_hd32_supported(T)) return fail(nullptr, TMAE_EINVAL, "tmae_attention_hd32_bf16: T = %d does not fit shared memory", T);
+    cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+    cudaError_t e = launch_attention_hd32(reinterpret_cast<const __nv_bfloat16*>(qkv), reinterpret_cast<__nv_bfloat16*>(out), N, T, H,
+                                          1.0f / sqrtf(32.0f), st);
     cudaError_t e2 = cudaStreamSynchronize(st);
     if (e != cudaSuccess || e2 != cudaSuccess) return fail(nullptr, TMAE_ECUDA, "attention launch: %s / %s", cudaGetErrorString(e), cudaGetErrorString(e2));
     return TMAE_OK;

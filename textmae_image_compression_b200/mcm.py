@@ -26,6 +26,14 @@ compressai-format byte strings and back.
 `decompress_symbols` is the decoder side of `MCM.decompress` (MCM.py:896-968) around the range decoder: symbols in (all at
 once, or group by group through a callback that receives the scale-table indexes), y_hat / z_hat / x_hat out, bit-exact
 with the encoder of the same accuracy mode.
+
+x_hat (g_s + MAE decoder + unpatchify) comes from one of two paths:
+    native_synthesis=False (default): recon.synthesize, stock fp32 PyTorch - the reference arithmetic that the conformance
+                    mode (`precise=`) and the parity tests rely on;
+    native_synthesis=True: `tmae_synthesize` on the engine (bf16 operands, fp32 accumulation, residual stream, LayerNorm
+                    statistics and softmax; one CUDA graph per batch size) on the call's stream, for forward(need_recon),
+                    decompress_symbols and decompress_bitstream.  The same accuracy-for-throughput choice `precise` offers for
+                    the rate path; it needs a decoder head dim of 32 (the reference's 512 / 16).
 """
 from __future__ import annotations
 
@@ -55,7 +63,7 @@ class MCM(nn.Module):
                  norm_layer=None, norm_pix_loss=False, latent_depth=384, hyperprior_depth=192, num_slices=12,
                  num_keep_patches=144, *, skip_dead_lrp: bool = False, debug_simt: bool = False,
                  softmax_isa: Optional[int] = None, extra_outputs: bool = False, share_sm: bool = False,
-                 precise: Optional[str] = None):
+                 precise: Optional[str] = None, native_synthesis: bool = False):
         super().__init__()
         self.cfg = PathConfig(img_size=img_size, patch_size=patch_size, in_chans=in_chans,
                               encoder_embed_dim=encoder_embed_dim, encoder_depth=encoder_depth,
@@ -76,6 +84,8 @@ class MCM(nn.Module):
         if precise not in (None, "rate", "all", "rate-x6", "all-x6"):
             raise ValueError("precise must be None, 'rate', 'all', 'rate-x6' or 'all-x6'")
         self.precise = precise
+        self.native_synthesis = native_synthesis  # x_hat on the engine (tmae_synthesize) instead of recon.synthesize
+        self._syn_on = False                     # the handle has synthesis enabled (native_synthesis and decoder weights)
         if softmax_isa is None:
             # lane order of the ATen CPU softmax the reference's host routine would have used on this machine
             softmax_isa = 16 if "AVX512" in torch.backends.cpu.get_cpu_capability().upper() else 8
@@ -163,18 +173,22 @@ class MCM(nn.Module):
             _native.check(lib.tmae_create(C.byref(cfg), C.byref(hp)), None, RuntimeError)
             self._handle = hp
             self._handle_device = dev
+            syn = self.native_synthesis and recon.has_decoder_weights(self._weights)
+            if syn:
+                _native.check(lib.tmae_enable_synthesis(hp, c.decoder_depth, c.decoder_num_heads), hp)
             ign = C.c_int(0)
             for name, t in self._weights.items():
                 if not t.is_floating_point():
                     continue
-                if not _native_needs(name):           # decoder-side tensors stay with recon.py (stock PyTorch)
-                    continue
+                if not (_native_needs(name) or (syn and name.startswith(recon.DECODER_PREFIXES))):
+                    continue                          # decoder-side tensors stay with recon.py unless synthesis is native
                 t = t.float().contiguous()            # .half() / .bfloat16() modules: the ABI takes fp32 (dtype 0)
                 shape = (C.c_int64 * max(t.dim(), 1))(*t.shape)
                 _native.check(lib.tmae_set_weight(hp, name.encode(), C.c_void_p(t.data_ptr()), 0, t.dim(), shape,
                                                   C.byref(ign)), hp)
             _native.check(lib.tmae_finalize_weights(hp), hp, RuntimeError)
         self._dirty = False
+        self._syn_on = syn
         self._scale_table_dirty = True           # a fresh handle has no scale table yet
         self._cdf_dirty = True                   # ... nor cdf tables
         self._last_stream = None
@@ -284,8 +298,8 @@ class MCM(nn.Module):
     @torch.no_grad()
     def forward(self, imgs: torch.Tensor, total_scores: torch.Tensor, need_recon: Optional[bool] = None):
         """MCM.forward (MCM.py:714-803).  The rate half runs in the library; with `need_recon` (default: whenever the
-        decoder-side weights are loaded) the reconstruction half follows in stock PyTorch and the dict also carries
-        the reference's "loss" 3-tuple and "x_hat"."""
+        decoder-side weights are loaded) the reconstruction half follows - x_hat in stock PyTorch, or on the engine with
+        native_synthesis=True - and the dict also carries the reference's "loss" 3-tuple and "x_hat"."""
         if need_recon is None:
             need_recon = recon.has_decoder_weights(self._weights)
         if need_recon and not recon.has_decoder_weights(self._weights):
@@ -304,10 +318,42 @@ class MCM(nn.Module):
     def _add_recon(self, out, t, imgs):
         c = self.cfg
         N = imgs.shape[0]
+        if self._syn_on:
+            with torch.cuda.device(self._handle_device):
+                cur = self._enter_stream(self._handle_device)
+                x_hat = self._synthesize(t["y_hat"], t["ids_restore"], cur)
+                self._leave_stream(cur)
+            out["loss"] = recon.forward_loss(imgs, x_hat, self.feature_loss)
+            out["x_hat"] = x_hat
+            return
         y_hat_tokens = t["y_hat"].reshape(N, c.num_keep_patches, c.latent_depth)      # NHWC == token matrix
         loss, x_hat = recon.reconstruct(self._weights, c, y_hat_tokens, t["ids_restore"], imgs, self.feature_loss)
         out["loss"] = loss
         out["x_hat"] = x_hat
+
+    def _synthesize(self, y_hat, ids_restore, cur):
+        """x_hat f32 [N,3,S,S] from channels-last y_hat [N,s,s,Cy] and ids_restore [N,L] on the engine (tmae_synthesize),
+        enqueued on `cur` (inside the handle's device context)."""
+        c = self.cfg
+        N = y_hat.shape[0]
+        ids = ids_restore.to(device=self._handle_device, dtype=torch.int64).contiguous()
+        x_hat = torch.empty((N, c.in_chans, c.img_size, c.img_size), dtype=torch.float32, device=self._handle_device)
+        _native.check(_native.load().tmae_synthesize(self._handle, C.c_void_p(y_hat.data_ptr()), C.c_void_p(ids.data_ptr()), N,
+                                                     C.c_void_p(x_hat.data_ptr()), C.c_void_p(cur.cuda_stream)),
+                      self._handle, RuntimeError)
+        return x_hat
+
+    def _ids_not_permutation(self, ids_restore):
+        """Device bool [N]: rows of ids_restore that are not a permutation of 0..L-1 (no host synchronisation)."""
+        L = self.cfg.num_patches
+        ids = ids_restore.to(device=self._handle_device, dtype=torch.int64)
+        return (ids.sort(dim=1).values != torch.arange(L, device=ids.device)).any(dim=1)
+
+    @staticmethod
+    def _raise_if_not_permutation(bad):
+        rows = [i for i, b in enumerate(bad) if b]
+        if rows:
+            raise ValueError(f"ids_restore rows {rows} are not permutations of 0..L-1")
 
     @torch.no_grad()
     def forward_encoder(self, imgs, total_scores) -> Tuple[torch.Tensor, torch.Tensor]:
@@ -516,7 +562,9 @@ class MCM(nn.Module):
         module of the same configuration (same `precise` mode) bit for bit.
         Returns {"y_hat": f32 [N,Cy,s,s], "z_hat": f32 [N,Cz,s/4,s/4], "y_indexes": i32 [N, Cy*s*s]} and, with `need_recon`
         (default: whenever the decoder-side weights are loaded), "x_hat": f32 [N,3,S,S] computed exactly as forward's
-        x_hat (recon.synthesize).  No post-processing (e.g. clamping) is applied to x_hat: it is forward's x_hat."""
+        x_hat (recon.synthesize, or tmae_synthesize with native_synthesis=True).  No post-processing (e.g. clamping) is
+        applied to x_hat: it is forward's x_hat.  With native_synthesis=True the x_hat is enqueued on the same stream, and a
+        row of ids_restore that is not a permutation of 0..L-1 raises ValueError (checked on the device, read once at the end)."""
         if (y_symbols is None) == (decode_fn is None):
             raise ValueError("give exactly one of y_symbols and decode_fn")
         if need_recon is None:
@@ -561,9 +609,13 @@ class MCM(nn.Module):
                         raise ValueError(f"decode_fn must return integer symbols [{N}, {cnt}, {sc}, {s}, {s}], got {sym.dtype} {tuple(sym.shape)}")
                     by_slice(ys)[:, first:first + cnt] = sym.to(device=dev, dtype=torch.int32)
                 _native.check(lib.tmae_decode_step(self._handle, g, C.c_void_p(ys.data_ptr()), C.byref(o), st), self._handle, RuntimeError)
+            x_hat = self._synthesize(y_hat, ids_restore, cur) if need_recon and self._syn_on else None
             self._leave_stream(cur)
         out = {"y_hat": self._nchw(y_hat), "z_hat": self._nchw(z_hat), "y_indexes": y_idx}
-        if need_recon:
+        if x_hat is not None:
+            self._raise_if_not_permutation(self._ids_not_permutation(ids_restore).tolist())
+            out["x_hat"] = x_hat
+        elif need_recon:
             out["x_hat"] = recon.synthesize(self._weights, c, y_hat.reshape(N, c.num_keep_patches, c.latent_depth), ids_restore.to(dev))
         return out
 
@@ -651,7 +703,9 @@ class MCM(nn.Module):
         to the device, then the range decoder and the network in one enqueued decode (no host round trip in between).
         Returns {"y_hat": f32 [N,Cy,s,s], "z_hat": f32 [N,Cz,s/4,s/4]} and, with `need_recon` (default: whenever the
         decoder-side weights are loaded), "x_hat" exactly as forward computes it.  Raises ValueError for malformed arguments,
-        and for images whose streams do not decode exactly to their end (naming them).  lanes=(W_y, W_z): the strings are in
+        and for images whose streams do not decode exactly to their end (naming them).  With native_synthesis=True the x_hat is
+        enqueued before the status read, which also carries the check that every row of ids_restore is a permutation of 0..L-1
+        (ValueError otherwise).  lanes=(W_y, W_z): the strings are in
         the laned format of `compress_bitstream(..., lanes=(W_y, W_z))`; a header with another lane count, or lane lengths
         that do not add up, is a stream that does not decode."""
         lanes = self._check_lanes(lanes)
@@ -704,13 +758,20 @@ class MCM(nn.Module):
                 rc = lib.tmae_decompress_streams_lanes(self._handle, yp, yo, lanes[0], zp, zo, lanes[1], N, C.byref(o),
                                                        C.c_void_p(status.data_ptr()), C.c_void_p(cur.cuda_stream))
             _native.check(rc, self._handle, RuntimeError)
+            x_hat = None
+            if need_recon and self._syn_on:   # enqueued before the status read: the one host round trip covers both
+                x_hat = self._synthesize(y_hat, ids_restore, cur)
+                status = torch.cat([status, self._ids_not_permutation(ids_restore).int()])
             self._leave_stream(cur)
         st = status.cpu()
         bad = [i for i in range(N) if st[i]]
         if bad:
             raise ValueError(f"the streams of images {bad} do not decode (status {[int(st[i]) for i in bad]}: truncated or corrupt)")
         out = {"y_hat": self._nchw(y_hat), "z_hat": self._nchw(z_hat)}
-        if need_recon:
+        if x_hat is not None:
+            self._raise_if_not_permutation(st[N:].tolist())
+            out["x_hat"] = x_hat
+        elif need_recon:
             out["x_hat"] = recon.synthesize(self._weights, c, y_hat.reshape(N, c.num_keep_patches, c.latent_depth), ids_restore.to(dev))
         return out
 
