@@ -82,22 +82,57 @@ struct Step {
     std::string tag;
 };
 
+// Plan kinds, and what each kind's steps and captured graphs read.  drop_plans(h, DEP_x) discards every plan that reads x
+// when x is freed or rewritten; the next call of that kind builds its plan again.
+enum PlanKind {
+    PLAN_FORWARD,                    // tmae_forward and the calls that run part of it
+    PLAN_FORCED,                     // tmae_forward_from_latent_forced
+    PLAN_DECODE,                     // tmae_decode_begin / _step
+    PLAN_STREAMS,                    // tmae_decompress_streams(_lanes): the decode with the range decoder in front
+    PLAN_SYNTH,                      // tmae_synthesize
+};
+enum PlanDep : unsigned {
+    DEP_WS = 1,                      // network workspace (ensure_workspace)
+    DEP_CODER = 2,                   // coder workspace (ensure_coder_workspace)
+    DEP_SYNTH = 4,                   // synthesis workspace (ensure_synth_workspace, tmae_enable_synthesis)
+    DEP_SCALE = 8,                   // scale table (tmae_set_scale_table)
+    DEP_CDF = 16,                    // CDF tables (tmae_set_cdf_tables)
+    DEP_ALL = ~0u,                   // weights (tmae_finalize_weights) and tmae_destroy: every plan
+};
+const unsigned kPlanDeps[] = {
+    DEP_WS | DEP_SCALE,                          // PLAN_FORWARD
+    DEP_WS | DEP_SCALE,                          // PLAN_FORCED
+    DEP_WS | DEP_SCALE,                          // PLAN_DECODE
+    DEP_WS | DEP_SCALE | DEP_CODER | DEP_CDF,    // PLAN_STREAMS
+    DEP_SYNTH,                                   // PLAN_SYNTH
+};
+// (kind, batch size, y lanes, z lanes); the lanes are nonzero for the laned PLAN_STREAMS only
+typedef std::tuple<int, int, int, int> PlanKey;
+
 struct Plan {
     int N = 0;
+    unsigned deps = 0;               // DEP_* bits of its kind
     std::vector<Step> steps;
     std::vector<GemmParams> host_params;
     GemmParams* d_params = nullptr;
     bool from_latent_ok = true;
-    cudaGraphExec_t graph = nullptr; // whole forward (steps + output copies), pointers via the device IoBlock
-    int calls = 0;                   // the first call runs plain launches (one-time function attributes), then capture
     bool attn_tc = false;           // tcgen05 attention: tensor maps of the Q and K / V tiles over this plan's qkv matrix
     CUtensorMap attn_q, attn_k;
     int first_rate_step = 0;        // index of the first step of the rate half (h_a)
     int encoder_end_step = 0;       // one past the final LayerNorm
-    // decode plans: stage k = steps [stage_begin[k], stage_begin[k + 1]), one CUDA graph per stage
-    std::vector<int> stage_begin;
+    // stage k = steps [stage_begin[k], stage_begin[k + 1]), one CUDA graph per stage (run_stage).  Builders add the cuts
+    // (the step-wise decode only); finish_plan closes the last stage.
+    std::vector<int> stage_begin{0};
     std::vector<cudaGraphExec_t> stage_graph;
     std::vector<int> stage_calls;
+
+    Plan() = default;
+    Plan(const Plan&) = delete;
+    Plan& operator=(const Plan&) = delete;
+    ~Plan() {
+        if (d_params) cudaFree(d_params);
+        for (cudaGraphExec_t g : stage_graph) if (g) cudaGraphExecDestroy(g);
+    }
 };
 
 struct Workspace {
@@ -156,6 +191,16 @@ struct SynthWorkspace {
     IoBlock* io = nullptr;           // per-call pointers (y_hat, ids_restore, x_hat)
 };
 
+// One profiled launch, or one run of consecutive same-family launches (tmae_profile_enable(h, 2)).
+struct ProfRecord {
+    cudaEvent_t begin = nullptr, end = nullptr;
+    int family = 0;
+    double flops = 0, bytes = 0, mma_flops = 0;
+    std::string tag;                 // the first step's tag
+    int ctas = 0, block_n = 0;       // the first step's GEMM grid and tile width (0: not a GEMM)
+    int launches = 0;
+};
+
 }  // namespace
 
 struct tmae_handle {
@@ -172,15 +217,11 @@ struct tmae_handle {
     bool gc_fuse = false;            // bf16 rate half: cc_transform_mean/scale[i].8 as one GEMM with the Gaussian conditional in its epilogue
     bool finalized = false;
     Workspace ws;
-    std::map<int, std::unique_ptr<Plan>> plans;
-    std::map<int, std::unique_ptr<Plan>> dec_plans;   // decode plans by batch size (tmae_decode_begin / _step)
-    // decode-from-streams plans by (batch size, y lanes, z lanes); lanes (0, 0) = compressai's format (tmae_decompress_streams)
-    std::map<std::tuple<int, int, int>, std::unique_ptr<Plan>> stream_plans;
-    // synthesis (tmae_enable_synthesis): g_s, the MAE decoder and unpatchify on the engine, one plan per batch size
+    std::map<PlanKey, std::unique_ptr<Plan>> plans;   // every launch plan of the handle (get_plan)
+    // synthesis (tmae_enable_synthesis): g_s, the MAE decoder and unpatchify on the engine
     int syn_depth = 0, syn_heads = 0;    // 0: synthesis disabled (the decoder-side weights are ignored)
     int Dd = 0, syn_mlp = 0, syn_out = 0; // decoder width, its MLP width, decoder_pred outputs (p * p * in_chans)
     SynthWorkspace sws;
-    std::map<int, std::unique_ptr<Plan>> syn_plans;
     CdfTables cdf[2];                // quantised CDF tables: [TMAE_MODEL_GAUSSIAN], [TMAE_MODEL_BOTTLENECK]
     CoderWorkspace cws;
     int dec_N = 0, dec_next = -1;    // decode in progress: batch size and the next group expected (-1 = none)
@@ -195,12 +236,7 @@ struct tmae_handle {
     // profiling
     bool profiling = false;
     bool prof_by_run = false;        // one event pair per run of consecutive same-family launches instead of per launch
-    std::vector<int> prof_launches;
-    std::vector<std::pair<cudaEvent_t, cudaEvent_t>> prof_events;
-    std::vector<int> prof_family;
-    std::vector<double> prof_flops, prof_bytes, prof_mma;
-    std::vector<std::string> prof_tag;
-    std::vector<int> prof_ctas, prof_bn;
+    std::vector<ProfRecord> prof;    // records of the profiled call; the events are kept for the next one
     size_t prof_used = 0;
     int dev = 0;
 };
@@ -699,14 +735,10 @@ int fill_params(tmae_handle* h, const GemmDesc& d, int groups_for_tiling, GemmPa
 }
 
 // ---- workspace -----------------------------------------------------------------------------------------
-template <typename Key>
-void drop_plans(std::map<Key, std::unique_ptr<Plan>>& plans) {
-    for (auto& kv : plans) {
-        if (kv.second->d_params) cudaFree(kv.second->d_params);
-        if (kv.second->graph) cudaGraphExecDestroy(kv.second->graph);
-        for (cudaGraphExec_t g : kv.second->stage_graph) if (g) cudaGraphExecDestroy(g);
-    }
-    plans.clear();
+// Discards the plans (and their captured graphs) that read any of the DEP_* bits in `mask`.
+void drop_plans(tmae_handle* h, unsigned mask) {
+    for (auto it = h->plans.begin(); it != h->plans.end();)
+        it = (it->second->deps & mask) ? h->plans.erase(it) : std::next(it);
 }
 
 void free_pool(std::vector<void*>& pool) {
@@ -717,10 +749,7 @@ void free_pool(std::vector<void*>& pool) {
 int ensure_workspace(tmae_handle* h, int N) {
     Workspace& w = h->ws;
     if (N <= w.cap_N) return TMAE_OK;
-    // plans hold pointers into the workspace: drop them
-    drop_plans(h->plans);
-    drop_plans(h->dec_plans);
-    drop_plans(h->stream_plans);
+    drop_plans(h, DEP_WS);
     free_pool(w.allocs);
     w = Workspace();
     size_t tot = 0;
@@ -1088,8 +1117,18 @@ int add_lrp_steps(tmae_handle* h, Plan& pl, int N, int i0, int cnt, bool forced)
     return TMAE_OK;
 }
 
-// Common tail of every plan: sanity check, weight-prefetch chain, parameter blocks to the device.
+// A step that launches one kernel from the plan's buffers (no GEMM parameter block).
+void add_step(Plan& pl, StepKind kind, int family, const std::string& tag, int slice = 0, int gc_slices = 1) {
+    Step st;
+    st.kind = kind; st.family = family; st.tag = tag; st.slice = slice; st.gc_slices = gc_slices;
+    pl.steps.push_back(st);
+}
+
+// Common tail of every plan: last stage, sanity check, weight-prefetch chain, parameter blocks to the device.
 int finish_plan(tmae_handle* h, Plan& pl) {
+    pl.stage_begin.push_back((int)pl.steps.size());
+    pl.stage_graph.assign(pl.stage_begin.size() - 1, nullptr);
+    pl.stage_calls.assign(pl.stage_begin.size() - 1, 0);
     for (const Step& st : pl.steps)
         if (st.kind == ST_GEMM && pl.host_params[st.param_index].num_segs < 1) return fail(h, TMAE_EINVAL, "bad plan");
     if (!getenv("TMAE_NO_WEIGHT_PREFETCH")) {      // each GEMM step prefetches the weights of the next one (cyclically)
@@ -1189,30 +1228,23 @@ int add_blocks(tmae_handle* h, Plan& pl, const BlockSet& b) {
 
 // forced = slice-wise teacher forcing (tmae_forward_from_latent_forced): after lrp_transform[i] the support columns of
 // slice i are overwritten with the caller's y_hat, so slice j > i never sees a symbol this run decided itself.
-int build_plan(tmae_handle* h, int N, Plan** out, bool forced = false) {
-    const int key = N * 2 + (forced ? 1 : 0);
-    auto it = h->plans.find(key);
-    if (it != h->plans.end()) { *out = it->second.get(); return TMAE_OK; }
+int build_plan(tmae_handle* h, Plan& pl, bool forced) {
+    const int N = pl.N;
     int rc = ensure_workspace(h, N);
     if (rc) return rc;
-    it = h->plans.find(key);        // ensure_workspace may have cleared the map
-    std::unique_ptr<Plan> plp(new Plan());
-    Plan& pl = *plp;
-    pl.N = N;
     Workspace& w = h->ws;
     const int C = h->C, T = h->T, K = h->K, s = h->s, Cy = h->Cy, Cz = h->Cz;
     const long long rt = (long long)N * T, rk = (long long)N * K;
     char tag[96];
     auto conv_in = [&](GemmDesc& d, int side) { conv_input(d, side, N); };
-    auto simple = [&](StepKind k, int fam, const char* t) { Step st; st.kind = k; st.family = fam; st.tag = t; pl.steps.push_back(st); };
 
     if (!h->precise_enc && !(h->cfg.flags & TMAE_FLAG_DEBUG_SIMT) && attention_tc_eligible(T)) {
         if ((rc = make_attention_maps(h, w.qkv.p, rt, C, T, (h->cfg.flags & TMAE_FLAG_SHARE_SM) ? 2 : 1, &pl.attn_q, &pl.attn_k))) return rc;
         pl.attn_tc = true;
     }
-    simple(ST_ZERO_RATE, FAM_MISC, "zero_rate");
-    simple(ST_MASK, FAM_MASK, "mask_select");
-    simple(ST_GATHER, FAM_GATHER, "gather_patches");
+    add_step(pl, ST_ZERO_RATE, FAM_MISC, "zero_rate");
+    add_step(pl, ST_MASK, FAM_MASK, "mask_select");
+    add_step(pl, ST_GATHER, FAM_GATHER, "gather_patches");
     {   // patch embed: conv k16 s16 == linear over (c,p,q) patches; + bias + pos_embed[id+1]  (MCM.py:615-618)
         GemmDesc d;
         d.layer = get_layer(h, "encoder_embed.proj");
@@ -1272,7 +1304,7 @@ int build_plan(tmae_handle* h, int N, Plan** out, bool forced = false) {
             rc = add_gemm_group(h, pl, &d, 1, tag); if (rc) return rc;
         }
     }
-    simple(ST_EB, FAM_ENTROPY, "entropy_bottleneck");
+    add_step(pl, ST_EB, FAM_ENTROPY, "entropy_bottleneck");
     if ((rc = add_hs_steps(h, pl, N))) return rc;
     const bool skip_dead = (h->cfg.flags & TMAE_FLAG_SKIP_DEAD_LRP) != 0;
     // Slice loop (MCM.py:755-784).  Slice i reads y_hat of slices [0, min(i, 6)): slices 0..5 form a serial chain,
@@ -1281,12 +1313,12 @@ int build_plan(tmae_handle* h, int N, Plan** out, bool forced = false) {
     for (int i0 = 0; i0 < h->nsl;) {
         const int cnt = i0 < half_sl ? 1 : h->nsl - i0;          // members of this slice group
         if ((rc = add_cc_steps(h, pl, N, i0, cnt, false))) return rc;
-        if (!h->gc_fuse) { Step g; g.kind = ST_GC; g.family = FAM_ENTROPY; g.slice = i0; g.gc_slices = cnt; g.tag = "gaussian." + std::to_string(i0); pl.steps.push_back(g); }
+        if (!h->gc_fuse) add_step(pl, ST_GC, FAM_ENTROPY, "gaussian." + std::to_string(i0), i0, cnt);
         if (!(skip_dead && i0 >= half_sl) && (rc = add_lrp_steps(h, pl, N, i0, cnt, forced))) return rc;
-        if (forced && i0 < half_sl) { Step f; f.kind = ST_FORCE; f.family = FAM_MISC; f.slice = i0; f.tag = "force." + std::to_string(i0); pl.steps.push_back(f); }
+        if (forced && i0 < half_sl) add_step(pl, ST_FORCE, FAM_MISC, "force." + std::to_string(i0), i0);
         i0 += cnt;
     }
-    simple(ST_RATE, FAM_ENTROPY, "rate_finalize");
+    add_step(pl, ST_RATE, FAM_ENTROPY, "rate_finalize");
 
     // algorithmic HBM bytes of the memory-bound kernels (bench.py reports them against the measured HBM peak)
     for (Step& st : pl.steps) {
@@ -1300,9 +1332,6 @@ int build_plan(tmae_handle* h, int N, Plan** out, bool forced = false) {
             default: break;
         }
     }
-    if ((rc = finish_plan(h, pl))) return rc;
-    *out = plp.get();
-    h->plans[key] = std::move(plp);
     return TMAE_OK;
 }
 
@@ -1318,50 +1347,10 @@ void slice_groups(int nsl, std::vector<std::pair<int, int>>& g) {
     }
 }
 
-// Decode plan (MCM.decompress, MCM.py:896-968, range decoder replaced by the caller's symbols): the rate half of the forward
-// with y replaced by symbols, cut into stages at the slice groups because the range decoder needs the scale-table indexes
-// of a group before it can supply the group's symbols.
-//   stage 0      z dequantise, h_s, cc layers + indexes of group 0
-//   stage g + 1  dequantise group g (symbols + mu), lrp_transform of group g, then cc layers + indexes of group g + 1
-//                (after the last group: y_hat / mu / sigma to the caller's buffers)
-// lrp_transform[6..11] always runs: y_hat is the product here (TMAE_FLAG_SKIP_DEAD_LRP applies to the forward only).
-int build_decode_plan(tmae_handle* h, int N, Plan** out) {
-    auto it = h->dec_plans.find(N);
-    if (it != h->dec_plans.end()) { *out = it->second.get(); return TMAE_OK; }
-    int rc = ensure_workspace(h, N);
-    if (rc) return rc;
-    std::unique_ptr<Plan> plp(new Plan());
-    Plan& pl = *plp;
-    pl.N = N;
-    auto simple = [&](StepKind k, int fam, const std::string& t, int slice = 0, int cnt = 1) {
-        Step st; st.kind = k; st.family = fam; st.tag = t; st.slice = slice; st.gc_slices = cnt; pl.steps.push_back(st);
-    };
-    std::vector<std::pair<int, int>> groups;
-    slice_groups(h->nsl, groups);
-    pl.stage_begin.push_back(0);
-    simple(ST_ZDEQ, FAM_ENTROPY, "z_dequantize");
-    if ((rc = add_hs_steps(h, pl, N))) return rc;
-    for (const auto& g : groups) {
-        if ((rc = add_cc_steps(h, pl, N, g.first, g.second, true))) return rc;
-        if (!h->gc_fuse) simple(ST_IDX, FAM_ENTROPY, "indexes." + std::to_string(g.first), g.first, g.second);
-        pl.stage_begin.push_back((int)pl.steps.size());
-        simple(ST_YDEQ, FAM_ENTROPY, "dequantize." + std::to_string(g.first), g.first, g.second);
-        if ((rc = add_lrp_steps(h, pl, N, g.first, g.second, false))) return rc;
-    }
-    simple(ST_DEC_OUT, FAM_MISC, "decode_outputs");
-    pl.stage_begin.push_back((int)pl.steps.size());
-    pl.stage_graph.assign(pl.stage_begin.size() - 1, nullptr);
-    pl.stage_calls.assign(pl.stage_begin.size() - 1, 0);
-    if ((rc = finish_plan(h, pl))) return rc;
-    *out = plp.get();
-    h->dec_plans[N] = std::move(plp);
-    return TMAE_OK;
-}
-
 int ensure_coder_workspace(tmae_handle* h, int N) {
     CoderWorkspace& c = h->cws;
     if (N <= c.cap_N) return TMAE_OK;
-    drop_plans(h->stream_plans);     // they hold pointers into these buffers
+    drop_plans(h, DEP_CODER);
     for (void* p : c.allocs) cudaFree(p);
     c.allocs.clear();
     c.cap_N = 0;
@@ -1374,52 +1363,50 @@ int ensure_coder_workspace(tmae_handle* h, int N) {
     return TMAE_OK;
 }
 
-// Decode plan fed by the range decoder (tmae_decompress_streams): the decode plan above with the coder in front of the two
-// dequantisations - ST_ZDEC decodes the z streams with the bottleneck tables before ST_ZDEQ, and ST_YDEC decodes slice group g
-// of the y streams, with the indexes the group's cc layers just wrote, before ST_YDEQ.  The y decoder's state stays in the
-// coder workspace between the groups.  One stage: the whole decode replays as one CUDA graph per (batch size, lanes).
-// lanes_y / lanes_z = 0: compressai's format; else the laned format with that many lanes per y / z stream.
-int build_stream_decode_plan(tmae_handle* h, int N, int lanes_y, int lanes_z, Plan** out) {
-    const auto key = std::make_tuple(N, lanes_y, lanes_z);
-    auto it = h->stream_plans.find(key);
-    if (it != h->stream_plans.end()) { *out = it->second.get(); return TMAE_OK; }
+// Decode plan (MCM.decompress, MCM.py:896-968): the rate half of the forward with y replaced by symbols.
+// lrp_transform[6..11] always runs: y_hat is the product here (TMAE_FLAG_SKIP_DEAD_LRP applies to the forward only).
+// Uncoded (tmae_decode_begin / _step, the caller's range decoder supplies the symbols): cut into stages at the slice groups,
+// because the range decoder needs the scale-table indexes of a group before it can supply the group's symbols.
+//   stage 0      z dequantise, h_s, cc layers + indexes of group 0
+//   stage g + 1  dequantise group g (symbols + mu), lrp_transform of group g, then cc layers + indexes of group g + 1
+//                (after the last group: y_hat / mu / sigma to the caller's buffers)
+// Coded (tmae_decompress_streams): the range decoder in front of the two dequantisations - ST_ZDEC decodes the z streams with
+// the bottleneck tables before ST_ZDEQ, and ST_YDEC decodes slice group g of the y streams, with the indexes the group's cc
+// layers just wrote, before ST_YDEQ.  The y decoder's state stays in the coder workspace between the groups.  One stage: the
+// whole decode replays as one CUDA graph per (batch size, lanes).  lanes_y / lanes_z = 0: compressai's format; else the laned
+// format with that many lanes per y / z stream.
+int build_decode_plan(tmae_handle* h, Plan& pl, bool coded, int lanes_y, int lanes_z) {
+    const int N = pl.N;
     int rc = ensure_workspace(h, N);
-    if (rc || (rc = ensure_coder_workspace(h, N))) return rc;
-    std::unique_ptr<Plan> plp(new Plan());
-    Plan& pl = *plp;
-    pl.N = N;
-    auto simple = [&](StepKind k, int fam, const std::string& t, int slice = 0, int cnt = 1) {
-        Step st; st.kind = k; st.family = fam; st.tag = t; st.slice = slice; st.gc_slices = cnt; pl.steps.push_back(st);
-    };
+    if (rc || (coded && (rc = ensure_coder_workspace(h, N)))) return rc;
     std::vector<std::pair<int, int>> groups;
     slice_groups(h->nsl, groups);
-    pl.stage_begin.push_back(0);
-    simple(ST_ZDEC, FAM_CODER, "rans_decode.z");
-    pl.steps.back().lanes = lanes_z;
-    simple(ST_ZDEQ, FAM_ENTROPY, "z_dequantize");
+    if (coded) {
+        add_step(pl, ST_ZDEC, FAM_CODER, "rans_decode.z");
+        pl.steps.back().lanes = lanes_z;
+    }
+    add_step(pl, ST_ZDEQ, FAM_ENTROPY, "z_dequantize");
     if ((rc = add_hs_steps(h, pl, N))) return rc;
     for (const auto& g : groups) {
         if ((rc = add_cc_steps(h, pl, N, g.first, g.second, true))) return rc;
-        if (!h->gc_fuse) simple(ST_IDX, FAM_ENTROPY, "indexes." + std::to_string(g.first), g.first, g.second);
-        simple(ST_YDEC, FAM_CODER, "rans_decode.y." + std::to_string(g.first), g.first, g.second);
-        pl.steps.back().lanes = lanes_y;
-        simple(ST_YDEQ, FAM_ENTROPY, "dequantize." + std::to_string(g.first), g.first, g.second);
+        if (!h->gc_fuse) add_step(pl, ST_IDX, FAM_ENTROPY, "indexes." + std::to_string(g.first), g.first, g.second);
+        if (coded) {
+            add_step(pl, ST_YDEC, FAM_CODER, "rans_decode.y." + std::to_string(g.first), g.first, g.second);
+            pl.steps.back().lanes = lanes_y;
+        } else {
+            pl.stage_begin.push_back((int)pl.steps.size());
+        }
+        add_step(pl, ST_YDEQ, FAM_ENTROPY, "dequantize." + std::to_string(g.first), g.first, g.second);
         if ((rc = add_lrp_steps(h, pl, N, g.first, g.second, false))) return rc;
     }
-    simple(ST_DEC_OUT, FAM_MISC, "decode_outputs");
-    pl.stage_begin.push_back((int)pl.steps.size());
-    pl.stage_graph.assign(1, nullptr);
-    pl.stage_calls.assign(1, 0);
-    if ((rc = finish_plan(h, pl))) return rc;
-    *out = plp.get();
-    h->stream_plans[key] = std::move(plp);
+    add_step(pl, ST_DEC_OUT, FAM_MISC, "decode_outputs");
     return TMAE_OK;
 }
 
 int ensure_synth_workspace(tmae_handle* h, int N) {
     SynthWorkspace& w = h->sws;
     if (N <= w.cap_N) return TMAE_OK;
-    drop_plans(h->syn_plans);        // they hold pointers into these buffers
+    drop_plans(h, DEP_SYNTH);
     free_pool(w.allocs);
     w = SynthWorkspace();
     const size_t rk = (size_t)N * h->K, rt = (size_t)N * (h->L + 1), Dd = h->Dd;
@@ -1440,19 +1427,14 @@ int ensure_synth_workspace(tmae_handle* h, int N) {
 // fp32 accumulation, fp32 residual stream / LayerNorm statistics / softmax, in every accuracy mode (the precise flags govern the
 // rate path; no symbol depends on x_hat).  Every LayerNorm is folded: block 0's norm1 into its QKV with the statistics the
 // unshuffle writes, decoder_norm into decoder_pred with the statistics of the last fc2.  One stage: one CUDA graph per N.
-int build_synth_plan(tmae_handle* h, int N, Plan** out) {
-    auto it = h->syn_plans.find(N);
-    if (it != h->syn_plans.end()) { *out = it->second.get(); return TMAE_OK; }
+int build_synth_plan(tmae_handle* h, Plan& pl) {
+    const int N = pl.N;
     int rc = ensure_synth_workspace(h, N);
     if (rc) return rc;
-    std::unique_ptr<Plan> plp(new Plan());
-    Plan& pl = *plp;
-    pl.N = N;
     SynthWorkspace& w = h->sws;
     const int Dd = h->Dd, T = h->L + 1, Cy = h->Cy;
     const long long rk = (long long)N * h->K, rt = (long long)N * T;
-    auto simple = [&](StepKind k, int fam, const char* t) { Step st; st.kind = k; st.family = fam; st.tag = t; pl.steps.push_back(st); };
-    simple(ST_SYN_IN, FAM_MISC, "synth_input");
+    add_step(pl, ST_SYN_IN, FAM_MISC, "synth_input");
     {   // g_s: four 1x1 ConvTranspose2d == per-token linears, GELU after the first three (MCM.py:96-112, 790)
         const int ch[5] = {Cy, h->ga_ch[3], h->ga_ch[2], h->ga_ch[1], h->C};
         const Bf srcs[4] = {w.y_bf, w.gs[0], w.gs[1], w.gs[2]}, dsts[4] = {w.gs[0], w.gs[1], w.gs[2], w.tok};
@@ -1476,7 +1458,7 @@ int build_synth_plan(tmae_handle* h, int N, Plan** out) {
         d.flops = 2.0 * rk * h->C * (double)Dd;
         if ((rc = add_gemm_group(h, pl, &d, 1, "decoder_embed"))) return rc;
     }
-    simple(ST_UNSHUF, FAM_GATHER, "unshuffle");
+    add_step(pl, ST_UNSHUF, FAM_GATHER, "unshuffle");
     {
         BlockSet b;
         b.prefix = "decoder_blocks"; b.tag = "dec_blk";
@@ -1494,7 +1476,7 @@ int build_synth_plan(tmae_handle* h, int N, Plan** out) {
         d.flops = 2.0 * rt * Dd * (double)h->syn_out;
         if ((rc = add_gemm_group(h, pl, &d, 1, "decoder_pred"))) return rc;
     }
-    simple(ST_UNPATCH, FAM_MISC, "unpatchify");
+    add_step(pl, ST_UNPATCH, FAM_MISC, "unpatchify");
     for (Step& st : pl.steps) {      // algorithmic HBM bytes of the elementwise steps
         switch (st.kind) {
             case ST_SYN_IN: st.bytes = (double)rk * Cy * (4 + 2); break;
@@ -1503,12 +1485,26 @@ int build_synth_plan(tmae_handle* h, int N, Plan** out) {
             default: break;
         }
     }
-    pl.stage_begin = {0, (int)pl.steps.size()};
-    pl.stage_graph.assign(1, nullptr);
-    pl.stage_calls.assign(1, 0);
-    if ((rc = finish_plan(h, pl))) return rc;
-    *out = plp.get();
-    h->syn_plans[N] = std::move(plp);
+    return TMAE_OK;
+}
+
+// The plan of `kind` for batch size N (lanes: PLAN_STREAMS only), built on first use and kept until drop_plans discards it.
+int get_plan(tmae_handle* h, PlanKind kind, int N, Plan** out, int lanes_y = 0, int lanes_z = 0) {
+    const PlanKey key(kind, N, lanes_y, lanes_z);
+    auto it = h->plans.find(key);
+    if (it != h->plans.end()) { *out = it->second.get(); return TMAE_OK; }
+    std::unique_ptr<Plan> pl(new Plan());
+    pl->N = N;
+    pl->deps = kPlanDeps[kind];
+    int rc = TMAE_OK;
+    switch (kind) {
+        case PLAN_FORWARD: case PLAN_FORCED: rc = build_plan(h, *pl, kind == PLAN_FORCED); break;
+        case PLAN_DECODE: case PLAN_STREAMS: rc = build_decode_plan(h, *pl, kind == PLAN_STREAMS, lanes_y, lanes_z); break;
+        case PLAN_SYNTH: rc = build_synth_plan(h, *pl); break;
+    }
+    if (rc || (rc = finish_plan(h, *pl))) return rc;
+    *out = pl.get();
+    h->plans[key] = std::move(pl);
     return TMAE_OK;
 }
 
@@ -1521,32 +1517,22 @@ struct RunArgs {
     const IoBlock* io = nullptr;     // non-null: kernels read the per-call pointers from the device IoBlock
 };
 
-int prof_slot(tmae_handle* h, const Step& st, cudaEvent_t* a, cudaEvent_t* b) {
-    if (h->prof_used == h->prof_events.size()) {
-        cudaEvent_t e0, e1;
-        CUDA_TRY(h, cudaEventCreate(&e0));
-        CUDA_TRY(h, cudaEventCreate(&e1));
-        h->prof_events.push_back({e0, e1});
-        h->prof_family.push_back(0);
-        h->prof_flops.push_back(0);
-        h->prof_bytes.push_back(0);
-        h->prof_mma.push_back(0);
-        h->prof_tag.push_back("");
-        h->prof_ctas.push_back(0);
-        h->prof_bn.push_back(0);
-        h->prof_launches.push_back(0);
+// The next profiling record, started at step `st` with no launches counted yet.
+int prof_slot(tmae_handle* h, const Step& st, ProfRecord** out) {
+    if (h->prof_used == h->prof.size()) {
+        ProfRecord r;
+        CUDA_TRY(h, cudaEventCreate(&r.begin));
+        CUDA_TRY(h, cudaEventCreate(&r.end));
+        h->prof.push_back(r);
     }
-    *a = h->prof_events[h->prof_used].first;
-    *b = h->prof_events[h->prof_used].second;
-    h->prof_family[h->prof_used] = st.family;
-    h->prof_flops[h->prof_used] = st.flops;
-    h->prof_bytes[h->prof_used] = st.bytes;
-    h->prof_mma[h->prof_used] = st.flops * st.mma_terms;
-    h->prof_tag[h->prof_used] = st.tag;
-    h->prof_ctas[h->prof_used] = st.kind == ST_GEMM ? ((st.max_M + kBlockM - 1) / kBlockM) * ((st.max_N + st.block_n - 1) / st.block_n) * st.groups : 0;
-    h->prof_bn[h->prof_used] = st.kind == ST_GEMM ? st.block_n : 0;
-    h->prof_launches[h->prof_used] = 1;
-    ++h->prof_used;
+    ProfRecord& r = h->prof[h->prof_used++];
+    r.family = st.family;
+    r.flops = r.bytes = r.mma_flops = 0;
+    r.tag = st.tag;
+    r.ctas = st.kind == ST_GEMM ? ((st.max_M + kBlockM - 1) / kBlockM) * ((st.max_N + st.block_n - 1) / st.block_n) * st.groups : 0;
+    r.block_n = st.kind == ST_GEMM ? st.block_n : 0;
+    r.launches = 0;
+    *out = &r;
     return TMAE_OK;
 }
 
@@ -1565,21 +1551,22 @@ int run_steps(tmae_handle* h, Plan& pl, const RunArgs& a, cudaStream_t st) {
     }
     for (int si = a.begin; si < a.end; ++si) {
         const Step& sp = pl.steps[si];
-        cudaEvent_t e0 = nullptr, e1 = nullptr;
         // profiling: per launch, or (prof_by_run) per run of consecutive launches of one kernel family, which keeps
         // the launch-to-launch overlap inside a run and drops the event gap between its members
         const bool run_start = !h->prof_by_run || si == a.begin || pl.steps[si - 1].family != sp.family;
         const bool run_end = !h->prof_by_run || si + 1 == a.end || pl.steps[si + 1].family != sp.family;
-        if (h->profiling && run_start) {
-            int rc = prof_slot(h, sp, &e0, &e1);
-            if (rc) return rc;
-            CUDA_TRY(h, cudaEventRecord(e0, st));
-        } else if (h->profiling) {
-            const size_t cur = h->prof_used - 1;
-            h->prof_flops[cur] += sp.flops;
-            h->prof_bytes[cur] += sp.bytes;
-            h->prof_mma[cur] += sp.flops * sp.mma_terms;
-            h->prof_launches[cur] += 1;
+        if (h->profiling) {
+            if (run_start) {
+                ProfRecord* r = nullptr;
+                int rc = prof_slot(h, sp, &r);
+                if (rc) return rc;
+                CUDA_TRY(h, cudaEventRecord(r->begin, st));
+            }
+            ProfRecord& r = h->prof[h->prof_used - 1];
+            r.flops += sp.flops;
+            r.bytes += sp.bytes;
+            r.mma_flops += sp.flops * sp.mma_terms;
+            r.launches += 1;
         }
         switch (sp.kind) {
             case ST_ZERO_RATE:
@@ -1687,7 +1674,7 @@ int run_steps(tmae_handle* h, Plan& pl, const RunArgs& a, cudaStream_t st) {
                 break;
             }
         }
-        if (h->profiling && run_end) CUDA_TRY(h, cudaEventRecord(h->prof_events[h->prof_used - 1].second, st));
+        if (h->profiling && run_end) CUDA_TRY(h, cudaEventRecord(h->prof[h->prof_used - 1].end, st));
     }
     return TMAE_OK;
 }
@@ -1708,23 +1695,32 @@ int copy_outputs(tmae_handle* h, int N, const tmae_outputs* out, bool rate_half,
     return TMAE_OK;
 }
 
-// Whole forward as one CUDA-graph replay: the per-call pointers travel through the device IoBlock, so the graph is
-// captured once per batch size.  Returns TMAE_OK with *done = false when graphs are disabled / profiling is on.
-int run_full_graph(tmae_handle* h, Plan& pl, const float* imgs, const float* scores, const tmae_outputs* out,
-                   cudaStream_t st, bool* done) {
-    *done = false;
-    if (!h->use_graph || h->profiling) return TMAE_OK;
-    if (pl.calls++ == 0) return TMAE_OK;
-    Workspace& w = h->ws;
-    const int N = pl.N;
-    if (!pl.graph) {
+// Stage `stage` of a plan.  Its first call runs plain launches (they set one-time function attributes), the second captures
+// the stage into a CUDA graph and every later call replays that graph; with graphs off (TMAE_NO_GRAPH) or profiling on,
+// every call runs plain launches.  The graph reads the per-call pointers `hio` from the device IoBlock `io`, uploaded on
+// each call, so one capture serves every call of the plan.
+// forward: the whole forward plan.  Its graph ends with the output copies (launch_copy_outputs); its plain launches read
+// imgs, scores and the outputs from `hio` on the host and copy with copy_outputs.
+int run_stage(tmae_handle* h, Plan& pl, int stage, const IoBlock& hio, IoBlock* io, cudaStream_t st, bool forward = false) {
+    RunArgs a;
+    a.begin = pl.stage_begin[stage]; a.end = pl.stage_begin[stage + 1];
+    const bool replay = h->use_graph && !h->profiling && pl.stage_calls[stage]++ > 0;
+    if (forward && !replay) {
+        a.imgs = hio.imgs; a.scores = hio.scores; a.out = &hio.out;
+        const int rc = run_steps(h, pl, a, st);
+        return rc ? rc : copy_outputs(h, pl.N, &hio.out, true, true, st);
+    }
+    CUDA_TRY(h, cudaMemcpyAsync(io, &hio, sizeof(hio), cudaMemcpyHostToDevice, st));   // pageable source: staged before return
+    a.io = io;
+    if (!replay) return run_steps(h, pl, a, st);
+    if (!pl.stage_graph[stage]) {
         if (!h->cap_stream) CUDA_TRY(h, cudaStreamCreateWithFlags(&h->cap_stream, cudaStreamNonBlocking));
         CUDA_TRY(h, cudaStreamBeginCapture(h->cap_stream, cudaStreamCaptureModeThreadLocal));
-        RunArgs a;
-        a.begin = 0; a.end = (int)pl.steps.size(); a.io = w.io;
         int rc = run_steps(h, pl, a, h->cap_stream);
-        if (rc == TMAE_OK) {
-            cudaError_t e = launch_copy_outputs(w.io, w.y, w.z, w.mu, w.sigma, w.yhat, w.ids_keep, (long long)N * h->K * h->Cy,
+        if (rc == TMAE_OK && forward) {
+            const Workspace& w = h->ws;
+            const int N = pl.N;
+            cudaError_t e = launch_copy_outputs(io, w.y, w.z, w.mu, w.sigma, w.yhat, w.ids_keep, (long long)N * h->K * h->Cy,
                                                 (long long)N * h->s4 * h->s4 * h->Cz, (long long)N * h->K, h->cap_stream);
             if (e != cudaSuccess) rc = fail(h, TMAE_ECUDA, "copy_outputs capture: %s", cudaGetErrorString(e));
         }
@@ -1732,23 +1728,25 @@ int run_full_graph(tmae_handle* h, Plan& pl, const float* imgs, const float* sco
         cudaError_t e = cudaStreamEndCapture(h->cap_stream, &g);
         if (rc != TMAE_OK) { if (g) cudaGraphDestroy(g); return rc; }
         if (e != cudaSuccess || !g) return fail(h, TMAE_ECUDA, "graph capture failed: %s", cudaGetErrorString(e));
-        e = cudaGraphInstantiate(&pl.graph, g, 0);
+        e = cudaGraphInstantiate(&pl.stage_graph[stage], g, 0);
         cudaGraphDestroy(g);
-        if (e != cudaSuccess) { pl.graph = nullptr; return fail(h, TMAE_ECUDA, "graph instantiate failed: %s", cudaGetErrorString(e)); }
+        if (e != cudaSuccess) { pl.stage_graph[stage] = nullptr; return fail(h, TMAE_ECUDA, "graph instantiate failed: %s", cudaGetErrorString(e)); }
     }
+    CUDA_TRY(h, cudaGraphLaunch(pl.stage_graph[stage], st));
+    return TMAE_OK;
+}
+
+// The whole forward from the caller's pointers (tmae_forward, tmae_forward_host).
+int run_forward(tmae_handle* h, Plan& pl, const float* imgs, const float* scores, const tmae_outputs* out, cudaStream_t st) {
     IoBlock hio;
     memset(&hio, 0, sizeof(hio));
     hio.imgs = imgs; hio.scores = scores;
     if (out) hio.out = *out;
-    CUDA_TRY(h, cudaMemcpyAsync(w.io, &hio, sizeof(hio), cudaMemcpyHostToDevice, st));   // pageable source: staged before return
-    CUDA_TRY(h, cudaGraphLaunch(pl.graph, st));
-    *done = true;
-    return TMAE_OK;
+    if (h->profiling) h->prof_used = 0;
+    return run_stage(h, pl, 0, hio, h->ws.io, st, true);
 }
 
-// One stage of a decode plan.  The per-call pointers (symbols in; z_hat, indexes, y_hat, mu, sigma out) always travel through
-// the device IoBlock, so the stage's first call runs plain launches and every later one replays a graph captured per
-// (N, stage), exactly as run_full_graph does for the forward.
+// The per-call pointers of a decode stage: symbols in; z_hat, indexes, y_hat, mu, sigma out.
 IoBlock decode_io(const int32_t* z_symbols, const int32_t* y_symbols, const tmae_outputs* out) {
     IoBlock hio;
     memset(&hio, 0, sizeof(hio));
@@ -1756,29 +1754,6 @@ IoBlock decode_io(const int32_t* z_symbols, const int32_t* y_symbols, const tmae
     hio.out.y_hat = out->y_hat; hio.out.mu = out->mu; hio.out.sigma = out->sigma;
     hio.z_symbols = z_symbols; hio.y_symbols = y_symbols;
     return hio;
-}
-
-// dev_io: the device IoBlock the stage reads (default: the workspace's; synthesis plans have their own)
-int run_decode_stage(tmae_handle* h, Plan& pl, int stage, const IoBlock& hio, cudaStream_t st, IoBlock* dev_io = nullptr) {
-    IoBlock* io = dev_io ? dev_io : h->ws.io;
-    CUDA_TRY(h, cudaMemcpyAsync(io, &hio, sizeof(hio), cudaMemcpyHostToDevice, st));   // pageable source: staged before return
-    RunArgs a;
-    a.begin = pl.stage_begin[stage]; a.end = pl.stage_begin[stage + 1]; a.io = io;
-    if (!h->use_graph || h->profiling || pl.stage_calls[stage]++ == 0) return run_steps(h, pl, a, st);
-    if (!pl.stage_graph[stage]) {
-        if (!h->cap_stream) CUDA_TRY(h, cudaStreamCreateWithFlags(&h->cap_stream, cudaStreamNonBlocking));
-        CUDA_TRY(h, cudaStreamBeginCapture(h->cap_stream, cudaStreamCaptureModeThreadLocal));
-        int rc = run_steps(h, pl, a, h->cap_stream);
-        cudaGraph_t g = nullptr;
-        cudaError_t e = cudaStreamEndCapture(h->cap_stream, &g);
-        if (rc != TMAE_OK) { if (g) cudaGraphDestroy(g); return rc; }
-        if (e != cudaSuccess || !g) return fail(h, TMAE_ECUDA, "decode graph capture failed: %s", cudaGetErrorString(e));
-        e = cudaGraphInstantiate(&pl.stage_graph[stage], g, 0);
-        cudaGraphDestroy(g);
-        if (e != cudaSuccess) { pl.stage_graph[stage] = nullptr; return fail(h, TMAE_ECUDA, "decode graph instantiate failed: %s", cudaGetErrorString(e)); }
-    }
-    CUDA_TRY(h, cudaGraphLaunch(pl.stage_graph[stage], st));
-    return TMAE_OK;
 }
 
 int check_ready(tmae_handle* h, int N) {
@@ -1846,10 +1821,7 @@ void tmae_destroy(tmae_handle* h) {
     if (!h) return;
     cudaDeviceSynchronize();
     for (auto& kv : h->raw) cudaFree(kv.second.ptr);
-    drop_plans(h->plans);
-    drop_plans(h->dec_plans);
-    drop_plans(h->stream_plans);
-    drop_plans(h->syn_plans);
+    drop_plans(h, DEP_ALL);
     for (CdfTables& t : h->cdf) rans_free_tables(&t);
     free_pool(h->cws.allocs);
     free_pool(h->sws.allocs);
@@ -1858,7 +1830,7 @@ void tmae_destroy(tmae_handle* h) {
     if (h->scale_table) cudaFree(h->scale_table);
     free_pool(h->ws.allocs);
     free_pool(h->weight_allocs);
-    for (auto& ev : h->prof_events) { cudaEventDestroy(ev.first); cudaEventDestroy(ev.second); }
+    for (ProfRecord& r : h->prof) { cudaEventDestroy(r.begin); cudaEventDestroy(r.end); }
     delete h;
 }
 
@@ -1887,10 +1859,7 @@ int tmae_set_weight(tmae_handle* h, const char* name, const void* data, int dtyp
 int tmae_finalize_weights(tmae_handle* h) {
     if (!h) return TMAE_EINVAL;
     // re-finalize: drop previous packs
-    drop_plans(h->plans);
-    drop_plans(h->dec_plans);
-    drop_plans(h->stream_plans);
-    drop_plans(h->syn_plans);
+    drop_plans(h, DEP_ALL);
     h->dec_next = -1;
     free_pool(h->weight_allocs);
     h->layers.clear();
@@ -2009,7 +1978,7 @@ int tmae_reserve(tmae_handle* h, int N) {
     int rc = check_ready(h, N);
     if (rc) return rc;
     Plan* pl = nullptr;
-    return build_plan(h, N, &pl);
+    return get_plan(h, PLAN_FORWARD, N, &pl);
 }
 
 int tmae_attention_plan(int T, int H, int N, int mode, int* out) {
@@ -2027,7 +1996,7 @@ int tmae_conv_geometry(int s, int n_img, int* out) {
 
 int tmae_launch_count(tmae_handle* h, int N) {
     Plan* pl = nullptr;
-    if (check_ready(h, N) || build_plan(h, N, &pl)) return -1;
+    if (check_ready(h, N) || get_plan(h, PLAN_FORWARD, N, &pl)) return -1;
     return (int)pl->steps.size();
 }
 
@@ -2036,16 +2005,8 @@ int tmae_forward(tmae_handle* h, const float* imgs, const float* scores, int N, 
     if (rc) return rc;
     if (!imgs || !scores) return fail(h, TMAE_EINVAL, "imgs / scores must not be null");
     Plan* pl = nullptr;
-    if ((rc = build_plan(h, N, &pl))) return rc;
-    cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
-    bool done = false;
-    if ((rc = run_full_graph(h, *pl, imgs, scores, out, st, &done))) return rc;
-    if (done) return TMAE_OK;
-    RunArgs a;
-    a.imgs = imgs; a.scores = scores; a.out = out; a.begin = 0; a.end = (int)pl->steps.size();
-    if (h->profiling) h->prof_used = 0;
-    if ((rc = run_steps(h, *pl, a, st))) return rc;
-    return copy_outputs(h, N, out, true, true, st);
+    if ((rc = get_plan(h, PLAN_FORWARD, N, &pl))) return rc;
+    return run_forward(h, *pl, imgs, scores, out, reinterpret_cast<cudaStream_t>(stream));
 }
 
 int tmae_forward_encoder(tmae_handle* h, const float* imgs, const float* scores, int N, const tmae_outputs* out,
@@ -2054,7 +2015,7 @@ int tmae_forward_encoder(tmae_handle* h, const float* imgs, const float* scores,
     if (rc) return rc;
     if (!imgs || !scores) return fail(h, TMAE_EINVAL, "imgs / scores must not be null");
     Plan* pl = nullptr;
-    if ((rc = build_plan(h, N, &pl))) return rc;
+    if ((rc = get_plan(h, PLAN_FORWARD, N, &pl))) return rc;
     cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
     RunArgs a;
     a.imgs = imgs; a.scores = scores; a.out = out; a.begin = 0; a.end = pl->encoder_end_step;
@@ -2068,7 +2029,7 @@ int tmae_forward_from_latent(tmae_handle* h, const float* y, int N, const tmae_o
     if (rc) return rc;
     if (!y) return fail(h, TMAE_EINVAL, "y must not be null");
     Plan* pl = nullptr;
-    if ((rc = build_plan(h, N, &pl))) return rc;
+    if ((rc = get_plan(h, PLAN_FORWARD, N, &pl))) return rc;
     cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
     Workspace& w = h->ws;
     const size_t rk = (size_t)N * h->K;
@@ -2089,7 +2050,7 @@ int tmae_forward_from_latent_forced(tmae_handle* h, const float* y, const float*
     if (!y || !y_hat_support) return fail(h, TMAE_EINVAL, "y / y_hat_support must not be null");
     if (h->cfg.flags & TMAE_FLAG_SKIP_DEAD_LRP) return fail(h, TMAE_EINVAL, "forced support needs every lrp_transform");
     Plan* pl = nullptr;
-    if ((rc = build_plan(h, N, &pl, true))) return rc;
+    if ((rc = get_plan(h, PLAN_FORCED, N, &pl))) return rc;
     cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
     Workspace& w = h->ws;
     const size_t rk = (size_t)N * h->K;
@@ -2113,7 +2074,7 @@ int tmae_forward_host(tmae_handle* h, const float* h_imgs, const float* h_scores
     if (rc) return rc;
     if (!h_imgs || !h_scores) return fail(h, TMAE_EINVAL, "h_imgs / h_scores must not be null");
     Plan* pl = nullptr;
-    if ((rc = build_plan(h, N, &pl))) return rc;
+    if ((rc = get_plan(h, PLAN_FORWARD, N, &pl))) return rc;
     cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
     Workspace& w = h->ws;
     const size_t img_elems = (size_t)N * h->cfg.in_chans * h->cfg.img_size * h->cfg.img_size;
@@ -2130,15 +2091,7 @@ int tmae_forward_host(tmae_handle* h, const float* h_imgs, const float* h_scores
     if (ho.y_symbols && !o.y_symbols_i16) o.y_symbols_i16 = w.st_ysym;
     if (ho.z_symbols && !o.z_symbols_i16) o.z_symbols_i16 = w.st_zsym;
     if (ho.ids_restore && !o.ids_restore) o.ids_restore = w.st_ids_restore;
-    bool done = false;
-    if ((rc = run_full_graph(h, *pl, w.st_imgs, w.st_scores, &o, st, &done))) return rc;
-    if (!done) {
-        RunArgs a;
-        a.imgs = w.st_imgs; a.scores = w.st_scores; a.out = &o; a.begin = 0; a.end = (int)pl->steps.size();
-        if (h->profiling) h->prof_used = 0;
-        if ((rc = run_steps(h, *pl, a, st))) return rc;
-        if ((rc = copy_outputs(h, N, out, true, true, st))) return rc;
-    }
+    if ((rc = run_forward(h, *pl, w.st_imgs, w.st_scores, &o, st))) return rc;
     const size_t ny = (size_t)N * h->K * h->Cy, nz = (size_t)N * h->s4 * h->s4 * h->Cz;
     if (ho.bpp) CUDA_TRY(h, cudaMemcpyAsync(ho.bpp, o.bpp, (size_t)N * sizeof(float), cudaMemcpyDeviceToHost, st));
     if (ho.rate_sums) CUDA_TRY(h, cudaMemcpyAsync(ho.rate_sums, o.rate_sums, 2 * sizeof(double), cudaMemcpyDeviceToHost, st));
@@ -2156,10 +2109,7 @@ int tmae_set_scale_table(tmae_handle* h, const float* table, int n) {
     CUDA_TRY(h, cudaDeviceSynchronize());
     CUDA_TRY(h, cudaMemcpy(h->scale_table, table, (size_t)n * sizeof(float), cudaMemcpyDefault));
     h->n_scale_table = n;
-    // plans (and their captured graphs) carry the table pointer / length: rebuild them on the next call
-    drop_plans(h->plans);
-    drop_plans(h->dec_plans);
-    drop_plans(h->stream_plans);
+    drop_plans(h, DEP_SCALE);        // plans and their graphs carry the table pointer / length
     h->dec_next = -1;
     return TMAE_OK;
 }
@@ -2183,9 +2133,9 @@ int tmae_decode_begin(tmae_handle* h, const int32_t* z_symbols, int N, const tma
     if (!z_symbols || !out || !out->y_indexes) return fail(h, TMAE_EINVAL, "z_symbols, out and out->y_indexes must not be null");
     if (!h->scale_table) return fail(h, TMAE_ESTATE, "decoding needs the scale table (call tmae_set_scale_table first)");
     Plan* pl = nullptr;
-    if ((rc = build_decode_plan(h, N, &pl))) return rc;
+    if ((rc = get_plan(h, PLAN_DECODE, N, &pl))) return rc;
     if (h->profiling) h->prof_used = 0;
-    if ((rc = run_decode_stage(h, *pl, 0, decode_io(z_symbols, nullptr, out), reinterpret_cast<cudaStream_t>(stream)))) return rc;
+    if ((rc = run_stage(h, *pl, 0, decode_io(z_symbols, nullptr, out), h->ws.io, reinterpret_cast<cudaStream_t>(stream)))) return rc;
     h->dec_N = N;
     h->dec_next = 0;
     return TMAE_OK;
@@ -2195,14 +2145,14 @@ int tmae_decode_step(tmae_handle* h, int group, const int32_t* y_symbols, const 
     if (!h) return TMAE_EINVAL;
     if (!y_symbols || !out || !out->y_indexes) return fail(h, TMAE_EINVAL, "y_symbols, out and out->y_indexes must not be null");
     const int expected = h->dec_next;
-    auto it = h->dec_plans.find(h->dec_N);
+    auto it = h->plans.find(PlanKey(PLAN_DECODE, h->dec_N, 0, 0));
     h->dec_next = -1;                // an out-of-order step ends the decode as well
-    if (expected < 0 || group != expected || it == h->dec_plans.end())
+    if (expected < 0 || group != expected || it == h->plans.end())
         return fail(h, TMAE_ESTATE, "decode step %d out of order (expected %s%d): steps follow tmae_decode_begin in group order, "
                     "and any other call on the handle in between ends the decode", group, expected < 0 ? "a new tmae_decode_begin, not step " : "step ",
                     expected < 0 ? group : expected);
     Plan& pl = *it->second;
-    const int rc = run_decode_stage(h, pl, group + 1, decode_io(nullptr, y_symbols, out), reinterpret_cast<cudaStream_t>(stream));
+    const int rc = run_stage(h, pl, group + 1, decode_io(nullptr, y_symbols, out), h->ws.io, reinterpret_cast<cudaStream_t>(stream));
     if (rc) return rc;
     if (group + 2 < (int)pl.stage_begin.size() - 1) h->dec_next = group + 1;
     return TMAE_OK;
@@ -2226,7 +2176,7 @@ int tmae_enable_synthesis(tmae_handle* h, int decoder_depth, int decoder_num_hea
     if (!attention_hd32_supported(h->L + 1))
         return fail(h, TMAE_EINVAL, "synthesis attention over %d tokens does not fit shared memory", h->L + 1);
     h->dec_next = -1;
-    drop_plans(h->syn_plans);
+    drop_plans(h, DEP_SYNTH);
     if (decoder_depth != h->syn_depth || Dd != h->Dd || mlp != h->syn_mlp) {   // buffers sized for another decoder
         free_pool(h->sws.allocs);
         h->sws = SynthWorkspace();
@@ -2250,12 +2200,12 @@ int tmae_synthesize(tmae_handle* h, const float* y_hat, const int64_t* ids_resto
         return fail(h, TMAE_EINVAL, "y_hat and x_hat must be 16-byte aligned");
     if (h->cfg.in_chans != 3) return fail(h, TMAE_EINVAL, "synthesis writes 3-channel images (in_chans %d)", h->cfg.in_chans);
     Plan* pl = nullptr;
-    if ((rc = build_synth_plan(h, N, &pl))) return rc;
+    if ((rc = get_plan(h, PLAN_SYNTH, N, &pl))) return rc;
     IoBlock hio;
     memset(&hio, 0, sizeof(hio));
     hio.syn_y_hat = y_hat; hio.syn_ids = ids_restore; hio.syn_x_hat = x_hat;
     if (h->profiling) h->prof_used = 0;
-    return run_decode_stage(h, *pl, 0, hio, reinterpret_cast<cudaStream_t>(stream), h->sws.io);
+    return run_stage(h, *pl, 0, hio, h->sws.io, reinterpret_cast<cudaStream_t>(stream));
 }
 
 // ---- entropy coder (compressai's rANS format) -----------------------------------------------------------
@@ -2287,7 +2237,7 @@ int tmae_set_cdf_tables(tmae_handle* h, int model, const int32_t* cdf, int n_tab
     char err[256] = {0};
     const int rc = rans_build_tables(c.data(), n_tables, stride, len.data(), off.data(), &t, err, sizeof(err));
     if (rc) return fail(h, rc, "cdf tables: %s", err);
-    drop_plans(h->stream_plans);                     // their graphs captured the previous tables
+    drop_plans(h, DEP_CDF);                          // their graphs captured the previous tables
     rans_free_tables(&h->cdf[model]);
     h->cdf[model] = t;
     return TMAE_OK;
@@ -2370,12 +2320,12 @@ int decompress_streams_impl(tmae_handle* h, const uint8_t* y_data, const int64_t
     if (h->cdf[TMAE_MODEL_GAUSSIAN].n != h->n_scale_table)
         return fail(h, TMAE_ESTATE, "%d Gaussian cdf tables for a scale table of %d entries", h->cdf[TMAE_MODEL_GAUSSIAN].n, h->n_scale_table);
     Plan* pl = nullptr;
-    if ((rc = build_stream_decode_plan(h, N, y_lanes, z_lanes, &pl))) return rc;
+    if ((rc = get_plan(h, PLAN_STREAMS, N, &pl, y_lanes, z_lanes))) return rc;
     IoBlock hio = decode_io(h->cws.zsym, h->cws.ysym, out);
     if (!hio.out.y_indexes) hio.out.y_indexes = h->cws.idx;
     hio.y_data = y_data; hio.y_offsets = y_offsets; hio.z_data = z_data; hio.z_offsets = z_offsets; hio.status = status;
     if (h->profiling) h->prof_used = 0;
-    return run_decode_stage(h, *pl, 0, hio, reinterpret_cast<cudaStream_t>(stream));
+    return run_stage(h, *pl, 0, hio, h->ws.io, reinterpret_cast<cudaStream_t>(stream));
 }
 }  // namespace
 
@@ -2913,15 +2863,16 @@ int tmae_profile_read(tmae_handle* h, tmae_profile_entry* entries, int max_entri
     memset(fam, 0, sizeof(fam));
     for (int f = 0; f < FAM_COUNT; ++f) snprintf(fam[f].name, sizeof(fam[f].name), "%s", kFamilyNames[f]);
     for (size_t i = 0; i < h->prof_used; ++i) {
+        const ProfRecord& r = h->prof[i];
         float ms = 0.f;
-        cudaError_t e = cudaEventElapsedTime(&ms, h->prof_events[i].first, h->prof_events[i].second);
+        cudaError_t e = cudaEventElapsedTime(&ms, r.begin, r.end);
         if (e != cudaSuccess) return fail(h, TMAE_ECUDA, "cudaEventElapsedTime: %s (synchronise the stream first)", cudaGetErrorString(e));
-        tmae_profile_entry& f = fam[h->prof_family[i]];
-        f.launches += h->prof_launches[i];
+        tmae_profile_entry& f = fam[r.family];
+        f.launches += r.launches;
         f.ms += ms;
-        f.flops += h->prof_flops[i];
-        f.bytes += h->prof_bytes[i];
-        f.mma_flops += h->prof_mma[i];
+        f.flops += r.flops;
+        f.bytes += r.bytes;
+        f.mma_flops += r.mma_flops;
     }
     int n = 0;
     for (int f = 0; f < FAM_COUNT && n < max_entries; ++f)
@@ -2934,15 +2885,16 @@ int tmae_profile_read_steps(tmae_handle* h, tmae_profile_step* steps, int max_st
     if (!h || !steps || !n_steps) return TMAE_EINVAL;
     int n = 0;
     for (size_t i = 0; i < h->prof_used && n < max_steps; ++i, ++n) {
+        const ProfRecord& r = h->prof[i];
         float ms = 0.f;
-        cudaError_t e = cudaEventElapsedTime(&ms, h->prof_events[i].first, h->prof_events[i].second);
+        cudaError_t e = cudaEventElapsedTime(&ms, r.begin, r.end);
         if (e != cudaSuccess) return fail(h, TMAE_ECUDA, "cudaEventElapsedTime: %s (synchronise the stream first)", cudaGetErrorString(e));
         memset(&steps[n], 0, sizeof(steps[n]));
-        snprintf(steps[n].name, sizeof(steps[n].name), "%s", h->prof_tag[i].c_str());
+        snprintf(steps[n].name, sizeof(steps[n].name), "%s", r.tag.c_str());
         steps[n].ms = ms;
-        steps[n].flops = h->prof_flops[i];
-        steps[n].ctas = h->prof_ctas[i];
-        steps[n].block_n = h->prof_bn[i];
+        steps[n].flops = r.flops;
+        steps[n].ctas = r.ctas;
+        steps[n].block_n = r.block_n;
     }
     *n_steps = n;
     return TMAE_OK;
