@@ -382,6 +382,17 @@ TMAE_API int  tmae_launch_count(tmae_handle* h, int N);
  * Q box rows, K/V box rows, form (0 full, 1 lite, 2 duo)}. */
 TMAE_API int  tmae_attention_plan(int T, int H, int N, int mode, int* out);
 
+/* Host-only (no device needed): the launch the GEMM engine's policy picks for one GEMM step.
+ * shape[17] = {groups, max_M, max_N, conv (0/1), side, n_img, output (0 other, 1 one bf16 same-row output, 2 fp32 same-row
+ * output + residual), act (0 none, 1 GELU, 2 0.5 tanh), fused Gaussian (0 none, 1 encoder, 2 decoder), LayerNorm statistics in,
+ * LayerNorm statistics out, PixelShuffle output, TMA-store aligned output, share-SM, debug SIMT, forced block_n (0 = policy),
+ * forced form (-1 = policy)}; conv shapes need max_M = m_tiles * 128 of tmae_conv_geometry.
+ * out[15] = {form (0 one tile per CTA, 1 one-CTA persistent, 2 CTA pairs, 3 persistent CTA pairs, 4 CUDA-core checker), act,
+ * store-phase kind, block_n, row tiles, column tiles, grid x, y, z, threads per CTA, dynamic shared memory, pipeline stages,
+ * k-blocks per stage, second producer warp, conv A-reuse stage bytes}.  Returns TMAE_EINVAL for an invalid shape or a forced
+ * form the shape rules out.  The A/B switches of INTEGRATION.md apply. */
+TMAE_API int  tmae_gemm_launch_plan(const int* shape, int* out);
+
 /* Host-only (no device needed): the CTA tiling the conv engine uses for an s x s grid of n_img images.
  * out[6] = {box_y, box_n, y_tiles, m_tiles, rows_used, reuse_ok}.  A tile covers image rows [y0, y0 + box_y) of images
  * [n0, n0 + box_n); rows_used = s * box_y * box_n <= 128 accumulator rows; reuse_ok = the haloed-box A reuse applies

@@ -118,6 +118,7 @@ SIGNATURES = {
     "tmae_profile_read_steps": (C.c_int, [_P, C.POINTER(TmaeProfileStep), C.c_int, C.POINTER(C.c_int)]),
     "tmae_launch_count": (C.c_int, [_P, C.c_int]),
     "tmae_attention_plan": (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_int)]),
+    "tmae_gemm_launch_plan": (C.c_int, [C.POINTER(C.c_int), C.POINTER(C.c_int)]),
     "tmae_conv_geometry": (C.c_int, [C.c_int, C.c_int, C.POINTER(C.c_int)]),
 }
 

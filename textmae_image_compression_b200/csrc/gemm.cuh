@@ -129,4 +129,71 @@ struct alignas(64) GemmParams {
     long long* dbg_ticks;             // optional [ctas][8] globaltimer stamps of the kernel phases (bring-up)
 };
 
+// EPI selects a compile-time specialisation of the store phase:
+//   EPI_GENERIC        any row map / two outputs / gathered residual (patch embed, g_a.6, strided, PixelShuffle, mu/sigma, LRP)
+//   EPI_BF16_SAME      one bf16 output at the accumulator's own row (QKV, fc1, g_a.0-4, every conv mid layer)
+//   EPI_F32_SAME_RESID one fp32 output at the accumulator's own row with an fp32 residual at the same row (proj, fc2)
+//   EPI_BF16_TMA       EPI_BF16_SAME when the tile is 128 consecutive output rows and block_n % 32 == 0: bias/activation in
+//                      registers, bf16 boxes of 32 columns staged in smem (64B swizzle) and written by TMA stores
+//   EPI_GAUSS          last layer of cc_transform_mean[i] + cc_transform_scale[i] as one block-diagonal 64-column GEMM: the
+//                      Gaussian conditional (quantise, likelihood, symbols, indexes, y_hat, rate) runs here, thread = pixel
+//   EPI_GAUSS_IDX      the same layer in the decoder (GemmParams::gc_on == 2): mu, sigma and scale-table indexes only
+enum EpiKind : int { EPI_GENERIC = 0, EPI_BF16_SAME = 1, EPI_F32_SAME_RESID = 2, EPI_BF16_TMA = 3, EPI_GAUSS = 4, EPI_GAUSS_IDX = 5 };
+
+// ---- launch policy (host) ------------------------------------------------------------------------------
+// The kernel a GEMM step launches.
+enum GemmForm : int {
+    ONE_CTA = 0,       // gemm_tc_kernel: one 128 x block_n tile per CTA
+    PERSISTENT,        // gemm_tc_persistent_kernel: one CTA per SM, tiles round-robin, double-buffered tensor memory
+    PAIR,              // gemm_tc_pair_kernel: CTA pairs (cta_group::2), 256-row tiles, each CTA stages half of the weight tile
+    PAIR_PERSISTENT,   // gemm_tc_pair_persistent_kernel: one cluster per TPC, pair tiles round-robin
+    SIMT               // gemm_simt_kernel: the CUDA-core checker (bring-up / tests)
+};
+// Output of every member of a step, as far as the store phase cares.
+enum GemmOut : int {
+    GOUT_OTHER = 0,
+    GOUT_BF16 = 1,         // one bf16 output at the accumulator's own row, no residual
+    GOUT_F32_RESID = 2     // one fp32 output at the accumulator's own row, fp32 residual read at the same row
+};
+
+// Tiling of a conv layer over an s x s grid: a CTA tile is box_y image rows of box_n images (s * box_y * box_n <= 128
+// accumulator rows).  reuse_ok: the tile allows the haloed-box A reuse (GemmParams::conv_reuse).
+struct ConvGeom { int box_y = 0, box_n = 0, y_tiles = 0, m_tiles = 0, rows_used = 0; bool reuse_ok = false; };
+
+// What the launch policy reads about one GEMM step (every member of a grouped launch).
+struct GemmShape {
+    int groups = 1, max_M = 0, max_N = 0;   // members, and the rows / output channels of the largest
+    bool conv = false;                      // IN_CONV members, all on the grid `side` x `side` of `n_img` images
+    int side = 0, n_img = 0;
+    int out = GOUT_OTHER;                   // GemmOut shared by every member (GOUT_OTHER if they differ)
+    int act = ACT_NONE;                     // shared by every member
+    int gauss = 0;                          // fused Gaussian conditional: 1 encoder (EPI_GAUSS), 2 decoder (EPI_GAUSS_IDX)
+    bool ln_in = false, ln_out = false;     // folded LayerNorm: statistics read (consumer) / written (producer)
+    bool shuffle = false;                   // a PixelShuffle output map
+    bool tma_store_ok = false;              // every member's output can take TMA stores (else the register store phase)
+    bool share_sm = false;                  // TMAE_FLAG_SHARE_SM
+    bool simt = false;                      // TMAE_FLAG_DEBUG_SIMT
+    // engine self-tests only: a forced tile width (0 = policy) and form (-1 = policy).  A forced form skips the plan's
+    // tile-width refinements; forced ONE_CTA still runs the one-CTA persistent kernel where that qualifies.
+    int force_block_n = 0, force_form = -1;
+};
+
+// Everything one GEMM launch needs, decided by gemm_resolve.
+struct GemmLaunch {
+    int form = ONE_CTA, act = ACT_NONE, epi = EPI_GENERIC, block_n = 0;
+    int m_tiles = 0, n_tiles = 0;           // tile grid of the largest member (128-row x block_n-column tiles)
+    int grid[3] = {0, 0, 0}, block = 0, smem = 0;
+    int stages = 0, kgroup = 1, two_producers = 0;
+    int conv_reuse_stage = 0;               // bytes of one stage of the haloed-box A reuse; 0 = one A box per tap
+};
+
+// A/B switches of the engine's launch policy, read from the environment once per process.
+struct GemmOptions {
+    bool no_persistent, no_tma_store, no_pair, no_pair_conv, no_pair_persistent, pp_share, no_conv_reuse,
+         no_weight_prefetch, plan_debug;
+    int two_producers;                      // TMAE_TWO_PRODUCERS, -1 = unset
+    int kgroup;                             // TMAE_KGROUP, 0 = unset
+    int bn_round;                           // TMAE_BN_ROUND: 0 never, 1 always, 2 linear layers only (default)
+};
+
 }  // namespace tmae

@@ -228,16 +228,7 @@ constexpr int kGemmThreads = 320;                     // warp 0 TMA, warp 1 MMA,
 constexpr int kEpiPitch = 36;                         // floats per staged accumulator row (32 + 4 pad)
 constexpr int kAStageBytes = kBlockM * kBlockK * 2;   // 16 KB
 
-// EPI selects a compile-time specialisation of the store phase:
-//   EPI_GENERIC        any row map / two outputs / gathered residual (patch embed, g_a.6, strided, PixelShuffle, mu/sigma, LRP)
-//   EPI_BF16_SAME      one bf16 output at the accumulator's own row (QKV, fc1, g_a.0-4, every conv mid layer)
-//   EPI_F32_SAME_RESID one fp32 output at the accumulator's own row with an fp32 residual at the same row (proj, fc2)
-//   EPI_BF16_TMA       EPI_BF16_SAME when the tile is 128 consecutive output rows and block_n % 32 == 0: bias/activation in
-//                      registers, bf16 boxes of 32 columns staged in smem (64B swizzle) and written by TMA stores
-//   EPI_GAUSS          last layer of cc_transform_mean[i] + cc_transform_scale[i] as one block-diagonal 64-column GEMM: the
-//                      Gaussian conditional (quantise, likelihood, symbols, indexes, y_hat, rate) runs here, thread = pixel
-//   EPI_GAUSS_IDX      the same layer in the decoder (GemmParams::gc_on == 2): mu, sigma and scale-table indexes only
-enum EpiKind : int { EPI_GENERIC = 0, EPI_BF16_SAME = 1, EPI_F32_SAME_RESID = 2, EPI_BF16_TMA = 3, EPI_GAUSS = 4, EPI_GAUSS_IDX = 5 };
+// EPI: the store-phase specialisation (EpiKind, gemm.cuh)
 constexpr uint32_t kStoreBoxBytes = kBlockM * 32 * 2;      // one 128 x 32 bf16 box
 
 // ---------------------------------------------------------------------------------------------------------
@@ -1275,10 +1266,78 @@ gemm_simt_kernel(const GemmParams* __restrict__ params) {
 }
 
 // ---------------------------------------------------------------------------------------------------------
-// host launchers
+// host launch policy: gemm_resolve decides every GEMM launch, gemm_launch only launches
 // ---------------------------------------------------------------------------------------------------------
+const GemmOptions& gemm_options() {
+    static const GemmOptions opts = [] {
+        auto on = [](const char* k) { return getenv(k) != nullptr; };
+        auto num = [](const char* k, int unset) { const char* v = getenv(k); return v ? atoi(v) : unset; };
+        GemmOptions o;
+        o.no_persistent = on("TMAE_NO_PERSISTENT");
+        o.no_tma_store = on("TMAE_NO_TMA_STORE");
+        o.no_pair = on("TMAE_NO_PAIR");
+        o.no_pair_conv = on("TMAE_NO_PAIR_CONV");
+        o.no_pair_persistent = on("TMAE_NO_PAIR_PERSISTENT");
+        o.pp_share = on("TMAE_PP_SHARE");                  // experiment: persistent pairs also while several streams share the GPU
+        o.no_conv_reuse = on("TMAE_NO_CONV_REUSE");
+        o.no_weight_prefetch = on("TMAE_NO_WEIGHT_PREFETCH");
+        o.plan_debug = on("TMAE_PLAN_DEBUG");
+        o.two_producers = num("TMAE_TWO_PRODUCERS", -1);
+        o.kgroup = num("TMAE_KGROUP", 0);
+        o.bn_round = num("TMAE_BN_ROUND", 2);
+        return o;
+    }();
+    return opts;
+}
+
+// Tiling of a conv layer over an s x s grid: pick the (box_y, box_n) pair with the fewest tiles.  A pair whose dy shift
+// (box_n * s rows) is a whole number of 8-row swizzle atoms can use the haloed-box A reuse (GemmParams::conv_reuse); such a
+// pair wins unless it costs more than 15 % extra tiles.
+bool conv_geom(int s, int n_img, ConvGeom* g) {
+    if (s <= 0 || s > kBlockM || n_img <= 0) return false;
+    long long best[2] = {-1, -1};          // [0] any pair, [1] reuse-compatible pair
+    ConvGeom cand[2];
+    for (int by = (s < kBlockM / s ? s : kBlockM / s); by >= 1; --by) {
+        for (int pass = 0; pass < 2; ++pass) {
+            int bn = kBlockM / (s * by);
+            if (bn > 256) bn = 256;
+            if (pass == 0) { if (bn > n_img) bn = n_img; }
+            else {
+                int q = 8; for (int d = 8; d >= 1; d >>= 1) if (s % d == 0) { q = 8 / d; break; }   // q = 8 / gcd(s, 8)
+                bn = bn / q * q;                                   // box_n * s must be a multiple of 8 rows
+                while (bn - q >= n_img && bn - q > 0) bn -= q;     // no more images per tile than needed
+                if (by < 2) bn = 0;                                // one row + two halo rows: nothing to reuse
+            }
+            if (bn <= 0) continue;
+            const int yt = (s + by - 1) / by;
+            const long long tiles = (long long)((n_img + bn - 1) / bn) * yt;
+            if (best[pass] < 0 || tiles < best[pass]) {
+                best[pass] = tiles;
+                cand[pass].box_y = by; cand[pass].box_n = bn; cand[pass].y_tiles = yt; cand[pass].m_tiles = (int)tiles;
+                cand[pass].rows_used = s * by * bn; cand[pass].reuse_ok = pass == 1;
+            }
+        }
+    }
+    if (best[0] < 0) return false;
+    *g = (!gemm_options().no_conv_reuse && best[1] > 0 && best[1] * 100 <= best[0] * 115) ? cand[1] : cand[0];
+    return true;
+}
+
+// Choose the N tile: fewest column tiles that still give the machine >= ~120 CTAs (148 SMs), multiple of 16.
+static int pick_block_n(int m_tiles, int N, int groups) {
+    auto round16 = [](int c) { return (c + 15) / 16 * 16; };
+    int best = round16(N) > 256 ? 256 : round16(N);
+    for (int nt = 1; nt <= 16; ++nt) {
+        int bn = round16((N + nt - 1) / nt);
+        if (bn > 256) continue;
+        best = bn;
+        if ((long long)m_tiles * nt * groups >= 120 || bn <= 64) break;
+    }
+    return best;
+}
+
 // conv_reuse launches: a stage is one haloed A box + three B atoms (`stage_bytes`); returns 0 if fewer than 2 fit
-int gemm_reuse_stages(int stage_bytes, int total_ctas, bool share_sm, int* smem_bytes) {
+static int reuse_stages(int stage_bytes, int total_ctas, bool share_sm, int* smem_bytes) {
     const int overhead = 256;
     const bool whole_sm = total_ctas <= 148 && !share_sm;
     const int budget = (whole_sm ? 226 : 113) * 1024 - overhead;
@@ -1289,13 +1348,12 @@ int gemm_reuse_stages(int stage_bytes, int total_ctas, bool share_sm, int* smem_
     return stages;
 }
 
-int gemm_pick_stages(int block_n, int total_ctas, bool share_sm, int* smem_bytes, int* kgroup) {
+static int pick_stages(int block_n, int total_ctas, bool share_sm, int force_g, int* smem_bytes, int* kgroup) {
     // Small tiles are bound by (a) the TMA round trip: bytes in flight per SM is what matters, and (b) the ~300-cycle
     // producer <-> MMA handshake per pipeline stage: see produce_tile.  A single wave (<= 148 CTAs) gets the whole
     // shared memory of its SM; larger grids run two CTAs per SM so that one CTA's epilogue overlaps the other's loop.
     // share_sm: several handles / streams are in flight on this GPU, so even a single-wave launch keeps to half the
     // shared memory and lets a CTA of another stream's kernel co-reside (measured +9 % throughput at 3 streams).
-    static const int force_g = getenv("TMAE_KGROUP") ? atoi(getenv("TMAE_KGROUP")) : 0;
     const int atom = kAStageBytes + block_n * kBlockK * 2;
     const int overhead = 256;                       // barriers + TMEM slot (the pipeline itself starts at offset 0)
     const bool whole_sm = total_ctas <= 148 && !share_sm;
@@ -1314,196 +1372,230 @@ int gemm_pick_stages(int block_n, int total_ctas, bool share_sm, int* smem_bytes
     return stages;
 }
 
-template <int ACT, int EPI>
-static cudaError_t configure_one() {
-    prefer_max_smem_carveout(gemm_tc_kernel<ACT, EPI>);
-    return cudaFuncSetAttribute(gemm_tc_kernel<ACT, EPI>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
+bool gemm_resolve(const GemmShape& s, GemmLaunch* out) {
+    const GemmOptions& o = gemm_options();
+    if (s.groups < 1 || s.max_M <= 0 || s.max_N <= 0 || s.force_block_n < 0) return false;
+    GemmLaunch L;
+    L.act = s.act;
+    L.m_tiles = (s.max_M + kBlockM - 1) / kBlockM;
+    const bool forced = s.force_form >= 0;
+
+    // ---- tile width
+    int bn = s.force_block_n > 0 ? s.force_block_n : pick_block_n(L.m_tiles, s.max_N, s.groups);
+    if (!forced) {
+        if (s.gauss) bn = 32;                  // fused Gaussian epilogue: one 32-column chunk (16 channels: mu | sigma) per CTA
+        if (!s.share_sm && s.groups == 1 && s.out == GOUT_BF16 && L.m_tiles * ((s.max_N + 255) / 256) > 2 * 148 - 1) {
+            // persistent-kernel candidate: tiles are dealt round-robin to 148 CTAs -> minimise rounds x (tile width + fixed cost)
+            long long best_cost = -1;
+            for (int cand = 256; cand >= 128; cand -= 16) {
+                const int tiles = L.m_tiles * ((s.max_N + cand - 1) / cand);
+                const long long cost = (long long)((tiles + 147) / 148) * (cand + 48);
+                if (best_cost < 0 || cost < best_cost) { best_cost = cost; bn = cand; }
+            }
+        }
+        // layers whose store phase can go through TMA: 32-column boxes -> block_n % 32 == 0.  conv layers keep their exact
+        // tile width (rounding 112 -> 128 or 80 -> 96 computes 14-20 % dead columns; such layers use the register/smem store
+        // phase instead): measured equal or slightly better at the power cap
+        const bool tma_layer = !o.no_tma_store && s.out == GOUT_BF16 && s.act != ACT_HALF_TANH;
+        if (tma_layer && bn % 32 != 0 && bn + 16 <= 256 && (o.bn_round == 1 || (o.bn_round == 2 && !s.conv))) bn += 16;
+        // PixelShuffle epilogue: a 32-column chunk must not straddle a quadrant; LayerNorm statistics: one slot per
+        // 32-column chunk, owned by exactly one tile
+        if (s.shuffle || s.ln_out) bn = (bn + 31) / 32 * 32;
+    }
+    L.block_n = bn;
+    L.n_tiles = (s.max_N + bn - 1) / bn;
+
+    // ---- store phase
+    if (s.gauss) L.epi = s.gauss == 2 ? EPI_GAUSS_IDX : EPI_GAUSS;
+    else if (s.out == GOUT_BF16 && s.act != ACT_HALF_TANH)
+        L.epi = (s.tma_store_ok && bn % 32 == 0 && !o.no_tma_store) ? EPI_BF16_TMA : EPI_BF16_SAME;
+    else if (s.out == GOUT_F32_RESID && !s.conv && s.act == ACT_NONE) L.epi = EPI_F32_SAME_RESID;
+    else L.epi = EPI_GENERIC;
+    const bool bf16_kernel = (L.epi == EPI_BF16_SAME || L.epi == EPI_BF16_TMA) && (s.act == ACT_NONE || s.act == ACT_GELU);
+
+    // ---- form
+    const int m_pairs = (L.m_tiles + 1) / 2;
+    L.form = s.force_form;
+    if (!forced) {
+        // CTA pairs.  Linear layers: one bf16 / fp32+residual same-row output and >= 8 row tiles (the encoder GEMMs).  3x3 conv
+        // layers: >= 8 row tiles and a weight tile of >= 64 columns (below that the B tile is too small for halving it to
+        // matter and the launch is latency bound).  The Gaussian epilogue lives in the one-CTA kernel.
+        const bool pair_layer = s.conv ? !o.no_pair_conv && bn >= 64
+                                       : s.groups == 1 && ((s.out == GOUT_BF16 && (s.act == ACT_NONE || s.act == ACT_GELU)) ||
+                                                           (s.out == GOUT_F32_RESID && s.act == ACT_NONE));
+        const bool pair = !s.simt && !s.gauss && !o.no_pair && (bn & 15) == 0 && s.max_M >= 8 * kBlockM && pair_layer;
+        // Persistent pairs: a linear layer that qualifies for pairs, bf16 same-row output, one batch in flight (a persistent
+        // launch owns every SM) and more pair tiles than one round of the 74 clusters.
+        const bool pair_persistent = pair && !o.no_pair_persistent && (!s.share_sm || o.pp_share) && !s.conv && s.groups == 1 &&
+                                     bf16_kernel && m_pairs * L.n_tiles > 74;
+        L.form = s.simt ? SIMT : pair_persistent ? PAIR_PERSISTENT : pair ? PAIR : ONE_CTA;
+    }
+    const bool pair_form = L.form == PAIR || L.form == PAIR_PERSISTENT;
+    if (pair_form && (bn & 15) != 0) return false;           // each CTA of a pair stages block_n / 2 rows of B
+
+    // ---- 3x3 conv: haloed-box A reuse when the geometry allows it and at least two stages (one haloed A box + three B atoms
+    // each) fit the launch's shared-memory budget.  A tap's MMA always reads 128 rows from its dy offset: with a partial tile
+    // the rows past the A box must still lie inside the stage (they land in the B atoms; the rows they feed are never stored).
+    ConvGeom cg;
+    if (s.conv && conv_geom(s.side, s.n_img, &cg) && cg.reuse_ok) {
+        const int bn_cta = pair_form ? bn / 2 : bn;          // B rows this CTA stages (a pair splits the weight tile)
+        const int stage = ((cg.box_y + 2) * cg.box_n * s.side + 3 * bn_cta) * kBlockK * 2;
+        int smem = 0;
+        if (cg.rows_used + 3 * bn_cta >= kBlockM && reuse_stages(stage, cg.m_tiles * L.n_tiles * s.groups, s.share_sm, &smem) >= 2)
+            L.conv_reuse_stage = stage;
+    }
+
+    // ---- launch geometry and pipeline depth
+    const int gx = L.m_tiles, gy = L.n_tiles, gz = s.groups;
+    auto set_grid = [&L](int x, int y, int z, int block) { L.grid[0] = x; L.grid[1] = y; L.grid[2] = z; L.block = block; };
+    const int persist_overhead = 1024 + 256 + kEpiStageBytes;
+    if (L.form == ONE_CTA && L.conv_reuse_stage == 0 && !o.no_persistent && !s.share_sm && gz == 1 && bf16_kernel && gx * gy > 2 * 148) {
+        // One-CTA persistent kernel: one group, bf16 same-row output, more tiles than 2 per SM.  Not used when several
+        // streams share the GPU: a persistent launch owns every SM (one CTA, all of its shared memory), which removes the
+        // cross-stream overlap that mode relies on (measured: 26.5k vs 25.9k images/s at 3 streams).
+        L.form = PERSISTENT;
+    }
+    switch (L.form) {
+        case SIMT:
+            set_grid(s.max_M, 1, gz, 128);
+            break;
+        case ONE_CTA:
+            L.stages = L.conv_reuse_stage > 0 ? reuse_stages(L.conv_reuse_stage, gx * gy * gz, s.share_sm, &L.smem)
+                                              : pick_stages(bn, gx * gy * gz, s.share_sm, o.kgroup, &L.smem, &L.kgroup);
+            if (L.stages == 0) return false;
+            // Second producer warp (TMAE_TWO_PRODUCERS=1): in isolation it shortens producer-bound main loops (64-wide GEMM
+            // tiles -20 %, fc2 -8 %), but since the conv layers moved to one haloed A box per three taps the whole forward is
+            // 4 % FASTER without it (25.6k vs 24.4k images/s, one batch in flight; equal with four) - off by default.
+            L.two_producers = o.two_producers >= 0 ? o.two_producers : 0;
+            set_grid(gx, gy, gz, kGemmThreads);
+            break;
+        case PERSISTENT: {
+            const int stage = kAStageBytes + bn * kBlockK * 2;
+            L.stages = (226 * 1024 - persist_overhead) / stage;
+            if (L.stages > 8) L.stages = 8;
+            L.smem = persist_overhead + L.stages * stage;
+            set_grid(gx * gy < 148 ? gx * gy : 148, 1, 1, kPersistThreads);
+            break;
+        }
+        case PAIR: {
+            const int px = m_pairs * 2;                      // whole pairs along x
+            const int stage = L.conv_reuse_stage > 0 ? L.conv_reuse_stage : kAStageBytes + (bn / 2) * kBlockK * 2;
+            const int overhead = 256;
+            const bool whole_sm = px * gy * gz <= 148 && !s.share_sm;
+            const int cap = L.conv_reuse_stage > 0 ? 4 : 8;
+            L.stages = ((whole_sm ? 226 : 113) * 1024 - overhead) / stage;
+            if (L.stages > cap) L.stages = cap;
+            if (L.stages < 2) return false;
+            L.smem = overhead + L.stages * stage;
+            set_grid(px, gy, gz, kGemmThreads);
+            break;
+        }
+        case PAIR_PERSISTENT: {
+            // one cluster per TPC, tiles round-robin
+            if (gz != 1 || L.conv_reuse_stage != 0 || !bf16_kernel) return false;
+            const int stage = kAStageBytes + (bn / 2) * kBlockK * 2;
+            L.stages = (226 * 1024 - persist_overhead) / stage;
+            if (L.stages > 8) L.stages = 8;
+            if (L.stages < 2) return false;
+            L.smem = persist_overhead + L.stages * stage;
+            const int tiles = m_pairs * gy;
+            set_grid(2 * (tiles < 74 ? tiles : 74), 1, 1, kPersistThreads);
+            break;
+        }
+        default:
+            return false;
+    }
+    *out = L;
+    return true;
+}
+
+// ---------------------------------------------------------------------------------------------------------
+// kernel tables: (act, epi) -> instantiated kernel, one table per form.  gemm_tc_configure sets up exactly these, and
+// gemm_launch launches nothing else.
+// ---------------------------------------------------------------------------------------------------------
+template <typename F>
+struct GemmKernel { int act, epi; F fn; };
+using OneCtaFn = void (*)(const GemmParams*, int, int, const GemmParams*, int, int);
+using PairFn = void (*)(const GemmParams*, int, const GemmParams*, int);
+using PersistentFn = void (*)(const GemmParams*, int, int, int, const GemmParams*, int);
+#define TMAE_GEMM_KERNEL(kernel, A, E) {A, E, kernel<A, E>}
+static const GemmKernel<OneCtaFn> kOneCtaKernels[] = {
+    TMAE_GEMM_KERNEL(gemm_tc_kernel, ACT_NONE, EPI_GENERIC),       TMAE_GEMM_KERNEL(gemm_tc_kernel, ACT_GELU, EPI_GENERIC),
+    TMAE_GEMM_KERNEL(gemm_tc_kernel, ACT_HALF_TANH, EPI_GENERIC),  TMAE_GEMM_KERNEL(gemm_tc_kernel, ACT_NONE, EPI_BF16_SAME),
+    TMAE_GEMM_KERNEL(gemm_tc_kernel, ACT_GELU, EPI_BF16_SAME),     TMAE_GEMM_KERNEL(gemm_tc_kernel, ACT_NONE, EPI_F32_SAME_RESID),
+    TMAE_GEMM_KERNEL(gemm_tc_kernel, ACT_NONE, EPI_GAUSS),         TMAE_GEMM_KERNEL(gemm_tc_kernel, ACT_NONE, EPI_GAUSS_IDX),
+    TMAE_GEMM_KERNEL(gemm_tc_kernel, ACT_NONE, EPI_BF16_TMA),      TMAE_GEMM_KERNEL(gemm_tc_kernel, ACT_GELU, EPI_BF16_TMA),
+};
+static const GemmKernel<PairFn> kPairKernels[] = {
+    TMAE_GEMM_KERNEL(gemm_tc_pair_kernel, ACT_NONE, EPI_BF16_TMA),       TMAE_GEMM_KERNEL(gemm_tc_pair_kernel, ACT_GELU, EPI_BF16_TMA),
+    TMAE_GEMM_KERNEL(gemm_tc_pair_kernel, ACT_NONE, EPI_BF16_SAME),      TMAE_GEMM_KERNEL(gemm_tc_pair_kernel, ACT_GELU, EPI_BF16_SAME),
+    TMAE_GEMM_KERNEL(gemm_tc_pair_kernel, ACT_NONE, EPI_F32_SAME_RESID), TMAE_GEMM_KERNEL(gemm_tc_pair_kernel, ACT_NONE, EPI_GENERIC),
+    TMAE_GEMM_KERNEL(gemm_tc_pair_kernel, ACT_GELU, EPI_GENERIC),        TMAE_GEMM_KERNEL(gemm_tc_pair_kernel, ACT_HALF_TANH, EPI_GENERIC),
+};
+static const GemmKernel<PersistentFn> kPersistentKernels[] = {
+    TMAE_GEMM_KERNEL(gemm_tc_persistent_kernel, ACT_NONE, EPI_BF16_TMA),  TMAE_GEMM_KERNEL(gemm_tc_persistent_kernel, ACT_GELU, EPI_BF16_TMA),
+    TMAE_GEMM_KERNEL(gemm_tc_persistent_kernel, ACT_NONE, EPI_BF16_SAME), TMAE_GEMM_KERNEL(gemm_tc_persistent_kernel, ACT_GELU, EPI_BF16_SAME),
+};
+static const GemmKernel<PersistentFn> kPairPersistentKernels[] = {
+    TMAE_GEMM_KERNEL(gemm_tc_pair_persistent_kernel, ACT_NONE, EPI_BF16_TMA),
+    TMAE_GEMM_KERNEL(gemm_tc_pair_persistent_kernel, ACT_GELU, EPI_BF16_TMA),
+    TMAE_GEMM_KERNEL(gemm_tc_pair_persistent_kernel, ACT_NONE, EPI_BF16_SAME),
+    TMAE_GEMM_KERNEL(gemm_tc_pair_persistent_kernel, ACT_GELU, EPI_BF16_SAME),
+};
+#undef TMAE_GEMM_KERNEL
+
+template <typename F, size_t N>
+static F find_kernel(const GemmKernel<F> (&table)[N], const GemmLaunch& L) {
+    for (const GemmKernel<F>& k : table)
+        if (k.act == L.act && k.epi == L.epi) return k.fn;
+    return nullptr;
+}
+
+template <typename F, size_t N>
+static cudaError_t configure_table(const GemmKernel<F> (&table)[N]) {
+    for (const GemmKernel<F>& k : table) {
+        prefer_max_smem_carveout(k.fn);
+        const cudaError_t e = cudaFuncSetAttribute(k.fn, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
+        if (e != cudaSuccess) return e;
+    }
+    return cudaSuccess;
 }
 
 cudaError_t gemm_tc_configure() {
     cudaError_t e;
-    if ((e = configure_one<ACT_NONE, EPI_GENERIC>()) != cudaSuccess) return e;
-    if ((e = configure_one<ACT_GELU, EPI_GENERIC>()) != cudaSuccess) return e;
-    if ((e = configure_one<ACT_HALF_TANH, EPI_GENERIC>()) != cudaSuccess) return e;
-    if ((e = configure_one<ACT_NONE, EPI_BF16_SAME>()) != cudaSuccess) return e;
-    if ((e = configure_one<ACT_GELU, EPI_BF16_SAME>()) != cudaSuccess) return e;
-    if ((e = configure_one<ACT_NONE, EPI_F32_SAME_RESID>()) != cudaSuccess) return e;
-    if ((e = configure_one<ACT_NONE, EPI_GAUSS>()) != cudaSuccess) return e;
-    if ((e = configure_one<ACT_NONE, EPI_GAUSS_IDX>()) != cudaSuccess) return e;
-    if ((e = configure_one<ACT_NONE, EPI_BF16_TMA>()) != cudaSuccess) return e;
-    if ((e = configure_one<ACT_GELU, EPI_BF16_TMA>()) != cudaSuccess) return e;
-    {
-        auto cfgp = [](auto kern) {
-            prefer_max_smem_carveout(kern);
-            return cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
-        };
-        if ((e = cfgp(gemm_tc_pair_kernel<ACT_NONE, EPI_BF16_TMA>)) != cudaSuccess) return e;
-        if ((e = cfgp(gemm_tc_pair_kernel<ACT_GELU, EPI_BF16_TMA>)) != cudaSuccess) return e;
-        if ((e = cfgp(gemm_tc_pair_kernel<ACT_NONE, EPI_BF16_SAME>)) != cudaSuccess) return e;
-        if ((e = cfgp(gemm_tc_pair_kernel<ACT_GELU, EPI_BF16_SAME>)) != cudaSuccess) return e;
-        if ((e = cfgp(gemm_tc_pair_kernel<ACT_NONE, EPI_F32_SAME_RESID>)) != cudaSuccess) return e;
-        if ((e = cfgp(gemm_tc_pair_kernel<ACT_NONE, EPI_GENERIC>)) != cudaSuccess) return e;
-        if ((e = cfgp(gemm_tc_pair_kernel<ACT_GELU, EPI_GENERIC>)) != cudaSuccess) return e;
-        if ((e = cfgp(gemm_tc_pair_kernel<ACT_HALF_TANH, EPI_GENERIC>)) != cudaSuccess) return e;
-    }
-    {
-        auto cfgpp = [](auto kernel) {
-            prefer_max_smem_carveout(kernel);
-            return cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
-        };
-        if ((e = cfgpp(gemm_tc_pair_persistent_kernel<ACT_NONE, EPI_BF16_TMA>)) != cudaSuccess) return e;
-        if ((e = cfgpp(gemm_tc_pair_persistent_kernel<ACT_GELU, EPI_BF16_TMA>)) != cudaSuccess) return e;
-        if ((e = cfgpp(gemm_tc_pair_persistent_kernel<ACT_NONE, EPI_BF16_SAME>)) != cudaSuccess) return e;
-        if ((e = cfgpp(gemm_tc_pair_persistent_kernel<ACT_GELU, EPI_BF16_SAME>)) != cudaSuccess) return e;
-    }
-    prefer_max_smem_carveout(gemm_tc_persistent_kernel<ACT_NONE, EPI_BF16_TMA>);
-    prefer_max_smem_carveout(gemm_tc_persistent_kernel<ACT_GELU, EPI_BF16_TMA>);
-    if ((e = cudaFuncSetAttribute(gemm_tc_persistent_kernel<ACT_NONE, EPI_BF16_TMA>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024)) != cudaSuccess) return e;
-    if ((e = cudaFuncSetAttribute(gemm_tc_persistent_kernel<ACT_GELU, EPI_BF16_TMA>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024)) != cudaSuccess) return e;
-    prefer_max_smem_carveout(gemm_tc_persistent_kernel<ACT_NONE, EPI_BF16_SAME>);
-    prefer_max_smem_carveout(gemm_tc_persistent_kernel<ACT_GELU, EPI_BF16_SAME>);
-    if ((e = cudaFuncSetAttribute(gemm_tc_persistent_kernel<ACT_NONE, EPI_BF16_SAME>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024)) != cudaSuccess) return e;
-    return cudaFuncSetAttribute(gemm_tc_persistent_kernel<ACT_GELU, EPI_BF16_SAME>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
+    if ((e = configure_table(kOneCtaKernels)) != cudaSuccess) return e;
+    if ((e = configure_table(kPairKernels)) != cudaSuccess) return e;
+    if ((e = configure_table(kPairPersistentKernels)) != cudaSuccess) return e;
+    return configure_table(kPersistentKernels);
 }
 
-// Persistent launch qualifies: one group, bf16 same-row output, more tiles than 2 per SM.
-// Not used when several streams share the GPU: a persistent launch owns every SM (one CTA, all of its shared memory),
-// which removes the cross-stream overlap that mode relies on (measured: 26.5k vs 25.9k images/s at 3 streams).
-bool gemm_use_persistent(int groups, int epi, int act, int tiles, bool share_sm) {
-    static const bool off = getenv("TMAE_NO_PERSISTENT") != nullptr;
-    return !off && !share_sm && groups == 1 && (epi == EPI_BF16_SAME || epi == EPI_BF16_TMA) && (act == ACT_NONE || act == ACT_GELU) && tiles > 2 * 148;
-}
-
-// Store-phase specialisation a parameter block qualifies for (every member of a grouped launch must agree).
-int gemm_epi_kind(const GemmParams& p) {
-    if (p.gc_on) return p.gc_on == 2 ? EPI_GAUSS_IDX : EPI_GAUSS;
-    const bool one_out = p.out[1].dtype == OUT_NONE && p.out[0].map == MAP_SAME;
-    static const bool no_tma_store = getenv("TMAE_NO_TMA_STORE") != nullptr;
-    if (one_out && p.out[0].dtype == OUT_BF16 && p.resid == nullptr && p.act != ACT_HALF_TANH)
-        return (p.tma_store_ok && (p.block_n & 31) == 0 && !no_tma_store) ? EPI_BF16_TMA : EPI_BF16_SAME;
-    if (one_out && p.in_mode != IN_CONV && p.out[0].dtype == OUT_F32 && p.resid != nullptr && p.resid_map == MAP_SAME && p.act == ACT_NONE)
-        return EPI_F32_SAME_RESID;
-    return EPI_GENERIC;
-}
-
-// CTA-pair policy.  Linear layers: one bf16 / fp32+residual same-row output and >= 8 row tiles (the encoder GEMMs).  3x3 conv
-// layers: >= 8 row tiles and a weight tile of >= 64 columns (below that the B tile is too small for halving it to matter and
-// the launch is latency bound).  block_n % 16 == 0 always holds.  TMAE_NO_PAIR=1 / TMAE_NO_PAIR_CONV=1 switch them off (A/B).
-bool gemm_use_pair(int groups, int epi, int act, int max_M, int block_n, bool pair_ok, bool conv) {
-    static const bool off = getenv("TMAE_NO_PAIR") != nullptr;
-    static const bool off_conv = getenv("TMAE_NO_PAIR_CONV") != nullptr;
-    if (off || !pair_ok || max_M < 8 * kBlockM) return false;
-    if (conv) return !off_conv && block_n >= 64;
-    if (groups != 1) return false;
-    if (epi == EPI_F32_SAME_RESID) return act == ACT_NONE;
-    return (epi == EPI_BF16_SAME || epi == EPI_BF16_TMA) && (act == ACT_NONE || act == ACT_GELU);
-}
-
-// Persistent pairs: a linear layer that already qualifies for pairs, bf16 same-row output, one batch in flight (a persistent
-// launch owns every SM) and more pair tiles than one round of the 74 clusters.  TMAE_NO_PAIR_PERSISTENT=1 = A/B switch.
-bool gemm_use_pair_persistent(int groups, int epi, int act, int max_M, int max_N, int block_n, bool share_sm, bool conv) {
-    static const bool off = getenv("TMAE_NO_PAIR_PERSISTENT") != nullptr;
-    static const bool in_share = getenv("TMAE_PP_SHARE") != nullptr;          // experiment: also while several streams share the GPU
-    if (off || (share_sm && !in_share) || conv || groups != 1) return false;
-    if ((epi != EPI_BF16_SAME && epi != EPI_BF16_TMA) || (act != ACT_NONE && act != ACT_GELU)) return false;
-    const int m_pairs = ((max_M + kBlockM - 1) / kBlockM + 1) / 2, n_tiles = (max_N + block_n - 1) / block_n;
-    return m_pairs * n_tiles > 74;
-}
-
-template <int ACT, int EPI>
-static cudaError_t launch_pair(dim3 grid, int smem, cudaStream_t stream, const GemmParams* d_params, int stages, const GemmParams* d_next,
-                               int next_groups) {
-    return launch_k_cluster(gemm_tc_pair_kernel<ACT, EPI>, grid, dim3(kGemmThreads), smem, stream, true, 2, d_params, stages, d_next, next_groups);
-}
-
-// params: device array of `groups` GemmParams; max_M / max_N / block_n describe the largest member.
-cudaError_t gemm_launch(const GemmParams* d_params, int groups, int max_M, int max_N, int block_n, int act, int epi,
-                        bool simt, bool share_sm, cudaStream_t stream, const GemmParams* d_next, int next_groups,
-                        int conv_reuse_stage_bytes, int pair) {
-    if (simt) {
-        dim3 grid(max_M, 1, groups);
-        gemm_simt_kernel<<<grid, 128, 0, stream>>>(d_params);
-        return cudaGetLastError();
+// d_params: device array of the step's GemmParams (one per group member); d_next / next_groups: the next GEMM step's (weight
+// prefetch), or nullptr.
+cudaError_t gemm_launch(const GemmLaunch& L, const GemmParams* d_params, const GemmParams* d_next, int next_groups, cudaStream_t stream) {
+    const dim3 grid(L.grid[0], L.grid[1], L.grid[2]), block(L.block);
+    switch (L.form) {
+        case SIMT:
+            gemm_simt_kernel<<<grid, block, 0, stream>>>(d_params);
+            return cudaGetLastError();
+        case ONE_CTA:
+            if (OneCtaFn k = find_kernel(kOneCtaKernels, L))
+                return launch_k(k, grid, block, L.smem, stream, true, d_params, L.stages, L.kgroup, d_next, next_groups, L.two_producers);
+            break;
+        case PERSISTENT:
+            if (PersistentFn k = find_kernel(kPersistentKernels, L))
+                return launch_k(k, grid, block, L.smem, stream, true, d_params, L.stages, L.m_tiles, L.n_tiles, d_next, next_groups);
+            break;
+        case PAIR:
+            if (PairFn k = find_kernel(kPairKernels, L))
+                return launch_k_cluster(k, grid, block, L.smem, stream, true, 2, d_params, L.stages, d_next, next_groups);
+            break;
+        case PAIR_PERSISTENT:
+            if (PersistentFn k = find_kernel(kPairPersistentKernels, L))
+                return launch_k_cluster(k, grid, block, L.smem, stream, true, 2, d_params, L.stages, (L.m_tiles + 1) / 2, L.n_tiles,
+                                        d_next, next_groups);
+            break;
     }
-    int smem = 0;
-    dim3 grid((max_M + kBlockM - 1) / kBlockM, (max_N + block_n - 1) / block_n, groups);
-    if (pair) {                                               // the plan's policy (gemm_use_pair) decided
-        if ((block_n & 15) != 0) return cudaErrorInvalidConfiguration;
-        dim3 pgrid((grid.x + 1) / 2 * 2, grid.y, groups);      // whole pairs along x
-        if (pair == 2) {
-            // persistent pairs (plan policy gemm_use_pair_persistent): one cluster per TPC, tiles round-robin
-            if (groups != 1 || conv_reuse_stage_bytes != 0 || (epi != EPI_BF16_SAME && epi != EPI_BF16_TMA) || (act != ACT_NONE && act != ACT_GELU))
-                return cudaErrorInvalidConfiguration;
-            const int stage_bytes = kAStageBytes + (block_n / 2) * kBlockK * 2;
-            const int overhead = 1024 + 256 + kEpiStageBytes;
-            int pst = (226 * 1024 - overhead) / stage_bytes;
-            if (pst > 8) pst = 8;
-            if (pst < 2) return cudaErrorInvalidConfiguration;
-            const int psmem = overhead + pst * stage_bytes;
-            const int m_pairs = (int)pgrid.x / 2, tiles = m_pairs * (int)grid.y;
-            const int pairs = tiles < 74 ? tiles : 74;
-            const dim3 g2(2 * pairs), blk(kPersistThreads);
-            if (epi == EPI_BF16_TMA && act == ACT_GELU) return launch_k_cluster(gemm_tc_pair_persistent_kernel<ACT_GELU, EPI_BF16_TMA>, g2, blk, psmem, stream, true, 2, d_params, pst, m_pairs, (int)grid.y, d_next, next_groups);
-            if (epi == EPI_BF16_TMA) return launch_k_cluster(gemm_tc_pair_persistent_kernel<ACT_NONE, EPI_BF16_TMA>, g2, blk, psmem, stream, true, 2, d_params, pst, m_pairs, (int)grid.y, d_next, next_groups);
-            if (act == ACT_GELU) return launch_k_cluster(gemm_tc_pair_persistent_kernel<ACT_GELU, EPI_BF16_SAME>, g2, blk, psmem, stream, true, 2, d_params, pst, m_pairs, (int)grid.y, d_next, next_groups);
-            return launch_k_cluster(gemm_tc_pair_persistent_kernel<ACT_NONE, EPI_BF16_SAME>, g2, blk, psmem, stream, true, 2, d_params, pst, m_pairs, (int)grid.y, d_next, next_groups);
-        }
-        // conv_reuse_stage_bytes is the PAIR stage here (haloed A box + three half B atoms), computed by the plan
-        const int stage_bytes = conv_reuse_stage_bytes > 0 ? conv_reuse_stage_bytes : kAStageBytes + (block_n / 2) * kBlockK * 2;
-        const int overhead = 256;
-        const bool whole_sm = (int)(pgrid.x * pgrid.y * pgrid.z) <= 148 && !share_sm;
-        const int budget = (whole_sm ? 226 : 113) * 1024 - overhead;
-        int pst = budget / stage_bytes;
-        if (pst > (conv_reuse_stage_bytes > 0 ? 4 : 8)) pst = conv_reuse_stage_bytes > 0 ? 4 : 8;
-        if (pst < 2) return cudaErrorInvalidConfiguration;
-        const int psmem = overhead + pst * stage_bytes;
-        if (epi == EPI_BF16_TMA) return act == ACT_GELU ? launch_pair<ACT_GELU, EPI_BF16_TMA>(pgrid, psmem, stream, d_params, pst, d_next, next_groups)
-                                                        : launch_pair<ACT_NONE, EPI_BF16_TMA>(pgrid, psmem, stream, d_params, pst, d_next, next_groups);
-        if (epi == EPI_BF16_SAME) return act == ACT_GELU ? launch_pair<ACT_GELU, EPI_BF16_SAME>(pgrid, psmem, stream, d_params, pst, d_next, next_groups)
-                                                         : launch_pair<ACT_NONE, EPI_BF16_SAME>(pgrid, psmem, stream, d_params, pst, d_next, next_groups);
-        if (epi == EPI_F32_SAME_RESID) return launch_pair<ACT_NONE, EPI_F32_SAME_RESID>(pgrid, psmem, stream, d_params, pst, d_next, next_groups);
-        if (act == ACT_GELU) return launch_pair<ACT_GELU, EPI_GENERIC>(pgrid, psmem, stream, d_params, pst, d_next, next_groups);
-        if (act == ACT_HALF_TANH) return launch_pair<ACT_HALF_TANH, EPI_GENERIC>(pgrid, psmem, stream, d_params, pst, d_next, next_groups);
-        return launch_pair<ACT_NONE, EPI_GENERIC>(pgrid, psmem, stream, d_params, pst, d_next, next_groups);
-    }
-    if (conv_reuse_stage_bytes == 0 && gemm_use_persistent(groups, epi, act, (int)(grid.x * grid.y), share_sm)) {
-        const int stage_bytes = kAStageBytes + block_n * kBlockK * 2;
-        const int overhead = 1024 + 256 + kEpiStageBytes;
-        int pst = (226 * 1024 - overhead) / stage_bytes;
-        if (pst > 8) pst = 8;
-        const int psmem = overhead + pst * stage_bytes;
-        const int tiles = (int)(grid.x * grid.y);
-        const int ctas = tiles < 148 ? tiles : 148;
-        if (epi == EPI_BF16_TMA && act == ACT_GELU) return launch_k(gemm_tc_persistent_kernel<ACT_GELU, EPI_BF16_TMA>, dim3(ctas), dim3(kPersistThreads), psmem, stream, true, d_params, pst, (int)grid.x, (int)grid.y, d_next, next_groups);
-        if (epi == EPI_BF16_TMA) return launch_k(gemm_tc_persistent_kernel<ACT_NONE, EPI_BF16_TMA>, dim3(ctas), dim3(kPersistThreads), psmem, stream, true, d_params, pst, (int)grid.x, (int)grid.y, d_next, next_groups);
-        if (act == ACT_GELU) return launch_k(gemm_tc_persistent_kernel<ACT_GELU, EPI_BF16_SAME>, dim3(ctas), dim3(kPersistThreads), psmem, stream, true, d_params, pst, (int)grid.x, (int)grid.y, d_next, next_groups);
-        return launch_k(gemm_tc_persistent_kernel<ACT_NONE, EPI_BF16_SAME>, dim3(ctas), dim3(kPersistThreads), psmem, stream, true, d_params, pst, (int)grid.x, (int)grid.y, d_next, next_groups);
-    }
-    static const int two_prod_env = getenv("TMAE_TWO_PRODUCERS") ? atoi(getenv("TMAE_TWO_PRODUCERS")) : -1;
-    int kgroup = 1;
-    int stages;
-    if (conv_reuse_stage_bytes > 0) {
-        stages = gemm_reuse_stages(conv_reuse_stage_bytes, (int)(grid.x * grid.y * grid.z), share_sm, &smem);
-        if (stages == 0) return cudaErrorInvalidConfiguration;      // the plan only marks launches whose stages fit
-    } else {
-        stages = gemm_pick_stages(block_n, (int)(grid.x * grid.y * grid.z), share_sm, &smem, &kgroup);
-    }
-    // Second producer warp (TMAE_TWO_PRODUCERS=1): in isolation it shortens producer-bound main loops (64-wide GEMM
-    // tiles -20 %, fc2 -8 %), but since the conv layers moved to one haloed A box per three taps the whole forward is
-    // 4 % FASTER without it (25.6k vs 24.4k images/s, one batch in flight; equal with four) - off by default.
-    const int two_prod = two_prod_env >= 0 ? two_prod_env : 0;
-    // every member of a grouped launch shares the activation and the store-phase specialisation
-    if (epi == EPI_GAUSS) return launch_k(gemm_tc_kernel<ACT_NONE, EPI_GAUSS>, grid, dim3(kGemmThreads), smem, stream, true, d_params, stages, kgroup, d_next, next_groups, two_prod);
-    if (epi == EPI_GAUSS_IDX) return launch_k(gemm_tc_kernel<ACT_NONE, EPI_GAUSS_IDX>, grid, dim3(kGemmThreads), smem, stream, true, d_params, stages, kgroup, d_next, next_groups, two_prod);
-    if (epi == EPI_BF16_TMA && act == ACT_GELU) return launch_k(gemm_tc_kernel<ACT_GELU, EPI_BF16_TMA>, grid, dim3(kGemmThreads), smem, stream, true, d_params, stages, kgroup, d_next, next_groups, two_prod);
-    else if (epi == EPI_BF16_TMA && act == ACT_NONE) return launch_k(gemm_tc_kernel<ACT_NONE, EPI_BF16_TMA>, grid, dim3(kGemmThreads), smem, stream, true, d_params, stages, kgroup, d_next, next_groups, two_prod);
-    else if (epi == EPI_BF16_SAME && act == ACT_GELU) return launch_k(gemm_tc_kernel<ACT_GELU, EPI_BF16_SAME>, grid, dim3(kGemmThreads), smem, stream, true, d_params, stages, kgroup, d_next, next_groups, two_prod);
-    else if (epi == EPI_BF16_SAME && act == ACT_NONE) return launch_k(gemm_tc_kernel<ACT_NONE, EPI_BF16_SAME>, grid, dim3(kGemmThreads), smem, stream, true, d_params, stages, kgroup, d_next, next_groups, two_prod);
-    else if (epi == EPI_F32_SAME_RESID && act == ACT_NONE) return launch_k(gemm_tc_kernel<ACT_NONE, EPI_F32_SAME_RESID>, grid, dim3(kGemmThreads), smem, stream, true, d_params, stages, kgroup, d_next, next_groups, two_prod);
-    else if (act == ACT_GELU) return launch_k(gemm_tc_kernel<ACT_GELU, EPI_GENERIC>, grid, dim3(kGemmThreads), smem, stream, true, d_params, stages, kgroup, d_next, next_groups, two_prod);
-    else if (act == ACT_HALF_TANH) return launch_k(gemm_tc_kernel<ACT_HALF_TANH, EPI_GENERIC>, grid, dim3(kGemmThreads), smem, stream, true, d_params, stages, kgroup, d_next, next_groups, two_prod);
-    else return launch_k(gemm_tc_kernel<ACT_NONE, EPI_GENERIC>, grid, dim3(kGemmThreads), smem, stream, true, d_params, stages, kgroup, d_next, next_groups, two_prod);
-    return cudaGetLastError();
+    return cudaErrorInvalidConfiguration;
 }
 
 }  // namespace tmae

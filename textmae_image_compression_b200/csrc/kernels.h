@@ -29,14 +29,11 @@ struct IoBlock {
 
 // gemm_tc.cu
 cudaError_t gemm_tc_configure();
-int gemm_pick_stages(int block_n, int total_ctas, bool share_sm, int* smem_bytes, int* kgroup);
-int gemm_epi_kind(const GemmParams& p);
-cudaError_t gemm_launch(const GemmParams* d_params, int groups, int max_M, int max_N, int block_n, int act, int epi,
-                        bool simt, bool share_sm, cudaStream_t stream,
-                        const GemmParams* d_next = nullptr, int next_groups = 0, int conv_reuse_stage_bytes = 0, int pair = 0);   // pair: 1 = CTA pairs, 2 = persistent CTA pairs
-bool gemm_use_pair(int groups, int epi, int act, int max_M, int block_n, bool pair_ok, bool conv);
-bool gemm_use_pair_persistent(int groups, int epi, int act, int max_M, int max_N, int block_n, bool share_sm, bool conv);
-int gemm_reuse_stages(int stage_bytes, int total_ctas, bool share_sm, int* smem_bytes);
+const GemmOptions& gemm_options();
+bool conv_geom(int s, int n_img, ConvGeom* g);
+// Host-only and pure: the launch a GEMM step of shape `s` runs.  false = no launch form fits (a forced form the shape rules out).
+bool gemm_resolve(const GemmShape& s, GemmLaunch* out);
+cudaError_t gemm_launch(const GemmLaunch& L, const GemmParams* d_params, const GemmParams* d_next, int next_groups, cudaStream_t stream);
 
 // mask.cu
 cudaError_t launch_mask_select(const float* scores, int N, int L, int K, int softmax_isa, int64_t* ids_shuffle,

@@ -64,11 +64,9 @@ struct Step {
     StepKind kind;
     int family = FAM_MISC;
     // GEMM
-    int param_index = 0, groups = 1, max_M = 0, max_N = 0, block_n = 0, act = 0, epi = 0;
+    int param_index = 0, groups = 1;
+    GemmLaunch launch;                         // what gemm_launch launches (gemm_resolve)
     int next_index = -1, next_groups = 0;      // parameter blocks of the next GEMM step (weight prefetch target)
-    int conv_reuse_stage_bytes = 0;            // > 0: 3x3 conv launch with haloed-box A reuse, stage size in bytes
-    bool pair = false;                         // CTA-pair (cta_group::2) launch
-    bool pair_persist = false;                 // ... as the persistent pair kernel (one batch in flight, several tiles per cluster)
     double flops = 0, bytes = 0;
     int mma_terms = 1;                         // 3 for precise (split-bf16) GEMM steps
     // LN
@@ -276,7 +274,6 @@ int dev_alloc(tmae_handle* h, std::vector<void*>& pool, Tp** out, size_t count, 
 }
 
 int pad64(int c) { return (c + 63) / 64 * 64; }
-int round16(int c) { return (c + 15) / 16 * 16; }
 
 // ---- geometry ------------------------------------------------------------------------------------------
 int derive_geometry(tmae_handle* h) {
@@ -541,54 +538,6 @@ int make_map4d(tmae_handle* h, CUtensorMap* map, const void* base, uint64_t cols
     return TMAE_OK;
 }
 
-// Tiling of a conv layer over an s x s grid: a CTA tile is box_y image rows of box_n images (s * box_y * box_n <= 128
-// accumulator rows).  Pick the pair with the fewest tiles.  A pair whose dy shift (box_n * s rows) is a whole number of
-// 8-row swizzle atoms can use the haloed-box A reuse (GemmParams::conv_reuse); such a pair wins unless it costs more
-// than 15 % extra tiles.
-struct ConvGeom { int box_y = 0, box_n = 0, y_tiles = 0, m_tiles = 0, rows_used = 0; bool reuse_ok = false; };
-bool conv_geom(int s, int n_img, ConvGeom* g) {
-    if (s <= 0 || s > kBlockM || n_img <= 0) return false;
-    long long best[2] = {-1, -1};          // [0] any pair, [1] reuse-compatible pair
-    ConvGeom cand[2];
-    for (int by = (s < kBlockM / s ? s : kBlockM / s); by >= 1; --by) {
-        for (int pass = 0; pass < 2; ++pass) {
-            int bn = kBlockM / (s * by);
-            if (bn > 256) bn = 256;
-            if (pass == 0) { if (bn > n_img) bn = n_img; }
-            else {
-                int q = 8; for (int d = 8; d >= 1; d >>= 1) if (s % d == 0) { q = 8 / d; break; }   // q = 8 / gcd(s, 8)
-                bn = bn / q * q;                                   // box_n * s must be a multiple of 8 rows
-                while (bn - q >= n_img && bn - q > 0) bn -= q;     // no more images per tile than needed
-                if (by < 2) bn = 0;                                // one row + two halo rows: nothing to reuse
-            }
-            if (bn <= 0) continue;
-            const int yt = (s + by - 1) / by;
-            const long long tiles = (long long)((n_img + bn - 1) / bn) * yt;
-            if (best[pass] < 0 || tiles < best[pass]) {
-                best[pass] = tiles;
-                cand[pass].box_y = by; cand[pass].box_n = bn; cand[pass].y_tiles = yt; cand[pass].m_tiles = (int)tiles;
-                cand[pass].rows_used = s * by * bn; cand[pass].reuse_ok = pass == 1;
-            }
-        }
-    }
-    if (best[0] < 0) return false;
-    static const bool no_reuse = getenv("TMAE_NO_CONV_REUSE") != nullptr;
-    *g = (!no_reuse && best[1] > 0 && best[1] * 100 <= best[0] * 115) ? cand[1] : cand[0];
-    return true;
-}
-
-// Choose the N tile: fewest column tiles that still give the machine >= ~120 CTAs (148 SMs), multiple of 16.
-int pick_block_n(int m_tiles, int N, int groups) {
-    int best = round16(N) > 256 ? 256 : round16(N);
-    for (int nt = 1; nt <= 16; ++nt) {
-        int bn = round16((N + nt - 1) / nt);
-        if (bn > 256) continue;
-        best = bn;
-        if ((long long)m_tiles * nt * groups >= 120 || bn <= 64) break;
-    }
-    return best;
-}
-
 struct SegSrc {
     const __nv_bfloat16* ptr;   // first column of the segment
     int cols;                   // channels in the segment
@@ -605,7 +554,6 @@ struct GemmDesc {
     int in_mode = IN_LINEAR;
     int side = 0;               // grid side for IN_COMPACT / IN_CONV
     int n_img = 0;              // IN_CONV: images
-    bool conv_reuse = false;    // IN_CONV: haloed-box A reuse (decided per launch in add_gemm_group)
     bool conv3 = false;
     int act = ACT_NONE;
     const float* resid = nullptr; int resid_ld = 0; int resid_map = MAP_SAME;
@@ -620,8 +568,17 @@ struct GemmDesc {
     bool gc_decode = false;     // ... decoder form: mu, sigma and scale-table indexes only (EPI_GAUSS_IDX)
 };
 
-int fill_params(tmae_handle* h, const GemmDesc& d, int groups_for_tiling, GemmParams* p, int force_block_n) {
+// The TMA-store epilogue can write this output: one bf16 output at the accumulator's own rows, one plane (two-plane outputs take
+// the register store phase), 16-byte aligned rows.
+bool tma_store_ok(const GemmDesc& d) {
+    return d.out0.dtype == OUT_BF16 && d.out0.map == MAP_SAME && d.out1.dtype == OUT_NONE && d.resid == nullptr && d.out0.lo_off == 0 &&
+           (reinterpret_cast<uintptr_t>(d.out0.ptr) & 15) == 0 && ((size_t)d.out0.ld * 2) % 16 == 0 && d.layer->Cout >= 32;
+}
+
+// One member's parameter block for the launch gemm_resolve decided (tile width, conv A reuse); builds its tensor maps.
+int fill_params(tmae_handle* h, const GemmDesc& d, const GemmLaunch& launch, GemmParams* p) {
     memset(p, 0, sizeof(*p));
+    const bool conv_reuse = launch.conv_reuse_stage > 0;
     const Layer& L = *d.layer;
     if (d.nseg != L.nseg) return fail(h, TMAE_EINVAL, "segment count mismatch");
     const bool conv = d.in_mode == IN_CONV;
@@ -660,7 +617,7 @@ int fill_params(tmae_handle* h, const GemmDesc& d, int groups_for_tiling, GemmPa
             p->seg_kblocks[j] = skb;
             p->seg_b_kb0[j] = kb0 + pw * L.kb_tap;
             int rc = conv ? make_map4d(h, &p->a_map[j], ptr, (uint64_t)d.seg[i].cols, d.side, d.n_img, (uint64_t)d.seg[i].ld, cg.box_n,
-                                       cg.box_y + (d.conv_reuse ? 2 : 0))
+                                       cg.box_y + (conv_reuse ? 2 : 0))
                           : make_map(h, &p->a_map[j], ptr, (uint64_t)d.seg[i].cols, (uint64_t)d.a_rows, (uint64_t)d.seg[i].ld, kBlockM);
             if (rc) return rc;
         }
@@ -673,13 +630,12 @@ int fill_params(tmae_handle* h, const GemmDesc& d, int groups_for_tiling, GemmPa
     p->K = d.side * d.side;
     p->T = p->K + 1;
     p->n_img = d.n_img; p->box_y = cg.box_y; p->box_n = cg.box_n; p->y_tiles = cg.y_tiles; p->rows_used = cg.rows_used;
-    if (d.conv_reuse && !(conv && cg.reuse_ok)) return fail(h, TMAE_EINVAL, "conv_reuse requested for an incompatible tile geometry");
-    p->conv_reuse = d.conv_reuse ? 1 : 0;
+    if (conv_reuse && !(conv && cg.reuse_ok)) return fail(h, TMAE_EINVAL, "conv_reuse requested for an incompatible tile geometry");
+    p->conv_reuse = conv_reuse ? 1 : 0;
     p->a_halo_rows = conv ? (cg.box_y + 2) * cg.box_n * d.side : 0;
     p->M = d.M;
     p->N = L.Cout;
-    const int m_tiles = (d.M + kBlockM - 1) / kBlockM;
-    p->block_n = force_block_n > 0 ? force_block_n : pick_block_n(m_tiles, L.Cout, groups_for_tiling);
+    p->block_n = launch.block_n;
     int rc = make_map(h, &p->b_map, L.w, (uint64_t)L.Kp, (uint64_t)L.Cout, (uint64_t)L.Kp, (uint32_t)p->block_n);
     if (rc) return rc;
     p->pair_ok = 0;
@@ -689,14 +645,10 @@ int fill_params(tmae_handle* h, const GemmDesc& d, int groups_for_tiling, GemmPa
         p->pair_ok = 1;
     }
     p->in_mode = d.in_mode;
-    // TMA-store epilogue: one bf16 output at the accumulator's own rows, and those rows are 128 consecutive output rows
+    // TMA-store epilogue: a linear tile is 128 consecutive output rows, a conv tile is stored as the 4-D box it is
     {
-        const bool one_bf16 = d.out0.dtype == OUT_BF16 && d.out0.map == MAP_SAME && d.out1.dtype == OUT_NONE && d.resid == nullptr &&
-                              d.out0.lo_off == 0;        // two-plane outputs take the register store phase
-        const bool rows_ok = true;        // conv tiles are stored as the 4-D box they are (any geometry)
-        const bool align_ok = (reinterpret_cast<uintptr_t>(d.out0.ptr) & 15) == 0 && ((size_t)d.out0.ld * 2) % 16 == 0;
         p->tma_store_ok = 0;
-        if (one_bf16 && rows_ok && align_ok && L.Cout >= 32) {
+        if (tma_store_ok(d)) {
             const uint64_t out_rows = conv ? (uint64_t)d.a_rows : (uint64_t)d.M;
             int rc2 = conv ? make_map4d(h, &p->out_map, d.out0.ptr, (uint64_t)L.Cout, d.side, d.n_img, (uint64_t)d.out0.ld, cg.box_n, cg.box_y,
                                         32, CU_TENSOR_MAP_SWIZZLE_64B)
@@ -849,21 +801,45 @@ double conv_flops(long long out_positions, int cin, int cout, int taps) {
     return 2.0 * (double)out_positions * cin * cout * taps;
 }
 
-// conv_reuse decision for one launch: the geometry must allow it and at least two stages (one haloed A box + three B
-// atoms each) must fit the launch's shared-memory budget.  Returns the stage size in bytes, 0 = per-tap loads.
-int conv_reuse_stage_bytes(const tmae_handle* h, const GemmDesc& d, int bn, int n_tiles, int groups, bool pair = false) {
-    if (d.in_mode != IN_CONV) return 0;
-    ConvGeom cg;
-    if (!conv_geom(d.side, d.n_img, &cg) || !cg.reuse_ok) return 0;
-    const int bn_cta = pair ? bn / 2 : bn;             // B rows this CTA stages (a pair splits the weight tile)
-    // a tap's MMA always reads 128 rows from its dy offset: with a partial tile the rows past the A box must still lie
-    // inside the stage (they land in the B atoms; the accumulator rows they feed are never stored)
-    if (cg.rows_used + 3 * bn_cta < kBlockM) return 0;
-    const int stage = ((cg.box_y + 2) * cg.box_n * d.side + 3 * bn_cta) * kBlockK * 2;
-    int smem = 0;
-    const bool share = (h->cfg.flags & TMAE_FLAG_SHARE_SM) != 0;
-    return gemm_reuse_stages(stage, cg.m_tiles * n_tiles * groups, share, &smem) >= 2 ? stage : 0;
+// Output kind of one member (GemmShape::out).
+int gemm_out_kind(const GemmDesc& d) {
+    if (d.out1.dtype != OUT_NONE || d.out0.map != MAP_SAME) return GOUT_OTHER;
+    if (d.out0.dtype == OUT_BF16 && d.resid == nullptr) return GOUT_BF16;
+    if (d.out0.dtype == OUT_F32 && d.resid != nullptr && d.resid_map == MAP_SAME) return GOUT_F32_RESID;
+    return GOUT_OTHER;
 }
+
+// What the launch policy (gemm_resolve) reads about a launch of `groups` members.  The members of a grouped launch share
+// the activation, the input geometry and the fused Gaussian form.
+int gemm_shape(tmae_handle* h, const GemmDesc* descs, int groups, const char* tag, GemmShape* s) {
+    const GemmDesc& d0 = descs[0];
+    *s = GemmShape();
+    s->groups = groups;
+    s->conv = d0.in_mode == IN_CONV; s->side = d0.side; s->n_img = d0.n_img;
+    s->out = gemm_out_kind(d0);
+    s->act = d0.act;
+    s->gauss = d0.gc_slice >= 0 ? (d0.gc_decode ? 2 : 1) : 0;
+    s->ln_in = d0.ln_stats_in != nullptr;
+    s->tma_store_ok = true;
+    s->share_sm = (h->cfg.flags & TMAE_FLAG_SHARE_SM) != 0;
+    s->simt = (h->cfg.flags & TMAE_FLAG_DEBUG_SIMT) != 0;
+    for (int g = 0; g < groups; ++g) {
+        const GemmDesc& d = descs[g];
+        if (d.act != d0.act) return fail(h, TMAE_EINVAL, "%s: grouped GEMM members must share the activation", tag);
+        if (d.in_mode != d0.in_mode || d.side != d0.side || d.n_img != d0.n_img || (d.gc_slice >= 0) != (d0.gc_slice >= 0) ||
+            d.gc_decode != d0.gc_decode)
+            return fail(h, TMAE_EINVAL, "%s: grouped GEMM members must share the input geometry and the Gaussian epilogue", tag);
+        if (gemm_out_kind(d) != s->out) s->out = GOUT_OTHER;
+        if (d.M > s->max_M) s->max_M = d.M;
+        if (d.layer->Cout > s->max_N) s->max_N = d.layer->Cout;
+        s->ln_out = s->ln_out || d.ln_stats_out != nullptr;
+        s->shuffle = s->shuffle || d.out0.map == MAP_SHUF || d.out1.map == MAP_SHUF;
+        s->tma_store_ok = s->tma_store_ok && tma_store_ok(d);
+    }
+    return TMAE_OK;
+}
+
+const char* const kGemmFormNames[] = {"one_cta", "persistent", "pair", "pair_persistent", "simt"};
 
 int add_gemm_group(tmae_handle* h, Plan& pl, const GemmDesc* descs, int groups, const char* tag) {
     Step st;
@@ -872,80 +848,28 @@ int add_gemm_group(tmae_handle* h, Plan& pl, const GemmDesc* descs, int groups, 
     st.param_index = (int)pl.host_params.size();
     st.groups = groups;
     st.tag = tag;
-    int max_M = 0, max_N = 0;
-    for (int g = 0; g < groups; ++g) {
-        if (descs[g].M > max_M) max_M = descs[g].M;
-        if (descs[g].layer->Cout > max_N) max_N = descs[g].layer->Cout;
-    }
-    const int m_tiles = (max_M + kBlockM - 1) / kBlockM;
-    int bn = pick_block_n(m_tiles, max_N, groups);
-    if (descs[0].gc_slice >= 0) bn = 32;        // fused Gaussian epilogue: one 32-column chunk (16 channels: mu | sigma) per CTA
-    if (!(h->cfg.flags & TMAE_FLAG_SHARE_SM) && groups == 1 && m_tiles * ((max_N + 255) / 256) > 2 * 148 - 1 && descs[0].out0.dtype == OUT_BF16 && descs[0].out0.map == MAP_SAME &&
-        descs[0].out1.dtype == OUT_NONE && descs[0].resid == nullptr) {
-        // persistent-kernel candidate: tiles are dealt round-robin to 148 CTAs -> minimise rounds x (tile width + fixed cost)
-        long long best_cost = -1;
-        for (int cand = 256; cand >= 128; cand -= 16) {
-            const int tiles = m_tiles * ((max_N + cand - 1) / cand);
-            const long long cost = (long long)((tiles + 147) / 148) * (cand + 48);
-            if (best_cost < 0 || cost < best_cost) { best_cost = cost; bn = cand; }
-        }
-    }
-    {   // layers whose store phase can go through TMA (one bf16 same-row output): 32-column boxes -> block_n % 32 == 0
-        bool all_bf16_same = !getenv("TMAE_NO_TMA_STORE");
-        for (int g = 0; g < groups; ++g)
-            all_bf16_same = all_bf16_same && descs[g].out0.dtype == OUT_BF16 && descs[g].out0.map == MAP_SAME &&
-                            descs[g].out1.dtype == OUT_NONE && descs[g].resid == nullptr && descs[g].act != ACT_HALF_TANH;
-        // conv layers keep their exact tile width (rounding 112 -> 128 or 80 -> 96 computes 14-20 % dead columns; such layers
-        // use the register/smem store phase instead): measured equal or slightly better at the power cap
-        static const int round_mode = getenv("TMAE_BN_ROUND") ? atoi(getenv("TMAE_BN_ROUND")) : 2;   // 0 never, 1 always, 2 only linear layers
-        const bool conv_layer = descs[0].in_mode == IN_CONV;
-        if (all_bf16_same && bn % 32 != 0 && bn + 16 <= 256 && (round_mode == 1 || (round_mode == 2 && !conv_layer))) bn += 16;
-    }
-    for (int g = 0; g < groups; ++g)       // PixelShuffle epilogue: a 32-column chunk must not straddle a quadrant;
-        if (descs[g].out0.map == MAP_SHUF || descs[g].out1.map == MAP_SHUF || descs[g].ln_stats_out != nullptr)
-            bn = (bn + 31) / 32 * 32;      // LayerNorm statistics: one slot per 32-column chunk, owned by exactly one tile
-    // CTA-pair launch?  (decided before the stage sizes: a pair stages half of the weight tile per CTA)
-    {
-        const bool conv_l = descs[0].in_mode == IN_CONV;
-        bool one_bf16 = descs[0].out0.dtype == OUT_BF16 && descs[0].out0.map == MAP_SAME && descs[0].out1.dtype == OUT_NONE && descs[0].resid == nullptr;
-        bool f32_resid = descs[0].out0.dtype == OUT_F32 && descs[0].out0.map == MAP_SAME && descs[0].out1.dtype == OUT_NONE &&
-                         descs[0].resid != nullptr && descs[0].resid_map == MAP_SAME && descs[0].act == ACT_NONE;
-        const int epi_hint = one_bf16 ? 1 : (f32_resid ? 2 : 0);
-        st.pair = !(h->cfg.flags & TMAE_FLAG_DEBUG_SIMT) && (bn & 15) == 0 &&
-                  gemm_use_pair(groups, epi_hint, descs[0].act, max_M, bn, true, conv_l);
-        for (int g = 1; g < groups; ++g) if (descs[g].in_mode != descs[0].in_mode) st.pair = false;
-        if (descs[0].gc_slice >= 0) st.pair = false;          // the Gaussian epilogue lives in the one-CTA kernel
-    }
-    // 3x3 conv launches: haloed-box A reuse when every member agrees on the geometry and the stages fit
-    st.conv_reuse_stage_bytes = conv_reuse_stage_bytes(h, descs[0], bn, (max_N + bn - 1) / bn, groups, st.pair);
-    for (int g = 1; g < groups; ++g)
-        if (descs[g].in_mode != descs[0].in_mode || descs[g].side != descs[0].side || descs[g].n_img != descs[0].n_img) st.conv_reuse_stage_bytes = 0;
+    GemmShape shape;
+    int rc = gemm_shape(h, descs, groups, tag, &shape);
+    if (rc) return rc;
+    if (!gemm_resolve(shape, &st.launch)) return fail(h, TMAE_EINVAL, "%s: no GEMM launch form fits this step", tag);
+    const GemmLaunch& L = st.launch;
+    if (shape.ln_in && L.epi != EPI_BF16_TMA)
+        return fail(h, TMAE_EINVAL, "%s: a LayerNorm-folded layer needs the TMA-store epilogue (epi %d)", tag, L.epi);
+    if (shape.ln_out && L.epi != EPI_F32_SAME_RESID)
+        return fail(h, TMAE_EINVAL, "%s: LayerNorm statistics need the fp32 residual epilogue (epi %d)", tag, L.epi);
     for (int g = 0; g < groups; ++g) {
         GemmParams p;
-        GemmDesc dg = descs[g];
-        dg.conv_reuse = st.conv_reuse_stage_bytes > 0;
-        int rc = fill_params(h, dg, groups, &p, bn);
-        if (rc) return rc;
-        const int ek = gemm_epi_kind(p);
-        if (g == 0) st.epi = ek;
-        else if (ek != st.epi) st.epi = ((ek == 1 || ek == 3) && (st.epi == 1 || st.epi == 3)) ? 1 : 0;   // mixed group -> common denominator
+        if ((rc = fill_params(h, descs[g], L, &p))) return rc;
+        if ((L.form == PAIR || L.form == PAIR_PERSISTENT) && !p.pair_ok) return fail(h, TMAE_EINVAL, "%s: CTA pairs need pair_ok", tag);
         pl.host_params.push_back(p);
         st.flops += descs[g].flops;
         st.mma_terms = p.mma_terms;
     }
-    if (descs[0].ln_stats_in != nullptr && st.epi != 3 /*EPI_BF16_TMA*/)
-        return fail(h, TMAE_EINVAL, "%s: a LayerNorm-folded layer needs the TMA-store epilogue (epi %d)", tag, st.epi);
-    if (descs[0].ln_stats_out != nullptr && st.epi != 2 /*EPI_F32_SAME_RESID*/)
-        return fail(h, TMAE_EINVAL, "%s: LayerNorm statistics need the fp32 residual epilogue (epi %d)", tag, st.epi);
-    st.max_M = max_M; st.max_N = max_N; st.block_n = bn; st.act = descs[0].act;
-    if (st.pair && !pl.host_params[st.param_index].pair_ok) st.pair = false;
-    st.pair_persist = st.pair && gemm_use_pair_persistent(groups, st.epi, st.act, max_M, max_N, bn, (h->cfg.flags & TMAE_FLAG_SHARE_SM) != 0,
-                                                          descs[0].in_mode == IN_CONV);
-    static const bool plan_debug = getenv("TMAE_PLAN_DEBUG") != nullptr;
-    if (plan_debug)
-        fprintf(stderr, "[plan] %-14s groups %2d M %6d N %4d bn %3d ctas %4d epi %d conv_reuse_stage %6d B pair %d\n", tag, groups, max_M, max_N, bn,
-                m_tiles * ((max_N + bn - 1) / bn) * groups, st.epi, st.conv_reuse_stage_bytes, (int)st.pair);
-    for (int g = 1; g < groups; ++g) if (descs[g].act != descs[0].act) return fail(h, TMAE_EINVAL, "grouped GEMM members must share the activation");
+    if (gemm_options().plan_debug)
+        fprintf(stderr, "[plan] %-14s groups %2d M %6d N %4d | %-15s act %d epi %d bn %3d tiles %4d x %2d grid %4d x %2d x %2d block %3d "
+                "smem %6d stages %d kgroup %d two_producers %d conv_reuse_stage %6d B\n", tag, groups, shape.max_M, shape.max_N,
+                kGemmFormNames[L.form], L.act, L.epi, L.block_n, L.m_tiles, L.n_tiles, L.grid[0], L.grid[1], L.grid[2], L.block, L.smem,
+                L.stages, L.kgroup, L.two_producers, L.conv_reuse_stage);
     pl.steps.push_back(st);
     return TMAE_OK;
 }
@@ -1131,7 +1055,7 @@ int finish_plan(tmae_handle* h, Plan& pl) {
     pl.stage_calls.assign(pl.stage_begin.size() - 1, 0);
     for (const Step& st : pl.steps)
         if (st.kind == ST_GEMM && pl.host_params[st.param_index].num_segs < 1) return fail(h, TMAE_EINVAL, "bad plan");
-    if (!getenv("TMAE_NO_WEIGHT_PREFETCH")) {      // each GEMM step prefetches the weights of the next one (cyclically)
+    if (!gemm_options().no_weight_prefetch) {      // each GEMM step prefetches the weights of the next one (cyclically)
         std::vector<int> gemm_steps;
         for (size_t i = 0; i < pl.steps.size(); ++i) if (pl.steps[i].kind == ST_GEMM) gemm_steps.push_back((int)i);
         for (size_t k = 0; k < gemm_steps.size(); ++k) {
@@ -1529,8 +1453,8 @@ int prof_slot(tmae_handle* h, const Step& st, ProfRecord** out) {
     r.family = st.family;
     r.flops = r.bytes = r.mma_flops = 0;
     r.tag = st.tag;
-    r.ctas = st.kind == ST_GEMM ? ((st.max_M + kBlockM - 1) / kBlockM) * ((st.max_N + st.block_n - 1) / st.block_n) * st.groups : 0;
-    r.block_n = st.kind == ST_GEMM ? st.block_n : 0;
+    r.ctas = st.kind == ST_GEMM ? st.launch.m_tiles * st.launch.n_tiles * st.groups : 0;
+    r.block_n = st.kind == ST_GEMM ? st.launch.block_n : 0;
     r.launches = 0;
     *out = &r;
     return TMAE_OK;
@@ -1541,7 +1465,6 @@ int run_steps(tmae_handle* h, Plan& pl, const RunArgs& a, cudaStream_t st) {
     const int N = pl.N, C = h->C, T = h->T, K = h->K, s = h->s;
     static const tmae_outputs kNoOut = {};
     const tmae_outputs& o = a.out ? *a.out : kNoOut;
-    const bool simt = (h->cfg.flags & TMAE_FLAG_DEBUG_SIMT) != 0;
     if (a.io == nullptr && h->gc_fuse) {
         // plain launches: the fused Gaussian epilogue always reads the caller's output pointers from the device IoBlock
         IoBlock hio;
@@ -1582,8 +1505,8 @@ int run_steps(tmae_handle* h, Plan& pl, const RunArgs& a, cudaStream_t st) {
                                                   h->cfg.in_chans, h->cfg.patch_size, w.patches.lo, st, a.io));
                 break;
             case ST_GEMM:
-                CUDA_TRY(h, gemm_launch(pl.d_params + sp.param_index, sp.groups, sp.max_M, sp.max_N, sp.block_n, sp.act, sp.epi, simt, (h->cfg.flags & TMAE_FLAG_SHARE_SM) != 0, st,
-                                        sp.next_index >= 0 ? pl.d_params + sp.next_index : nullptr, sp.next_groups, sp.conv_reuse_stage_bytes, sp.pair ? (sp.pair_persist ? 2 : 1) : 0));
+                CUDA_TRY(h, gemm_launch(sp.launch, pl.d_params + sp.param_index, sp.next_index >= 0 ? pl.d_params + sp.next_index : nullptr,
+                                        sp.next_groups, st));
                 break;
             case ST_FORCE:
                 CUDA_TRY(h, launch_f32_to_bf16_cols(w.yhat_force + sp.slice * h->sc, w.yhat_bf.p + sp.slice * h->sc, (long long)N * K, h->sc,
@@ -1811,7 +1734,7 @@ int tmae_create(const tmae_config* cfg, tmae_handle** out) {
     h->precise_rate = h->precise_enc || (h->cfg.flags & TMAE_FLAG_PRECISE_RATE) != 0;
     h->planes = (h->cfg.flags & TMAE_FLAG_PRECISE_X6) ? 3 : 2;
     // the fold needs the thread-per-row TMA-store epilogue; the CUDA-core checker keeps the stand-alone LayerNorm path
-    h->ln_fold = !h->precise_enc && !(h->cfg.flags & TMAE_FLAG_DEBUG_SIMT) && !getenv("TMAE_NO_LN_FOLD") && !getenv("TMAE_NO_TMA_STORE");
+    h->ln_fold = !h->precise_enc && !(h->cfg.flags & TMAE_FLAG_DEBUG_SIMT) && !getenv("TMAE_NO_LN_FOLD") && !gemm_options().no_tma_store;
     h->gc_fuse = !h->precise_rate && !(h->cfg.flags & TMAE_FLAG_DEBUG_SIMT) && !getenv("TMAE_NO_GC_FUSE") && h->sc % 16 == 0;
     *out = h.release();
     return TMAE_OK;
@@ -1984,6 +1907,27 @@ int tmae_reserve(tmae_handle* h, int N) {
 int tmae_attention_plan(int T, int H, int N, int mode, int* out) {
     if (!out || T <= 0 || H <= 0 || N <= 0 || mode < 1 || mode > 3) return fail(nullptr, TMAE_EINVAL, "tmae_attention_plan: invalid argument");
     attention_tc_describe(T, H, N, mode, out);
+    return TMAE_OK;
+}
+
+int tmae_gemm_launch_plan(const int* shape, int* out) {
+    if (!shape || !out) return fail(nullptr, TMAE_EINVAL, "tmae_gemm_launch_plan: invalid argument");
+    GemmShape s;
+    s.groups = shape[0]; s.max_M = shape[1]; s.max_N = shape[2];
+    s.conv = shape[3] != 0; s.side = shape[4]; s.n_img = shape[5];
+    s.out = shape[6]; s.act = shape[7]; s.gauss = shape[8];
+    s.ln_in = shape[9] != 0; s.ln_out = shape[10] != 0; s.shuffle = shape[11] != 0; s.tma_store_ok = shape[12] != 0;
+    s.share_sm = shape[13] != 0; s.simt = shape[14] != 0;
+    s.force_block_n = shape[15]; s.force_form = shape[16];
+    ConvGeom cg;
+    if (s.out < GOUT_OTHER || s.out > GOUT_F32_RESID || s.act < ACT_NONE || s.act > ACT_HALF_TANH || s.gauss < 0 || s.gauss > 2 ||
+        s.force_form < -1 || s.force_form > SIMT || (s.conv && (!conv_geom(s.side, s.n_img, &cg) || s.max_M != cg.m_tiles * kBlockM)))
+        return fail(nullptr, TMAE_EINVAL, "tmae_gemm_launch_plan: invalid shape");
+    GemmLaunch L;
+    if (!gemm_resolve(s, &L)) return fail(nullptr, TMAE_EINVAL, "tmae_gemm_launch_plan: no launch form fits this shape");
+    const int r[15] = {L.form, L.act, L.epi, L.block_n, L.m_tiles, L.n_tiles, L.grid[0], L.grid[1], L.grid[2], L.block, L.smem,
+                       L.stages, L.kgroup, L.two_producers, L.conv_reuse_stage};
+    memcpy(out, r, sizeof(r));
     return TMAE_OK;
 }
 
@@ -2168,7 +2112,7 @@ int tmae_enable_synthesis(tmae_handle* h, int decoder_depth, int decoder_num_hea
     if (Dd / decoder_num_heads != 32)
         return fail(h, TMAE_EINVAL, "synthesis supports a decoder head dim of 32 only (decoder_embed_dim %d / %d heads = %d)", Dd,
                     decoder_num_heads, Dd / decoder_num_heads);
-    if ((h->cfg.flags & TMAE_FLAG_DEBUG_SIMT) || getenv("TMAE_NO_TMA_STORE"))
+    if ((h->cfg.flags & TMAE_FLAG_DEBUG_SIMT) || gemm_options().no_tma_store)
         return fail(h, TMAE_EINVAL, "synthesis folds its LayerNorms into the TMA-store phase of the tensor-core GEMMs: not available with "
                     "TMAE_FLAG_DEBUG_SIMT or TMAE_NO_TMA_STORE");
     const int mlp = (int)(Dd * h->cfg.mlp_ratio);
@@ -2429,146 +2373,6 @@ int tmae_generate_scores(const uint8_t* gray, int n, int height, int width, int 
 }
 
 // ---- engine self-tests ---------------------------------------------------------------------------------
-static int engine_common(tmae_handle* tmp, const GemmDesc& d_in, int block_n, int impl, cudaStream_t st, int pair = 0) {
-    GemmParams p;
-    GemmDesc d = d_in;
-    int reuse_bytes = 0;
-    if (d.in_mode == IN_CONV) {          // same decision as add_gemm_group (block_n first, then whether the reuse stages fit)
-        const int mt = (d.M + kBlockM - 1) / kBlockM;
-        const int bn = block_n > 0 ? block_n : pick_block_n(mt, d.layer->Cout, 1);
-        block_n = bn;
-        reuse_bytes = conv_reuse_stage_bytes(tmp, d, bn, (d.layer->Cout + bn - 1) / bn, 1, pair != 0 && impl == 0);
-        d.conv_reuse = reuse_bytes > 0;
-    }
-    int rc = fill_params(tmp, d, 1, &p, block_n);
-    if (rc) return rc;
-    GemmParams* dp = nullptr;
-    if (cudaMalloc(reinterpret_cast<void**>(&dp), sizeof(GemmParams)) != cudaSuccess) return fail(tmp, TMAE_ENOMEM, "cudaMalloc params");
-    // bring-up aid: TMAE_GEMM_TIMING=1 prints the per-phase globaltimer profile of the tensor-core kernel
-    const bool timing = getenv("TMAE_GEMM_TIMING") != nullptr && impl == 0;
-    __nv_bfloat16* bf16_out = nullptr;
-    if (timing && getenv("TMAE_TIMING_BF16")) {      // time the bf16 same-row store path (persistent kernel for big grids); output discarded
-        cudaMalloc(reinterpret_cast<void**>(&bf16_out), (size_t)p.M * p.N * 2);
-        p.out[0].ptr = bf16_out; p.out[0].dtype = OUT_BF16; p.out[0].map = MAP_SAME; p.out[0].ld = p.N;
-        if (getenv("TMAE_TIMING_GELU")) p.act = ACT_GELU;
-    }
-    const int ctas = ((p.M + kBlockM - 1) / kBlockM) * ((p.N + p.block_n - 1) / p.block_n);
-    long long* dticks = nullptr;
-    if (timing) {
-        cudaMalloc(reinterpret_cast<void**>(&dticks), (size_t)ctas * 16 * sizeof(long long));
-        cudaMemset(dticks, 0, (size_t)ctas * 16 * sizeof(long long));
-        p.dbg_ticks = dticks;
-    }
-    cudaMemcpyAsync(dp, &p, sizeof(p), cudaMemcpyHostToDevice, st);
-    if (pair && !p.pair_ok) { cudaFree(dp); return fail(tmp, TMAE_EINVAL, "pair launch needs a linear layer with block_n %% 32 == 0"); }
-    if (pair == 2 && getenv("TMAE_GEMM_TIMING") != nullptr && impl == 0) {
-        // bring-up aid for the persistent pair kernel: phase stamps of the first three tiles of every CTA
-        long long* dt = nullptr;
-        cudaMalloc(reinterpret_cast<void**>(&dt), (size_t)148 * 16 * sizeof(long long));
-        cudaMemset(dt, 0, (size_t)148 * 16 * sizeof(long long));
-        p.dbg_ticks = dt;
-        cudaMemcpyAsync(dp, &p, sizeof(p), cudaMemcpyHostToDevice, st);
-        gemm_launch(dp, 1, p.M, p.N, p.block_n, p.act, gemm_epi_kind(p), false, false, st, nullptr, 0, 0, 2);      // cold
-        cudaStreamSynchronize(st);
-        cudaEvent_t ev0, ev1; cudaEventCreate(&ev0); cudaEventCreate(&ev1);
-        cudaEventRecord(ev0, st);
-        cudaError_t e2 = gemm_launch(dp, 1, p.M, p.N, p.block_n, p.act, gemm_epi_kind(p), false, false, st, nullptr, 0, 0, 2);
-        cudaEventRecord(ev1, st);
-        cudaStreamSynchronize(st);
-        float ms = 0; cudaEventElapsedTime(&ms, ev0, ev1);
-        std::vector<long long> t((size_t)148 * 16);
-        cudaMemcpy(t.data(), dt, t.size() * sizeof(long long), cudaMemcpyDeviceToHost);
-        double avg[16] = {0}; int nc = 0;
-        for (int c = 0; c < 148; c += 2) if (t[c * 16]) { ++nc; for (int k = 1; k < 14; ++k) avg[k] += (double)(t[c * 16 + k] - t[c * 16]); }
-        for (int k = 1; k < 14; ++k) avg[k] /= nc > 0 ? nc : 1;
-        fprintf(stderr, "[pair-persistent timing] M=%d N=%d K=%d bn=%d leaders=%d | kernel %.1f us | ns since entry, tiles 0/1/2: mma_first %.0f/%.0f/%.0f  mma_last %.0f/%.0f/%.0f  "
-                "accum_seen %.0f/%.0f/%.0f  epi_done %.0f/%.0f/%.0f | exit %.0f (%s)\n", p.M, p.N, p.b_kb_per_tap * 64, p.block_n, nc, ms * 1e3,
-                avg[1], avg[5], avg[9], avg[2], avg[6], avg[10], avg[3], avg[7], avg[11], avg[4], avg[8], avg[12], avg[13], cudaGetErrorString(e2));
-        p.dbg_ticks = nullptr;
-        cudaMemcpyAsync(dp, &p, sizeof(p), cudaMemcpyHostToDevice, st);
-        cudaStreamSynchronize(st);
-        cudaFree(dt);
-        // steady state, 50 launches back to back on the stream (PDL overlaps ramp and drain): the three bf16 store kernels
-        for (int variant = 0; variant < 3; ++variant) {
-            for (int i = 0; i < 3; ++i) gemm_launch(dp, 1, p.M, p.N, p.block_n, p.act, gemm_epi_kind(p), false, false, st, nullptr, 0, 0, variant);
-            cudaStreamSynchronize(st);
-            cudaEventRecord(ev0, st);
-            for (int i = 0; i < 50; ++i) gemm_launch(dp, 1, p.M, p.N, p.block_n, p.act, gemm_epi_kind(p), false, false, st, nullptr, 0, 0, variant);
-            cudaEventRecord(ev1, st);
-            cudaStreamSynchronize(st);
-            float msv = 0; cudaEventElapsedTime(&msv, ev0, ev1);
-            fprintf(stderr, "[pair-persistent timing]   back-to-back x50, %s: %.2f us/launch = %.0f TFLOP/s\n",
-                    variant == 0 ? "one CTA per tile / one-CTA persistent" : (variant == 1 ? "CTA pairs" : "persistent CTA pairs"),
-                    msv * 1e3 / 50, 2.0 * p.M * p.N * p.b_kb_per_tap * 64 / (msv * 1e-3 / 50) / 1e12);
-        }
-    }
-    cudaError_t e = gemm_launch(dp, 1, p.M, p.N, p.block_n, p.act, gemm_epi_kind(p), impl == 1, false, st, nullptr, 0, reuse_bytes, impl == 0 ? pair : 0);
-    if (timing) {                      // second, warm launch is the one reported
-        cudaStreamSynchronize(st);
-        cudaEvent_t ev0, ev1; cudaEventCreate(&ev0); cudaEventCreate(&ev1);
-        cudaEventRecord(ev0, st);
-        e = gemm_launch(dp, 1, p.M, p.N, p.block_n, p.act, gemm_epi_kind(p), false, false, st, nullptr, 0, reuse_bytes);
-        cudaEventRecord(ev1, st);
-        cudaStreamSynchronize(st);
-        float ms = 0; cudaEventElapsedTime(&ms, ev0, ev1);
-        std::vector<long long> t((size_t)ctas * 16);
-        cudaMemcpy(t.data(), dticks, t.size() * sizeof(long long), cudaMemcpyDeviceToHost);
-        long long tmin = t[0], tend = 0;
-        for (int c = 0; c < ctas; ++c) { if (t[c * 16] < tmin) tmin = t[c * 16]; if (t[c * 16 + 6] > tend) tend = t[c * 16 + 6]; }
-        double avg[16] = {0};
-        for (int c = 0; c < ctas; ++c) for (int k = 1; k < 12; ++k) avg[k] += (double)(t[c * 16 + k] - t[c * 16]) / ctas;
-        int smem = 0, kgroup = 1; const int stages = gemm_pick_stages(p.block_n, ctas, false, &smem, &kgroup);
-        fprintf(stderr, "[gemm timing] M=%d N=%d Kb=%d taps=%d bn=%d ctas=%d stages=%d x%d smem=%d | kernel %.1f us (events), first-start..last-end %.1f us | "
-                "per-CTA avg ns since entry: setup %.0f, tma0 %.0f, full0 %.0f, mma_done_issue %.0f, accum_seen %.0f, epi_done %.0f | first chunk: ldtm_done %.0f, staged %.0f, batch0 %.0f, batch1 %.0f\n",
-                p.M, p.N, p.b_kb_per_tap, p.num_taps, p.block_n, ctas, stages, kgroup, smem, ms * 1e3,
-                (tend - tmin) * 1e-3, avg[1], avg[2], avg[3], avg[4], avg[5], avg[6], avg[8], avg[9], avg[10], avg[11]);
-        // steady-state cost of back-to-back dependent launches of this kernel: plain stream vs CUDA graph
-        {
-            p.dbg_ticks = nullptr;
-            cudaMemcpyAsync(dp, &p, sizeof(p), cudaMemcpyHostToDevice, st);
-            const int reps = 50;
-            cudaStreamSynchronize(st);
-            cudaEventRecord(ev0, st);
-            for (int i = 0; i < reps; ++i) gemm_launch(dp, 1, p.M, p.N, p.block_n, p.act, gemm_epi_kind(p), false, false, st, nullptr, 0, reuse_bytes);
-            cudaEventRecord(ev1, st);
-            cudaStreamSynchronize(st);
-            float ms_plain = 0; cudaEventElapsedTime(&ms_plain, ev0, ev1);
-            cudaStream_t cs; cudaStreamCreateWithFlags(&cs, cudaStreamNonBlocking);
-            cudaGraph_t graph = nullptr; cudaGraphExec_t gexec = nullptr;
-            cudaStreamBeginCapture(cs, cudaStreamCaptureModeThreadLocal);
-            for (int i = 0; i < reps; ++i) gemm_launch(dp, 1, p.M, p.N, p.block_n, p.act, gemm_epi_kind(p), false, false, cs, nullptr, 0, reuse_bytes);
-            cudaStreamEndCapture(cs, &graph);
-            float ms_graph = -1;
-            if (graph && cudaGraphInstantiate(&gexec, graph, 0) == cudaSuccess) {
-                cudaGraphLaunch(gexec, cs); cudaStreamSynchronize(cs);
-                cudaEventRecord(ev0, cs); cudaGraphLaunch(gexec, cs); cudaEventRecord(ev1, cs);
-                cudaStreamSynchronize(cs);
-                cudaEventElapsedTime(&ms_graph, ev0, ev1);
-                cudaGraphExecDestroy(gexec);
-            }
-            if (graph) cudaGraphDestroy(graph);
-            cudaStreamDestroy(cs);
-            fprintf(stderr, "[gemm timing]   back-to-back x%d: %.2f us/launch (stream), %.2f us/launch (graph)\n", reps,
-                    ms_plain * 1e3 / reps, ms_graph * 1e3 / reps);
-        }
-        if (bf16_out) {
-            double a2[16] = {0};
-            const int pc = ctas < 148 ? ctas : 148;
-            for (int c = 0; c < pc; ++c) for (int k = 1; k < 13; ++k) a2[k] += (double)(t[c * 16 + k] - t[c * 16]) / pc;
-            fprintf(stderr, "[gemm timing]   persistent tiles (ns since CTA entry): t0 mma %.0f-%.0f epi %.0f-%.0f | t1 mma %.0f-%.0f epi %.0f-%.0f | t2 mma %.0f-%.0f epi %.0f-%.0f\n",
-                    a2[1], a2[2], a2[3], a2[4], a2[5], a2[6], a2[7], a2[8], a2[9], a2[10], a2[11], a2[12]);
-            cudaFree(bf16_out);
-        }
-        cudaFree(dticks);
-        cudaEventDestroy(ev0); cudaEventDestroy(ev1);
-    }
-    cudaError_t e2 = cudaStreamSynchronize(st);
-    cudaFree(dp);
-    if (e != cudaSuccess || e2 != cudaSuccess)
-        return fail(tmp, TMAE_ECUDA, "engine launch: %s / %s", cudaGetErrorString(e), cudaGetErrorString(e2));
-    return TMAE_OK;
-}
-
 static int make_tmp_handle(std::unique_ptr<tmae_handle>& tmp) {
     tmp.reset(new tmae_handle());
     void* fn = nullptr;
@@ -2581,35 +2385,228 @@ static int make_tmp_handle(std::unique_ptr<tmae_handle>& tmp) {
     return TMAE_OK;
 }
 
+// One GEMM-engine call on the caller's buffers: a temporary handle and one packed layer staged from the caller's weights and
+// bias.  The entry points report errors through tmae_last_error(NULL) (`done`).
+struct EngineTest {
+    std::unique_ptr<tmae_handle> tmp;
+    std::vector<void*> pool;
+    Layer L;
+    cudaStream_t st = nullptr;
+    ~EngineTest() { free_pool(pool); }
+    int done(int rc) {
+        if (rc && tmp && !tmp->err.empty()) g_create_error = tmp->err;
+        return rc;
+    }
+};
+
+// Weights: w_bf16 [Cout, Cin] bf16 (one tap, one plane) copied into the zero-padded pack, or w_f32 [Cout, Cin, taps] fp32 packed
+// into `planes` split-bf16 planes.  A null bias is zero.
+static int engine_stage(EngineTest& t, void* stream, const void* w_bf16, const float* w_f32, const float* bias, int Cout, int Cin,
+                        int taps, int planes) {
+    int rc = make_tmp_handle(t.tmp);
+    if (rc) return rc;
+    tmae_handle* h = t.tmp.get();
+    t.st = reinterpret_cast<cudaStream_t>(stream);
+    Layer& L = t.L;
+    const int kp_tap = pad64(Cin);
+    L.Cout = Cout; L.Cin = Cin; L.taps = taps; L.nseg = 1; L.segc[0] = Cin; L.planes = planes; L.kb_tap = kp_tap / 64;
+    L.Kp = kp_tap * taps * planes;
+    if ((rc = dev_alloc(h, t.pool, &L.w, (size_t)Cout * L.Kp)) || (rc = dev_alloc(h, t.pool, &L.bias, (size_t)Cout))) return rc;
+    cudaError_t e;
+    if (w_bf16) {
+        e = cudaMemcpy2DAsync(L.w, (size_t)L.Kp * 2, w_bf16, (size_t)Cin * 2, (size_t)Cin * 2, Cout, cudaMemcpyDeviceToDevice, t.st);
+    } else {
+        int sg[1] = {Cin};
+        e = launch_prepack_weight(w_f32, L.w, Cout, Cin, taps, 1, sg, 0, planes, t.st);
+    }
+    if (e == cudaSuccess && bias) e = cudaMemcpyAsync(L.bias, bias, (size_t)Cout * 4, cudaMemcpyDeviceToDevice, t.st);
+    if (e != cudaSuccess) return fail(h, TMAE_ECUDA, "engine staging: %s", cudaGetErrorString(e));
+    return TMAE_OK;
+}
+
+// fp32 activations split into `planes` bf16 planes, as a precise layer reads them.
+static int engine_split(EngineTest& t, const float* src, long long count, int planes, SegSrc* seg_out, int cols) {
+    const size_t plane = ((size_t)count + 63) / 64 * 64;
+    const long long lo = planes == 2 ? (long long)plane : -(long long)plane;
+    __nv_bfloat16* p = nullptr;
+    int rc = dev_alloc(t.tmp.get(), t.pool, &p, plane * planes);
+    if (rc) return rc;
+    const cudaError_t e = launch_f32_to_bf16(src, p, count, lo, t.st);
+    if (e != cudaSuccess) return fail(t.tmp.get(), TMAE_ECUDA, "engine staging: %s", cudaGetErrorString(e));
+    *seg_out = seg(p, cols, cols, lo);
+    return TMAE_OK;
+}
+
+// Bring-up aid (TMAE_GEMM_TIMING=1): globaltimer phase profiles of the tensor-core kernels and back-to-back launch costs, on
+// stderr.  TMAE_TIMING_BF16=1 times the bf16 same-row store phase instead (output discarded; TMAE_TIMING_GELU=1 adds GELU).
+// Launches the resolved record of the self-test (persistent CTA pairs: also the three bf16 store forms).
+static cudaError_t engine_timing(EngineTest& et, GemmShape shape, GemmLaunch L, GemmParams p, GemmParams* dp) {
+    tmae_handle* h = et.tmp.get();
+    const cudaStream_t st = et.st;
+    __nv_bfloat16* bf16_out = nullptr;
+    if (getenv("TMAE_TIMING_BF16")) {
+        if (dev_alloc(h, et.pool, &bf16_out, (size_t)p.M * p.N)) return cudaErrorMemoryAllocation;
+        p.out[0].ptr = bf16_out; p.out[0].dtype = OUT_BF16; p.out[0].map = MAP_SAME; p.out[0].ld = p.N;
+        shape.out = p.resid == nullptr ? GOUT_BF16 : GOUT_OTHER;
+        shape.tma_store_ok = false;                        // no store map was built for the scratch output
+        if (getenv("TMAE_TIMING_GELU")) p.act = shape.act = ACT_GELU;
+        shape.force_block_n = p.block_n;
+        if (!gemm_resolve(shape, &L)) return cudaErrorInvalidConfiguration;
+    }
+    auto resolve = [&](int form) {
+        GemmShape s = shape;
+        s.force_form = form;
+        GemmLaunch r;
+        return gemm_resolve(s, &r) ? r : L;
+    };
+    const int ctas = L.m_tiles * L.n_tiles;
+    long long* dticks = nullptr;
+    if (dev_alloc(h, et.pool, &dticks, (size_t)(ctas > 148 ? ctas : 148) * 16)) return cudaErrorMemoryAllocation;
+    cudaEvent_t ev0, ev1; cudaEventCreate(&ev0); cudaEventCreate(&ev1);
+    if (L.form == PAIR_PERSISTENT) {
+        // phase stamps of the first three tiles of every CTA
+        p.dbg_ticks = dticks;
+        cudaMemcpyAsync(dp, &p, sizeof(p), cudaMemcpyHostToDevice, st);
+        gemm_launch(L, dp, nullptr, 0, st);      // cold
+        cudaStreamSynchronize(st);
+        cudaEventRecord(ev0, st);
+        cudaError_t e2 = gemm_launch(L, dp, nullptr, 0, st);
+        cudaEventRecord(ev1, st);
+        cudaStreamSynchronize(st);
+        float ms = 0; cudaEventElapsedTime(&ms, ev0, ev1);
+        std::vector<long long> t((size_t)148 * 16);
+        cudaMemcpy(t.data(), dticks, t.size() * sizeof(long long), cudaMemcpyDeviceToHost);
+        double avg[16] = {0}; int nc = 0;
+        for (int c = 0; c < 148; c += 2) if (t[c * 16]) { ++nc; for (int k = 1; k < 14; ++k) avg[k] += (double)(t[c * 16 + k] - t[c * 16]); }
+        for (int k = 1; k < 14; ++k) avg[k] /= nc > 0 ? nc : 1;
+        fprintf(stderr, "[pair-persistent timing] M=%d N=%d K=%d bn=%d leaders=%d | kernel %.1f us | ns since entry, tiles 0/1/2: mma_first %.0f/%.0f/%.0f  mma_last %.0f/%.0f/%.0f  "
+                "accum_seen %.0f/%.0f/%.0f  epi_done %.0f/%.0f/%.0f | exit %.0f (%s)\n", p.M, p.N, p.b_kb_per_tap * 64, p.block_n, nc, ms * 1e3,
+                avg[1], avg[5], avg[9], avg[2], avg[6], avg[10], avg[3], avg[7], avg[11], avg[4], avg[8], avg[12], avg[13], cudaGetErrorString(e2));
+        p.dbg_ticks = nullptr;
+        cudaMemcpyAsync(dp, &p, sizeof(p), cudaMemcpyHostToDevice, st);
+        cudaStreamSynchronize(st);
+        cudaMemsetAsync(dticks, 0, (size_t)148 * 16 * sizeof(long long), st);
+        // steady state, 50 launches back to back on the stream (PDL overlaps ramp and drain): the three bf16 store kernels
+        const int forms[3] = {ONE_CTA, PAIR, PAIR_PERSISTENT};
+        for (int variant = 0; variant < 3; ++variant) {
+            const GemmLaunch V = resolve(forms[variant]);
+            for (int i = 0; i < 3; ++i) gemm_launch(V, dp, nullptr, 0, st);
+            cudaStreamSynchronize(st);
+            cudaEventRecord(ev0, st);
+            for (int i = 0; i < 50; ++i) gemm_launch(V, dp, nullptr, 0, st);
+            cudaEventRecord(ev1, st);
+            cudaStreamSynchronize(st);
+            float msv = 0; cudaEventElapsedTime(&msv, ev0, ev1);
+            fprintf(stderr, "[pair-persistent timing]   back-to-back x50, %s: %.2f us/launch = %.0f TFLOP/s\n",
+                    variant == 0 ? "one CTA per tile / one-CTA persistent" : (variant == 1 ? "CTA pairs" : "persistent CTA pairs"),
+                    msv * 1e3 / 50, 2.0 * p.M * p.N * p.b_kb_per_tap * 64 / (msv * 1e-3 / 50) / 1e12);
+        }
+    }
+    p.dbg_ticks = dticks;
+    cudaMemcpyAsync(dp, &p, sizeof(p), cudaMemcpyHostToDevice, st);
+    cudaError_t e = gemm_launch(L, dp, nullptr, 0, st);
+    cudaStreamSynchronize(st);                            // second, warm launch is the one reported
+    cudaEventRecord(ev0, st);
+    if (e == cudaSuccess) e = gemm_launch(L, dp, nullptr, 0, st);
+    cudaEventRecord(ev1, st);
+    cudaStreamSynchronize(st);
+    float ms = 0; cudaEventElapsedTime(&ms, ev0, ev1);
+    std::vector<long long> t((size_t)ctas * 16);
+    cudaMemcpy(t.data(), dticks, t.size() * sizeof(long long), cudaMemcpyDeviceToHost);
+    long long tmin = t[0], tend = 0;
+    for (int c = 0; c < ctas; ++c) { if (t[c * 16] < tmin) tmin = t[c * 16]; if (t[c * 16 + 6] > tend) tend = t[c * 16 + 6]; }
+    double avg[16] = {0};
+    for (int c = 0; c < ctas; ++c) for (int k = 1; k < 12; ++k) avg[k] += (double)(t[c * 16 + k] - t[c * 16]) / ctas;
+    fprintf(stderr, "[gemm timing] M=%d N=%d Kb=%d taps=%d bn=%d ctas=%d stages=%d x%d smem=%d | kernel %.1f us (events), first-start..last-end %.1f us | "
+            "per-CTA avg ns since entry: setup %.0f, tma0 %.0f, full0 %.0f, mma_done_issue %.0f, accum_seen %.0f, epi_done %.0f | first chunk: ldtm_done %.0f, staged %.0f, batch0 %.0f, batch1 %.0f\n",
+            p.M, p.N, p.b_kb_per_tap, p.num_taps, p.block_n, ctas, L.stages, L.kgroup, L.smem, ms * 1e3,
+            (tend - tmin) * 1e-3, avg[1], avg[2], avg[3], avg[4], avg[5], avg[6], avg[8], avg[9], avg[10], avg[11]);
+    // steady-state cost of back-to-back dependent launches of this kernel: plain stream vs CUDA graph
+    {
+        p.dbg_ticks = nullptr;
+        cudaMemcpyAsync(dp, &p, sizeof(p), cudaMemcpyHostToDevice, st);
+        const int reps = 50;
+        cudaStreamSynchronize(st);
+        cudaEventRecord(ev0, st);
+        for (int i = 0; i < reps; ++i) gemm_launch(L, dp, nullptr, 0, st);
+        cudaEventRecord(ev1, st);
+        cudaStreamSynchronize(st);
+        float ms_plain = 0; cudaEventElapsedTime(&ms_plain, ev0, ev1);
+        cudaStream_t cs; cudaStreamCreateWithFlags(&cs, cudaStreamNonBlocking);
+        cudaGraph_t graph = nullptr; cudaGraphExec_t gexec = nullptr;
+        cudaStreamBeginCapture(cs, cudaStreamCaptureModeThreadLocal);
+        for (int i = 0; i < reps; ++i) gemm_launch(L, dp, nullptr, 0, cs);
+        cudaStreamEndCapture(cs, &graph);
+        float ms_graph = -1;
+        if (graph && cudaGraphInstantiate(&gexec, graph, 0) == cudaSuccess) {
+            cudaGraphLaunch(gexec, cs); cudaStreamSynchronize(cs);
+            cudaEventRecord(ev0, cs); cudaGraphLaunch(gexec, cs); cudaEventRecord(ev1, cs);
+            cudaStreamSynchronize(cs);
+            cudaEventElapsedTime(&ms_graph, ev0, ev1);
+            cudaGraphExecDestroy(gexec);
+        }
+        if (graph) cudaGraphDestroy(graph);
+        cudaStreamDestroy(cs);
+        fprintf(stderr, "[gemm timing]   back-to-back x%d: %.2f us/launch (stream), %.2f us/launch (graph)\n", reps,
+                ms_plain * 1e3 / reps, ms_graph * 1e3 / reps);
+    }
+    if (bf16_out) {
+        double a2[16] = {0};
+        const int pc = ctas < 148 ? ctas : 148;
+        for (int c = 0; c < pc; ++c) for (int k = 1; k < 13; ++k) a2[k] += (double)(t[c * 16 + k] - t[c * 16]) / pc;
+        fprintf(stderr, "[gemm timing]   persistent tiles (ns since CTA entry): t0 mma %.0f-%.0f epi %.0f-%.0f | t1 mma %.0f-%.0f epi %.0f-%.0f | t2 mma %.0f-%.0f epi %.0f-%.0f\n",
+                a2[1], a2[2], a2[3], a2[4], a2[5], a2[6], a2[7], a2[8], a2[9], a2[10], a2[11], a2[12]);
+    }
+    cudaEventDestroy(ev0); cudaEventDestroy(ev1);
+    return e;
+}
+
+// Runs the staged layer on `d` (its layer is set here) in `form` (GemmShape::force_form), block_n 0 = the engine's pick, and
+// waits for it.
+static int engine_run(EngineTest& t, GemmDesc d, int block_n, int form) {
+    tmae_handle* h = t.tmp.get();
+    d.layer = &t.L;
+    GemmShape shape;
+    int rc = gemm_shape(h, &d, 1, "engine", &shape);
+    if (rc) return rc;
+    shape.force_block_n = block_n;
+    shape.force_form = form;
+    GemmLaunch L;
+    if (!gemm_resolve(shape, &L))
+        return fail(h, TMAE_EINVAL, "engine: no %s launch fits this shape (CTA pairs need block_n %% 16 == 0)", kGemmFormNames[form]);
+    GemmParams p;
+    GemmParams* dp = nullptr;
+    if ((rc = fill_params(h, d, L, &p)) || (rc = dev_alloc(h, t.pool, &dp, 1))) return rc;
+    cudaError_t e;
+    if (form != SIMT && getenv("TMAE_GEMM_TIMING") != nullptr) {
+        e = engine_timing(t, shape, L, p, dp);
+    } else {
+        e = cudaMemcpyAsync(dp, &p, sizeof(p), cudaMemcpyHostToDevice, t.st);
+        if (e == cudaSuccess) e = gemm_launch(L, dp, nullptr, 0, t.st);
+    }
+    const cudaError_t e2 = cudaStreamSynchronize(t.st);
+    if (e != cudaSuccess || e2 != cudaSuccess)
+        return fail(h, TMAE_ECUDA, "engine launch: %s / %s", cudaGetErrorString(e), cudaGetErrorString(e2));
+    return TMAE_OK;
+}
+
+static GemmDesc linear_desc(const __nv_bfloat16* A, int M, int K) {
+    GemmDesc d;
+    d.seg[0] = seg(A, K, K);
+    d.a_rows = M; d.M = M;
+    return d;
+}
+
 int tmae_gemm_bf16(const void* A, const void* B, const float* bias, float* Cmat, int M, int N, int K, int block_n,
                    int impl, void* stream) {
     if (!A || !B || !Cmat || M <= 0 || N <= 0 || K <= 0 || K % 8 != 0 || N % 8 != 0)
         return fail(nullptr, TMAE_EINVAL, "tmae_gemm_bf16: invalid shape (need K %% 8 == 0, N %% 8 == 0)");
-    std::unique_ptr<tmae_handle> tmp;
-    int rc = make_tmp_handle(tmp);
-    if (rc) return rc;
-    cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
-    // pack B [N, K] bf16 into [N, pad64(K)] (zero padded) and a zero bias if none
-    const int Kp = pad64(K);
-    __nv_bfloat16* wp = nullptr;
-    float* bz = nullptr;
-    std::vector<void*> pool;
-    if ((rc = dev_alloc(tmp.get(), pool, &wp, (size_t)N * Kp)) || (rc = dev_alloc(tmp.get(), pool, &bz, (size_t)N))) {
-        g_create_error = tmp->err; free_pool(pool); return rc;
-    }
-    cudaMemcpy2DAsync(wp, (size_t)Kp * 2, B, (size_t)K * 2, (size_t)K * 2, N, cudaMemcpyDeviceToDevice, st);
-    if (bias) cudaMemcpyAsync(bz, bias, (size_t)N * 4, cudaMemcpyDeviceToDevice, st);
-    Layer L;
-    L.w = wp; L.bias = bz; L.Cout = N; L.Cin = K; L.taps = 1; L.nseg = 1; L.segc[0] = K; L.Kp = Kp; L.kb_tap = Kp / 64;
-    GemmDesc d;
-    d.layer = &L;
-    d.seg[0] = seg(reinterpret_cast<const __nv_bfloat16*>(A), K, K);
-    d.a_rows = M; d.M = M;
+    EngineTest t;
+    int rc = engine_stage(t, stream, B, nullptr, bias, N, K, 1, 1);
+    if (rc) return t.done(rc);
+    GemmDesc d = linear_desc(reinterpret_cast<const __nv_bfloat16*>(A), M, K);
     d.out0 = outspec(Cmat, N, OUT_F32, MAP_SAME);
-    rc = engine_common(tmp.get(), d, block_n, impl, st);
-    if (rc) g_create_error = tmp->err;
-    free_pool(pool);
-    return rc;
+    return t.done(engine_run(t, d, block_n, impl == 1 ? SIMT : ONE_CTA));
 }
 
 // C (bf16) = act(A B^T + bias): the bf16 same-row store phases (TMA-store epilogue when block_n % 32 == 0).  variant 0 = one
@@ -2619,66 +2616,31 @@ int tmae_gemm_bf16_out(const void* A, const void* B, const float* bias, void* Cm
                        int variant, void* stream) {
     if (!A || !B || !Cmat || M <= 0 || N <= 0 || K <= 0 || K % 8 != 0 || N % 8 != 0 || variant < 0 || variant > 3)
         return fail(nullptr, TMAE_EINVAL, "tmae_gemm_bf16_out: invalid argument (need K %% 8 == 0, N %% 8 == 0, variant 0..3)");
-    std::unique_ptr<tmae_handle> tmp;
-    int rc = make_tmp_handle(tmp);
-    if (rc) return rc;
-    cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
-    const int Kp = pad64(K);
-    __nv_bfloat16* wp = nullptr;
-    float* bz = nullptr;
-    std::vector<void*> pool;
-    if ((rc = dev_alloc(tmp.get(), pool, &wp, (size_t)N * Kp)) || (rc = dev_alloc(tmp.get(), pool, &bz, (size_t)N))) {
-        g_create_error = tmp->err; free_pool(pool); return rc;
-    }
-    cudaMemcpy2DAsync(wp, (size_t)Kp * 2, B, (size_t)K * 2, (size_t)K * 2, N, cudaMemcpyDeviceToDevice, st);
-    if (bias) cudaMemcpyAsync(bz, bias, (size_t)N * 4, cudaMemcpyDeviceToDevice, st);
-    Layer L;
-    L.w = wp; L.bias = bz; L.Cout = N; L.Cin = K; L.taps = 1; L.nseg = 1; L.segc[0] = K; L.Kp = Kp; L.kb_tap = Kp / 64;
-    GemmDesc d;
-    d.layer = &L;
-    d.seg[0] = seg(reinterpret_cast<const __nv_bfloat16*>(A), K, K);
-    d.a_rows = M; d.M = M;
+    static const int kForms[4] = {ONE_CTA, PAIR, PAIR_PERSISTENT, SIMT};
+    EngineTest t;
+    int rc = engine_stage(t, stream, B, nullptr, bias, N, K, 1, 1);
+    if (rc) return t.done(rc);
+    GemmDesc d = linear_desc(reinterpret_cast<const __nv_bfloat16*>(A), M, K);
     d.act = gelu ? ACT_GELU : ACT_NONE;
     d.out0 = outspec(Cmat, N, OUT_BF16, MAP_SAME);
-    rc = engine_common(tmp.get(), d, block_n, variant == 3 ? 1 : 0, st, variant == 3 ? 0 : variant);
-    if (rc) g_create_error = tmp->err;
-    free_pool(pool);
-    return rc;
+    return t.done(engine_run(t, d, block_n, kForms[variant]));
 }
 
 int tmae_conv3x3_bf16(const void* x, const float* wgt, const float* bias, float* out, int N, int s, int Cin, int Cout,
                       int gelu, int impl, void* stream) {
     if (!x || !wgt || !out || N <= 0 || s <= 0 || Cin % 8 != 0 || Cout % 8 != 0)
         return fail(nullptr, TMAE_EINVAL, "tmae_conv3x3_bf16: invalid shape");
-    std::unique_ptr<tmae_handle> tmp;
-    int rc = make_tmp_handle(tmp);
-    if (rc) return rc;
-    cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
-    const int Kp = pad64(Cin) * 9;
-    std::vector<void*> pool;
-    __nv_bfloat16* wp = nullptr;
-    float* bz = nullptr;
-    if ((rc = dev_alloc(tmp.get(), pool, &wp, (size_t)Cout * Kp)) || (rc = dev_alloc(tmp.get(), pool, &bz, (size_t)Cout))) {
-        g_create_error = tmp->err; free_pool(pool); return rc;
-    }
-    int sg[1] = {Cin};
-    cudaError_t e = launch_prepack_weight(wgt, wp, Cout, Cin, 9, 1, sg, 0, 1, st);
-    if (bias) cudaMemcpyAsync(bz, bias, (size_t)Cout * 4, cudaMemcpyDeviceToDevice, st);
-    if (e != cudaSuccess) { free_pool(pool); return fail(nullptr, TMAE_ECUDA, "conv3x3 staging: %s", cudaGetErrorString(e)); }
-    Layer L;
-    L.w = wp; L.bias = bz; L.Cout = Cout; L.Cin = Cin; L.taps = 9; L.nseg = 1; L.segc[0] = Cin; L.Kp = Kp; L.kb_tap = pad64(Cin) / 64;
     ConvGeom cg;
-    if (!conv_geom(s, N, &cg)) { free_pool(pool); return fail(nullptr, TMAE_EINVAL, "tmae_conv3x3_bf16: grid side %d unsupported (1..128)", s); }
+    if (!conv_geom(s, N, &cg)) return fail(nullptr, TMAE_EINVAL, "tmae_conv3x3_bf16: grid side %d unsupported (1..128)", s);
+    EngineTest t;
+    int rc = engine_stage(t, stream, nullptr, wgt, bias, Cout, Cin, 9, 1);
+    if (rc) return t.done(rc);
     GemmDesc d;
-    d.layer = &L;
     d.seg[0] = seg(reinterpret_cast<const __nv_bfloat16*>(x), Cin, Cin);      // compact NHWC, read in place by 4-D TMA boxes
-    d.a_rows = (long long)N * s * s; d.M = cg.m_tiles * kBlockM; d.in_mode = IN_CONV; d.side = s; d.n_img = N;
+    conv_input(d, s, N);
     d.act = gelu ? ACT_GELU : ACT_NONE;
     d.out0 = outspec(out, Cout, OUT_F32, MAP_SAME);
-    rc = engine_common(tmp.get(), d, 0, impl == 2 ? 0 : impl, st, impl == 2);      // impl 2: CTA-pair (cta_group::2) launch
-    if (rc) g_create_error = tmp->err;
-    free_pool(pool);
-    return rc;
+    return t.done(engine_run(t, d, 0, impl == 1 ? SIMT : impl == 2 ? PAIR : ONE_CTA));      // impl 2: CTA-pair (cta_group::2) launch
 }
 
 // softmax(q k^T / sqrt(64)) v for qkv bf16 [N*T, 3C] (columns [3][H][64]) -> out bf16 [N*T, C]: the attention kernels of the
@@ -2743,31 +2705,13 @@ int tmae_gemm_bf16_resid(const void* A, const void* B, const float* bias, const 
                          int block_n, int pair, int impl, void* stream) {
     if (!A || !B || !Cmat || !resid || M <= 0 || N <= 0 || K <= 0 || K % 8 != 0 || N % 8 != 0)
         return fail(nullptr, TMAE_EINVAL, "tmae_gemm_bf16_resid: invalid shape (need K %% 8 == 0, N %% 8 == 0)");
-    std::unique_ptr<tmae_handle> tmp;
-    int rc = make_tmp_handle(tmp);
-    if (rc) return rc;
-    cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
-    const int Kp = pad64(K);
-    __nv_bfloat16* wp = nullptr;
-    float* bz = nullptr;
-    std::vector<void*> pool;
-    if ((rc = dev_alloc(tmp.get(), pool, &wp, (size_t)N * Kp)) || (rc = dev_alloc(tmp.get(), pool, &bz, (size_t)N))) {
-        g_create_error = tmp->err; free_pool(pool); return rc;
-    }
-    cudaMemcpy2DAsync(wp, (size_t)Kp * 2, B, (size_t)K * 2, (size_t)K * 2, N, cudaMemcpyDeviceToDevice, st);
-    if (bias) cudaMemcpyAsync(bz, bias, (size_t)N * 4, cudaMemcpyDeviceToDevice, st);
-    Layer L;
-    L.w = wp; L.bias = bz; L.Cout = N; L.Cin = K; L.taps = 1; L.nseg = 1; L.segc[0] = K; L.Kp = Kp; L.kb_tap = Kp / 64;
-    GemmDesc d;
-    d.layer = &L;
-    d.seg[0] = seg(reinterpret_cast<const __nv_bfloat16*>(A), K, K);
-    d.a_rows = M; d.M = M;
+    EngineTest t;
+    int rc = engine_stage(t, stream, B, nullptr, bias, N, K, 1, 1);
+    if (rc) return t.done(rc);
+    GemmDesc d = linear_desc(reinterpret_cast<const __nv_bfloat16*>(A), M, K);
     d.resid = resid; d.resid_ld = N; d.resid_map = MAP_SAME;
     d.out0 = outspec(Cmat, N, OUT_F32, MAP_SAME);
-    rc = engine_common(tmp.get(), d, block_n, impl, st, pair != 0);
-    if (rc) g_create_error = tmp->err;
-    free_pool(pool);
-    return rc;
+    return t.done(engine_run(t, d, block_n, impl == 1 ? SIMT : pair ? PAIR : ONE_CTA));
 }
 
 // Precise (split-bf16) engine self-tests: fp32 operands in, split into (hi, lo) bf16 planes here, three tensor-core
@@ -2776,76 +2720,31 @@ int tmae_gemm_split(const float* A, const float* B, const float* bias, float* Cm
                     int planes, int impl, void* stream) {
     if (!A || !B || !Cmat || M <= 0 || N <= 0 || K <= 0 || K % 8 != 0 || N % 8 != 0 || (planes != 2 && planes != 3))
         return fail(nullptr, TMAE_EINVAL, "tmae_gemm_split: invalid shape (need K %% 8 == 0, N %% 8 == 0)");
-    std::unique_ptr<tmae_handle> tmp;
-    int rc = make_tmp_handle(tmp);
-    if (rc) return rc;
-    cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
-    const int Kp = pad64(K);
-    __nv_bfloat16 *wp = nullptr, *ap = nullptr;
-    float* bz = nullptr;
-    std::vector<void*> pool;
-    const size_t a_plane = ((size_t)M * K + 63) / 64 * 64;
-    const long long a_lo = planes == 2 ? (long long)a_plane : -(long long)a_plane;
-    if ((rc = dev_alloc(tmp.get(), pool, &wp, (size_t)N * Kp * planes)) || (rc = dev_alloc(tmp.get(), pool, &bz, (size_t)N)) ||
-        (rc = dev_alloc(tmp.get(), pool, &ap, a_plane * planes))) {
-        g_create_error = tmp->err; free_pool(pool); return rc;
-    }
-    int sg[1] = {K};
-    cudaError_t e = launch_prepack_weight(B, wp, N, K, 1, 1, sg, 0, planes, st);
-    if (e == cudaSuccess) e = launch_f32_to_bf16(A, ap, (long long)M * K, a_lo, st);
-    if (bias) cudaMemcpyAsync(bz, bias, (size_t)N * 4, cudaMemcpyDeviceToDevice, st);
-    if (e != cudaSuccess) { free_pool(pool); return fail(nullptr, TMAE_ECUDA, "gemm_split staging: %s", cudaGetErrorString(e)); }
-    Layer L;
-    L.w = wp; L.bias = bz; L.Cout = N; L.Cin = K; L.taps = 1; L.nseg = 1; L.segc[0] = K; L.planes = planes; L.kb_tap = Kp / 64; L.Kp = Kp * planes;
+    EngineTest t;
     GemmDesc d;
-    d.layer = &L;
-    d.seg[0] = seg(ap, K, K, a_lo);
+    int rc = engine_stage(t, stream, nullptr, B, bias, N, K, 1, planes);
+    if (!rc) rc = engine_split(t, A, (long long)M * K, planes, &d.seg[0], K);
+    if (rc) return t.done(rc);
     d.a_rows = M; d.M = M;
     d.out0 = outspec(Cmat, N, OUT_F32, MAP_SAME);
-    rc = engine_common(tmp.get(), d, block_n, impl, st);
-    if (rc) g_create_error = tmp->err;
-    free_pool(pool);
-    return rc;
+    return t.done(engine_run(t, d, block_n, impl == 1 ? SIMT : ONE_CTA));
 }
 
 int tmae_conv3x3_split(const float* x, const float* wgt, const float* bias, float* out, int N, int s, int Cin, int Cout,
                        int gelu, int planes, int impl, void* stream) {
     if (!x || !wgt || !out || N <= 0 || s <= 0 || Cin % 8 != 0 || Cout % 8 != 0 || (planes != 2 && planes != 3))
         return fail(nullptr, TMAE_EINVAL, "tmae_conv3x3_split: invalid shape");
-    std::unique_ptr<tmae_handle> tmp;
-    int rc = make_tmp_handle(tmp);
-    if (rc) return rc;
-    cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
-    const int kp_tap = pad64(Cin);
-    std::vector<void*> pool;
-    __nv_bfloat16 *wp = nullptr, *xp = nullptr;
-    float* bz = nullptr;
-    const size_t x_plane = ((size_t)N * s * s * Cin + 63) / 64 * 64;
-    const long long x_lo = planes == 2 ? (long long)x_plane : -(long long)x_plane;
-    if ((rc = dev_alloc(tmp.get(), pool, &wp, (size_t)Cout * kp_tap * 9 * planes)) || (rc = dev_alloc(tmp.get(), pool, &bz, (size_t)Cout)) ||
-        (rc = dev_alloc(tmp.get(), pool, &xp, x_plane * planes))) {
-        g_create_error = tmp->err; free_pool(pool); return rc;
-    }
-    int sg[1] = {Cin};
-    cudaError_t e = launch_prepack_weight(wgt, wp, Cout, Cin, 9, 1, sg, 0, planes, st);
-    if (e == cudaSuccess) e = launch_f32_to_bf16(x, xp, (long long)N * s * s * Cin, x_lo, st);
-    if (bias) cudaMemcpyAsync(bz, bias, (size_t)Cout * 4, cudaMemcpyDeviceToDevice, st);
-    if (e != cudaSuccess) { free_pool(pool); return fail(nullptr, TMAE_ECUDA, "conv3x3_split staging: %s", cudaGetErrorString(e)); }
-    Layer L;
-    L.w = wp; L.bias = bz; L.Cout = Cout; L.Cin = Cin; L.taps = 9; L.nseg = 1; L.segc[0] = Cin; L.planes = planes; L.kb_tap = kp_tap / 64;
-    L.Kp = kp_tap * 9 * planes;
     ConvGeom cg;
-    if (!conv_geom(s, N, &cg)) { free_pool(pool); return fail(nullptr, TMAE_EINVAL, "tmae_conv3x3_split: grid side %d unsupported (1..128)", s); }
+    if (!conv_geom(s, N, &cg)) return fail(nullptr, TMAE_EINVAL, "tmae_conv3x3_split: grid side %d unsupported (1..128)", s);
+    EngineTest t;
     GemmDesc d;
-    d.layer = &L;
-    d.seg[0] = seg(xp, Cin, Cin, x_lo);
-    d.a_rows = (long long)N * s * s; d.M = cg.m_tiles * kBlockM; d.in_mode = IN_CONV; d.side = s; d.n_img = N;
+    int rc = engine_stage(t, stream, nullptr, wgt, bias, Cout, Cin, 9, planes);
+    if (!rc) rc = engine_split(t, x, (long long)N * s * s * Cin, planes, &d.seg[0], Cin);
+    if (rc) return t.done(rc);
+    conv_input(d, s, N);
     d.act = gelu ? ACT_GELU : ACT_NONE;
     d.out0 = outspec(out, Cout, OUT_F32, MAP_SAME);
-    rc = engine_common(tmp.get(), d, 0, impl, st);
-    if (rc) g_create_error = tmp->err;
-    free_pool(pool);
-    return rc;
+    return t.done(engine_run(t, d, 0, impl == 1 ? SIMT : ONE_CTA));
 }
 
 // ---- profiling -----------------------------------------------------------------------------------------
