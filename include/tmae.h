@@ -265,6 +265,43 @@ TMAE_API int  tmae_decompress_streams_lanes(tmae_handle* h, const uint8_t* y_dat
                                             const uint8_t* z_data, const int64_t* z_offsets, int z_lanes, int N,
                                             const tmae_outputs* out, int32_t* status, void* stream);
 
+/* Image containers (DESIGN.md section 7): one self-contained byte string per image - a 28-byte header (magic "TMAE", version,
+ * accuracy mode, lane counts, img_size, patch_size, K, model tag, z and y stream lengths), the kept patch ids ids_keep[0..K)
+ * bit-packed in max(1, bit_length(L - 1)) bits each, then the z and the y stream exactly as tmae_rans_encode(_lanes) writes them.
+ * Lanes: 0 = compressai's format, 1..32 = the laned format with that many lanes.  Status bits above the coder's (ORed with them
+ * per image): */
+#define TMAE_IMG_HEADER         64   /* decode: bad magic / version / reserved bits, or section lengths that do not add up to the
+                                        container's byte range (or a range outside [0, n_bytes)) */
+#define TMAE_IMG_CONFIG         128  /* decode: img_size, patch_size, K, accuracy mode or lane counts other than the handle's / call's */
+#define TMAE_IMG_MODEL          256  /* decode: model tag other than the handle's (other scale table or CDF tables) */
+#define TMAE_IMG_IDS            512  /* decode: a patch id >= L, or two equal ids */
+/* Host-only: FNV-1a (32-bit) over the scale table (fp32) and then, Gaussian set first, every table's cdf length, offset and cdf
+ * entries (int32), all little-endian: what a container's model tag must equal.  TMAE_ESTATE until the scale table and both CDF
+ * table sets are installed; TMAE_EINVAL for null pointers.  The synthesis weights are not covered. */
+TMAE_API int  tmae_model_tag(const tmae_handle* h, uint32_t* tag);
+/* Host-only: bytes that always suffice for the containers of N images (the ABI's worst case of both streams plus the header and
+ * the patch ids, per image); -1 for a null handle, N < 1 or lanes outside {0} and 1..32. */
+TMAE_API int64_t tmae_images_bound(const tmae_handle* h, int N, int y_lanes, int z_lanes);
+/* The forward of N images (imgs / scores as tmae_forward), then both rANS encodes and the packing of one container per image,
+ * all enqueued on `stream` without a host synchronisation.  Container n is bytes [offsets[n], offsets[n + 1]) of `out` (device,
+ * 4-byte aligned; capacity bytes, tmae_images_bound always suffices); offsets i64 [N + 1] (8-byte aligned), status i32 [N]
+ * (device, 4-byte aligned): the coder's
+ * encode bits, TMAE_RANS_OVERFLOW when the container does not fit `capacity` (not written).  Needs the scale table and both CDF
+ * table sets (TMAE_ESTATE). */
+TMAE_API int  tmae_compress_images(tmae_handle* h, const float* imgs, const float* scores, int N, int y_lanes, int z_lanes,
+                                   uint8_t* out, int64_t capacity, int64_t* offsets, int32_t* status, void* stream);
+/* Decode of N containers, bytes [offsets[n], offsets[n + 1]) of data (device, 4-byte aligned, n_bytes long; offsets i64 [N + 1]
+ * on the device; offsets, ids_restore and out->ids_keep 8-byte aligned, status 4-byte aligned: TMAE_EINVAL otherwise), enqueued without a host synchronisation: a parse-and-validate kernel, then the decode of
+ * tmae_decompress_streams(_lanes) from the streams inside the containers, then (x_hat non-NULL) the synthesis of
+ * tmae_synthesize.  Writes out->y_hat / z_hat (and out->ids_keep i64 [N, K] when non-NULL), ids_restore i64 [N, L] - the
+ * canonical one: ids_restore[ids_keep[j]] = j, the other positions in ascending order K .. L-1 - and x_hat f32 [N, 3, S, S].
+ * status i32 [N]: 0 = decoded exactly; TMAE_IMG_* for a container the parse refuses (its streams are then not read), TMAE_RANS_*
+ * for streams that do not decode.  A bad container never affects another.  y_lanes / z_lanes: the lane counts every container
+ * must carry.  Replays as one CUDA graph per (N, y_lanes, z_lanes); x_hat needs tmae_enable_synthesis (TMAE_ESTATE). */
+TMAE_API int  tmae_decompress_images(tmae_handle* h, const uint8_t* data, int64_t n_bytes, const int64_t* offsets, int N,
+                                     int y_lanes, int z_lanes, const tmae_outputs* out, int64_t* ids_restore, float* x_hat,
+                                     int32_t* status, void* stream);
+
 /* Stand-alone operators on the path (each mirrors one reference call) ---------------------------------- */
 /* MCM.get_ids_shuffle + random_masking index work (MCM.py:364-423, 579-583). Outputs may be NULL. */
 TMAE_API int  tmae_mask_select(const float* scores, int N, int L, int K, int softmax_isa,

@@ -24,6 +24,7 @@ SOURCES = {
     "mask.cu": ["-fmad=false"],
     "scores.cu": ["-fmad=false"],
     "rans.cu": [],
+    "container.cu": [],
     "huffman.cpp": [],
     "tmae_api.cu": [],
 }

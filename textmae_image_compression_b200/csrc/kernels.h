@@ -18,10 +18,17 @@ struct IoBlock {
     const int32_t* z_symbols;        // decode: z symbols [N, Cz, s/4, s/4] (range-coder order)
     const int32_t* y_symbols;        // decode: y symbols [N, Cy * s * s], per image slice by slice in (c, y, x) order
     const uint8_t* y_data;           // decode from streams (tmae_decompress_streams): image n's y stream is bytes
-    const int64_t* y_offsets;        //   [y_offsets[n], y_offsets[n + 1]) of y_data; likewise z
+    const int64_t* y_offsets;        //   [y_offsets[n], y_ends[n]) of y_data; likewise z.  Streams packed back to back:
+    const int64_t* y_ends;           //   y_ends = y_offsets + 1; inside image containers: the ranges image_parse_kernel wrote
     const uint8_t* z_data;
     const int64_t* z_offsets;
-    int32_t* status;                 //   [N] per-image coder status (RANS_ST_* bits)
+    const int64_t* z_ends;
+    int32_t* status;                 //   [N] per-image coder status (RANS_ST_* bits, and IMG_ST_* from the container parse)
+    const uint8_t* img_data;         // decode from image containers (tmae_decompress_images): container n is bytes
+    const int64_t* img_offsets;      //   [img_offsets[n], img_offsets[n + 1]) of img_data, inside [0, img_n_bytes)
+    long long img_n_bytes;
+    int64_t* img_ids_restore;        //   [N, L] out: the canonical ids_restore of every container
+    int64_t* img_ids_keep;           //   [N, K] out (may be null): the kept patch ids of every container
     const float* syn_y_hat;          // synthesis (tmae_synthesize): y_hat f32 [N, s, s, Cy] in,
     const int64_t* syn_ids;          //   ids_restore [N, L] in,
     float* syn_x_hat;                //   x_hat f32 [N, 3, S, S] out
@@ -132,8 +139,9 @@ struct RansDecArgs {
     int entries = 0, n_tab = 0;
     int lanes = 0;                   // 0: compressai's format (warp per stream); 1..32: laned format (thread per lane), state [s * lanes + l]
     int use_smem = 0, streams_per_block = 1;                 // set by launch_rans_decode
-    const uint8_t* data = nullptr;   // streams: bytes [offsets[s], offsets[s + 1]) of data
-    const int64_t* offsets = nullptr;
+    const uint8_t* data = nullptr;   // streams: bytes [begins[s], ends[s]) of data (packed back to back: ends = begins + 1)
+    const int64_t* begins = nullptr;
+    const int64_t* ends = nullptr;
     const int32_t* indexes = nullptr;                        // [s * idx_stride + i]; nullptr: table (i / idx_div)
     long long idx_stride = 0;
     int idx_div = 1;
@@ -144,7 +152,7 @@ struct RansDecArgs {
     int status_reset = 1;            // init: overwrite status[s] (else OR into it)
     RansDecState* state = nullptr;   // between stages (init == 0 reads it, fin == 0 writes it)
     int32_t* status = nullptr;
-    const IoBlock* io = nullptr;     // non-null: data / offsets / status (and, io_stream 1, the indexes io->out.y_indexes)
+    const IoBlock* io = nullptr;     // non-null: data / begins / ends / status (and, io_stream 1, the indexes io->out.y_indexes)
     int io_stream = 0;               //   come from the IoBlock: 1 = the y streams, 2 = the z streams
 };
 int pmf_to_quantized_cdf(const float* pmf, int n, int32_t* cdf_out);          // host; cdf_out holds n + 1 entries
@@ -158,6 +166,29 @@ cudaError_t launch_rans_encode(const int32_t* sym, const int32_t* idx, int n_str
                                uint2* rec, uint32_t* scratch, long long cap_words, long long* n_words, uint8_t* out, long long capacity,
                                int64_t* offsets, int32_t* status, cudaStream_t st);
 cudaError_t launch_rans_decode(RansDecArgs a, cudaStream_t st);
+
+// container.cu: image containers (DESIGN.md section 7)
+enum : int32_t {                     // per-image status bits of the container parse (include/tmae.h TMAE_IMG_*)
+    IMG_ST_HEADER = 64,              // magic / version / reserved bits, or section lengths other than the container's byte range
+    IMG_ST_CONFIG = 128,             // geometry, accuracy mode or lane counts other than the handle's / call's
+    IMG_ST_MODEL = 256,              // model tag other than the handle's
+    IMG_ST_IDS = 512,                // a patch id >= L, or two equal ids
+};
+constexpr uint32_t kImageMagic = 0x45414D54u;    // bytes "TMAE"
+struct ImageFields {                 // what the handle writes into (and expects of) words 1 to 4 of a container
+    uint32_t word1;                  // version | accuracy mode << 8 | W_y << 16 | W_z << 24
+    uint32_t word2;                  // img_size | patch_size << 16
+    uint32_t word3;                  // K
+    uint32_t tag;                    // model tag
+    int L, K, id_bits;               // patches, kept patches, bits per packed id
+};
+// after the encodes of N images (stream offsets / status of each kind): container n at offsets[n] of out
+cudaError_t launch_image_pack(const int64_t* ids_keep, const uint8_t* y_bytes, const int64_t* y_off, const int32_t* y_st,
+                              const uint8_t* z_bytes, const int64_t* z_off, const int32_t* z_st, const ImageFields& f, int N,
+                              uint8_t* out, long long capacity, int64_t* offsets, int32_t* status, cudaStream_t st);
+// the containers of io->img_*: canonical ids_restore (io->img_ids_restore), io->img_ids_keep when non-null, io->status, and the
+// stream ranges [4 N] (z begin, z end, y begin, y end)
+cudaError_t launch_image_parse(const IoBlock* io, const ImageFields& f, int N, int64_t* ranges, cudaStream_t st);
 
 // ---- patch-score generation (scores.cu; generate_scores_file.py:19-31, utils/map.py, utils/distribution.py) ----
 constexpr int kScoreMaxLevels = 16;

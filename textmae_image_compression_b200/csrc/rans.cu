@@ -335,8 +335,8 @@ struct LaneReader {
 
 // The table set, [cdf entries | meta 3 per table], staged in shared memory when a.use_smem (the tables are constant: staged
 // while the predecessor finishes); then the per-call pointers, from the IoBlock in a decode-plan replay.
-__device__ __forceinline__ const int* dec_prologue(const RansDecArgs& a, int* smem_tab, const uint8_t*& data, const int64_t*& offsets,
-                                                   const int32_t*& indexes, int32_t*& status) {
+__device__ __forceinline__ const int* dec_prologue(const RansDecArgs& a, int* smem_tab, const uint8_t*& data, const int64_t*& begins,
+                                                   const int64_t*& ends, const int32_t*& indexes, int32_t*& status) {
     const int* tab = a.cdf;
     if (a.use_smem) {
         const int n_words_tab = a.entries + 3 * a.n_tab;
@@ -346,13 +346,15 @@ __device__ __forceinline__ const int* dec_prologue(const RansDecArgs& a, int* sm
     }
     pdl_wait();
     data = a.data;
-    offsets = a.offsets;
+    begins = a.begins;
+    ends = a.ends;
     indexes = a.indexes;
     status = a.status;
     if (a.io) {
         const bool y = a.io_stream == 1;
         data = y ? a.io->y_data : a.io->z_data;
-        offsets = y ? a.io->y_offsets : a.io->z_offsets;
+        begins = y ? a.io->y_offsets : a.io->z_offsets;
+        ends = y ? a.io->y_ends : a.io->z_ends;
         status = a.io->status;
         if (y) indexes = a.io->out.y_indexes;
     }
@@ -390,17 +392,17 @@ __global__ void __launch_bounds__(256)
 rans_decode_kernel(RansDecArgs a) {
     extern __shared__ int smem_tab[];
     const uint8_t* data;
-    const int64_t* offsets;
+    const int64_t *begins, *ends;
     const int32_t* indexes;
     int32_t* status;
-    const int* tab = dec_prologue(a, smem_tab, data, offsets, indexes, status);
+    const int* tab = dec_prologue(a, smem_tab, data, begins, ends, indexes, status);
     const int* meta = tab + a.entries;
     const int lane = threadIdx.x & 31;
     const int s = blockIdx.x * a.streams_per_block + (threadIdx.x >> 5);
     if ((int)(threadIdx.x >> 5) >= a.streams_per_block || s >= a.n_streams) return;
 
-    // the stream: bytes [offsets[s], offsets[s + 1]) of data; a malformed range decodes nothing (reads as zeros)
-    const long long b0 = offsets[s], b1 = offsets[s + 1];
+    // the stream: bytes [begins[s], ends[s]) of data; a malformed range decodes nothing (reads as zeros)
+    const long long b0 = begins[s], b1 = ends[s];
     WordReader rd;
     rd.bad = 0;
     if (b0 < 0 || b1 < b0 || (b0 & 3) || ((b1 - b0) & 3) || (b1 - b0) / 4 > 0xffffffffll) {
@@ -469,10 +471,10 @@ rans_decode_lanes_kernel(RansDecArgs a) {
     extern __shared__ int smem_tab[];
     __shared__ int st_img[256];
     const uint8_t* data;
-    const int64_t* offsets;
+    const int64_t *begins, *ends;
     const int32_t* indexes;
     int32_t* status;
-    const int* tab = dec_prologue(a, smem_tab, data, offsets, indexes, status);
+    const int* tab = dec_prologue(a, smem_tab, data, begins, ends, indexes, status);
     const int* meta = tab + a.entries;
     const int W = a.lanes;
     const int j = threadIdx.x / W, l = threadIdx.x - j * W;
@@ -480,7 +482,7 @@ rans_decode_lanes_kernel(RansDecArgs a) {
     if ((int)threadIdx.x < a.streams_per_block) st_img[threadIdx.x] = 0;
     __syncthreads();
     if (j < a.streams_per_block && s < a.n_streams) {
-        const long long b0 = offsets[s], b1 = offsets[s + 1];
+        const long long b0 = begins[s], b1 = ends[s];
         const bool range_ok = !(b0 < 0 || b1 < b0 || (b0 & 3) || ((b1 - b0) & 3) || (b1 - b0) / 4 > 0xffffffffll);
         LaneReader rd;
         rd.w = reinterpret_cast<const uint32_t*>(data + (range_ok ? b0 : 0));

@@ -55,6 +55,7 @@ struct Bf {
 enum StepKind { ST_MASK, ST_GATHER, ST_GEMM, ST_FORCE, ST_LN, ST_ATTN, ST_EB, ST_GC, ST_RATE, ST_ZERO_RATE,
                 ST_ZDEQ, ST_IDX, ST_YDEQ, ST_DEC_OUT,        // decode plans only
                 ST_ZDEC, ST_YDEC,                            // decode-from-streams plans only: the range decoder
+                ST_PARSE,                                    // image-container plans only: parse and validate the containers
                 ST_SYN_IN, ST_UNSHUF, ST_ATTN32, ST_UNPATCH };  // synthesis plans only
 enum Family { FAM_GEMM = 0, FAM_ATTN, FAM_LN, FAM_MASK, FAM_GATHER, FAM_ENTROPY, FAM_MISC, FAM_CODER, FAM_COUNT };
 const char* kFamilyNames[FAM_COUNT] = {"gemm_tc", "attention", "layernorm", "mask_select", "gather_patches",
@@ -75,8 +76,10 @@ struct Step {
     int ln_final = 0;
     // GC
     int slice = 0, gc_slices = 1;
-    // ST_ZDEC / ST_YDEC: lanes per stream (0 = compressai's format)
+    // ST_ZDEC / ST_YDEC: lanes per stream (0 = compressai's format); ST_PARSE: y lanes, parse_z_lanes z lanes
     int lanes = 0;
+    int parse_z_lanes = 0;
+    bool status_or = false;                    // ST_ZDEC: OR into the status ST_PARSE wrote instead of overwriting it
     std::string tag;
 };
 
@@ -88,6 +91,7 @@ enum PlanKind {
     PLAN_DECODE,                     // tmae_decode_begin / _step
     PLAN_STREAMS,                    // tmae_decompress_streams(_lanes): the decode with the range decoder in front
     PLAN_SYNTH,                      // tmae_synthesize
+    PLAN_IMAGES,                     // tmae_decompress_images: PLAN_STREAMS behind the container parse
 };
 enum PlanDep : unsigned {
     DEP_WS = 1,                      // network workspace (ensure_workspace)
@@ -103,8 +107,9 @@ const unsigned kPlanDeps[] = {
     DEP_WS | DEP_SCALE,                          // PLAN_DECODE
     DEP_WS | DEP_SCALE | DEP_CODER | DEP_CDF,    // PLAN_STREAMS
     DEP_SYNTH,                                   // PLAN_SYNTH
+    DEP_WS | DEP_SCALE | DEP_CODER | DEP_CDF,    // PLAN_IMAGES
 };
-// (kind, batch size, y lanes, z lanes); the lanes are nonzero for the laned PLAN_STREAMS only
+// (kind, batch size, y lanes, z lanes); the lanes are nonzero for the laned PLAN_STREAMS / PLAN_IMAGES only
 typedef std::tuple<int, int, int, int> PlanKey;
 
 struct Plan {
@@ -171,8 +176,19 @@ struct CoderWorkspace {
     int32_t* ysym = nullptr;         // [N, Cy * K] decoded y symbols (ST_YDEC -> ST_YDEQ)
     int32_t* idx = nullptr;          // [N, Cy * K] scale-table indexes, when the caller does not ask for them
     RansDecState* state = nullptr;   // [N * 32] y decoder state between the slice groups (per image, or per image and lane)
+    int64_t* ranges = nullptr;       // [4 N] decode from image containers: z begin, z end, y begin, y end (ST_PARSE -> ST_*DEC)
     size_t enc_bytes = 0;            // tmae_rans_encode scratch: records, per-stream word regions, word counts
     void* enc = nullptr;
+    // tmae_compress_images, grown on demand: the forward's symbols / indexes, the coder-order copies, both encodes' outputs
+    std::vector<void*> img_allocs;
+    int img_cap_N = 0;
+    int32_t *img_fwd = nullptr;      // [2 ny + nz] y symbols, y indexes, z symbols (channels-last)
+    int32_t *img_coder = nullptr;    // [2 ny + nz] y symbols, y indexes, z symbols (coder order)
+    int32_t *img_zidx = nullptr;     // [nz] z indexes: the channel of every element, coder order
+    uint8_t *img_y = nullptr, *img_z = nullptr;     // encoded streams, img_y_cap / img_z_cap bytes
+    long long img_y_cap = 0, img_z_cap = 0;
+    int64_t* img_off = nullptr;      // [2 (N + 1)] y, z stream offsets
+    int32_t* img_st = nullptr;       // [2 N] y, z encode status
 };
 
 // Buffers of the synthesis plans (tmae_synthesize), allocated only on handles with synthesis enabled.  All bf16 buffers hold
@@ -221,6 +237,12 @@ struct tmae_handle {
     int Dd = 0, syn_mlp = 0, syn_out = 0; // decoder width, its MLP width, decoder_pred outputs (p * p * in_chans)
     SynthWorkspace sws;
     CdfTables cdf[2];                // quantised CDF tables: [TMAE_MODEL_GAUSSIAN], [TMAE_MODEL_BOTTLENECK]
+    // model tag of the image containers (tmae_model_tag): the hashed bytes of the scale table and of both table sets, and the tag
+    // over them once all three are installed
+    std::vector<float> tag_scale;
+    std::vector<int32_t> tag_tables[2];
+    bool tag_ok = false;
+    uint32_t tag = 0;
     CoderWorkspace cws;
     int dec_N = 0, dec_next = -1;    // decode in progress: batch size and the next group expected (-1 = none)
     PFN_encodeTiled encode = nullptr;
@@ -1281,7 +1303,8 @@ int ensure_coder_workspace(tmae_handle* h, int N) {
     const size_t ny = (size_t)N * h->Cy * h->K, nz = (size_t)N * h->Cz * h->s4 * h->s4;
     int rc;
     if ((rc = dev_alloc(h, c.allocs, &c.zsym, nz)) || (rc = dev_alloc(h, c.allocs, &c.ysym, ny)) ||
-        (rc = dev_alloc(h, c.allocs, &c.idx, ny)) || (rc = dev_alloc(h, c.allocs, &c.state, (size_t)N * 32)))
+        (rc = dev_alloc(h, c.allocs, &c.idx, ny)) || (rc = dev_alloc(h, c.allocs, &c.state, (size_t)N * 32)) ||
+        (rc = dev_alloc(h, c.allocs, &c.ranges, (size_t)N * 4)))
         return rc;
     c.cap_N = N;
     return TMAE_OK;
@@ -1299,15 +1322,23 @@ int ensure_coder_workspace(tmae_handle* h, int N) {
 // layers just wrote, before ST_YDEQ.  The y decoder's state stays in the coder workspace between the groups.  One stage: the
 // whole decode replays as one CUDA graph per (batch size, lanes).  lanes_y / lanes_z = 0: compressai's format; else the laned
 // format with that many lanes per y / z stream.
-int build_decode_plan(tmae_handle* h, Plan& pl, bool coded, int lanes_y, int lanes_z) {
+// Images (tmae_decompress_images): the coded plan behind ST_PARSE, which validates the containers, writes the canonical
+// ids_restore and the streams' byte ranges in the blob, and resets the status the decoders then OR into.
+int build_decode_plan(tmae_handle* h, Plan& pl, bool coded, int lanes_y, int lanes_z, bool images = false) {
     const int N = pl.N;
     int rc = ensure_workspace(h, N);
     if (rc || (coded && (rc = ensure_coder_workspace(h, N)))) return rc;
     std::vector<std::pair<int, int>> groups;
     slice_groups(h->nsl, groups);
+    if (images) {
+        add_step(pl, ST_PARSE, FAM_CODER, "image_parse");
+        pl.steps.back().lanes = lanes_y;
+        pl.steps.back().parse_z_lanes = lanes_z;
+    }
     if (coded) {
         add_step(pl, ST_ZDEC, FAM_CODER, "rans_decode.z");
         pl.steps.back().lanes = lanes_z;
+        pl.steps.back().status_or = images;
     }
     add_step(pl, ST_ZDEQ, FAM_ENTROPY, "z_dequantize");
     if ((rc = add_hs_steps(h, pl, N))) return rc;
@@ -1412,7 +1443,7 @@ int build_synth_plan(tmae_handle* h, Plan& pl) {
     return TMAE_OK;
 }
 
-// The plan of `kind` for batch size N (lanes: PLAN_STREAMS only), built on first use and kept until drop_plans discards it.
+// The plan of `kind` for batch size N (lanes: PLAN_STREAMS / PLAN_IMAGES only), built on first use and kept until drop_plans discards it.
 int get_plan(tmae_handle* h, PlanKind kind, int N, Plan** out, int lanes_y = 0, int lanes_z = 0) {
     const PlanKey key(kind, N, lanes_y, lanes_z);
     auto it = h->plans.find(key);
@@ -1425,11 +1456,27 @@ int get_plan(tmae_handle* h, PlanKind kind, int N, Plan** out, int lanes_y = 0, 
         case PLAN_FORWARD: case PLAN_FORCED: rc = build_plan(h, *pl, kind == PLAN_FORCED); break;
         case PLAN_DECODE: case PLAN_STREAMS: rc = build_decode_plan(h, *pl, kind == PLAN_STREAMS, lanes_y, lanes_z); break;
         case PLAN_SYNTH: rc = build_synth_plan(h, *pl); break;
+        case PLAN_IMAGES: rc = build_decode_plan(h, *pl, true, lanes_y, lanes_z, true); break;
     }
     if (rc || (rc = finish_plan(h, *pl))) return rc;
     *out = pl.get();
     h->plans[key] = std::move(pl);
     return TMAE_OK;
+}
+
+// Words 1 to 4 of this handle's containers with y_lanes / z_lanes lanes (0 = compressai's format).
+ImageFields image_fields(const tmae_handle* h, int y_lanes, int z_lanes) {
+    ImageFields f;
+    f.word1 = 1u | (((unsigned)h->cfg.flags >> 3) & 7u) << 8 | (unsigned)y_lanes << 16 | (unsigned)z_lanes << 24;
+    f.word2 = (unsigned)h->cfg.img_size | (unsigned)h->cfg.patch_size << 16;
+    f.word3 = (unsigned)h->K;
+    f.tag = h->tag;
+    f.L = h->L;
+    f.K = h->K;
+    int w = 1;
+    while ((1ll << w) < h->L) ++w;                  // max(1, bit_length(L - 1))
+    f.id_bits = w;
+    return f;
 }
 
 // ---- execution -----------------------------------------------------------------------------------------
@@ -1564,10 +1611,14 @@ int run_steps(tmae_handle* h, Plan& pl, const RunArgs& a, cudaStream_t st) {
                 d.symbols = h->cws.zsym; d.sym_stride = (long long)h->Cz * h->s4 * h->s4;
                 d.n_streams = N; d.begin = 0; d.end = h->Cz * h->s4 * h->s4;
                 d.lanes = sp.lanes;
+                d.status_reset = !sp.status_or;
                 d.io = a.io; d.io_stream = 2;
                 CUDA_TRY(h, launch_rans_decode(d, st));
                 break;
             }
+            case ST_PARSE:
+                CUDA_TRY(h, launch_image_parse(a.io, image_fields(h, sp.lanes, sp.parse_z_lanes), N, h->cws.ranges, st));
+                break;
             case ST_SYN_IN:
                 CUDA_TRY(h, launch_synth_input(h->sws.y_bf.p, (long long)N * K * h->Cy, st, a.io));
                 break;
@@ -1679,6 +1730,20 @@ IoBlock decode_io(const int32_t* z_symbols, const int32_t* y_symbols, const tmae
     return hio;
 }
 
+// FNV-1a (32-bit) of the model tag over the installed tables (include/tmae.h tmae_model_tag)
+void update_model_tag(tmae_handle* h) {
+    h->tag_ok = h->scale_table && h->cdf[0].n && h->cdf[1].n;
+    if (!h->tag_ok) return;
+    uint32_t x = 2166136261u;
+    auto eat = [&](const void* p, size_t bytes) {
+        const uint8_t* b = static_cast<const uint8_t*>(p);
+        for (size_t i = 0; i < bytes; ++i) x = (x ^ b[i]) * 16777619u;
+    };
+    eat(h->tag_scale.data(), h->tag_scale.size() * 4);          // the host is little-endian (x86-64 / aarch64)
+    for (const auto& t : h->tag_tables) eat(t.data(), t.size() * 4);
+    h->tag = x;
+}
+
 int check_ready(tmae_handle* h, int N) {
     if (!h) return TMAE_EINVAL;
     h->dec_next = -1;                // any other call on the handle ends a decode in progress
@@ -1747,6 +1812,7 @@ void tmae_destroy(tmae_handle* h) {
     drop_plans(h, DEP_ALL);
     for (CdfTables& t : h->cdf) rans_free_tables(&t);
     free_pool(h->cws.allocs);
+    free_pool(h->cws.img_allocs);
     free_pool(h->sws.allocs);
     if (h->cws.enc) cudaFree(h->cws.enc);
     if (h->cap_stream) cudaStreamDestroy(h->cap_stream);
@@ -2052,7 +2118,10 @@ int tmae_set_scale_table(tmae_handle* h, const float* table, int n) {
     if (!h->scale_table) CUDA_TRY(h, cudaMalloc(reinterpret_cast<void**>(&h->scale_table), 256 * sizeof(float)));
     CUDA_TRY(h, cudaDeviceSynchronize());
     CUDA_TRY(h, cudaMemcpy(h->scale_table, table, (size_t)n * sizeof(float), cudaMemcpyDefault));
+    h->tag_scale.resize(n);
+    CUDA_TRY(h, cudaMemcpy(h->tag_scale.data(), h->scale_table, (size_t)n * sizeof(float), cudaMemcpyDeviceToHost));
     h->n_scale_table = n;
+    update_model_tag(h);
     drop_plans(h, DEP_SCALE);        // plans and their graphs carry the table pointer / length
     h->dec_next = -1;
     return TMAE_OK;
@@ -2184,6 +2253,14 @@ int tmae_set_cdf_tables(tmae_handle* h, int model, const int32_t* cdf, int n_tab
     drop_plans(h, DEP_CDF);                          // their graphs captured the previous tables
     rans_free_tables(&h->cdf[model]);
     h->cdf[model] = t;
+    std::vector<int32_t>& tw = h->tag_tables[model];
+    tw.clear();
+    for (int i = 0; i < n_tables; ++i) {
+        tw.push_back(len[i]);
+        tw.push_back(off[i]);
+        tw.insert(tw.end(), c.begin() + (size_t)i * stride, c.begin() + (size_t)i * stride + len[i]);
+    }
+    update_model_tag(h);
     return TMAE_OK;
 }
 
@@ -2201,6 +2278,41 @@ int coder_tables(tmae_handle* h, int model, const CdfTables** out) {
 namespace {
 bool bad_lanes(int lanes) { return lanes < 1 || lanes > 32; }
 
+// Encode scratch of n_streams streams of n_per symbols: records, one word region per (stream, lane) sized for the longest lane,
+// word counts.
+struct EncScratch {
+    long long cap_words;
+    size_t rec_bytes, words_bytes, total;
+};
+EncScratch enc_scratch_bytes(int n_streams, int n_per, int lanes) {
+    EncScratch e;
+    const int chains = lanes ? lanes : 1;
+    e.cap_words = rans_bound_bytes((n_per + chains - 1) / chains) / 4;
+    e.rec_bytes = ((size_t)n_streams * n_per * sizeof(uint2) + 255) / 256 * 256;
+    e.words_bytes = ((size_t)n_streams * chains * e.cap_words * 4 + 255) / 256 * 256;
+    e.total = e.rec_bytes + e.words_bytes + (size_t)n_streams * chains * 8;
+    return e;
+}
+int grow_enc_scratch(tmae_handle* h, const EncScratch& need) {
+    CoderWorkspace& c = h->cws;
+    if (need.total <= c.enc_bytes) return TMAE_OK;
+    if (c.enc) { cudaFree(c.enc); c.enc = nullptr; c.enc_bytes = 0; }
+    cudaError_t e = cudaMalloc(&c.enc, need.total);
+    if (e != cudaSuccess) return fail(h, TMAE_ENOMEM, "rans_encode scratch (%zu bytes): %s", need.total, cudaGetErrorString(e));
+    c.enc_bytes = need.total;
+    return TMAE_OK;
+}
+// one encode in the handle's scratch (grown by the caller)
+int enqueue_encode(tmae_handle* h, const CdfTables& t, const int32_t* symbols, const int32_t* indexes, int n_streams, int n_per,
+                   int lanes, uint8_t* out, int64_t capacity, int64_t* offsets, int32_t* status, cudaStream_t st) {
+    const EncScratch sz = enc_scratch_bytes(n_streams, n_per, lanes);
+    char* base = static_cast<char*>(h->cws.enc);
+    CUDA_TRY(h, launch_rans_encode(symbols, indexes, n_streams, n_per, lanes, t, reinterpret_cast<uint2*>(base),
+                                   reinterpret_cast<uint32_t*>(base + sz.rec_bytes), sz.cap_words,
+                                   reinterpret_cast<long long*>(base + sz.rec_bytes + sz.words_bytes), out, capacity, offsets, status, st));
+    return TMAE_OK;
+}
+
 // lanes = 0: compressai's format, else the laned format
 int rans_encode_impl(tmae_handle* h, int model, const int32_t* symbols, const int32_t* indexes, int n_streams, int n_per_stream,
                      int lanes, uint8_t* out, int64_t capacity, int64_t* offsets, int32_t* status, void* stream) {
@@ -2210,24 +2322,9 @@ int rans_encode_impl(tmae_handle* h, int model, const int32_t* symbols, const in
     if (n_streams < 1 || n_per_stream < 0 || (n_per_stream > 0 && (!symbols || !indexes)) || !out || !offsets || !status || capacity < 0)
         return fail(h, TMAE_EINVAL, "rans_encode: null pointer or bad size");
     if (reinterpret_cast<uintptr_t>(out) & 3) return fail(h, TMAE_EINVAL, "rans_encode: out must be 4-byte aligned");
-    const int chains = lanes ? lanes : 1;           // scratch: one region per (stream, lane), sized for the longest lane
-    const long long cap_words = rans_bound_bytes((n_per_stream + chains - 1) / chains) / 4;
-    const size_t rec_bytes = ((size_t)n_streams * n_per_stream * sizeof(uint2) + 255) / 256 * 256;
-    const size_t words_bytes = ((size_t)n_streams * chains * cap_words * 4 + 255) / 256 * 256;
-    const size_t need = rec_bytes + words_bytes + (size_t)n_streams * chains * 8;
-    CoderWorkspace& c = h->cws;
-    if (need > c.enc_bytes) {
-        if (c.enc) { cudaFree(c.enc); c.enc = nullptr; c.enc_bytes = 0; }
-        cudaError_t e = cudaMalloc(&c.enc, need);
-        if (e != cudaSuccess) return fail(h, TMAE_ENOMEM, "rans_encode scratch (%zu bytes): %s", need, cudaGetErrorString(e));
-        c.enc_bytes = need;
-    }
-    char* base = static_cast<char*>(c.enc);
-    CUDA_TRY(h, launch_rans_encode(symbols, indexes, n_streams, n_per_stream, lanes, *t, reinterpret_cast<uint2*>(base),
-                                   reinterpret_cast<uint32_t*>(base + rec_bytes), cap_words,
-                                   reinterpret_cast<long long*>(base + rec_bytes + words_bytes), out, capacity, offsets, status,
-                                   reinterpret_cast<cudaStream_t>(stream)));
-    return TMAE_OK;
+    if ((rc = grow_enc_scratch(h, enc_scratch_bytes(n_streams, n_per_stream, lanes)))) return rc;
+    return enqueue_encode(h, *t, symbols, indexes, n_streams, n_per_stream, lanes, out, capacity, offsets, status,
+                          reinterpret_cast<cudaStream_t>(stream));
 }
 
 int rans_decode_impl(tmae_handle* h, int model, const uint8_t* data, const int64_t* offsets, int n_streams, const int32_t* indexes,
@@ -2241,7 +2338,7 @@ int rans_decode_impl(tmae_handle* h, int model, const uint8_t* data, const int64
     RansDecArgs d;
     d.cdf = t->cdf; d.entries = t->entries; d.n_tab = t->n;
     d.lanes = lanes;
-    d.data = data; d.offsets = offsets;
+    d.data = data; d.begins = offsets; d.ends = offsets + 1;
     d.indexes = indexes; d.idx_stride = n_per_stream;
     d.symbols = symbols; d.sym_stride = n_per_stream;
     d.n_streams = n_streams; d.begin = 0; d.end = n_per_stream;
@@ -2267,7 +2364,8 @@ int decompress_streams_impl(tmae_handle* h, const uint8_t* y_data, const int64_t
     if ((rc = get_plan(h, PLAN_STREAMS, N, &pl, y_lanes, z_lanes))) return rc;
     IoBlock hio = decode_io(h->cws.zsym, h->cws.ysym, out);
     if (!hio.out.y_indexes) hio.out.y_indexes = h->cws.idx;
-    hio.y_data = y_data; hio.y_offsets = y_offsets; hio.z_data = z_data; hio.z_offsets = z_offsets; hio.status = status;
+    hio.y_data = y_data; hio.y_offsets = y_offsets; hio.y_ends = y_offsets + 1;
+    hio.z_data = z_data; hio.z_offsets = z_offsets; hio.z_ends = z_offsets + 1; hio.status = status;
     if (h->profiling) h->prof_used = 0;
     return run_stage(h, *pl, 0, hio, h->ws.io, reinterpret_cast<cudaStream_t>(stream));
 }
@@ -2311,6 +2409,139 @@ int tmae_decompress_streams_lanes(tmae_handle* h, const uint8_t* y_data, const i
     if (!h || bad_lanes(y_lanes) || bad_lanes(z_lanes) || !y_data || !y_offsets || !z_data || !z_offsets || !out || !status)
         return fail(h, TMAE_EINVAL, "decompress_streams_lanes: null pointer, or lanes (%d, %d) outside 1..32", y_lanes, z_lanes);
     return decompress_streams_impl(h, y_data, y_offsets, y_lanes, z_data, z_offsets, z_lanes, N, out, status, stream);
+}
+
+// ---- image containers (DESIGN.md section 7) ---------------------------------------------------------------
+namespace {
+bool bad_img_lanes(int lanes) { return lanes < 0 || lanes > 32; }
+
+long long stream_bound(long long n, int lanes) { return lanes ? rans_bound_lanes_bytes(n, lanes) : rans_bound_bytes(n); }
+
+long long image_bound(const tmae_handle* h, int y_lanes, int z_lanes) {
+    const ImageFields f = image_fields(h, y_lanes, z_lanes);
+    return 28 + 4 * (((long long)f.K * f.id_bits + 31) / 32) + stream_bound((long long)h->Cy * h->K, y_lanes) +
+           stream_bound((long long)h->Cz * h->s4 * h->s4, z_lanes);
+}
+
+// The handle can write / read containers: geometry that fits the header fields, the scale table and both table sets (the tag).
+int images_ready(tmae_handle* h) {
+    if (h->cfg.img_size > 0xffff || h->cfg.patch_size > 0xff || h->K > 0xffff)
+        return fail(h, TMAE_EINVAL, "image containers hold img_size < 65536, patch_size < 256 and K < 65536");
+    if (!h->scale_table) return fail(h, TMAE_ESTATE, "image containers need the scale table (call tmae_set_scale_table first)");
+    if (!h->tag_ok) return fail(h, TMAE_ESTATE, "image containers need both cdf table sets (tmae_set_cdf_tables)");
+    if (h->cdf[TMAE_MODEL_GAUSSIAN].n != h->n_scale_table)
+        return fail(h, TMAE_ESTATE, "%d Gaussian cdf tables for a scale table of %d entries", h->cdf[TMAE_MODEL_GAUSSIAN].n, h->n_scale_table);
+    return TMAE_OK;
+}
+
+// Buffers of tmae_compress_images for N images, sized for the larger (32-lane) stream bound of either format.
+int ensure_image_workspace(tmae_handle* h, int N) {
+    CoderWorkspace& c = h->cws;
+    if (N <= c.img_cap_N) return TMAE_OK;
+    free_pool(c.img_allocs);
+    c.img_cap_N = 0;
+    const size_t hw4 = (size_t)h->s4 * h->s4, ny = (size_t)N * h->Cy * h->K, nz = (size_t)N * h->Cz * hw4;
+    c.img_y_cap = N * rans_bound_lanes_bytes((long long)h->Cy * h->K, 32);
+    c.img_z_cap = N * rans_bound_lanes_bytes((long long)h->Cz * hw4, 32);
+    int rc;
+    if ((rc = dev_alloc(h, c.img_allocs, &c.img_fwd, 2 * ny + nz)) || (rc = dev_alloc(h, c.img_allocs, &c.img_coder, 2 * ny + nz)) ||
+        (rc = dev_alloc(h, c.img_allocs, &c.img_zidx, nz)) ||
+        (rc = dev_alloc(h, c.img_allocs, &c.img_y, (size_t)c.img_y_cap)) || (rc = dev_alloc(h, c.img_allocs, &c.img_z, (size_t)c.img_z_cap)) ||
+        (rc = dev_alloc(h, c.img_allocs, &c.img_off, 2 * ((size_t)N + 1))) || (rc = dev_alloc(h, c.img_allocs, &c.img_st, 2 * (size_t)N)))
+        return rc;
+    std::vector<int32_t> zidx(nz);                  // the z indexes never change: the channel of every element, coder order
+    for (size_t i = 0; i < nz; ++i) zidx[i] = (int32_t)((i / hw4) % h->Cz);
+    CUDA_TRY(h, cudaMemcpy(c.img_zidx, zidx.data(), nz * sizeof(int32_t), cudaMemcpyHostToDevice));
+    c.img_cap_N = N;
+    return TMAE_OK;
+}
+}  // namespace
+
+int tmae_model_tag(const tmae_handle* h, uint32_t* tag) {
+    if (!h || !tag) return TMAE_EINVAL;
+    if (!h->tag_ok) return TMAE_ESTATE;
+    *tag = h->tag;
+    return TMAE_OK;
+}
+
+int64_t tmae_images_bound(const tmae_handle* h, int N, int y_lanes, int z_lanes) {
+    if (!h || N < 1 || bad_img_lanes(y_lanes) || bad_img_lanes(z_lanes)) return -1;
+    return N * image_bound(h, y_lanes, z_lanes);
+}
+
+int tmae_compress_images(tmae_handle* h, const float* imgs, const float* scores, int N, int y_lanes, int z_lanes, uint8_t* out,
+                         int64_t capacity, int64_t* offsets, int32_t* status, void* stream) {
+    if (!h) return TMAE_EINVAL;
+    if (!imgs || !scores || !out || !offsets || !status || N < 1 || capacity < 0 || bad_img_lanes(y_lanes) || bad_img_lanes(z_lanes))
+        return fail(h, TMAE_EINVAL, "compress_images: null pointer, N < 1, capacity < 0 or lanes (%d, %d) outside 0..32", y_lanes, z_lanes);
+    if ((reinterpret_cast<uintptr_t>(out) | reinterpret_cast<uintptr_t>(status)) & 3 || reinterpret_cast<uintptr_t>(offsets) & 7)
+        return fail(h, TMAE_EINVAL, "compress_images: out and status must be 4-byte aligned, offsets 8-byte aligned");
+    int rc = check_ready(h, N);
+    if (rc || (rc = images_ready(h))) return rc;
+    const long long hw = (long long)h->s * h->s, hw4 = (long long)h->s4 * h->s4;
+    const int ny = h->Cy * h->K, nz = (int)(h->Cz * hw4);
+    const EncScratch ys = enc_scratch_bytes(N, ny, y_lanes), zs = enc_scratch_bytes(N, nz, z_lanes);
+    if ((rc = ensure_image_workspace(h, N)) || (rc = grow_enc_scratch(h, ys.total > zs.total ? ys : zs))) return rc;
+    Plan* pl = nullptr;
+    if ((rc = get_plan(h, PLAN_FORWARD, N, &pl))) return rc;
+    CoderWorkspace& c = h->cws;
+    const size_t sy = (size_t)N * ny;
+    int32_t *f_ysym = c.img_fwd, *f_yidx = f_ysym + sy, *f_zsym = f_yidx + sy;
+    int32_t *ysym = c.img_coder, *yidx = ysym + sy, *zsym = yidx + sy, *zidx = c.img_zidx;
+    tmae_outputs o;
+    memset(&o, 0, sizeof(o));
+    o.y_symbols = f_ysym; o.y_indexes = f_yidx; o.z_symbols = f_zsym;
+    cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+    if (h->profiling) h->prof_used = 0;
+    if ((rc = run_forward(h, *pl, imgs, scores, &o, st))) return rc;
+    CUDA_TRY(h, launch_pack_nchw_i32(f_ysym, ysym, N, (int)hw, h->Cy, st));
+    CUDA_TRY(h, launch_pack_nchw_i32(f_yidx, yidx, N, (int)hw, h->Cy, st));
+    CUDA_TRY(h, launch_pack_nchw_i32(f_zsym, zsym, N, (int)hw4, h->Cz, st));
+    int64_t *y_off = c.img_off, *z_off = c.img_off + N + 1;
+    int32_t *y_st = c.img_st, *z_st = c.img_st + N;
+    if ((rc = enqueue_encode(h, h->cdf[TMAE_MODEL_GAUSSIAN], ysym, yidx, N, ny, y_lanes, c.img_y, c.img_y_cap, y_off, y_st, st)) ||
+        (rc = enqueue_encode(h, h->cdf[TMAE_MODEL_BOTTLENECK], zsym, zidx, N, nz, z_lanes, c.img_z, c.img_z_cap, z_off, z_st, st)))
+        return rc;
+    CUDA_TRY(h, launch_image_pack(h->ws.ids_keep, c.img_y, y_off, y_st, c.img_z, z_off, z_st, image_fields(h, y_lanes, z_lanes), N,
+                                  out, capacity, offsets, status, st));
+    return TMAE_OK;
+}
+
+int tmae_decompress_images(tmae_handle* h, const uint8_t* data, int64_t n_bytes, const int64_t* offsets, int N, int y_lanes,
+                           int z_lanes, const tmae_outputs* out, int64_t* ids_restore, float* x_hat, int32_t* status, void* stream) {
+    if (!h) return TMAE_EINVAL;
+    if (!data || !offsets || !out || !out->y_hat || !out->z_hat || !ids_restore || !status || N < 1 || n_bytes < 0 ||
+        bad_img_lanes(y_lanes) || bad_img_lanes(z_lanes))
+        return fail(h, TMAE_EINVAL, "decompress_images: null pointer, N < 1, n_bytes < 0 or lanes (%d, %d) outside 0..32", y_lanes, z_lanes);
+    if ((reinterpret_cast<uintptr_t>(data) | reinterpret_cast<uintptr_t>(status)) & 3 ||
+        (reinterpret_cast<uintptr_t>(offsets) | reinterpret_cast<uintptr_t>(ids_restore) | reinterpret_cast<uintptr_t>(out->ids_keep)) & 7)
+        return fail(h, TMAE_EINVAL, "decompress_images: data and status must be 4-byte aligned, offsets, ids_restore and "
+                    "out->ids_keep 8-byte aligned");
+    if (x_hat && ((reinterpret_cast<uintptr_t>(out->y_hat) | reinterpret_cast<uintptr_t>(x_hat)) & 15))
+        return fail(h, TMAE_EINVAL, "decompress_images: y_hat and x_hat must be 16-byte aligned");
+    int rc = check_ready(h, N);
+    if (rc || (rc = images_ready(h))) return rc;
+    if (x_hat && h->syn_depth == 0) return fail(h, TMAE_ESTATE, "x_hat needs synthesis (call tmae_enable_synthesis)");
+    if (x_hat && h->cfg.in_chans != 3) return fail(h, TMAE_EINVAL, "synthesis writes 3-channel images (in_chans %d)", h->cfg.in_chans);
+    Plan* pl = nullptr;
+    Plan* syn = nullptr;
+    if ((rc = get_plan(h, PLAN_IMAGES, N, &pl, y_lanes, z_lanes)) || (x_hat && (rc = get_plan(h, PLAN_SYNTH, N, &syn)))) return rc;
+    IoBlock hio = decode_io(h->cws.zsym, h->cws.ysym, out);
+    if (!hio.out.y_indexes) hio.out.y_indexes = h->cws.idx;
+    const int64_t* r = h->cws.ranges;               // the parse's stream ranges (build order of launch_image_parse)
+    hio.y_data = data; hio.y_offsets = r + 2 * N; hio.y_ends = r + 3 * N;
+    hio.z_data = data; hio.z_offsets = r; hio.z_ends = r + N;
+    hio.status = status;
+    hio.img_data = data; hio.img_offsets = offsets; hio.img_n_bytes = n_bytes; hio.img_ids_restore = ids_restore;
+    hio.img_ids_keep = out->ids_keep;
+    cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+    if (h->profiling) h->prof_used = 0;
+    if ((rc = run_stage(h, *pl, 0, hio, h->ws.io, st))) return rc;
+    if (!x_hat) return TMAE_OK;
+    IoBlock sio;
+    memset(&sio, 0, sizeof(sio));
+    sio.syn_y_hat = out->y_hat; sio.syn_ids = ids_restore; sio.syn_x_hat = x_hat;
+    return run_stage(h, *syn, 0, sio, h->sws.io, st);
 }
 
 int tmae_pack_nchw_i32(const int32_t* nhwc, int32_t* nchw, int N, int hw, int C, void* stream) {

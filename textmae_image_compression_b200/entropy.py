@@ -173,6 +173,21 @@ def decode_lanes(handle, model: int, data: torch.Tensor, offsets: torch.Tensor, 
     return sym, status
 
 
+def images_bound(handle, n_images: int, y_lanes: int, z_lanes: int) -> int:
+    """Bytes that always suffice for the image containers of n_images images (include/tmae.h tmae_images_bound)."""
+    return int(_native.load().tmae_images_bound(handle, n_images, y_lanes, z_lanes))
+
+
+_IMAGE_REASONS = ((_native.IMG_HEADER, "header"), (_native.IMG_CONFIG, "configuration"), (_native.IMG_MODEL, "model"),
+                  (_native.IMG_IDS, "patch ids"))
+
+
+def image_status_reason(status: int) -> str:
+    """Why a container did not decode, from its status: the container checks that failed, else the streams'."""
+    reasons = [name for bit, name in _IMAGE_REASONS if status & bit]
+    return ", ".join(reasons) if reasons else "a stream that does not decode"
+
+
 def pack_strings(strings) -> Tuple[torch.Tensor, torch.Tensor]:
     """list of bytes -> (uint8 [total] host tensor, int64 [n + 1] byte offsets)."""
     lens = [len(s) for s in strings]

@@ -23,6 +23,8 @@ include/tmae.h.  PyTorch is used for device memory, streams and the module plumb
 order `encode_with_indexes` consumes, z symbols / channel indexes for `entropy_bottleneck.compress` (SURVEY 8f-1).
 `compress_bitstream` / `decompress_bitstream` add the GPU rANS coder (entropy.py, csrc/rans.cu) on either side: images to
 compressai-format byte strings and back.
+`compress_images` / `decompress_images` wrap both streams, the patch selection and a header into one self-contained byte string per
+image (DESIGN.md section 7), decoded on the GPU from nothing but those bytes.
 `decompress_symbols` is the decoder side of `MCM.decompress` (MCM.py:896-968) around the range decoder: symbols in (all at
 once, or group by group through a callback that receives the scale-table indexes), y_hat / z_hat / x_hat out, bit-exact
 with the encoder of the same accuracy mode.
@@ -38,7 +40,7 @@ x_hat (g_s + MAE decoder + unpatchify) comes from one of two paths:
 from __future__ import annotations
 
 import ctypes as C
-from typing import Callable, Dict, Iterator, Optional, Tuple
+from typing import Callable, Dict, Iterator, List, Optional, Tuple
 
 import torch
 import torch.nn as nn
@@ -773,6 +775,114 @@ class MCM(nn.Module):
             out["x_hat"] = x_hat
         elif need_recon:
             out["x_hat"] = recon.synthesize(self._weights, c, y_hat.reshape(N, c.num_keep_patches, c.latent_depth), ids_restore.to(dev))
+        return out
+
+    # ------------------------------------------------------------------ image containers (DESIGN.md section 7)
+    @staticmethod
+    def _check_image_lanes(lanes):
+        """(W_y, W_z) of a container: (0, 0) for compressai's format (lanes=None)."""
+        checked = MCM._check_lanes(lanes)
+        return (0, 0) if checked is None else checked
+
+    @torch.no_grad()
+    def compress_images(self, imgs: torch.Tensor, total_scores: torch.Tensor, lanes=(32, 4)) -> List[bytes]:
+        """One self-contained byte string per image: a header (geometry, accuracy mode, lane counts, the tag of the entropy model),
+        the kept patch ids bit-packed, then the z and y rANS streams of `compress_bitstream(imgs, total_scores, lanes)`.
+        `decompress_images` needs nothing else.  The forward, both encodes and the packing are enqueued on the current stream;
+        the host then reads the container offsets and status, and exactly the containers' bytes.  lanes=None puts
+        compressai-format streams inside.  Raises RuntimeError naming the images whose encode failed."""
+        y_lanes, z_lanes = self._check_image_lanes(lanes)
+        self._ensure_handle()
+        self._check_inputs(imgs, total_scores)
+        self._install_coder_tables()
+        dev = self._handle_device
+        imgs = imgs.to(device=dev, dtype=torch.float32).contiguous()
+        total_scores = total_scores.to(device=dev, dtype=torch.float32).contiguous()
+        N = imgs.shape[0]
+        lib = _native.load()
+        cap = entropy.images_bound(self._handle, N, y_lanes, z_lanes)
+        with torch.cuda.device(dev):
+            out = torch.empty(cap, dtype=torch.uint8, device=dev)
+            meta = torch.empty(2 * N + 1, dtype=torch.int64, device=dev)        # offsets [N + 1] | status int32 [N] (padded)
+            status = meta[N + 1:].view(torch.int32)[:N]
+            cur = self._enter_stream(dev)
+            _native.check(lib.tmae_compress_images(self._handle, C.c_void_p(imgs.data_ptr()), C.c_void_p(total_scores.data_ptr()), N,
+                                                   y_lanes, z_lanes, C.c_void_p(out.data_ptr()), cap, C.c_void_p(meta.data_ptr()),
+                                                   C.c_void_p(status.data_ptr()), C.c_void_p(cur.cuda_stream)),
+                          self._handle, RuntimeError)
+            self._leave_stream(cur)
+            host_meta = meta.cpu()
+            offs = host_meta[: N + 1].tolist()
+            st = host_meta[N + 1:].view(torch.int32)[:N].tolist()
+            bad = [i for i in range(N) if st[i]]
+            if bad:
+                raise RuntimeError(f"image container encode failed for images {bad} (status {[st[i] for i in bad]})")
+            host = out[: offs[-1]].cpu().numpy().tobytes()
+        return [host[offs[i]: offs[i + 1]] for i in range(N)]
+
+    @torch.no_grad()
+    def decompress_images(self, strings, need_recon: Optional[bool] = None) -> Dict[str, torch.Tensor]:
+        """Decode `compress_images`' byte strings with nothing else: one copy of the containers (and their offsets) to the device,
+        the container parse, the rANS decode and the network in one enqueued decode, one status read at the end.
+        Returns {"y_hat": f32 [N,Cy,s,s], "z_hat": f32 [N,Cz,s/4,s/4], "ids_restore": i64 [N,L], "ids_keep": i64 [N,K]} and, with
+        `need_recon` (default: whenever the decoder-side weights are loaded), "x_hat" exactly as forward computes it (on the
+        engine with native_synthesis=True, else recon.synthesize).  ids_restore is the canonical one (the kept ids at their
+        positions, the other positions ascending); x_hat reads no more of it than that.  The lane counts are the first
+        container's; a container with other lane counts, or any geometry, accuracy mode or entropy model other than this
+        module's, is refused.  Raises ValueError naming each image that does not decode and why."""
+        if need_recon is None:
+            need_recon = recon.has_decoder_weights(self._weights)
+        if need_recon and not recon.has_decoder_weights(self._weights):
+            raise RuntimeError("need_recon=True but the loaded state dict has no g_s / decoder tensors")
+        if not isinstance(strings, (list, tuple)) or len(strings) < 1:
+            raise ValueError("strings must be a non-empty list of byte strings")
+        strings = list(strings)
+        bad = [i for i, b in enumerate(strings) if not isinstance(b, (bytes, bytearray, memoryview)) or len(b) % 4 or len(b) < 28]
+        if bad:
+            raise ValueError(f"images {bad} do not decode (header: a container is bytes of a length that is a multiple of 4 and >= 28)")
+        self._ensure_handle()
+        self._install_coder_tables()
+        c = self.cfg
+        s, s4 = c.side, c.side // 4
+        N = len(strings)
+        lanes = (bytes(strings[0][6:7])[0], bytes(strings[0][7:8])[0])          # bytes 2 and 3 of word 1
+        if not all(w <= 32 for w in lanes):
+            lanes = (0, 0)                       # not a lane count: the call decodes compressai-format containers, and refuses
+                                                 # (configuration) every container with lanes, the first one included
+        dev = self._handle_device
+        data, off = entropy.pack_strings([bytes(b) for b in strings])
+        host = torch.cat([off.view(torch.uint8), data])       # offsets int64 [N + 1] | containers
+        f32 = torch.float32
+        y_hat = torch.empty((N, s, s, c.latent_depth), dtype=f32, device=dev)
+        z_hat = torch.empty((N, s4, s4, c.hyperprior_depth), dtype=f32, device=dev)
+        ids_restore = torch.empty((N, c.num_patches), dtype=torch.int64, device=dev)
+        ids_keep = torch.empty((N, c.num_keep_patches), dtype=torch.int64, device=dev)
+        status = torch.empty(N, dtype=torch.int32, device=dev)
+        native_x = need_recon and self._syn_on
+        x_hat = torch.empty((N, c.in_chans, c.img_size, c.img_size), dtype=f32, device=dev) if native_x else None
+        o = _native.TmaeOutputs()
+        o.y_hat, o.z_hat, o.ids_keep = y_hat.data_ptr(), z_hat.data_ptr(), ids_keep.data_ptr()
+        lib = _native.load()
+        with torch.cuda.device(dev):
+            cur = self._enter_stream(dev)
+            buf = host.pin_memory().to(dev, non_blocking=True)
+            b0 = buf.data_ptr()
+            _native.check(lib.tmae_decompress_images(self._handle, C.c_void_p(b0 + 8 * (N + 1)), data.numel(), C.c_void_p(b0), N,
+                                                     lanes[0], lanes[1], C.byref(o), C.c_void_p(ids_restore.data_ptr()),
+                                                     C.c_void_p(x_hat.data_ptr()) if native_x else None,
+                                                     C.c_void_p(status.data_ptr()), C.c_void_p(cur.cuda_stream)),
+                          self._handle, RuntimeError)
+            self._leave_stream(cur)
+        st = status.cpu().tolist()
+        bad = [i for i in range(N) if st[i]]
+        if bad:
+            why = "; ".join(f"image {i}: {entropy.image_status_reason(st[i])} (status {st[i]})" for i in bad)
+            raise ValueError(f"images {bad} do not decode - {why}")
+        out = {"y_hat": self._nchw(y_hat), "z_hat": self._nchw(z_hat), "ids_restore": ids_restore, "ids_keep": ids_keep}
+        if native_x:
+            out["x_hat"] = x_hat
+        elif need_recon:
+            out["x_hat"] = recon.synthesize(self._weights, c, y_hat.reshape(N, c.num_keep_patches, c.latent_depth), ids_restore)
         return out
 
     def compress(self, *args, **kwargs):
