@@ -302,6 +302,48 @@ TMAE_API int  tmae_decompress_images(tmae_handle* h, const uint8_t* data, int64_
                                      int y_lanes, int z_lanes, const tmae_outputs* out, int64_t* ids_restore, float* x_hat,
                                      int32_t* status, void* stream);
 
+/* Picture containers (DESIGN.md section 7, "The picture container"): a picture of any size H x W (1..65535 each) in one byte
+ * string.  The picture is zero-padded on the bottom / right to whole tiles of side S = img_size and cut into T = rows * cols tiles
+ * in raster order (tiling.py's policy); every tile is coded as the image container tmae_compress_images writes for it, with the
+ * scores the score generator makes from the tile's grey pixels (out_side = img_size).  Little-endian 32-bit words: magic "TMAP",
+ * version 1 (byte 0; bytes 1-3 reserved, 0), H | W << 16, T, the byte length of each tile container, then the T tile containers.
+ * A picture is 4 (4 + T) + sum of the lengths bytes.  Status bit above the image containers' (ORed with its tiles' status): */
+#define TMAE_PIC_HEADER         1024 /* decode: bad magic / version / reserved bits, H / W / T other than the call's, lengths that are
+                                        not multiples of 4 or do not add up to the picture's byte range (or a range outside
+                                        [0, n_bytes)); every tile of the picture is then refused as well (TMAE_IMG_HEADER) */
+/* Stand-alone: pictures f32 [P, 3, H, W] -> tiles f32 [P T, 3, tile, tile] and grey tiles u8 [P T, tile, tile] (either output may
+ * be NULL), zero padding, equal to tiling.tile_image.  The grey tiles are cut from gray u8 [P, H, W], or, with gray NULL, made from
+ * the RGB as OpenCV's cvtColor(RGB2GRAY) of v = saturate_u8(rint(255 x)): (9798 R + 19235 G + 3735 B + 16384) >> 15. */
+TMAE_API int  tmae_picture_tiles(const float* imgs, const uint8_t* gray, int P, int H, int W, int tile, float* tiles,
+                                 uint8_t* gray_tiles, void* stream);
+/* Stand-alone: tiles f32 [P T, 3, tile, tile] -> canvas f32 [P, 3, H, W], padding dropped (tiling.untile_image of each picture). */
+TMAE_API int  tmae_picture_untile(const float* tiles, int P, int H, int W, int tile, float* canvas, void* stream);
+/* Host-only: H, W and T of the picture in h_data [n_bytes] and the lane counts of its first tile (any output may be NULL).
+ * TMAE_EINVAL for bytes that are not a picture (magic, version, reserved bits, a first tile that is not an image container, or a
+ * T other than the tile grid of H x W at the first tile's img_size). */
+TMAE_API int  tmae_picture_geometry(const uint8_t* h_data, int64_t n_bytes, int* H, int* W, int* T, int* y_lanes, int* z_lanes);
+/* Host-only: bytes that always suffice for P pictures of H x W; -1 for a null handle, P < 1, H or W outside 1..65535 or lanes
+ * outside {0} and 1..32. */
+TMAE_API int64_t tmae_pictures_bound(const tmae_handle* h, int P, int H, int W, int y_lanes, int z_lanes);
+/* P pictures imgs f32 [P, 3, H, W] (gray u8 [P, H, W] or NULL as in tmae_picture_tiles) to one picture container each, enqueued on
+ * `stream` without a host synchronisation: the tiling, the score generator on the grey tiles, the forward of the P T tiles, both
+ * rANS encodes and the pack, which writes the tile containers straight into the picture layout.  Picture p is bytes
+ * [offsets[p], offsets[p + 1]) of `out` (capacity bytes; tmae_pictures_bound always suffices).  status i32 [P]: the OR of its tiles'
+ * encode bits, or TMAE_RANS_OVERFLOW.  P T <= 65535.  Argument checks as tmae_compress_images (out and status 4-byte aligned,
+ * offsets 8-byte aligned), and in_chans must be 3.  Scratch (tiles, grey tiles, scores) is the handle's, grown on first use. */
+TMAE_API int  tmae_compress_pictures(tmae_handle* h, const float* imgs, const uint8_t* gray, int P, int H, int W, int y_lanes,
+                                     int z_lanes, uint8_t* out, int64_t capacity, int64_t* offsets, int32_t* status, void* stream);
+/* Decode of P pictures of H x W, bytes [offsets[p], offsets[p + 1]) of data (n_bytes long), enqueued without a host
+ * synchronisation: the picture parse, then the image-container decode of the P T tiles (tmae_decompress_images), replayed as one
+ * CUDA graph per (tiles, lanes, H x W); then, x_hat non-NULL, the synthesis of the tiles and their untiling into x_hat
+ * f32 [P, 3, H, W].  tile_out (may be NULL): y_hat / z_hat / ids_keep and the other decode outputs of the tiles, as in
+ * tmae_decompress_images; ids_restore i64 [P T, L] (may be NULL).  status i32 [P]: TMAE_PIC_HEADER ORed with the status of every
+ * tile of the picture.  A bad picture never affects another; the pixels of a picture with nonzero status are unspecified, but every
+ * write stays inside its canvas.  Alignment: data and status 4 bytes, offsets, ids_restore and ids_keep 8, y_hat and x_hat 16. */
+TMAE_API int  tmae_decompress_pictures(tmae_handle* h, const uint8_t* data, int64_t n_bytes, const int64_t* offsets, int P, int H,
+                                       int W, int y_lanes, int z_lanes, const tmae_outputs* tile_out, int64_t* ids_restore,
+                                       float* x_hat, int32_t* status, void* stream);
+
 /* Stand-alone operators on the path (each mirrors one reference call) ---------------------------------- */
 /* MCM.get_ids_shuffle + random_masking index work (MCM.py:364-423, 579-583). Outputs may be NULL. */
 TMAE_API int  tmae_mask_select(const float* scores, int N, int L, int K, int softmax_isa,

@@ -20,6 +20,7 @@ FLAG_PRECISE_X6 = 32
 MODEL_GAUSSIAN, MODEL_BOTTLENECK = 0, 1
 RANS_OVERRUN, RANS_UNFINISHED, RANS_BAD_INDEX, RANS_RANGE, RANS_OVERFLOW, RANS_MALFORMED = 1, 2, 4, 8, 16, 32
 IMG_HEADER, IMG_CONFIG, IMG_MODEL, IMG_IDS = 64, 128, 256, 512
+PIC_HEADER = 1024
 
 
 class TmaeConfig(C.Structure):
@@ -98,6 +99,14 @@ SIGNATURES = {
     "tmae_images_bound": (C.c_int64, [_P, C.c_int, C.c_int, C.c_int]),
     "tmae_compress_images": (C.c_int, [_P, _P, _P, C.c_int, C.c_int, C.c_int, _P, C.c_int64, _P, _P, _P]),
     "tmae_decompress_images": (C.c_int, [_P, _P, C.c_int64, _P, C.c_int, C.c_int, C.c_int, C.POINTER(TmaeOutputs), _P, _P, _P, _P]),
+    "tmae_picture_tiles": (C.c_int, [_P, _P, C.c_int, C.c_int, C.c_int, C.c_int, _P, _P, _P]),
+    "tmae_picture_untile": (C.c_int, [_P, C.c_int, C.c_int, C.c_int, C.c_int, _P, _P]),
+    "tmae_picture_geometry": (C.c_int, [_P, C.c_int64, C.POINTER(C.c_int), C.POINTER(C.c_int), C.POINTER(C.c_int),
+                                        C.POINTER(C.c_int), C.POINTER(C.c_int)]),
+    "tmae_pictures_bound": (C.c_int64, [_P, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int]),
+    "tmae_compress_pictures": (C.c_int, [_P, _P, _P, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, _P, C.c_int64, _P, _P, _P]),
+    "tmae_decompress_pictures": (C.c_int, [_P, _P, C.c_int64, _P, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int,
+                                           C.POINTER(TmaeOutputs), _P, _P, _P, _P]),
     "tmae_mask_select": (C.c_int, [_P, C.c_int, C.c_int, C.c_int, C.c_int, _P, _P, _P, _P]),
     "tmae_gaussian_rate": (C.c_int, [_P, _P, _P, C.c_int64, _P, _P, _P, _P]),
     "tmae_bottleneck_rate": (C.c_int, [_P, _P, C.c_int64, _P, _P, _P, _P]),

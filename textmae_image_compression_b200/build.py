@@ -25,6 +25,7 @@ SOURCES = {
     "scores.cu": ["-fmad=false"],
     "rans.cu": [],
     "container.cu": [],
+    "picture.cu": [],
     "huffman.cpp": [],
     "tmae_api.cu": [],
 }

@@ -3,7 +3,7 @@
 //   | 3 K (16 bits), reserved (16) | 4 model tag | 5 z stream bytes | 6 y stream bytes
 //   | ids_keep[0..K) in w = max(1, bit_length(L - 1)) bits each, LSB-first, zero-padded to a word | z stream | y stream
 // Pack: one CTA per image after the two rANS encodes; the container's offset is the sum of the earlier containers' lengths,
-// which the encodes' stream offsets (exclusive prefix sums) already give.  Parse: one CTA per container, the first stage of the
+// which the encodes' stream offsets (exclusive prefix sums) already give (for the tiles of pictures, plus the picture headers).  Parse: one CTA per container, the first stage of the
 // decode; it validates the container against the handle and hands the decoders the byte ranges of the two streams (empty for a
 // container it refuses, so nothing outside a container is ever read).
 #include "common.cuh"
@@ -37,37 +37,73 @@ __device__ __forceinline__ uint32_t unpack_id(const uint32_t* p, int w, int j) {
 }
 }  // namespace
 
+// Byte offset and length of container n in the output: the containers before it back to back, plus (pictures) the header and
+// length table of its picture and of every picture before it.
+__device__ __forceinline__ void image_extent(const int64_t* y_off, const int64_t* z_off, long long fixed, int T, int n,
+                                             long long* off, long long* len) {
+    const long long gap = T ? (long long)(n / T + 1) * 4 * (4 + T) : 0;
+    *off = n * fixed + (y_off[n] - y_off[0]) + (z_off[n] - z_off[0]) + gap;
+    *len = fixed + (y_off[n + 1] - y_off[n]) + (z_off[n + 1] - z_off[n]);
+}
+
 __global__ void __launch_bounds__(256)
 image_pack_kernel(const int64_t* __restrict__ ids_keep, const uint8_t* __restrict__ y_bytes, const int64_t* __restrict__ y_off,
                   const int32_t* __restrict__ y_st, const uint8_t* __restrict__ z_bytes, const int64_t* __restrict__ z_off,
                   const int32_t* __restrict__ z_st, ImageFields f, int N, uint8_t* __restrict__ out, long long capacity,
-                  int64_t* __restrict__ offsets, int32_t* __restrict__ status) {
+                  int64_t* __restrict__ offsets, int32_t* __restrict__ status, PictureGroup g) {
     const int n = blockIdx.x;
     const int id_words = (int)(((long long)f.K * f.id_bits + 31) / 32);
     const long long fixed = 4ll * (kHeaderWords + id_words);
-    const long long off = n * fixed + (y_off[n] - y_off[0]) + (z_off[n] - z_off[0]);
+    long long off, len;
+    image_extent(y_off, z_off, fixed, g.T, n, &off, &len);
     const long long y_len = y_off[n + 1] - y_off[n], z_len = z_off[n + 1] - z_off[n];
-    const long long len = fixed + z_len + y_len;
     const bool fits = off + len <= capacity;
     if (threadIdx.x == 0) {
         offsets[n] = off;
         if (n == N - 1) offsets[N] = off + len;
         status[n] = y_st[n] | z_st[n] | (fits ? 0 : RANS_ST_OVERFLOW);
     }
-    if (!fits) return;
-    uint32_t* dst = reinterpret_cast<uint32_t*>(out + off);           // off, the header and every section: multiples of 4
-    if (threadIdx.x == 0) {
-        dst[0] = kImageMagic; dst[1] = f.word1; dst[2] = f.word2; dst[3] = f.word3; dst[4] = f.tag;
-        dst[5] = (uint32_t)z_len; dst[6] = (uint32_t)y_len;
+    if (fits) {
+        uint32_t* dst = reinterpret_cast<uint32_t*>(out + off);       // off, the header and every section: multiples of 4
+        if (threadIdx.x == 0) {
+            dst[0] = kImageMagic; dst[1] = f.word1; dst[2] = f.word2; dst[3] = f.word3; dst[4] = f.tag;
+            dst[5] = (uint32_t)z_len; dst[6] = (uint32_t)y_len;
+        }
+        const int64_t* ids = ids_keep + (size_t)n * f.K;
+        for (int i = threadIdx.x; i < id_words; i += blockDim.x) dst[kHeaderWords + i] = pack_id_word(ids, f.K, f.id_bits, i);
+        dst += kHeaderWords + id_words;
+        const uint32_t* zs = reinterpret_cast<const uint32_t*>(z_bytes + z_off[n]);
+        for (long long i = threadIdx.x; i < z_len / 4; i += blockDim.x) dst[i] = zs[i];
+        dst += z_len / 4;
+        const uint32_t* ys = reinterpret_cast<const uint32_t*>(y_bytes + y_off[n]);
+        for (long long i = threadIdx.x; i < y_len / 4; i += blockDim.x) dst[i] = ys[i];
     }
-    const int64_t* ids = ids_keep + (size_t)n * f.K;
-    for (int i = threadIdx.x; i < id_words; i += blockDim.x) dst[kHeaderWords + i] = pack_id_word(ids, f.K, f.id_bits, i);
-    dst += kHeaderWords + id_words;
-    const uint32_t* zs = reinterpret_cast<const uint32_t*>(z_bytes + z_off[n]);
-    for (long long i = threadIdx.x; i < z_len / 4; i += blockDim.x) dst[i] = zs[i];
-    dst += z_len / 4;
-    const uint32_t* ys = reinterpret_cast<const uint32_t*>(y_bytes + y_off[n]);
-    for (long long i = threadIdx.x; i < y_len / 4; i += blockDim.x) dst[i] = ys[i];
+    if (g.T) {
+        // the picture of this tile: header words (first tile), length word t (tile t), and the picture's offset and status
+        const int t = n % g.T, n0 = n - t;
+        const long long hdr = 4ll * (4 + g.T);
+        long long off0, len0;
+        image_extent(y_off, z_off, fixed, g.T, n0, &off0, &len0);
+        uint32_t* pic = reinterpret_cast<uint32_t*>(out + (off0 - hdr));
+        if (threadIdx.x == 0) {
+            if (fits) pic[4 + t] = (uint32_t)len;
+            if (t == 0 && fits) { pic[0] = kPictureMagic; pic[1] = 1u; pic[2] = g.hw; pic[3] = (uint32_t)g.T; }
+            if (n == N - 1) g.offsets[N / g.T] = off + len;
+        }
+        if (t == 0 && threadIdx.x < 32) {            // one warp: OR of the group's tile status
+            int st = 0;
+            for (int j = threadIdx.x; j < g.T; j += 32) {
+                long long o, l;
+                image_extent(y_off, z_off, fixed, g.T, n0 + j, &o, &l);
+                st |= y_st[n0 + j] | z_st[n0 + j] | (o + l <= capacity ? 0 : RANS_ST_OVERFLOW);
+            }
+            st = __reduce_or_sync(0xffffffffu, st);
+            if (threadIdx.x == 0) {
+                g.offsets[n / g.T] = off0 - hdr;
+                g.status[n / g.T] = st;
+            }
+        }
+    }
 }
 
 // ranges [4 N]: z begin, z end, y begin, y end of every container (byte offsets into the blob; all 0 for a refused container)
@@ -80,7 +116,7 @@ image_parse_kernel(const IoBlock* __restrict__ io, ImageFields f, int N, int64_t
     for (int i = threadIdx.x; i < map_words; i += blockDim.x) seen[i] = 0;
     if (threadIdx.x == 0) s_st = 0;
     const uint8_t* data = io->img_data;
-    const long long c0 = io->img_offsets[n], c1 = io->img_offsets[n + 1];
+    const long long c0 = io->img_offsets[n], c1 = io->img_ends[n];
     const bool range_ok = c0 >= 0 && c1 >= c0 && c1 <= io->img_n_bytes && !(c0 & 3) && !((c1 - c0) & 3);
     const long long n_words = range_ok ? (c1 - c0) / 4 : 0;
     const uint32_t* cw = reinterpret_cast<const uint32_t*>(data + (range_ok ? c0 : 0));
@@ -146,8 +182,9 @@ image_parse_kernel(const IoBlock* __restrict__ io, ImageFields f, int N, int64_t
 
 cudaError_t launch_image_pack(const int64_t* ids_keep, const uint8_t* y_bytes, const int64_t* y_off, const int32_t* y_st,
                               const uint8_t* z_bytes, const int64_t* z_off, const int32_t* z_st, const ImageFields& f, int N,
-                              uint8_t* out, long long capacity, int64_t* offsets, int32_t* status, cudaStream_t st) {
-    image_pack_kernel<<<N, 256, 0, st>>>(ids_keep, y_bytes, y_off, y_st, z_bytes, z_off, z_st, f, N, out, capacity, offsets, status);
+                              uint8_t* out, long long capacity, int64_t* offsets, int32_t* status, cudaStream_t st,
+                              const PictureGroup& g) {
+    image_pack_kernel<<<N, 256, 0, st>>>(ids_keep, y_bytes, y_off, y_st, z_bytes, z_off, z_st, f, N, out, capacity, offsets, status, g);
     return cudaGetLastError();
 }
 

@@ -25,10 +25,16 @@ struct IoBlock {
     const int64_t* z_ends;
     int32_t* status;                 //   [N] per-image coder status (RANS_ST_* bits, and IMG_ST_* from the container parse)
     const uint8_t* img_data;         // decode from image containers (tmae_decompress_images): container n is bytes
-    const int64_t* img_offsets;      //   [img_offsets[n], img_offsets[n + 1]) of img_data, inside [0, img_n_bytes)
+    const int64_t* img_offsets;      //   [img_offsets[n], img_ends[n]) of img_data, inside [0, img_n_bytes).  Containers packed back
+    const int64_t* img_ends;         //   to back: img_ends = img_offsets + 1; the tiles of pictures: the ranges picture_parse_kernel wrote
     long long img_n_bytes;
     int64_t* img_ids_restore;        //   [N, L] out: the canonical ids_restore of every container
     int64_t* img_ids_keep;           //   [N, K] out (may be null): the kept patch ids of every container
+    const int64_t* pic_offsets;      // decode from picture containers (tmae_decompress_pictures): picture p is bytes
+                                     //   [pic_offsets[p], pic_offsets[p + 1]) of img_data; its T tiles are images p T .. p T + T - 1
+    int64_t* pic_ranges;             //   [2 N] out: begin, then end byte of every tile container (-> img_offsets / img_ends)
+    int32_t* pic_status;             //   [P] out: PIC_ST_HEADER, ORed with the status of every tile of the picture
+    int pic_P, pic_H, pic_W;         //   pictures and their height / width
     const float* syn_y_hat;          // synthesis (tmae_synthesize): y_hat f32 [N, s, s, Cy] in,
     const int64_t* syn_ids;          //   ids_restore [N, L] in,
     float* syn_x_hat;                //   x_hat f32 [N, 3, S, S] out
@@ -182,13 +188,36 @@ struct ImageFields {                 // what the handle writes into (and expects
     uint32_t tag;                    // model tag
     int L, K, id_bits;               // patches, kept patches, bits per packed id
 };
+// Images packed as the tiles of pictures (tmae_compress_pictures): every group of T consecutive images is one picture, whose
+// header and length table take the 4 (4 + T) bytes in front of its first tile.  T = 0: plain image containers, back to back.
+struct PictureGroup {
+    int T = 0;                       // tiles per picture
+    uint32_t hw = 0;                 // word 2 of the picture header: H | W << 16
+    int64_t* offsets = nullptr;      // [N / T + 1] out: picture offsets
+    int32_t* status = nullptr;       // [N / T] out: OR of the picture's tile status
+};
 // after the encodes of N images (stream offsets / status of each kind): container n at offsets[n] of out
 cudaError_t launch_image_pack(const int64_t* ids_keep, const uint8_t* y_bytes, const int64_t* y_off, const int32_t* y_st,
                               const uint8_t* z_bytes, const int64_t* z_off, const int32_t* z_st, const ImageFields& f, int N,
-                              uint8_t* out, long long capacity, int64_t* offsets, int32_t* status, cudaStream_t st);
+                              uint8_t* out, long long capacity, int64_t* offsets, int32_t* status, cudaStream_t st,
+                              const PictureGroup& g = PictureGroup());
 // the containers of io->img_*: canonical ids_restore (io->img_ids_restore), io->img_ids_keep when non-null, io->status, and the
 // stream ranges [4 N] (z begin, z end, y begin, y end)
 cudaError_t launch_image_parse(const IoBlock* io, const ImageFields& f, int N, int64_t* ranges, cudaStream_t st);
+
+// picture.cu: pictures of any size as tiles of img_size (DESIGN.md section 7, "The picture container")
+constexpr int32_t PIC_ST_HEADER = 1024;          // include/tmae.h TMAE_PIC_HEADER
+constexpr uint32_t kPictureMagic = 0x50414D54u;  // bytes "TMAP"
+// pictures f32 [P, 3, H, W] -> tiles f32 [P T, 3, S, S] and grey tiles u8 [P T, S, S] (either may be null), zero-padded; the grey
+// tiles are cut from gray u8 [P, H, W], or made from the RGB (cv2 RGB2GRAY of the 8-bit pixels) when gray is null
+cudaError_t launch_picture_tile(const float* imgs, const uint8_t* gray, int P, int H, int W, int S, float* tiles,
+                                uint8_t* gray_tiles, cudaStream_t st);
+// tiles f32 [P T, 3, S, S] -> canvas f32 [P, 3, H, W]
+cudaError_t launch_picture_untile(const float* tiles, int P, int H, int W, int S, float* canvas, cudaStream_t st);
+// the picture headers of io->pic_*: io->pic_ranges, io->pic_status (S = img_size)
+cudaError_t launch_picture_parse(const IoBlock* io, int P, int S, cudaStream_t st);
+// io->pic_status[p] |= io->status of its T tiles
+cudaError_t launch_picture_status(const IoBlock* io, int P, int T, cudaStream_t st);
 
 // ---- patch-score generation (scores.cu; generate_scores_file.py:19-31, utils/map.py, utils/distribution.py) ----
 constexpr int kScoreMaxLevels = 16;

@@ -137,7 +137,7 @@ mask_select_kernel(const float* __restrict__ scores, int L, int Lp2, int K, int 
     int* scan = pos + Lp2;                            // scratch for scans
     __shared__ float thr[NQ], means[NG];
     __shared__ int gsize[NG], goff[NG + 1], taken[NQ], base[NQ], warp_tmp[kWarps];
-    __shared__ int sh_nu, sh_total_sel;
+    __shared__ int sh_nu;
 
     const int n = blockIdx.x, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const float* sc = scores + (size_t)n * L;
@@ -259,7 +259,6 @@ mask_select_kernel(const float* __restrict__ scores, int L, int Lp2, int K, int 
             base[g] = acc;
             acc += taken[g];
         }
-        sh_total_sel = acc;
     }
     __syncthreads();
 
@@ -301,10 +300,11 @@ mask_select_kernel(const float* __restrict__ scores, int L, int Lp2, int K, int 
     __syncthreads();
 
     // ---- unselected indices ascending: MCM.py:418-420 ----
+    // They follow the selected ones.  A NaN score equals no value (MCM.py:410-416 selects nothing for it), so a row of NaN scores
+    // (0/0 of a flat image) selects fewer indices than the take counts add up to: ids 0, 1, 2, ... for an all-NaN row.
     for (int i = tid; i < Lp2; i += kThreads) scan[i] = (i < L && pos[i] == -1) ? 1 : 0;
     __syncthreads();
-    block_exclusive_scan(scan, Lp2, warp_tmp);
-    const int total_sel = sh_total_sel;
+    const int total_sel = L - block_exclusive_scan(scan, Lp2, warp_tmp);
     for (int i = tid; i < L; i += kThreads) {
         const int p = pos[i] == -1 ? total_sel + scan[i] : pos[i];
         if (ids_shuffle) ids_shuffle[(size_t)n * L + p] = i;

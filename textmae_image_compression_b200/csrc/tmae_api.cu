@@ -56,6 +56,7 @@ enum StepKind { ST_MASK, ST_GATHER, ST_GEMM, ST_FORCE, ST_LN, ST_ATTN, ST_EB, ST
                 ST_ZDEQ, ST_IDX, ST_YDEQ, ST_DEC_OUT,        // decode plans only
                 ST_ZDEC, ST_YDEC,                            // decode-from-streams plans only: the range decoder
                 ST_PARSE,                                    // image-container plans only: parse and validate the containers
+                ST_PICPARSE, ST_PICSTATUS,                   // picture plans only: the picture headers, the picture status
                 ST_SYN_IN, ST_UNSHUF, ST_ATTN32, ST_UNPATCH };  // synthesis plans only
 enum Family { FAM_GEMM = 0, FAM_ATTN, FAM_LN, FAM_MASK, FAM_GATHER, FAM_ENTROPY, FAM_MISC, FAM_CODER, FAM_COUNT };
 const char* kFamilyNames[FAM_COUNT] = {"gemm_tc", "attention", "layernorm", "mask_select", "gather_patches",
@@ -80,6 +81,7 @@ struct Step {
     int lanes = 0;
     int parse_z_lanes = 0;
     bool status_or = false;                    // ST_ZDEC: OR into the status ST_PARSE wrote instead of overwriting it
+    int pic_P = 0;                             // ST_PICPARSE / ST_PICSTATUS: pictures (of pl.N / pic_P tiles each)
     std::string tag;
 };
 
@@ -92,6 +94,7 @@ enum PlanKind {
     PLAN_STREAMS,                    // tmae_decompress_streams(_lanes): the decode with the range decoder in front
     PLAN_SYNTH,                      // tmae_synthesize
     PLAN_IMAGES,                     // tmae_decompress_images: PLAN_STREAMS behind the container parse
+    PLAN_PICTURES,                   // tmae_decompress_pictures: PLAN_IMAGES of the tiles behind the picture parse
 };
 enum PlanDep : unsigned {
     DEP_WS = 1,                      // network workspace (ensure_workspace)
@@ -108,12 +111,16 @@ const unsigned kPlanDeps[] = {
     DEP_WS | DEP_SCALE | DEP_CODER | DEP_CDF,    // PLAN_STREAMS
     DEP_SYNTH,                                   // PLAN_SYNTH
     DEP_WS | DEP_SCALE | DEP_CODER | DEP_CDF,    // PLAN_IMAGES
+    DEP_WS | DEP_SCALE | DEP_CODER | DEP_CDF,    // PLAN_PICTURES
 };
-// (kind, batch size, y lanes, z lanes); the lanes are nonzero for the laned PLAN_STREAMS / PLAN_IMAGES only
-typedef std::tuple<int, int, int, int> PlanKey;
+// (kind, batch size, y lanes, z lanes, picture geometry); the lanes are nonzero for the laned PLAN_STREAMS / PLAN_IMAGES /
+// PLAN_PICTURES only, the geometry (H << 16 | W) for PLAN_PICTURES only: the batch size counts tiles, and two geometries with
+// as many tiles have plans (and graphs) of their own
+typedef std::tuple<int, int, int, int, long long> PlanKey;
 
 struct Plan {
     int N = 0;
+    int pic_H = 0, pic_W = 0;        // PLAN_PICTURES: picture height and width (N tiles)
     unsigned deps = 0;               // DEP_* bits of its kind
     std::vector<Step> steps;
     std::vector<GemmParams> host_params;
@@ -191,6 +198,20 @@ struct CoderWorkspace {
     int32_t* img_st = nullptr;       // [2 N] y, z encode status
 };
 
+// Scratch of the picture calls (tmae_compress_pictures / tmae_decompress_pictures) for N tiles, grown on demand.
+struct PictureWorkspace {
+    std::vector<void*> allocs;
+    int cap_N = 0;
+    float* tiles = nullptr;          // [N, 3, S, S] encode: the tiles of the pictures; decode: the tiles' x_hat
+    uint8_t* gray = nullptr;         // [N, S, S] grey tiles (encode)
+    float* scores = nullptr;         // [N, L] the tiles' scores (encode)
+    uint8_t* score_ws = nullptr;     // workspace of the score generator, score_bytes
+    size_t score_bytes = 0;
+    int64_t* offsets = nullptr;      // [N + 1] encode: tile container offsets; decode: [2 N] tile begins, tile ends
+    int32_t* status = nullptr;       // [N] tile status
+    int64_t* ids = nullptr;          // [N, L] decode: ids_restore of the tiles, when the caller does not ask for it
+};
+
 // Buffers of the synthesis plans (tmae_synthesize), allocated only on handles with synthesis enabled.  All bf16 buffers hold
 // one plane: synthesis runs bf16 operands in every accuracy mode.
 struct SynthWorkspace {
@@ -244,6 +265,7 @@ struct tmae_handle {
     bool tag_ok = false;
     uint32_t tag = 0;
     CoderWorkspace cws;
+    PictureWorkspace pws;
     int dec_N = 0, dec_next = -1;    // decode in progress: batch size and the next group expected (-1 = none)
     PFN_encodeTiled encode = nullptr;
     std::vector<void*> weight_allocs;
@@ -1324,12 +1346,19 @@ int ensure_coder_workspace(tmae_handle* h, int N) {
 // format with that many lanes per y / z stream.
 // Images (tmae_decompress_images): the coded plan behind ST_PARSE, which validates the containers, writes the canonical
 // ids_restore and the streams' byte ranges in the blob, and resets the status the decoders then OR into.
-int build_decode_plan(tmae_handle* h, Plan& pl, bool coded, int lanes_y, int lanes_z, bool images = false) {
+// Pictures (tmae_decompress_pictures, pic_P pictures of pl.N / pic_P tiles): the images plan of the tiles behind ST_PICPARSE,
+// which validates the picture headers and writes the tiles' byte ranges, and ST_PICSTATUS at the end, which ORs every tile's
+// status into its picture's.
+int build_decode_plan(tmae_handle* h, Plan& pl, bool coded, int lanes_y, int lanes_z, bool images = false, int pic_P = 0) {
     const int N = pl.N;
     int rc = ensure_workspace(h, N);
     if (rc || (coded && (rc = ensure_coder_workspace(h, N)))) return rc;
     std::vector<std::pair<int, int>> groups;
     slice_groups(h->nsl, groups);
+    if (pic_P) {
+        add_step(pl, ST_PICPARSE, FAM_CODER, "picture_parse");
+        pl.steps.back().pic_P = pic_P;
+    }
     if (images) {
         add_step(pl, ST_PARSE, FAM_CODER, "image_parse");
         pl.steps.back().lanes = lanes_y;
@@ -1355,6 +1384,10 @@ int build_decode_plan(tmae_handle* h, Plan& pl, bool coded, int lanes_y, int lan
         if ((rc = add_lrp_steps(h, pl, N, g.first, g.second, false))) return rc;
     }
     add_step(pl, ST_DEC_OUT, FAM_MISC, "decode_outputs");
+    if (pic_P) {
+        add_step(pl, ST_PICSTATUS, FAM_CODER, "picture_status");
+        pl.steps.back().pic_P = pic_P;
+    }
     return TMAE_OK;
 }
 
@@ -1443,13 +1476,15 @@ int build_synth_plan(tmae_handle* h, Plan& pl) {
     return TMAE_OK;
 }
 
-// The plan of `kind` for batch size N (lanes: PLAN_STREAMS / PLAN_IMAGES only), built on first use and kept until drop_plans discards it.
-int get_plan(tmae_handle* h, PlanKind kind, int N, Plan** out, int lanes_y = 0, int lanes_z = 0) {
-    const PlanKey key(kind, N, lanes_y, lanes_z);
+// The plan of `kind` for batch size N (lanes: PLAN_STREAMS / PLAN_IMAGES / PLAN_PICTURES only; pic_H / pic_W: PLAN_PICTURES only),
+// built on first use and kept until drop_plans discards it.
+int get_plan(tmae_handle* h, PlanKind kind, int N, Plan** out, int lanes_y = 0, int lanes_z = 0, int pic_H = 0, int pic_W = 0) {
+    const PlanKey key(kind, N, lanes_y, lanes_z, (long long)pic_H << 16 | pic_W);
     auto it = h->plans.find(key);
     if (it != h->plans.end()) { *out = it->second.get(); return TMAE_OK; }
     std::unique_ptr<Plan> pl(new Plan());
     pl->N = N;
+    pl->pic_H = pic_H; pl->pic_W = pic_W;
     pl->deps = kPlanDeps[kind];
     int rc = TMAE_OK;
     switch (kind) {
@@ -1457,6 +1492,11 @@ int get_plan(tmae_handle* h, PlanKind kind, int N, Plan** out, int lanes_y = 0, 
         case PLAN_DECODE: case PLAN_STREAMS: rc = build_decode_plan(h, *pl, kind == PLAN_STREAMS, lanes_y, lanes_z); break;
         case PLAN_SYNTH: rc = build_synth_plan(h, *pl); break;
         case PLAN_IMAGES: rc = build_decode_plan(h, *pl, true, lanes_y, lanes_z, true); break;
+        case PLAN_PICTURES: {
+            const int S = h->cfg.img_size, T = ((pic_H + S - 1) / S) * ((pic_W + S - 1) / S);
+            rc = build_decode_plan(h, *pl, true, lanes_y, lanes_z, true, N / T);
+            break;
+        }
     }
     if (rc || (rc = finish_plan(h, *pl))) return rc;
     *out = pl.get();
@@ -1618,6 +1658,12 @@ int run_steps(tmae_handle* h, Plan& pl, const RunArgs& a, cudaStream_t st) {
             }
             case ST_PARSE:
                 CUDA_TRY(h, launch_image_parse(a.io, image_fields(h, sp.lanes, sp.parse_z_lanes), N, h->cws.ranges, st));
+                break;
+            case ST_PICPARSE:
+                CUDA_TRY(h, launch_picture_parse(a.io, sp.pic_P, h->cfg.img_size, st));
+                break;
+            case ST_PICSTATUS:
+                CUDA_TRY(h, launch_picture_status(a.io, sp.pic_P, N / sp.pic_P, st));
                 break;
             case ST_SYN_IN:
                 CUDA_TRY(h, launch_synth_input(h->sws.y_bf.p, (long long)N * K * h->Cy, st, a.io));
@@ -1813,6 +1859,7 @@ void tmae_destroy(tmae_handle* h) {
     for (CdfTables& t : h->cdf) rans_free_tables(&t);
     free_pool(h->cws.allocs);
     free_pool(h->cws.img_allocs);
+    free_pool(h->pws.allocs);
     free_pool(h->sws.allocs);
     if (h->cws.enc) cudaFree(h->cws.enc);
     if (h->cap_stream) cudaStreamDestroy(h->cap_stream);
@@ -2158,7 +2205,7 @@ int tmae_decode_step(tmae_handle* h, int group, const int32_t* y_symbols, const 
     if (!h) return TMAE_EINVAL;
     if (!y_symbols || !out || !out->y_indexes) return fail(h, TMAE_EINVAL, "y_symbols, out and out->y_indexes must not be null");
     const int expected = h->dec_next;
-    auto it = h->plans.find(PlanKey(PLAN_DECODE, h->dec_N, 0, 0));
+    auto it = h->plans.find(PlanKey(PLAN_DECODE, h->dec_N, 0, 0, 0));
     h->dec_next = -1;                // an out-of-order step ends the decode as well
     if (expected < 0 || group != expected || it == h->plans.end())
         return fail(h, TMAE_ESTATE, "decode step %d out of order (expected %s%d): steps follow tmae_decode_begin in group order, "
@@ -2469,19 +2516,22 @@ int64_t tmae_images_bound(const tmae_handle* h, int N, int y_lanes, int z_lanes)
     return N * image_bound(h, y_lanes, z_lanes);
 }
 
-int tmae_compress_images(tmae_handle* h, const float* imgs, const float* scores, int N, int y_lanes, int z_lanes, uint8_t* out,
-                         int64_t capacity, int64_t* offsets, int32_t* status, void* stream) {
-    if (!h) return TMAE_EINVAL;
-    if (!imgs || !scores || !out || !offsets || !status || N < 1 || capacity < 0 || bad_img_lanes(y_lanes) || bad_img_lanes(z_lanes))
-        return fail(h, TMAE_EINVAL, "compress_images: null pointer, N < 1, capacity < 0 or lanes (%d, %d) outside 0..32", y_lanes, z_lanes);
-    if ((reinterpret_cast<uintptr_t>(out) | reinterpret_cast<uintptr_t>(status)) & 3 || reinterpret_cast<uintptr_t>(offsets) & 7)
-        return fail(h, TMAE_EINVAL, "compress_images: out and status must be 4-byte aligned, offsets 8-byte aligned");
-    int rc = check_ready(h, N);
-    if (rc || (rc = images_ready(h))) return rc;
+namespace {
+// The image workspace and the encode scratch of N images (tmae_compress_images, tmae_compress_pictures).
+int ensure_encode_scratch(tmae_handle* h, int N, int y_lanes, int z_lanes) {
+    const int ny = h->Cy * h->K, nz = h->Cz * h->s4 * h->s4;
+    const EncScratch ys = enc_scratch_bytes(N, ny, y_lanes), zs = enc_scratch_bytes(N, nz, z_lanes);
+    int rc = ensure_image_workspace(h, N);
+    return rc ? rc : grow_enc_scratch(h, ys.total > zs.total ? ys : zs);
+}
+
+// The forward of N images, both encodes and the pack (tmae_compress_images; the tiles of pictures with g.T > 0), after the
+// argument and state checks and ensure_encode_scratch.
+int compress_images_impl(tmae_handle* h, const float* imgs, const float* scores, int N, int y_lanes, int z_lanes, uint8_t* out,
+                         int64_t capacity, int64_t* offsets, int32_t* status, cudaStream_t st, const PictureGroup& g) {
+    int rc;
     const long long hw = (long long)h->s * h->s, hw4 = (long long)h->s4 * h->s4;
     const int ny = h->Cy * h->K, nz = (int)(h->Cz * hw4);
-    const EncScratch ys = enc_scratch_bytes(N, ny, y_lanes), zs = enc_scratch_bytes(N, nz, z_lanes);
-    if ((rc = ensure_image_workspace(h, N)) || (rc = grow_enc_scratch(h, ys.total > zs.total ? ys : zs))) return rc;
     Plan* pl = nullptr;
     if ((rc = get_plan(h, PLAN_FORWARD, N, &pl))) return rc;
     CoderWorkspace& c = h->cws;
@@ -2491,7 +2541,6 @@ int tmae_compress_images(tmae_handle* h, const float* imgs, const float* scores,
     tmae_outputs o;
     memset(&o, 0, sizeof(o));
     o.y_symbols = f_ysym; o.y_indexes = f_yidx; o.z_symbols = f_zsym;
-    cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
     if (h->profiling) h->prof_used = 0;
     if ((rc = run_forward(h, *pl, imgs, scores, &o, st))) return rc;
     CUDA_TRY(h, launch_pack_nchw_i32(f_ysym, ysym, N, (int)hw, h->Cy, st));
@@ -2503,8 +2552,22 @@ int tmae_compress_images(tmae_handle* h, const float* imgs, const float* scores,
         (rc = enqueue_encode(h, h->cdf[TMAE_MODEL_BOTTLENECK], zsym, zidx, N, nz, z_lanes, c.img_z, c.img_z_cap, z_off, z_st, st)))
         return rc;
     CUDA_TRY(h, launch_image_pack(h->ws.ids_keep, c.img_y, y_off, y_st, c.img_z, z_off, z_st, image_fields(h, y_lanes, z_lanes), N,
-                                  out, capacity, offsets, status, st));
+                                  out, capacity, offsets, status, st, g));
     return TMAE_OK;
+}
+}  // namespace
+
+int tmae_compress_images(tmae_handle* h, const float* imgs, const float* scores, int N, int y_lanes, int z_lanes, uint8_t* out,
+                         int64_t capacity, int64_t* offsets, int32_t* status, void* stream) {
+    if (!h) return TMAE_EINVAL;
+    if (!imgs || !scores || !out || !offsets || !status || N < 1 || capacity < 0 || bad_img_lanes(y_lanes) || bad_img_lanes(z_lanes))
+        return fail(h, TMAE_EINVAL, "compress_images: null pointer, N < 1, capacity < 0 or lanes (%d, %d) outside 0..32", y_lanes, z_lanes);
+    if ((reinterpret_cast<uintptr_t>(out) | reinterpret_cast<uintptr_t>(status)) & 3 || reinterpret_cast<uintptr_t>(offsets) & 7)
+        return fail(h, TMAE_EINVAL, "compress_images: out and status must be 4-byte aligned, offsets 8-byte aligned");
+    int rc = check_ready(h, N);
+    if (rc || (rc = images_ready(h)) || (rc = ensure_encode_scratch(h, N, y_lanes, z_lanes))) return rc;
+    return compress_images_impl(h, imgs, scores, N, y_lanes, z_lanes, out, capacity, offsets, status,
+                                reinterpret_cast<cudaStream_t>(stream), PictureGroup());
 }
 
 int tmae_decompress_images(tmae_handle* h, const uint8_t* data, int64_t n_bytes, const int64_t* offsets, int N, int y_lanes,
@@ -2532,7 +2595,8 @@ int tmae_decompress_images(tmae_handle* h, const uint8_t* data, int64_t n_bytes,
     hio.y_data = data; hio.y_offsets = r + 2 * N; hio.y_ends = r + 3 * N;
     hio.z_data = data; hio.z_offsets = r; hio.z_ends = r + N;
     hio.status = status;
-    hio.img_data = data; hio.img_offsets = offsets; hio.img_n_bytes = n_bytes; hio.img_ids_restore = ids_restore;
+    hio.img_data = data; hio.img_offsets = offsets; hio.img_ends = offsets + 1; hio.img_n_bytes = n_bytes;
+    hio.img_ids_restore = ids_restore;
     hio.img_ids_keep = out->ids_keep;
     cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
     if (h->profiling) h->prof_used = 0;
@@ -2542,6 +2606,163 @@ int tmae_decompress_images(tmae_handle* h, const uint8_t* data, int64_t n_bytes,
     memset(&sio, 0, sizeof(sio));
     sio.syn_y_hat = out->y_hat; sio.syn_ids = ids_restore; sio.syn_x_hat = x_hat;
     return run_stage(h, *syn, 0, sio, h->sws.io, st);
+}
+
+// ---- picture containers (DESIGN.md section 7, "The picture container") --------------------------------------------------
+namespace {
+bool bad_side(int v) { return v < 1 || v > 0xffff; }
+long long tile_count(int H, int W, int S) { return (long long)((H + S - 1) / S) * ((W + S - 1) / S); }
+
+// Picture scratch of N tiles: tiles (and the tiles' x_hat), grey tiles, scores and the score generator's workspace, tile offsets
+// (or ranges) and status, tile ids_restore.
+int ensure_picture_workspace(tmae_handle* h, int N) {
+    PictureWorkspace& w = h->pws;
+    if (N <= w.cap_N) return TMAE_OK;
+    free_pool(w.allocs);
+    w = PictureWorkspace();
+    const int S = h->cfg.img_size;
+    ScoreGeom g;
+    if (!score_geometry(S, S, S, &g)) return fail(h, TMAE_EINVAL, "pictures: tiles of side %d have no patch scores", S);
+    const size_t px = (size_t)N * S * S;
+    w.score_bytes = score_workspace_bytes(g, N);
+    int rc;
+    if ((rc = dev_alloc(h, w.allocs, &w.tiles, 3 * px)) || (rc = dev_alloc(h, w.allocs, &w.gray, px)) ||
+        (rc = dev_alloc(h, w.allocs, &w.scores, (size_t)N * h->L)) || (rc = dev_alloc(h, w.allocs, &w.score_ws, w.score_bytes)) ||
+        (rc = dev_alloc(h, w.allocs, &w.offsets, 2 * (size_t)N + 1)) || (rc = dev_alloc(h, w.allocs, &w.status, (size_t)N)) ||
+        (rc = dev_alloc(h, w.allocs, &w.ids, (size_t)N * h->L)))
+        return rc;
+    w.cap_N = N;
+    return TMAE_OK;
+}
+
+// The checks shared by both picture calls; *N = tiles of the call.
+int pictures_args(tmae_handle* h, const char* what, int P, int H, int W, int y_lanes, int z_lanes, int* N) {
+    if (P < 1 || bad_side(H) || bad_side(W) || bad_img_lanes(y_lanes) || bad_img_lanes(z_lanes))
+        return fail(h, TMAE_EINVAL, "%s: P = %d < 1, H x W = %d x %d outside 1..65535 or lanes (%d, %d) outside 0..32", what, P, H, W,
+                    y_lanes, z_lanes);
+    const long long n = (long long)P * tile_count(H, W, h->cfg.img_size);
+    if (n > 65535) return fail(h, TMAE_EINVAL, "%s: %lld tiles, at most 65535 per call", what, n);
+    if (h->cfg.in_chans != 3) return fail(h, TMAE_EINVAL, "%s: pictures are RGB (in_chans %d)", what, h->cfg.in_chans);
+    *N = (int)n;
+    return TMAE_OK;
+}
+}  // namespace
+
+int tmae_picture_tiles(const float* imgs, const uint8_t* gray, int P, int H, int W, int tile, float* tiles, uint8_t* gray_tiles,
+                       void* stream) {
+    if (!imgs || P < 1 || bad_side(H) || bad_side(W) || tile < 1 || tile > 0xffff)
+        return fail(nullptr, TMAE_EINVAL, "picture_tiles: null imgs, P < 1, or H, W, tile outside 1..65535");
+    if (!tiles && !gray_tiles) return TMAE_OK;
+    CUDA_TRY(nullptr, launch_picture_tile(imgs, gray, P, H, W, tile, tiles, gray_tiles, reinterpret_cast<cudaStream_t>(stream)));
+    return TMAE_OK;
+}
+
+int tmae_picture_untile(const float* tiles, int P, int H, int W, int tile, float* canvas, void* stream) {
+    if (!tiles || !canvas || P < 1 || bad_side(H) || bad_side(W) || tile < 1 || tile > 0xffff)
+        return fail(nullptr, TMAE_EINVAL, "picture_untile: null pointer, P < 1, or H, W, tile outside 1..65535");
+    CUDA_TRY(nullptr, launch_picture_untile(tiles, P, H, W, tile, canvas, reinterpret_cast<cudaStream_t>(stream)));
+    return TMAE_OK;
+}
+
+int tmae_picture_geometry(const uint8_t* h_data, int64_t n_bytes, int* H, int* W, int* T, int* y_lanes, int* z_lanes) {
+    if (!h_data || n_bytes < 16 || (n_bytes & 3)) return TMAE_EINVAL;
+    uint32_t w[4];
+    memcpy(w, h_data, 16);                          // the host is little-endian (x86-64 / aarch64)
+    const long long t = w[3];
+    const int h = (int)(w[2] & 0xffffu), wd = (int)(w[2] >> 16);
+    if (w[0] != kPictureMagic || w[1] != 1u || h < 1 || wd < 1 || t < 1 || 4 * (4 + t) + 28 > n_bytes) return TMAE_EINVAL;
+    uint32_t len0, img[3];
+    memcpy(&len0, h_data + 16, 4);
+    const uint8_t* tile0 = h_data + 4 * (4 + t);
+    memcpy(img, tile0, 12);
+    const int S = (int)(img[2] & 0xffffu);
+    if (len0 < 28 || 4 * (4 + t) + len0 > n_bytes || img[0] != kImageMagic || (img[1] & 0xffu) != 1u || S < 1 ||
+        tile_count(h, wd, S) != t)
+        return TMAE_EINVAL;
+    if (H) *H = h;
+    if (W) *W = wd;
+    if (T) *T = (int)t;
+    if (y_lanes) *y_lanes = (int)((img[1] >> 16) & 0xffu);
+    if (z_lanes) *z_lanes = (int)(img[1] >> 24);
+    return TMAE_OK;
+}
+
+int64_t tmae_pictures_bound(const tmae_handle* h, int P, int H, int W, int y_lanes, int z_lanes) {
+    if (!h || P < 1 || bad_side(H) || bad_side(W) || bad_img_lanes(y_lanes) || bad_img_lanes(z_lanes)) return -1;
+    const long long T = tile_count(H, W, h->cfg.img_size);
+    return P * (4 * (4 + T) + T * image_bound(h, y_lanes, z_lanes));
+}
+
+int tmae_compress_pictures(tmae_handle* h, const float* imgs, const uint8_t* gray, int P, int H, int W, int y_lanes, int z_lanes,
+                           uint8_t* out, int64_t capacity, int64_t* offsets, int32_t* status, void* stream) {
+    if (!h) return TMAE_EINVAL;
+    if (!imgs || !out || !offsets || !status || capacity < 0)
+        return fail(h, TMAE_EINVAL, "compress_pictures: null pointer or capacity < 0");
+    int N = 0;
+    int rc = pictures_args(h, "compress_pictures", P, H, W, y_lanes, z_lanes, &N);
+    if (rc) return rc;
+    if ((reinterpret_cast<uintptr_t>(out) | reinterpret_cast<uintptr_t>(status)) & 3 || reinterpret_cast<uintptr_t>(offsets) & 7)
+        return fail(h, TMAE_EINVAL, "compress_pictures: out and status must be 4-byte aligned, offsets 8-byte aligned");
+    if ((rc = check_ready(h, N)) || (rc = images_ready(h)) || (rc = ensure_picture_workspace(h, N)) ||
+        (rc = ensure_encode_scratch(h, N, y_lanes, z_lanes)))
+        return rc;
+    const int S = h->cfg.img_size;
+    PictureWorkspace& w = h->pws;
+    cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+    CUDA_TRY(h, launch_picture_tile(imgs, gray, P, H, W, S, w.tiles, w.gray, st));
+    ScoreGeom g;
+    score_geometry(S, S, S, &g);
+    CUDA_TRY(h, launch_generate_scores(w.gray, N, g, w.scores, nullptr, nullptr, nullptr, w.score_ws, st));
+    PictureGroup pg;
+    pg.T = N / P; pg.hw = (uint32_t)H | (uint32_t)W << 16; pg.offsets = offsets; pg.status = status;
+    return compress_images_impl(h, w.tiles, w.scores, N, y_lanes, z_lanes, out, capacity, w.offsets, w.status, st, pg);
+}
+
+int tmae_decompress_pictures(tmae_handle* h, const uint8_t* data, int64_t n_bytes, const int64_t* offsets, int P, int H, int W,
+                             int y_lanes, int z_lanes, const tmae_outputs* tile_out, int64_t* ids_restore, float* x_hat,
+                             int32_t* status, void* stream) {
+    if (!h) return TMAE_EINVAL;
+    if (!data || !offsets || !status || n_bytes < 0) return fail(h, TMAE_EINVAL, "decompress_pictures: null pointer or n_bytes < 0");
+    int N = 0;
+    int rc = pictures_args(h, "decompress_pictures", P, H, W, y_lanes, z_lanes, &N);
+    if (rc) return rc;
+    const tmae_outputs none = {};
+    const tmae_outputs& o = tile_out ? *tile_out : none;
+    if ((reinterpret_cast<uintptr_t>(data) | reinterpret_cast<uintptr_t>(status)) & 3 ||
+        (reinterpret_cast<uintptr_t>(offsets) | reinterpret_cast<uintptr_t>(ids_restore) | reinterpret_cast<uintptr_t>(o.ids_keep)) & 7 ||
+        (reinterpret_cast<uintptr_t>(o.y_hat) | reinterpret_cast<uintptr_t>(x_hat)) & 15)
+        return fail(h, TMAE_EINVAL, "decompress_pictures: data and status must be 4-byte aligned, offsets, ids_restore and "
+                    "tile_out->ids_keep 8-byte aligned, tile_out->y_hat and x_hat 16-byte aligned");
+    if ((rc = check_ready(h, N)) || (rc = images_ready(h))) return rc;
+    if (x_hat && h->syn_depth == 0) return fail(h, TMAE_ESTATE, "x_hat needs synthesis (call tmae_enable_synthesis)");
+    Plan* pl = nullptr;
+    Plan* syn = nullptr;
+    if ((rc = ensure_picture_workspace(h, N)) || (rc = get_plan(h, PLAN_PICTURES, N, &pl, y_lanes, z_lanes, H, W)) ||
+        (x_hat && (rc = get_plan(h, PLAN_SYNTH, N, &syn))))
+        return rc;
+    PictureWorkspace& w = h->pws;
+    int64_t* ids = ids_restore ? ids_restore : w.ids;
+    IoBlock hio = decode_io(h->cws.zsym, h->cws.ysym, &o);
+    if (!hio.out.y_indexes) hio.out.y_indexes = h->cws.idx;
+    const int64_t* r = h->cws.ranges;               // the container parse's stream ranges
+    hio.y_data = data; hio.y_offsets = r + 2 * N; hio.y_ends = r + 3 * N;
+    hio.z_data = data; hio.z_offsets = r; hio.z_ends = r + N;
+    hio.status = w.status;
+    hio.img_data = data; hio.img_offsets = w.offsets; hio.img_ends = w.offsets + N; hio.img_n_bytes = n_bytes;
+    hio.img_ids_restore = ids; hio.img_ids_keep = o.ids_keep;
+    hio.pic_offsets = offsets; hio.pic_ranges = w.offsets; hio.pic_status = status;
+    hio.pic_P = P; hio.pic_H = H; hio.pic_W = W;
+    cudaStream_t st = reinterpret_cast<cudaStream_t>(stream);
+    if (h->profiling) h->prof_used = 0;
+    if ((rc = run_stage(h, *pl, 0, hio, h->ws.io, st))) return rc;
+    if (!x_hat) return TMAE_OK;
+    IoBlock sio;
+    memset(&sio, 0, sizeof(sio));
+    sio.syn_y_hat = o.y_hat ? o.y_hat : h->ws.yhat;  // the decode's y_hat stays in the workspace when the caller does not ask for it
+    sio.syn_ids = ids; sio.syn_x_hat = w.tiles;
+    if ((rc = run_stage(h, *syn, 0, sio, h->sws.io, st))) return rc;
+    CUDA_TRY(h, launch_picture_untile(w.tiles, P, H, W, h->cfg.img_size, x_hat, st));
+    return TMAE_OK;
 }
 
 int tmae_pack_nchw_i32(const int32_t* nhwc, int32_t* nchw, int N, int hw, int C, void* stream) {

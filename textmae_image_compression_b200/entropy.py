@@ -173,17 +173,30 @@ def decode_lanes(handle, model: int, data: torch.Tensor, offsets: torch.Tensor, 
     return sym, status
 
 
+def pictures_bound(handle, n_pictures: int, height: int, width: int, y_lanes: int, z_lanes: int) -> int:
+    """Bytes that always suffice for n_pictures picture containers of height x width (include/tmae.h tmae_pictures_bound)."""
+    return int(_native.load().tmae_pictures_bound(handle, n_pictures, height, width, y_lanes, z_lanes))
+
+
+def picture_geometry(data: bytes):
+    """(H, W, T, y_lanes, z_lanes) of a picture container, or None for bytes that are not one (tmae_picture_geometry)."""
+    out = [C.c_int(0) for _ in range(5)]
+    buf = bytes(data)
+    rc = _native.load().tmae_picture_geometry(buf, len(buf), *[C.byref(v) for v in out])
+    return None if rc else tuple(v.value for v in out)
+
+
 def images_bound(handle, n_images: int, y_lanes: int, z_lanes: int) -> int:
     """Bytes that always suffice for the image containers of n_images images (include/tmae.h tmae_images_bound)."""
     return int(_native.load().tmae_images_bound(handle, n_images, y_lanes, z_lanes))
 
 
-_IMAGE_REASONS = ((_native.IMG_HEADER, "header"), (_native.IMG_CONFIG, "configuration"), (_native.IMG_MODEL, "model"),
+_IMAGE_REASONS = ((_native.PIC_HEADER, "picture header"), (_native.IMG_HEADER, "header"), (_native.IMG_CONFIG, "configuration"), (_native.IMG_MODEL, "model"),
                   (_native.IMG_IDS, "patch ids"))
 
 
 def image_status_reason(status: int) -> str:
-    """Why a container did not decode, from its status: the container checks that failed, else the streams'."""
+    """Why a container (image or picture) did not decode, from its status: the container checks that failed, else the streams'."""
     reasons = [name for bit, name in _IMAGE_REASONS if status & bit]
     return ", ".join(reasons) if reasons else "a stream that does not decode"
 

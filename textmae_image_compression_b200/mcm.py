@@ -25,6 +25,8 @@ order `encode_with_indexes` consumes, z symbols / channel indexes for `entropy_b
 compressai-format byte strings and back.
 `compress_images` / `decompress_images` wrap both streams, the patch selection and a header into one self-contained byte string per
 image (DESIGN.md section 7), decoded on the GPU from nothing but those bytes.
+`compress_pictures` / `decompress_pictures` do the same for pictures of any size: tiled on the GPU (tiling.py's policy), one byte
+string per picture, x_hat back at the picture's own size.
 `decompress_symbols` is the decoder side of `MCM.decompress` (MCM.py:896-968) around the range decoder: symbols in (all at
 once, or group by group through a callback that receives the scale-table indexes), y_hat / z_hat / x_hat out, bit-exact
 with the encoder of the same accuracy mode.
@@ -884,6 +886,181 @@ class MCM(nn.Module):
         elif need_recon:
             out["x_hat"] = recon.synthesize(self._weights, c, y_hat.reshape(N, c.num_keep_patches, c.latent_depth), ids_restore)
         return out
+
+    # ------------------------------------------------------------------ picture containers (DESIGN.md section 7)
+    @torch.no_grad()
+    def compress_pictures(self, pictures, gray=None, lanes=(32, 4)) -> List[bytes]:
+        """One self-contained byte string per picture of any size: the picture is zero-padded and cut into img_size tiles
+        (tiling.py's policy), every tile is coded as `compress_images` codes an image, with the scores the score generator makes
+        from the tile's grey pixels, and the tile containers follow a header with H, W and the tile lengths.
+        pictures: a list of f32 [3, H, W] tensors, or one [P, 3, H, W] tensor.  gray: None (grey made from the RGB as OpenCV's
+        cvtColor(RGB2GRAY) of the 8-bit pixels) or one uint8 [H, W] per picture (cv2.imread(..., IMREAD_GRAYSCALE) reproduces the
+        reference's scores).  Pictures of one size go in one library call (tiling, scores, forward, encodes and packing enqueued on
+        the current stream); the output order is the input order.  Raises RuntimeError naming the pictures whose encode failed."""
+        y_lanes, z_lanes = self._check_image_lanes(lanes)
+        self._ensure_handle()
+        c = self.cfg
+        if isinstance(pictures, torch.Tensor):
+            if pictures.dim() != 4:
+                raise ValueError(f"expected pictures [P,3,H,W] or a list of [3,H,W], got {tuple(pictures.shape)}")
+            pictures = list(pictures.unbind(0))
+        pictures = list(pictures)
+        if not pictures:
+            raise ValueError("pictures must be a non-empty list")
+        if gray is not None:
+            gray = list(gray.unbind(0)) if isinstance(gray, torch.Tensor) and gray.dim() == 3 else list(gray)
+            if len(gray) != len(pictures):
+                raise ValueError(f"need one grey picture per picture, got {len(gray)} for {len(pictures)}")
+        for i, x in enumerate(pictures):
+            if not isinstance(x, torch.Tensor) or x.dim() != 3 or x.shape[0] != c.in_chans or c.in_chans != 3:
+                raise ValueError(f"picture {i}: expected an RGB tensor [3, H, W], got {getattr(x, 'shape', type(x))}")
+            if not (1 <= x.shape[1] <= 65535 and 1 <= x.shape[2] <= 65535):
+                raise ValueError(f"picture {i}: H and W must be in 1..65535, got {tuple(x.shape[1:])}")
+            if gray is not None and (not isinstance(gray[i], torch.Tensor) or gray[i].dtype != torch.uint8
+                                     or tuple(gray[i].shape) != tuple(x.shape[1:])):
+                raise ValueError(f"picture {i}: gray must be uint8 [{x.shape[1]}, {x.shape[2]}]")
+        self._install_coder_tables()
+        dev = self._handle_device
+        lib = _native.load()
+        groups: Dict[Tuple[int, int], List[int]] = {}
+        for i, x in enumerate(pictures):
+            groups.setdefault((int(x.shape[1]), int(x.shape[2])), []).append(i)
+        result: List[Optional[bytes]] = [None] * len(pictures)
+        failed = []
+        with torch.cuda.device(dev):
+            for (H, W), idx in groups.items():
+                P = len(idx)
+                imgs = torch.stack([pictures[i].to(device=dev, dtype=torch.float32) for i in idx]).contiguous()
+                g = torch.stack([gray[i].to(dev) for i in idx]).contiguous() if gray is not None else None
+                cap = entropy.pictures_bound(self._handle, P, H, W, y_lanes, z_lanes)
+                out = torch.empty(cap, dtype=torch.uint8, device=dev)
+                meta = torch.empty(2 * P + 1, dtype=torch.int64, device=dev)     # offsets [P + 1] | status int32 [P] (padded)
+                status = meta[P + 1:].view(torch.int32)[:P]
+                cur = self._enter_stream(dev)
+                _native.check(lib.tmae_compress_pictures(self._handle, C.c_void_p(imgs.data_ptr()),
+                                                         C.c_void_p(g.data_ptr()) if g is not None else None, P, H, W, y_lanes,
+                                                         z_lanes, C.c_void_p(out.data_ptr()), cap, C.c_void_p(meta.data_ptr()),
+                                                         C.c_void_p(status.data_ptr()), C.c_void_p(cur.cuda_stream)),
+                              self._handle, RuntimeError)
+                self._leave_stream(cur)
+                host_meta = meta.cpu()
+                offs = host_meta[: P + 1].tolist()
+                st = host_meta[P + 1:].view(torch.int32)[:P].tolist()
+                failed += [(idx[k], st[k]) for k in range(P) if st[k]]
+                host = out[: offs[-1]].cpu().numpy().tobytes()
+                for k, i in enumerate(idx):
+                    result[i] = host[offs[k]: offs[k + 1]]
+        if failed:
+            failed.sort()
+            raise RuntimeError(f"picture container encode failed for pictures {[i for i, _ in failed]} "
+                               f"(status {[s for _, s in failed]})")
+        return result
+
+    def _tile_status(self, tiles: List[bytes], lanes) -> List[int]:
+        """Per-tile status of a picture that did not decode: its tile containers decoded on their own (the error path only)."""
+        N = len(tiles)
+        c = self.cfg
+        s, s4 = c.side, c.side // 4
+        dev = self._handle_device
+        data, off = entropy.pack_strings(tiles)
+        host = torch.cat([off.view(torch.uint8), data])
+        y_hat = torch.empty((N, s, s, c.latent_depth), dtype=torch.float32, device=dev)
+        z_hat = torch.empty((N, s4, s4, c.hyperprior_depth), dtype=torch.float32, device=dev)
+        ids_restore = torch.empty((N, c.num_patches), dtype=torch.int64, device=dev)
+        status = torch.empty(N, dtype=torch.int32, device=dev)
+        o = _native.TmaeOutputs()
+        o.y_hat, o.z_hat = y_hat.data_ptr(), z_hat.data_ptr()
+        with torch.cuda.device(dev):
+            cur = self._enter_stream(dev)
+            buf = host.pin_memory().to(dev, non_blocking=True)
+            b0 = buf.data_ptr()
+            _native.check(_native.load().tmae_decompress_images(
+                self._handle, C.c_void_p(b0 + 8 * (N + 1)), data.numel(), C.c_void_p(b0), N, lanes[0], lanes[1], C.byref(o),
+                C.c_void_p(ids_restore.data_ptr()), None, C.c_void_p(status.data_ptr()), C.c_void_p(cur.cuda_stream)),
+                self._handle, RuntimeError)
+            self._leave_stream(cur)
+        return status.cpu().tolist()
+
+    @torch.no_grad()
+    def decompress_pictures(self, strings) -> List[torch.Tensor]:
+        """Decode `compress_pictures`' byte strings with nothing else: x_hat f32 [3, H, W] per picture, at the picture's own size
+        (forward's x_hat of every tile, unclamped, padding dropped).  Needs the decoder-side weights.  Pictures are grouped by
+        geometry and lane counts (tmae_picture_geometry); per group one copy of the bytes to the device and one library call
+        decodes the tiles (picture parse, container parse, rANS decode, the network) - with native_synthesis=True it also
+        synthesises the tiles and untiles them into the canvas; otherwise recon.synthesize runs on the tiles' y_hat and
+        tmae_picture_untile builds the canvas.  Raises ValueError naming every picture that does not decode, why, and its
+        failing tiles."""
+        if not recon.has_decoder_weights(self._weights):
+            raise RuntimeError("decompress_pictures needs the decoder-side weights (g_s / decoder tensors) for x_hat")
+        if not isinstance(strings, (list, tuple)) or len(strings) < 1:
+            raise ValueError("strings must be a non-empty list of byte strings")
+        strings = [bytes(b) if isinstance(b, (bytes, bytearray, memoryview)) else None for b in strings]
+        self._ensure_handle()
+        self._install_coder_tables()
+        c = self.cfg
+        dev = self._handle_device
+        lib = _native.load()
+        failures = {}
+        groups: Dict[Tuple[int, int, int, int], List[int]] = {}
+        for i, b in enumerate(strings):
+            geo = entropy.picture_geometry(b) if b is not None else None
+            if geo is None:
+                failures[i] = "header: not a picture container"
+            elif geo[3] > 32 or geo[4] > 32:
+                failures[i] = "configuration: lane counts outside 0..32"
+            else:
+                groups.setdefault((geo[0], geo[1], geo[3], geo[4]), []).append(i)
+        result: List[Optional[torch.Tensor]] = [None] * len(strings)
+        K, s = c.num_keep_patches, c.side
+        for (H, W, y_lanes, z_lanes), idx in groups.items():
+            P = len(idx)
+            T = (-(-H // c.img_size)) * (-(-W // c.img_size))
+            N = P * T
+            data, off = entropy.pack_strings([strings[i] for i in idx])
+            host = torch.cat([off.view(torch.uint8), data])
+            canvas = torch.empty((P, 3, H, W), dtype=torch.float32, device=dev)
+            status = torch.empty(P, dtype=torch.int32, device=dev)
+            with torch.cuda.device(dev):
+                cur = self._enter_stream(dev)
+                buf = host.pin_memory().to(dev, non_blocking=True)
+                b0 = buf.data_ptr()
+                args = (self._handle, C.c_void_p(b0 + 8 * (P + 1)), data.numel(), C.c_void_p(b0), P, H, W, y_lanes, z_lanes)
+                if self._syn_on:
+                    _native.check(lib.tmae_decompress_pictures(*args, None, None, C.c_void_p(canvas.data_ptr()),
+                                                               C.c_void_p(status.data_ptr()), C.c_void_p(cur.cuda_stream)),
+                                  self._handle, RuntimeError)
+                else:
+                    y_hat = torch.empty((N, s, s, c.latent_depth), dtype=torch.float32, device=dev)
+                    ids_restore = torch.empty((N, c.num_patches), dtype=torch.int64, device=dev)
+                    o = _native.TmaeOutputs()
+                    o.y_hat = y_hat.data_ptr()
+                    _native.check(lib.tmae_decompress_pictures(*args, C.byref(o), C.c_void_p(ids_restore.data_ptr()), None,
+                                                               C.c_void_p(status.data_ptr()), C.c_void_p(cur.cuda_stream)),
+                                  self._handle, RuntimeError)
+                    x_tiles = recon.synthesize(self._weights, c, y_hat.reshape(N, K, c.latent_depth), ids_restore)
+                    x_tiles = x_tiles.to(torch.float32).contiguous()
+                    _native.check(lib.tmae_picture_untile(C.c_void_p(x_tiles.data_ptr()), P, H, W, c.img_size,
+                                                          C.c_void_p(canvas.data_ptr()), C.c_void_p(cur.cuda_stream)))
+                self._leave_stream(cur)
+            st = status.cpu().tolist()
+            for k, i in enumerate(idx):
+                if not st[k]:
+                    result[i] = canvas[k]
+                    continue
+                if st[k] & _native.PIC_HEADER:
+                    tiles = "all"
+                else:
+                    b = strings[i]
+                    lens = [int.from_bytes(b[16 + 4 * t: 20 + 4 * t], "little") for t in range(T)]
+                    starts = [4 * (4 + T) + sum(lens[:t]) for t in range(T)]
+                    tile_st = self._tile_status([b[a: a + n] for a, n in zip(starts, lens)], (y_lanes, z_lanes))
+                    tiles = [t for t in range(T) if tile_st[t]]
+                failures[i] = f"{entropy.image_status_reason(st[k])} (status {st[k]}), tiles {tiles}"
+        if failures:
+            bad = sorted(failures)
+            why = "; ".join(f"picture {i}: {failures[i]}" for i in bad)
+            raise ValueError(f"pictures {bad} do not decode - {why}")
+        return result
 
     def compress(self, *args, **kwargs):
         raise NotImplementedError("MCM.compress is not provided under the reference's name until the bitstream format has been "
